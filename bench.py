@@ -1,7 +1,8 @@
 #!/usr/bin/env python3
-"""Benchmark of the score-and-rank hot path (contract: see the task prompt / DESIGN.md §Measurement).
+"""Benchmark of the score-and-rank hot path (see DESIGN.md §Measurement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config marco|c5] [--batch B]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of B synthetic queries: fused
 score(Q . P^T) -> history mask (set -1e6) -> per-row top-k.
@@ -21,6 +22,11 @@ e2e    : the same through the public host API from HOST buffers: pinned fp32 que
          and encodes 1/G of the rows, all-gathered over NVLink) + the mask CSR are copied H2D, the mask
          is column-sharded on the device, and rank 0 copies the [B,k] scores + ids back D2H, all inside
          the timed region.
+
+--dump-outputs DIR writes the [B,k] scores (float32) and global ids (float64) of the last timed resident
+step as DIR/scores.npy and DIR/ids.npy (above 60 MB, a fixed seeded sample of rows, numbered in
+DIR/rows.npy).  Every input is generated from fixed seeds, so two builds run with the same arguments can be
+compared output for output.  Inside the tree, bench_out/ is the directory git ignores for this.
 """
 import argparse
 import json
@@ -62,7 +68,13 @@ def parse():
     ap.add_argument("--k", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-library-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's scores / ids as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours only")
     cfg = CONFIGS[a.config]
     a.custom_shape = a.n_items is not None or a.k is not None
     a.batch = a.batch or cfg["batch"]
@@ -105,6 +117,28 @@ def rows_to_csr(rows):
     np.cumsum([len(r) for r in rows], out=indptr[1:])
     cols = np.concatenate(rows).astype(np.int32) if len(rows) else np.zeros(0, np.int32)
     return indptr, cols, np.full(len(cols), -1e6)
+
+
+DUMP_BYTES = 60 * 10**6  # under 64 MB with room for the .npy headers
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_BYTES):
+    """Write host arrays (float32 / float64, one row per query) as out_dir/<name>.npy.  When they hold more
+    than `limit` bytes, the same fixed, seeded sample of rows is taken from each and the sampled row
+    numbers are written as rows.npy."""
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"{name}: {a.dtype} (float32 / float64 only)")
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if n * row_bytes > limit:
+        keep = limit // (row_bytes + 8)
+        rows = np.sort(np.random.RandomState(0).choice(n, size=keep, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
 
 
 # ----------------------------------------------------------------------------------------------
@@ -386,12 +420,15 @@ def run_ours(args):
         e0.record()
         for it in range(args.steps):
             L.ccr_set_profile_events(ev_k0[it].cuda_event, ev_k1[it].cuda_event)
-            step_resident()
+            out = step_resident()
         L.ccr_set_profile_events(None, None)
         e1.record()
         barrier()
     ms_total = e0.elapsed_time(e1)
     kern_ms = float(np.mean([a.elapsed_time(b) for a, b in zip(ev_k0, ev_k1)]))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"scores": out[0].cpu().numpy(),
+                                         "ids": out[1].cpu().numpy().astype(np.float64)})
 
     for _ in range(max(1, args.warmup // 2)):
         step_e2e()

@@ -12,6 +12,7 @@ rule, for EVERY query row:
 
 One 12.5 M x 768 bf16 table (19.2 GB) is generated once per module exactly like bench.py generates
 its corpus (same per-chunk seeds); the smaller corpora are its prefixes.  Needs a B200."""
+import json
 import os
 import sys
 
@@ -233,3 +234,34 @@ def test_device_mask_column_shard_equals_host(ccr):
         np.testing.assert_array_equal(g.cols.cpu().numpy()[:n], h.host[1])
         np.testing.assert_array_equal(g.vals.cpu().numpy()[:n], h.host[2])
         assert g.nnz >= n and g.max_row_nnz >= h.max_row_nnz
+
+
+def test_bench_dump_outputs_are_the_timed_step(ccr, bench, tmp_path, monkeypatch, capsys):
+    """`bench.py --dump-outputs` writes the bits of the timed resident step: a direct search over the
+    same seeded table, queries and history mask gives them again.  `--steps` sets how many searches the
+    timed loops issue (counted at the table, next to the warm-up ones)."""
+    N, B, k, steps, warmup = 300_000, 256, 100, 3, 2
+    calls = []
+    search = ccr.EmbeddingTable.search
+    monkeypatch.setattr(ccr.EmbeddingTable, "search",
+                        lambda self, *a, **kw: calls.append(kw.get("encoded", False)) or search(self, *a, **kw))
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", str(steps), "--warmup", str(warmup), "--n-items", str(N),
+                                      "--batch", str(B), "--no-cpu-baseline", "--no-library-baseline",
+                                      "--dump-outputs", str(tmp_path)])
+    bench.run_ours(bench.parse())
+    line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
+    assert line["steps"] == steps
+    assert calls.count(True) == warmup + steps              # resident: warm-up + timed
+    assert calls.count(False) == max(1, warmup // 2) + steps  # e2e from host buffers: warm-up + timed
+    monkeypatch.setattr(ccr.EmbeddingTable, "search", search)
+    s, i = np.load(tmp_path / "scores.npy"), np.load(tmp_path / "ids.npy")
+    assert s.dtype == np.float32 and i.dtype == np.float64 and s.shape == i.shape == (B, k)
+    dev = torch.device("cuda:0")
+    table = ccr.EmbeddingTable(N, DIM, device=dev)
+    bench.build_shard(table, 0, N, dev)
+    q = table.encode_queries(torch.randn((B, DIM), generator=torch.Generator().manual_seed(7)))
+    indptr, cols, vals = bench.rows_to_csr(bench.history_mask_rows(B, N))
+    mask = ccr.SparseMask(indptr, cols, vals, N, ccr.MASK_SET, dev)
+    s2, i2 = table.search(q, k, mask=mask, encoded=True)
+    np.testing.assert_array_equal(s, s2.cpu().numpy())
+    np.testing.assert_array_equal(i, i2.cpu().numpy().astype(np.float64))

@@ -137,6 +137,52 @@ def test_lazy_algebra_matches_reference_classes():
                                type(rows_r[0]).collate_fn(rows_r).as_tensor("cpu"))
 
 
+@pytest.mark.parametrize("name", list(cases.RIME_CASES))
+def test_lazy_algebra_matches_stored_reference_output(name, golden_dir, monkeypatch):
+    """Every operation test_lazy_algebra_matches_reference_classes compares, without the reference tree:
+    the full matrix against the reference's stored output of the same expression (tests/golden/
+    rime_<case>.npz: dtype, shape, head block), everything derived from it against the oracle's restatement
+    of ``as_tensor`` (pinned to that stored output by test_oracle_golden.py)."""
+    import ccr_b200 as C
+    from oracle import ccr_oracle as O
+
+    g = np.load(os.path.join(golden_dir, f"rime_{name}.npz"))
+    c = cases.rime_case(name)
+    S = C.LazyDenseMatrix(c["U"]) @ C.LazyDenseMatrix(c["V"]).T
+    if c["prior"] is not None:
+        S = S + c["prior"]
+    ref = O.lazy_score_dense_ref(c["U"], c["V"], c["prior"])
+    dense = S.as_tensor("cpu")
+    assert str(dense.dtype) == str(g["dense_dtype"]) and tuple(dense.shape) == tuple(g["shape"])
+    np.testing.assert_array_equal(dense[:4, :16].numpy().astype(np.float64), g["dense_head"])
+    torch.testing.assert_close(dense, ref, rtol=0, atol=0)
+    B, N = S.shape
+    assert S.shape == tuple(ref.shape) and len(S) == B and S.size == B * N
+    # the reference's row-batch heuristic (score_array.py:8-18), set small enough to stream several batches
+    monkeypatch.setenv("BATCH_SIZE_FRAC", "1e-9")
+    mem = torch.cuda.get_device_properties(0).total_memory if torch.cuda.device_count() else 16e9
+    n_batches = int(B / (mem / 8 / N * 1e-9)) + 1
+    assert S.batch_size == int(np.ceil(B / n_batches)) < B
+    for key in (slice(0, 5), slice(3, B), [1, 4, B - 1]):
+        assert S[key].shape == tuple(ref[key].shape)
+        torch.testing.assert_close(S[key].as_tensor("cpu"), ref[key])
+    torch.testing.assert_close(S.T.as_tensor("cpu"), ref.T)
+    parts = [S[i:min(B, i + 4)] for i in range(0, B, 4)]
+    torch.testing.assert_close(S.collate_fn(parts).as_tensor("cpu"), ref)
+    b = S.batch_size
+    prior_rows = (lambda i: c["prior"][i:i + b]) if c["prior"] is not None else (lambda i: None)
+    want = max(float(O.lazy_score_dense_ref(c["U"][i:i + b], c["V"], prior_rows(i)).max()) for i in range(0, B, b))
+    assert float(C.score_op(S, "max")) == want == pytest.approx(float(ref.max()), rel=1e-6)
+    # values only: no stored reference output pins the dtype of a float32 matrix times a Python scalar
+    torch.testing.assert_close((S * 0.5).sigmoid().as_tensor("cpu").double(), (ref * 0.5).sigmoid().double())
+    if c["prior"] is not None:
+        prior = torch.as_tensor(c["prior"].toarray())
+        P = C.auto_cast_lazy_score(c["prior"])
+        torch.testing.assert_close(P[2:6].as_tensor("cpu"), prior[2:6])
+        rows = [P[i] for i in range(3)]
+        torch.testing.assert_close(type(rows[0]).collate_fn(rows).as_tensor("cpu"), prior[:3])
+
+
 def test_mask_helpers_on_cpu_arrays():
     """SparseMask canonicalisation / row slicing / column sharding arithmetic (host arrays only)."""
     from ccr_b200 import engine
@@ -186,7 +232,7 @@ def test_sparse_mask_from_flat_equals_from_lists(monkeypatch):
         engine.SparseMask.from_flat([1], [50], 50, -1e6, engine.MASK_SET, "cpu")
 
 
-def test_expression_recognition_factor_vs_materialised():
+def test_expression_recognition_factor_vs_materialised(monkeypatch):
     """Which expressions go to the fused kernel (factor pair), which to the dense top-k
     (materialised matrix), which are refused -- host-side logic only."""
     import scipy.sparse as sps
@@ -205,6 +251,7 @@ def test_expression_recognition_factor_vs_materialised():
     assert ccr.dense_plan(dense + dense) is None and ccr.fused_plan(mm + mm) is None   # two dense terms
     assert ccr.dense_plan(dense.exp()) is None and ccr.fused_plan(mm.exp()) is None    # non-linear
     assert ccr.dense_plan(ccr.auto_cast_lazy_score(np.zeros((2, 2)))) is not None      # plain ndarray
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)                       # also where a GPU is
     with pytest.raises(RuntimeError, match="CUDA"):                                      # no CPU path behind it
         ccr._assign_topk(dense, 2)
 
@@ -251,3 +298,37 @@ def test_bench_reference_arm_contract(capsys, monkeypatch):
     assert line["config"]["queries_per_step"] == 4096 and "plan" not in line["config"]
     assert line["e2e"] == {"value": line["value"], "unit": "queries/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["value"] == line["value"]
+
+
+def test_bench_dump_outputs_and_steps_option(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float32 / float64 .npy files; above the size limit the same seeded row
+    sample of every array plus its row numbers, identical from run to run.  `--steps` below 1 and a dump of the
+    reference arm are refused."""
+    import bench
+
+    s = np.arange(40 * 3, dtype=np.float32).reshape(40, 3)
+    i = s.astype(np.float64) * 2
+    bench.dump_outputs(str(tmp_path / "all"), {"scores": s, "ids": i})
+    np.testing.assert_array_equal(np.load(tmp_path / "all" / "scores.npy"), s)
+    np.testing.assert_array_equal(np.load(tmp_path / "all" / "ids.npy"), i)
+    assert not (tmp_path / "all" / "rows.npy").exists()
+    limit = 10 * (3 * 4 + 3 * 8 + 8)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"scores": s, "ids": i}, limit=limit)
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("scores", "ids", "rows")}
+    rows = got["rows"].astype(np.int64)
+    assert got["rows"].dtype == np.float64 and len(rows) == 10 and (np.diff(rows) > 0).all()
+    assert sum(a.nbytes for a in got.values()) <= limit
+    np.testing.assert_array_equal(got["scores"], s[rows])
+    np.testing.assert_array_equal(got["ids"], i[rows])
+    for n, a in got.items():
+        np.testing.assert_array_equal(np.load(tmp_path / "b" / f"{n}.npy"), a)
+    with pytest.raises(TypeError):
+        bench.dump_outputs(str(tmp_path / "c"), {"ids": i.astype(np.int64)})
+    monkeypatch.setattr("sys.argv", ["bench.py", "--steps", "3", "--dump-outputs", str(tmp_path)])
+    a = bench.parse()
+    assert a.steps == 3 and a.dump_outputs == str(tmp_path)
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr("sys.argv", ["bench.py", *argv])
+        with pytest.raises(SystemExit):
+            bench.parse()
