@@ -15,16 +15,12 @@ static thread_local char g_err[512] = "";
 static void* g_status_record = nullptr;  // see ccr_set_status_record
 static thread_local cudaEvent_t g_prof_start = nullptr, g_prof_stop = nullptr;  // see ccr_set_profile_events
 
-// Diagnostic knobs (DESIGN.md §7b).  The environment is parsed ONCE, on first use; a test or A/B
-// harness that changes it inside a live process calls ccr_debug_reload_env().  None is needed in
-// production.
+// Test levers (DESIGN.md §7b): each forces a choice the planner otherwise makes itself, so that the
+// tests can check that results do not depend on it.  The environment is parsed ONCE, on first use; a
+// test that changes it inside a live process calls ccr_debug_reload_env().  None is needed in production.
 namespace {
 struct Knobs {
-  int mask_exclude = 0, two_cta = -1, split_mult = 0, cap_mult = 0, no_share = 0, no_seed = 0, no_hist = 0;
-  long long seed_m = 0;
-  int debug = 0, debug_grid = 0, keep_tau = 0, throttle = -1, lead = 0, no_qpad = 0;
-  int bm25_blockwide = 0, thr_mode = -1;
-  float debug_tau = 0.f;
+  int two_cta = -1, lead = 0, no_hist = 0, bm25_blockwide = 0;
 };
 Knobs g_knobs;
 std::once_flag g_knobs_once;
@@ -32,23 +28,10 @@ std::once_flag g_knobs_once;
 int env_int(const char* name, int dflt) { const char* v = getenv(name); return v ? atoi(v) : dflt; }
 void load_knobs() {
   Knobs k;
-  k.mask_exclude = getenv("CCR_MASK_EXCLUDE") != nullptr;
   k.two_cta = env_int("CCR_2CTA", -1);
-  k.split_mult = env_int("CCR_SPLIT_MULT", 0);
-  k.cap_mult = env_int("CCR_CAP_MULT", 0);
-  k.no_share = getenv("CCR_NO_SHARE") != nullptr;
-  k.no_seed = getenv("CCR_NO_SEED") != nullptr;
-  k.no_hist = getenv("CCR_NO_HIST") != nullptr;
-  { const char* v = getenv("CCR_SEED_M"); k.seed_m = v ? atoll(v) : 0; }
-  k.debug = env_int("CCR_DEBUG", 0);
-  k.debug_grid = env_int("CCR_DEBUG_GRID", 0);
-  k.keep_tau = getenv("CCR_DEBUG_KEEP_TAU") != nullptr;
-  k.throttle = env_int("CCR_THROTTLE", -1);
   k.lead = env_int("CCR_LEAD", 0);
-  k.no_qpad = getenv("CCR_NO_QPAD") != nullptr;
+  k.no_hist = getenv("CCR_NO_HIST") != nullptr;
   k.bm25_blockwide = getenv("CCR_BM25_BLOCKWIDE") != nullptr;
-  k.thr_mode = env_int("CCR_THR_MODE", -1);
-  { const char* v = getenv("CCR_DEBUG_TAU"); k.debug_tau = v ? (float)atof(v) : 0.f; }
   g_knobs = k;
 }
 const Knobs& knobs() {
@@ -92,9 +75,14 @@ struct Plan {
   int two_cta;           // tensor-core kernel variant: CTA pairs (cta_group::2)
   int include_mask;      // 1: masked items stream through and are dropped in finalize (k + h candidates/row)
   int k_keep;            // k + h_max in include mode, else k
-  int seed_m;            // sampled items of the threshold-seeding pre-pass (0 = off)
+  int seed_m;            // sampled items of the threshold-seeding pre-pass (0 = no pre-pass)
   long long seed_stride; // item-row stride of the sample
   long long seed_ld;     // row pitch of the sampled score matrix (floats)
+  int use_hist;          // the pre-pass also sets up the per-row score histograms (histogram sharing)
+  int throttle;          // bounded-drift throttle between the units of one item split (tensor-core kernel)
+  int lead_tiles;        // throttle: max lead (item tiles) of a producer over its slowest peer
+  int lead_every;        // throttle: progress is published / checked every lead_every tiles (power of two)
+  int throttle_poller;   // throttle: 1 a dedicated warp watches the peers, 0 the producer polls inline
   size_t off_seed;
   size_t off_progress;
   size_t off_qpad;       // zero-padded copy of a short query batch (B < 128): every TMA box in bounds
@@ -129,13 +117,12 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
   const int sms = device_sm_count();
   const Knobs& kn = knobs();
   pl->algo = algo;
-  pl->include_mask = (algo == CCR_ALGO_TCGEN05 && nnz > 0 && h_max >= 0 && h_max <= 256 && k + h_max <= CCR_MAX_K &&
-                      !kn.mask_exclude) ? 1 : 0;
+  pl->include_mask = (algo == CCR_ALGO_TCGEN05 && nnz > 0 && h_max >= 0 && h_max <= 256 && k + h_max <= CCR_MAX_K) ? 1 : 0;
   pl->k_keep = pl->include_mask ? (int)(k + h_max) : k;
   if (algo == CCR_ALGO_TCGEN05) {
     // CTA pairs (cta_group::2, 256 query rows per unit) stream each item tile once for 256 queries:
     // a third less operand traffic from L2 into the SMs and a GEMM pipeline that is ~9 % faster on its
-    // own.  With the bounded-drift throttle (see ccr_score_topk_bf16) they win at every batch size
+    // own.  With the bounded-drift throttle (below) they win at every batch size
     // measured on B200 (8.84M x 768, k=100, same box, profiles/r01_pairs_throttle_ab.txt): B=256 2.95 vs
     // 3.27 ms, 512 5.7 vs 6.05, 1024 11.2-11.7 vs 12.2, 2048 21.7 vs 23.4, 4096 43.3 vs 46.8, 8192 90.0 vs
     // 92.6; bench.py's sustained loop 94.3-95.0 k vs 87.1-87.4 k queries/s.  A pair pads the batch to 256
@@ -152,13 +139,8 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
     pl->rows_pad = pl->n_q_tiles * unit_rows;
     long long tiles = (n_items + kITile - 1) / kITile;
     pl->S = splits_tc(pl->n_q_tiles, tiles, pl->two_cta ? sms / 2 : sms);
-    if (kn.split_mult > 0) {  // experiment knob: finer units (more waves)
-      long long s2 = (long long)pl->S * kn.split_mult;
-      if (s2 >= 1 && s2 <= tiles && s2 * 2 <= 1024) pl->S = (int)s2;
-    }
     pl->halves = 2;
     pl->C = cand_capacity(pl->k_keep, 128);
-    if (kn.cap_mult >= 1 && kn.cap_mult <= 16) pl->C *= kn.cap_mult;  // experiment knob: fewer prunes
     {
       // streams of one row that run in the first wave; use half of them for the bound so a few
       // late streams do not hold it back
@@ -173,10 +155,26 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
       const int kk = pl->k_keep;  // m * j distinct items must cover k plus every possibly-masked one
       while ((kk + j - 1) / j > use) j <<= 1;
       if (j > k) j = k;
-      pl->share_j = (s_row > 1 && !kn.no_share) ? j : 0;
+      pl->share_j = s_row > 1 ? j : 0;
       pl->share_m = (kk + j - 1) / j;
       if (pl->share_m > 256 || pl->share_m > s_row) pl->share_j = 0;
     }
+    // Bounded-drift throttle of the units that stream one item split (they only share its tiles through
+    // L2 while they stay close; without it a leader runs away from its followers and every follower
+    // misses L2 too: 99 GB instead of 15 GB of DRAM reads were measured for CTA pairs at B=4096).
+    // Same-box A/B on B200, 8.84M x 768 (profiles/r02_throttle_ab.md):
+    //  * lead: 16 tiles below 4 units per split (no throttle needed at 2: 6.27 vs 6.30 ms), 8 tiles from
+    //    4 units per split on (B=1024 11.71 vs 11.75, 2048 21.6 vs 22.0, 4096 42.6 vs 42.9 ms); leads of
+    //    2-4 tiles stall the producers on the polling itself and lose 10-30 %.
+    //  * who polls: the producer itself every lead/2 tiles ("inline") is fastest up to 16 units per split
+    //    (B <= 4096: 42.6 vs 46.0 ms at B=4096, 21.6 vs 28.0 at 2048); from 32 units per split on, reading
+    //    32 counters serially stalls the producer and a dedicated poller warp that keeps
+    //    "slowest + lead" in shared memory wins (B=8192: 84.9 vs 89.2 ms).
+    //  * single CTAs (odd tile counts, B > 8192) gain from the same throttle: B=640 8.63 vs 9.16 ms, 1152
+    //    13.8 vs 14.9, 16384 (poller) 183.1 vs 186.8.
+    pl->throttle = pl->n_q_tiles > 1 ? 1 : 0;
+    pl->lead_tiles = pl->n_q_tiles >= 4 ? 8 : 16;
+    pl->throttle_poller = pl->n_q_tiles >= 32 ? 1 : 0;
   } else {
     pl->n_q_tiles = (int)((B + kSimtRows - 1) / kSimtRows);
     if (pl->n_q_tiles < 1) pl->n_q_tiles = 1;
@@ -190,7 +188,11 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
     pl->two_cta = 0;
     pl->C = cand_capacity(k, kSimtChunk);
     pl->share_j = 0; pl->share_m = 0;
+    pl->throttle = 0; pl->lead_tiles = 0; pl->throttle_poller = 0;
   }
+  if (kn.lead >= 1 && kn.lead <= 4096) pl->lead_tiles = kn.lead;
+  pl->lead_every = 1;
+  while (pl->lead_every * 2 <= pl->lead_tiles && pl->lead_every < 8) pl->lead_every *= 2;  // 16 -> 8, 8 -> 8, 4 -> 4
   size_t off = 0;
   pl->off_cand = off;   off = align_up(off + (size_t)pl->rows_pad * pl->S * pl->halves * pl->C * sizeof(u64), 256);
   pl->off_counts = off; off = align_up(off + (size_t)pl->rows_pad * pl->S * pl->halves * sizeof(int), 256);
@@ -204,8 +206,8 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
   pl->off_hist = off;   off = align_up(off + (size_t)pl->rows_pad * kHistBins * sizeof(u32), 256);
   pl->off_hpar = off;   off = align_up(off + (size_t)pl->rows_pad * sizeof(uint2), 256);
   pl->off_qpad = off;     off = align_up(off + (size_t)kQTile * 4096 * sizeof(__nv_bfloat16), 256);
-  pl->seed_m = 0; pl->seed_stride = 1; pl->seed_ld = 0; pl->off_seed = off;
-  if (algo == CCR_ALGO_TCGEN05 && pl->share_j >= 0 && n_items >= (1 << 18) && !kn.no_seed) {
+  pl->seed_m = 0; pl->seed_stride = 1; pl->seed_ld = 0; pl->off_seed = off; pl->use_hist = 0;
+  if (algo == CCR_ALGO_TCGEN05 && n_items >= (1 << 18)) {
     // strided sample of max(N/256, 64k) items (4096..131072, <= N/8); the pre-pass keeps one fp32 value
     // per 8 sampled items (their best score), capped so that matrix stays <= 512 MB
     // With histogram sharing (no mask / include mode) the seed only has to be a sensible origin for the
@@ -223,32 +225,20 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
     if (m > n_items / 8) m = n_items / 8;
     long long cap = 8LL * (512LL << 20) / (4LL * pl->rows_pad);
     if (m > cap) m = cap;
-    if (kn.seed_m >= 1024 && kn.seed_m < m) m = kn.seed_m;  // experiment knob
     m = m / 256 * 256;
     if (m >= 1024 && 16LL * pl->k_keep <= m) {
       pl->seed_m = (int)m;
       pl->seed_stride = n_items / m;
       pl->seed_ld = m / 8;
+      // the histogram needs the seed bound as its origin and counts every streamed item, so it is
+      // off in exclude-mask mode (masked items must not be counted)
+      pl->use_hist = hist_ok && !kn.no_hist;
       off = align_up(off + (size_t)pl->rows_pad * (size_t)pl->seed_ld * sizeof(float), 256);
     }
   }
   pl->total = off;
   return true;
 }
-
-// Bounded-drift throttle of the units that stream one item split (they only share its tiles through L2
-// while they stay close).  Same-box A/B on B200, 8.84M x 768 (profiles/r02_throttle_ab.md):
-//  * who polls: the producer itself every lead/2 tiles ("inline") is fastest up to 16 units per split
-//    (B <= 4096: 42.6 vs 46.0 ms at B=4096, 21.6 vs 28.0 at 2048); from 32 units per split on, reading
-//    32 counters serially stalls the producer and a dedicated poller warp that keeps
-//    "slowest + lead" in shared memory wins (B=8192: 84.9 vs 89.2 ms).
-//  * lead: 16 tiles below 4 units per split (no throttle needed at 2: 6.27 vs 6.30 ms), 8 tiles from
-//    4 units per split on (B=1024 11.71 vs 11.75, 2048 21.6 vs 22.0, 4096 42.6 vs 42.9 ms); leads of 2-4
-//    tiles stall the producers on the polling itself and lose 10-30 %.
-int default_lead_tiles(const Plan& pl) { return pl.n_q_tiles >= 4 ? 8 : 16; }
-//  * single CTAs (odd tile counts, B > 8192) gain from the same throttle: B=640 8.63 vs 9.16 ms, 1152 13.8
-//    vs 14.9, 16384 (poller) 183.1 vs 186.8.
-int default_throttle_poller(const Plan& pl) { return pl.n_q_tiles >= 32 ? 1 : 0; }
 
 int check_shape(long long B, long long n_items, int D, int k, int flags) {
   if (B < 0 || n_items < 0) return fail(CCR_EINVAL, "negative size B=%lld n_items=%lld", B, n_items);
@@ -303,19 +293,16 @@ int ccr_plan_info(int64_t B, int64_t n_items, int D, int k, int64_t mask_nnz, in
   if (!info8) return fail(CCR_EINVAL, "info8 is null");
   Plan pl;
   make_plan(B, n_items, D, k, mask_nnz, mask_nnz > 0 ? mask_max_row_nnz : -1, flags, &pl);
-  const bool seeded = pl.seed_m > 0 && n_items > 0 && !knobs().keep_tau;
-  int lead = pl.algo == CCR_ALGO_TCGEN05 ? default_lead_tiles(pl) : 0;
-  if (knobs().lead >= 1 && knobs().lead <= 4096) lead = knobs().lead;
   info8[0] = pl.n_q_tiles;
   info8[1] = pl.S;
   info8[2] = pl.C;
   info8[3] = pl.algo;
   info8[4] = pl.two_cta;
-  info8[5] = seeded ? pl.seed_m : 0;
+  info8[5] = pl.seed_m;
   // kernels one ccr_score_topk_bf16 call launches: [seeding GEMM, seed select,] fused score+select,
   // [mask overrides,] finalize  (memsets / the short-batch query copy are not kernels of this library)
-  info8[6] = (B > 0) ? (seeded ? 2 : 0) + (n_items > 0 ? 1 : 0) + (mask_nnz > 0 ? 1 : 0) + 1 : 0;
-  info8[7] = lead;
+  info8[6] = (B > 0) ? (pl.seed_m > 0 ? 2 : 0) + (n_items > 0 ? 1 : 0) + (mask_nnz > 0 ? 1 : 0) + 1 : 0;
+  info8[7] = pl.lead_tiles;
   return CCR_OK;
 }
 
@@ -349,12 +336,11 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   if (!workspace || workspace_bytes < pl.total)
     return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, pl.total);
   unsigned char* ws = (unsigned char*)workspace;
-  const Knobs& kn = knobs();
   // watchdog record: the caller's host-mapped one (readable after a device trap) or a workspace slot
   DeviceStatus* status = g_status_record ? (DeviceStatus*)g_status_record : (DeviceStatus*)(ws + pl.off_status);
-  // one memset for everything that must start from zero: status slot, throttle counters and (unless
-  // the debug knob keeps them) thresholds, published quantiles, histograms and their parameters
-  cudaError_t e = cudaMemsetAsync(ws + pl.off_status, 0, (kn.keep_tau ? pl.off_gtau : pl.off_qpad) - pl.off_status, st);
+  // one memset for everything that must start from zero: status slot, throttle counters, thresholds,
+  // published quantiles, histograms and their parameters
+  cudaError_t e = cudaMemsetAsync(ws + pl.off_status, 0, pl.off_qpad - pl.off_status, st);
   if (e != cudaSuccess) return fail(CCR_ECUDA, "memset call state: %s", cudaGetErrorString(e));
 
   SelectParams sp = {};
@@ -366,37 +352,23 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   sp.cand = (u64*)(ws + pl.off_cand);
   sp.counts = (int*)(ws + pl.off_counts);
   sp.status = status;
-  sp.debug = kn.debug; sp.debug_tau = kn.debug_tau; sp.debug_grid = kn.debug_grid;
   sp.g_tau = nullptr; sp.g_q = nullptr; sp.S_row = pl.S * pl.halves; sp.share_j = pl.share_j; sp.share_m = pl.share_m;
   sp.dense_out = nullptr; sp.ld_out = 0; sp.store_max8 = 0;
-  sp.progress = nullptr;
   sp.g_hist = nullptr; sp.g_hpar = nullptr;
-  // bounded drift between the units that stream the same item split (see default_lead_tiles): without
-  // it a leader runs away from its followers and every follower misses L2 too (99 GB instead of 15 GB
-  // of DRAM reads were measured for CTA pairs at B=4096)
-  bool use_throttle = pl.n_q_tiles > 1;
-  if (kn.throttle >= 0) use_throttle = kn.throttle != 0;
-  sp.lead_tiles = pl.algo == CCR_ALGO_TCGEN05 ? default_lead_tiles(pl) : 16;
-  if (kn.lead >= 1 && kn.lead <= 4096) sp.lead_tiles = kn.lead;
-  sp.lead_every = 1;
-  while (sp.lead_every * 2 <= sp.lead_tiles && sp.lead_every < 8) sp.lead_every *= 2;  // 16 -> 8, 8 -> 8, 4 -> 4
-  sp.throttle_poller = kn.thr_mode >= 0 ? kn.thr_mode : default_throttle_poller(pl);
-  if (pl.algo == CCR_ALGO_TCGEN05 && use_throttle) sp.progress = (int*)(ws + pl.off_progress);
+  sp.progress = pl.throttle ? (int*)(ws + pl.off_progress) : nullptr;
+  sp.lead_tiles = pl.lead_tiles; sp.lead_every = pl.lead_every; sp.throttle_poller = pl.throttle_poller;
   if (pl.share_j > 0 || pl.seed_m > 0) {
     sp.g_tau = (u32*)(ws + pl.off_gtau);
     sp.g_q = (u32*)(ws + pl.off_gq);
   }
-  if (pl.seed_m > 0 && n_items > 0 && !kn.keep_tau) {
+  if (pl.seed_m > 0) {
     // threshold seeding pre-pass: scores of a strided item sample -> per-row lower bound in g_tau
     SelectParams ss = sp;
     ss.n_items = pl.seed_m; ss.ldi = ldi * pl.seed_stride;
     ss.mask_indptr = nullptr; ss.mask_cols = nullptr;
     ss.dense_out = (float*)(ws + pl.off_seed); ss.ld_out = pl.seed_ld; ss.store_max8 = 1;
     ss.g_tau = nullptr; ss.g_q = nullptr; ss.share_j = 0; ss.progress = nullptr;
-    // the histogram needs the seed bound as its origin and counts every streamed item, so it is
-    // off in exclude-mask mode (masked items must not be counted)
-    const bool use_hist = sp.mask_cols == nullptr && !kn.no_hist;
-    if (use_hist) { sp.g_hist = (u32*)(ws + pl.off_hist); sp.g_hpar = (const uint2*)(ws + pl.off_hpar); }
+    if (pl.use_hist) { sp.g_hist = (u32*)(ws + pl.off_hist); sp.g_hpar = (const uint2*)(ws + pl.off_hpar); }
     ss.two_cta = 0; ss.n_q_tiles = pl.rows_pad / kQTile;
     long long tiles = (pl.seed_m + kITile - 1) / kITile;
     ss.S = splits_tc(ss.n_q_tiles, tiles, device_sm_count());
@@ -404,11 +376,11 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
     if (lr0) return fail(CCR_ECUDA, "seed GEMM launch failed (%d)", lr0);
     // per row: the (k + h)-th largest of the seed_m / 8 group maxima
     lr0 = launch_seed_tau(ss.dense_out, pl.seed_ld, (int)pl.seed_ld, (int)B, k, has_mask ? (const long long*)mask_indptr : nullptr,
-                          sp.g_tau, use_hist ? (uint2*)(ws + pl.off_hpar) : nullptr, st);
+                          sp.g_tau, pl.use_hist ? (uint2*)(ws + pl.off_hpar) : nullptr, st);
     if (lr0) return fail(CCR_ECUDA, "seed select launch failed: %s", cudaGetErrorString((cudaError_t)lr0));
   }
 
-  if (pl.algo == CCR_ALGO_TCGEN05 && B < kQTile && n_items > 0 && !kn.no_qpad) {
+  if (pl.algo == CCR_ALGO_TCGEN05 && B < kQTile && n_items > 0) {
     // short batch: stage the queries in a [128, D] block so that no TMA box of the query operand is
     // out of bounds (measurably faster than hardware zero-fill of 120+ rows); only the padding rows
     // are zeroed

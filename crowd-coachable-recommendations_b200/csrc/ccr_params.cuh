@@ -63,9 +63,6 @@ struct SelectParams {
   float* dense_out;      // [rows_pad][ld_out], null in select mode
   long long ld_out;      // floats per row: >= n_items rounded up to 256 (full) or / 8 (store_max8)
   int store_max8;
-  float debug_tau;  // CCR_DEBUG & 16: fixed threshold, no prune (cnt wraps); & 32: also no store
-  int debug;  // CCR_DEBUG bits (env, diagnostics only): 1 = skip selection, keep pipeline
-  int debug_grid;  // CCR_DEBUG_GRID: cap on the persistent grid (0 = none)
 };
 
 struct FinalizeParams {

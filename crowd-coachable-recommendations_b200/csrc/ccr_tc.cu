@@ -15,8 +15,6 @@
 // query tile varying fastest so CTAs running concurrently share item tiles through L2.
 #include <cuda.h>
 #include <stddef.h>
-#include <stdio.h>
-#include <stdlib.h>
 
 #include "ccr_params.cuh"
 
@@ -208,7 +206,6 @@ struct SelState {
   int stream;      // index of this stream among the row's streams
   u32* hist;       // the row's score histogram (null: off for this row)
   u32 hbase, hshift;  // bucket b covers ord32 scores [hbase + (b << hshift), hbase + ((b + 1) << hshift))
-  unsigned n_slow, n_prune;  // debug counters (CCR_DEBUG & 4)
 };
 
 __device__ __forceinline__ float max8(const u32 (&v)[32], int g) {
@@ -276,13 +273,11 @@ static __device__ __noinline__ u32 hist_bound(const u32* hist, int need, u32 hba
 // lowest-id tie rule because a stream sees its items in ascending id order.
 template <bool kMask>
 __device__ __forceinline__ void filter_chunk(const u32 (&v)[32], u32 col0, SelState& st, const SelectParams& p) {
-  if (p.debug & 1) return;
   float m8[4];
 #pragma unroll
   for (int g = 0; g < 4; ++g) m8[g] = max8(v, g);
   const float m = fmaxf(fmaxf(m8[0], m8[1]), fmaxf(m8[2], m8[3]));
   if (!__any_sync(0xffffffffu, m >= st.tau_f)) return;
-  st.n_slow++;
   const u32 nlo0 = 0xFFFFFFFFu - col0;  // low key word of column col0; column col0+j -> nlo0 - j
 #define CCR_APPEND(J)                                                                            \
   if (kMask) {                                                                                   \
@@ -302,7 +297,6 @@ __device__ __forceinline__ void filter_chunk(const u32 (&v)[32], u32 col0, SelSt
     CCR_APPEND(G * 8 + 4) CCR_APPEND(G * 8 + 5) CCR_APPEND(G * 8 + 6) CCR_APPEND(G * 8 + 7)      \
   }
   CCR_GROUP(0) CCR_GROUP(1) CCR_GROUP(2) CCR_GROUP(3)
-  if (p.debug & 16) st.cnt &= 127;
 #undef CCR_GROUP
 #undef CCR_APPEND
   asm volatile("" ::: "memory");  // appended keys are read back by the prune
@@ -364,7 +358,7 @@ static __device__ __noinline__ u64 exact_prune(u64* b, int n, int k, int j, bool
 // Prune one stream's buffer (all 32 lanes cooperate), publish its share_j-th best, refresh the
 // row's shared bound.  Returns (kept << 32) | float bits of the stream's new threshold.
 static __device__ __noinline__ u64 prune_stream(u64* b, int n, int k, int C, int row_s, int stream_s, ShareArgs sh,
-                                                u32 hist_s, u32 stage_s, int debug) {
+                                                u32 hist_s, u32 stage_s) {
   const int lane = threadIdx.x & 31;
   const bool staged = C <= kStageKeys;
   const int jj = sh.share_j > 0 ? sh.share_j : k;
@@ -372,11 +366,9 @@ static __device__ __noinline__ u64 prune_stream(u64* b, int n, int k, int C, int
   int kept = k;
   u32 j_ord = 0u, pivot_ord = 0u;
   // fast path: one histogram pass; leaves between k and (k + C-128)/2 survivors
-  bool fast = false;
-  if (!(debug & 64)) {
-    if (staged) fast = warp_prune_hist<true>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord);
-    else fast = warp_prune_hist<false>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord);
-  }
+  const bool fast =
+      staged ? warp_prune_hist<true>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord)
+             : warp_prune_hist<false>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord);
   if (fast) {
     new_tau = unord32(pivot_ord);  // ">=": every key at or above the pivot bucket was kept
   } else {
@@ -396,23 +388,12 @@ static __device__ __noinline__ u64 prune_stream(u64* b, int n, int k, int C, int
   return ((u64)(u32)kept << 32) | (u64)__float_as_uint(new_tau);
 }
 
-// CCR_DEBUG & 512: invariant checks that end in an error record + trap instead of a wild access
-__device__ __forceinline__ void debug_fail(DeviceStatus* st, int where, int extra) {
-  if (st) { st->code = 2; st->where = where; st->block = blockIdx.x; st->extra = extra; }
-  __threadfence_system();
-  __trap();
-}
-
 // Prune every stream of this warp whose buffer could overflow during the next half tile.  Runs
 // after the accumulator has been handed back, i.e. off the MMA critical path.
-__device__ __forceinline__ void prune_pending(SelState& st, const ShareArgs& sh, int k, int C, u32 hist_s,
-                                              u32 stage_s, int debug, DeviceStatus* status) {
+__device__ __forceinline__ void prune_pending(SelState& st, const ShareArgs& sh, int C, u32 hist_s, u32 stage_s) {
   const int lane = threadIdx.x & 31;
-  if ((debug & 512) && (st.cnt > C || st.cnt < 0 || st.k_row > C - 128 || st.k_row < 1))
-    debug_fail(status, 500, st.cnt > C || st.cnt < 0 ? st.cnt : -st.k_row);
   unsigned need = __ballot_sync(0xffffffffu, st.cnt > C - 128);
   while (need) {
-    st.n_prune++;
     const int src = __ffs(need) - 1;
     need &= need - 1;
     u64* b = reinterpret_cast<u64*>(__shfl_sync(0xffffffffu, (u64)(uintptr_t)st.buf, src));
@@ -420,8 +401,7 @@ __device__ __forceinline__ void prune_pending(SelState& st, const ShareArgs& sh,
     const int row_s = __shfl_sync(0xffffffffu, st.row, src);
     const int stream_s = __shfl_sync(0xffffffffu, st.stream, src);
     const int k_s = __shfl_sync(0xffffffffu, st.k_row, src);
-    const u64 r = prune_stream(b, n, k_s, C, row_s, stream_s, sh, hist_s, stage_s, debug);
-    if ((debug & 512) && ((int)(r >> 32) > n || (int)(r >> 32) < k_s)) debug_fail(status, 501, (int)(r >> 32));
+    const u64 r = prune_stream(b, n, k_s, C, row_s, stream_s, sh, hist_s, stage_s);
     if (lane == src) { st.cnt = (int)(r >> 32); st.tau_f = __uint_as_float((u32)r); }
   }
 }
@@ -552,18 +532,15 @@ select_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
           for (int kb = 0; kb < num_kb; ++kb) {
             mbar_wait(&sh->empty[stage], phase ^ 1u, p.status, 100 + stage);
             unsigned char* sa = smem + (size_t)stage * kStageBytes;
-            // CCR_DEBUG & 1024 (experiment, results invalid): stream the query operand only for the first
-            // tile of a unit -- what the pipeline would cost if the query tile were resident on chip
-            const bool skip_q = (p.debug & 1024) && t > t0;
             if (kCta == 2) {
               // both CTAs' bytes are accounted on the leader's barrier; only the leader arms it
-              if (crank == 0) mbar_expect_tx(&sh->full[stage], 2 * (skip_q ? G::kItemBytes : kStageBytes));
+              if (crank == 0) mbar_expect_tx(&sh->full[stage], 2 * kStageBytes);
               const u32 lbar = mapa_u32(&sh->full[stage], 0);
-              if (!skip_q) tma_load_2d_2cta(sa, &tmap_q, kb * kKBlock, qt * kQRows + crank * kQTile, lbar);
+              tma_load_2d_2cta(sa, &tmap_q, kb * kKBlock, qt * kQRows + crank * kQTile, lbar);
               tma_load_2d_2cta(sa + kBytesA, &tmap_items, kb * kKBlock, (int)(t * kITile) + crank * G::kItemRows, lbar);
             } else {
-              mbar_expect_tx(&sh->full[stage], skip_q ? G::kItemBytes : kStageBytes);
-              if (!skip_q) tma_load_2d(sa, &tmap_q, kb * kKBlock, qt * kQTile, &sh->full[stage]);
+              mbar_expect_tx(&sh->full[stage], kStageBytes);
+              tma_load_2d(sa, &tmap_q, kb * kKBlock, qt * kQTile, &sh->full[stage]);
               tma_load_2d(sa + kBytesA, &tmap_items, kb * kKBlock, (int)(t * kITile), &sh->full[stage]);
             }
             if (++stage == kStages) { stage = 0; phase ^= 1u; }
@@ -736,14 +713,10 @@ select_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
       const long long t0 = (long long)u * tiles_total / p.S, t1 = (long long)(u + 1) * tiles_total / p.S;
       const int row = qt * kQRows + crank * kQTile + row_in_tile;
       const bool valid_row = row < p.B;
-      unsigned long long t_start = 0;
-      if (p.debug & (4 | 128)) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_start));
       SelState st;
-      st.n_slow = st.n_prune = 0;
       st.buf = p.cand + (((long long)row * p.S + u) * 2 + half) * C;
       st.cnt = 0;
-      st.tau_f = (valid_row && !(p.debug & 2)) ? -INFINITY : INFINITY;  // debug 2: reject everything
-      if ((p.debug & 16) && valid_row) st.tau_f = p.debug_tau;
+      st.tau_f = valid_row ? -INFINITY : INFINITY;
       st.mbeg = 0; st.mend = 0; st.sig = 0ull; st.sig2 = 0ull;
       st.row = row; st.stream = u * 2 + half;
       st.hist = nullptr; st.hbase = 0u; st.hshift = 0u;
@@ -763,15 +736,14 @@ select_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
           st.sig |= 1ull << (mc & 63u);
           st.sig2 |= 1ull << ((mc >> 6) & 63u);
         }
-        if (p.debug & 256) { st.sig = 0ull; st.sig2 = 0ull; }  // experiment: never run the exact search
       }
 
       for (long long t = t0; t < t1; ++t) {
         u32 gt = 0u;
-        if (p.g_tau && valid_row && !(p.debug & 8)) gt = __ldcg(p.g_tau + row);  // issued before the wait
+        if (p.g_tau && valid_row) gt = __ldcg(p.g_tau + row);  // issued before the wait
         mbar_wait(&sh->tmem_full[acc], acc_phase, p.status, 400 + acc);
         tc_fence_after();
-        if (gt > ord32(st.tau_f) && !(p.debug & 16)) st.tau_f = unord32(gt);
+        if (gt > ord32(st.tau_f)) st.tau_f = unord32(gt);
         const u32 taddr0 = tmem_base + ((u32)(quad * 32) << 16) + (u32)(acc * kITile + half * 128);
         const long long col0 = t * kITile + half * 128;
         const bool ragged = col0 + 128 > p.n_items;
@@ -802,7 +774,7 @@ select_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             for (int j = 0; j < 32; ++j) { v[j] = w2[j]; w1[j] = w3[j]; }
           }
         }
-        if (!(p.debug & 16)) prune_pending(st, sa, k, C, hist_s, stage_s, p.debug, p.status);
+        prune_pending(st, sa, C, hist_s, stage_s);
         if (!kMask && p.g_hist) {
           // refresh the row bound from the histogram at tiles 4, 8, 16, ... 256 and every 256 after
           const long long ti = t - t0 + 1;
@@ -814,26 +786,9 @@ select_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             }
           }
         }
-        if ((p.debug & 128) && blockIdx.x == 0 && ew == 0 && lane == 0) {
-          const long long ti = t - t0 + 1;
-          if ((ti & (ti - 1)) == 0 || t + 1 == t1) {
-            unsigned long long now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            printf("[ccr tl] unit %d tile %lld us %llu slow %u prunes %u cnt %d tau %f\n", unit, ti,
-                   (now - t_start) / 1000ull, st.n_slow, st.n_prune, st.cnt, st.tau_f);
-          }
-        }
         if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
       }
       p.counts[((long long)row * p.S + u) * 2 + half] = st.cnt;
-      if ((p.debug & 4) && blockIdx.x < 2) {
-        unsigned long long t_end;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_end));
-        if (lane == 0)
-          printf("[ccr stats] cta %d unit %d warp %d tiles %lld slow %u prunes %u cnt(lane0) %d tau %f us %llu\n",
-                 blockIdx.x, unit, ew, t1 - t0, st.n_slow, st.n_prune, st.cnt, st.tau_f,
-                 (t_end - t_start) / 1000ull);
-      }
     }
    }
   }
@@ -986,7 +941,6 @@ static int launch_variant(const CUtensorMap& tq, const CUtensorMap& ti, const Se
   const int n_units = p.n_q_tiles * p.S;
   int workers = num_sms / kCta;  // persistent CTAs (kCta = 1) or CTA pairs (kCta = 2)
   if (n_units < workers) workers = n_units;
-  if (p.debug_grid > 0 && p.debug_grid / kCta < workers) workers = p.debug_grid / kCta;
   if (workers < 1) workers = 1;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)(workers * kCta));

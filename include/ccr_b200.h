@@ -16,7 +16,7 @@
  *   - return value: 0 on success, negative CCR_E* on failure; ccr_last_error_string()
  *     returns a thread-local description of the last failure;
  *   - re-entrant and stream-ordered.  Process-wide state is limited to: a per-device cache of
- *     immutable device attributes; the diagnostic CCR_* environment knobs, parsed once on first
+ *     immutable device attributes; the CCR_* environment test levers, parsed once on first
  *     use (ccr_debug_reload_env re-reads them); the optional watchdog record pointer
  *     (ccr_set_status_record).  The measurement hook (ccr_set_profile_events) is per host thread.
  *     Calls that share a workspace must be ordered on one stream.
@@ -298,8 +298,8 @@ int ccr_plan_info(int64_t B, int64_t n_items, int D, int k, int64_t mask_nnz, in
  */
 void ccr_set_status_record(void* host_mapped_ptr);
 
-/* Diagnostics: re-read the CCR_* environment knobs (DESIGN.md section 7b).  They are parsed once on
- * first use; an A/B harness that changes the environment of a live process calls this afterwards.
+/* Tests: re-read the CCR_* environment test levers (DESIGN.md section 7b).  They are parsed once on
+ * first use; a test that changes the environment of a live process calls this afterwards.
  * Not thread-safe against concurrent ccr_* calls. */
 void ccr_debug_reload_env(void);
 

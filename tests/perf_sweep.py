@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Batch sweep x variant A/B on ONE box (builder tool; feeds profiles/r02_*.md).
 
-    python tests/perf_sweep.py --batches 256,512,4096 --variants "base=;pf4=CCR_PREFETCH=4" [--k 100] [--mask 1]
+    python tests/perf_sweep.py --batches 256,512,4096 --variants "base=;single=CCR_2CTA=0" [--k 100] [--mask 1]
                                [--n 8841823] [--secs 0.4] [--md out.md]
 
 The table is built once (bench.py's generator).  For every batch size the variants are run round-robin
