@@ -13,6 +13,7 @@ MASK_NONE, MASK_SET, MASK_ADD = 0, 1, 2
 ALGO_AUTO, ALGO_SIMT, ALGO_TCGEN05 = 0, 1, 2
 FLAG_ALLOW_SHORT = 0x10
 FLAG_PACKED_KEYS = 0x20
+FLAG_F16 = 0x40  # q and items hold fp16 instead of bf16
 MAX_K = 2048
 ABI_VERSION = 6
 
@@ -30,7 +31,10 @@ EXPORTS = [
     "ccr_mask_column_shard",
     "ccr_ingest_rows_f32",
     "ccr_normalize_rows_bf16",
+    "ccr_ingest_rows_f32_f16",
+    "ccr_normalize_rows_f16",
     "ccr_score_dense_f32",
+    "ccr_score_dense_f16",
     "ccr_choose_algo",
     "ccr_plan_info",
     "ccr_set_profile_events",
@@ -93,6 +97,12 @@ def lib():
     L.ccr_normalize_rows_bf16.argtypes = [vp, i64, i32, i64, vp, i64, vp]
     L.ccr_score_dense_f32.restype = i32
     L.ccr_score_dense_f32.argtypes = [vp, i64, i64, vp, i64, i64, i32, vp, i64, vp]
+    L.ccr_ingest_rows_f32_f16.restype = i32
+    L.ccr_ingest_rows_f32_f16.argtypes = [vp, i64, i32, i64, vp, i64, i32, vp, vp]
+    L.ccr_normalize_rows_f16.restype = i32
+    L.ccr_normalize_rows_f16.argtypes = [vp, i64, i32, i64, vp, i64, vp]
+    L.ccr_score_dense_f16.restype = i32
+    L.ccr_score_dense_f16.argtypes = [vp, i64, i64, vp, i64, i64, i32, vp, i64, vp]
     L.ccr_choose_algo.restype = i32
     L.ccr_choose_algo.argtypes = [i64, i64, i32, i32]
     L.ccr_set_profile_events.restype = None

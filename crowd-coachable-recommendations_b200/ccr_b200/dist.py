@@ -10,7 +10,7 @@ import torch
 import torch.distributed as dist
 
 from . import engine
-from .table import EmbeddingTable
+from .table import EmbeddingTable, check_table_dtype
 
 
 def shard_bounds(n_items, world_size, rank):
@@ -24,7 +24,8 @@ def shard_bounds(n_items, world_size, rank):
 class ShardedIndex:
     """Each rank holds rows [lo, hi) of the global table in an EmbeddingTable with id_offset=lo."""
 
-    def __init__(self, n_items, dim=768, normalize=False, device=None, group=None):
+    def __init__(self, n_items, dim=768, normalize=False, device=None, group=None, dtype=torch.bfloat16):
+        self.dtype = check_table_dtype(dtype)  # element type of the local table (bf16 or fp16)
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -34,7 +35,8 @@ class ShardedIndex:
         self.table = self._make_table(self.hi - self.lo, dim, normalize)
 
     def _make_table(self, capacity, dim, normalize):
-        return EmbeddingTable(capacity, dim, device=self.device, normalize=normalize, id_offset=self.lo)
+        return EmbeddingTable(capacity, dim, device=self.device, normalize=normalize, id_offset=self.lo,
+                              dtype=self.dtype)
 
     # ---- the device steps; CPU gloo tests replace them to exercise the plumbing ----
     def _local_topk(self, q_encoded, k, mask):
@@ -84,8 +86,8 @@ class ShardedIndex:
         return mask.column_shard(self.lo, self.hi)
 
     def _encode_replicated(self, queries):
-        """bf16 queries on every rank.  Host queries are uploaded and encoded in G row slices, one per
-        rank, and all-gathered over NVLink: B*D*4/G bytes cross each PCIe link instead of B*D*4."""
+        """Encoded queries (the table's dtype) on every rank.  Host queries are uploaded and encoded in G row
+        slices, one per rank, and all-gathered over NVLink: B*D*4/G bytes cross each PCIe link instead of B*D*4."""
         if self.world == 1 or not isinstance(queries, torch.Tensor) or queries.is_cuda or queries.dim() != 2:
             return self._encode(queries)
         B = queries.shape[0]
@@ -93,7 +95,7 @@ class ShardedIndex:
         a, b = min(B, self.rank * per), min(B, (self.rank + 1) * per)
         part = self._encode(queries[a:b]) if b > a else None
         ld = part.shape[1] if part is not None else self._encode(queries[:1]).shape[1]
-        mine = torch.zeros((per, ld), dtype=torch.bfloat16 if part is None else part.dtype,
+        mine = torch.zeros((per, ld), dtype=self.dtype if part is None else part.dtype,
                            device=self.device if part is None else part.device)
         if part is not None:
             mine[: b - a].copy_(part)

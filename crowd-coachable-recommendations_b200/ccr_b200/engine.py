@@ -217,19 +217,31 @@ class SparseMask:
         return SparseMask(new_ip, c[keep] - lo, v[keep], hi - lo, self.mode, self.device)
 
 
+def _operand_f16(q, items):
+    """True for two fp16 operands, False for two bf16 ones; anything else is a TypeError."""
+    if q.dtype == items.dtype == torch.float16:
+        return True
+    if q.dtype == items.dtype == torch.bfloat16:
+        return False
+    if {q.dtype, items.dtype} <= {torch.bfloat16, torch.float16}:
+        raise TypeError(f"q is {q.dtype} but items are {items.dtype}: encode the queries with the table "
+                        "(EmbeddingTable.encode_queries) so both share its dtype")
+    raise TypeError("q and items must both be bfloat16 or both float16 (use EmbeddingTable / ingest_rows to convert)")
+
+
 def score_topk(q, items, k, mask: SparseMask | None = None, id_offset=0, algo=_lib.ALGO_AUTO,
                allow_short=False, want_f64=False, n_items=None, D=None, want_keys=False):
     """Fused ``topk(q @ items.T [mask], k)`` on the device (C ABI: ccr_score_topk_bf16).
 
-    q [B, ldq] bf16 cuda, items [N, ldi] bf16 cuda (row-major, last dim contiguous).
+    q [B, ldq] bf16 cuda, items [N, ldi] bf16 cuda (row-major, last dim contiguous); or both fp16
+    (CCR_FLAG_F16: fp16 operands, fp32 accumulation, fp32 scores).
     Returns (scores float32 [B,k] descending, ids int64 [B,k]) and, with ``want_f64``, the
     float64 values the order was decided on; with ``want_keys`` instead the packed uint64
     exchange keys (CCR_FLAG_PACKED_KEYS; int64 tensor holding the bit pattern).
     """
     _require_cuda(q, "q")
     _require_cuda(items, "items")
-    if q.dtype != torch.bfloat16 or items.dtype != torch.bfloat16:
-        raise TypeError("q and items must be bfloat16 (use EmbeddingTable / ingest_rows to convert)")
+    f16 = _operand_f16(q, items)
     if q.dim() != 2 or items.dim() != 2 or q.stride(1) != 1 or items.stride(1) != 1:
         raise ValueError("q and items must be 2-d with a contiguous last dimension")
     dev = q.device
@@ -239,7 +251,7 @@ def score_topk(q, items, k, mask: SparseMask | None = None, id_offset=0, algo=_l
     ldq = q.stride(0) if B > 1 else max(q.stride(0), q.shape[1])
     ldi = items.stride(0) if items.shape[0] > 1 else max(items.stride(0), items.shape[1])
     k = int(k)
-    flags = int(algo) | (_lib.FLAG_ALLOW_SHORT if allow_short else 0)
+    flags = int(algo) | (_lib.FLAG_ALLOW_SHORT if allow_short else 0) | (_lib.FLAG_F16 if f16 else 0)
     if want_keys:
         if want_f64:
             raise ValueError("want_keys and want_f64 are exclusive (one 8-byte slot per entry)")
@@ -416,12 +428,14 @@ def first_hit_rank(ids, rel_indptr, rel_ids):
     return out
 
 
-def ingest_rows(src, dst, normalize=False):
-    """fp32 (or bf16) rows on the device -> bf16 table rows, optional fp32 L2 normalisation."""
+def ingest_rows(src, dst, normalize=False, overflow=None):
+    """fp32 (or bf16 / fp16) rows on the device -> bf16 or fp16 table rows (``dst.dtype``), optional fp32
+    L2 normalisation.  fp16 destinations: ``overflow`` (a device int32 [1] tensor, optional) has the
+    number of stored values that are not finite added to it (|x| >= 65520 rounds to inf)."""
     _require_cuda(src, "src")
     _require_cuda(dst, "dst")
-    if dst.dtype != torch.bfloat16 or dst.stride(1) != 1 or src.stride(1) != 1:
-        raise ValueError("dst must be bf16 and both must have a contiguous last dimension")
+    if dst.dtype not in (torch.bfloat16, torch.float16) or dst.stride(1) != 1 or src.stride(1) != 1:
+        raise ValueError("dst must be bf16 or fp16 and both must have a contiguous last dimension")
     n, D = src.shape
     if dst.shape[0] != n or dst.shape[1] < D:
         raise ValueError("dst shape mismatch")
@@ -429,21 +443,34 @@ def ingest_rows(src, dst, normalize=False):
         # the kernel zero-fills every column up to the row pitch: a column slice of a wider tensor
         # would have its neighbours overwritten
         raise ValueError("dst rows must be dense (stride(0) == shape[1])")
+    f16 = dst.dtype == torch.float16
+    if f16 and src.dtype == torch.bfloat16:
+        src = src.float()  # bf16 -> fp32 is exact; the fp16 rounding happens once, in the kernel
+    if not f16 and src.dtype == torch.float16:
+        raise TypeError("fp16 rows do not go into a bf16 table: pass them as float32")
+    if overflow is not None and (not f16 or overflow.dtype != torch.int32 or not overflow.is_cuda):
+        raise ValueError("overflow must be a device int32 tensor, for fp16 destinations only")
     ld_src = src.stride(0) if n > 1 else max(src.stride(0), D)
     ld_dst = dst.stride(0) if n > 1 else max(dst.stride(0), dst.shape[1])
     L = _lib.lib()
     with torch.cuda.device(src.device):
         if src.dtype == torch.float32:
-            rc = L.ccr_ingest_rows_f32(src.data_ptr(), n, D, ld_src, dst.data_ptr(), ld_dst, int(bool(normalize)),
-                                       _stream_ptr(src.device))
-        elif src.dtype == torch.bfloat16:
+            if f16:
+                rc = L.ccr_ingest_rows_f32_f16(src.data_ptr(), n, D, ld_src, dst.data_ptr(), ld_dst,
+                                               int(bool(normalize)),
+                                               overflow.data_ptr() if overflow is not None else None,
+                                               _stream_ptr(src.device))
+            else:
+                rc = L.ccr_ingest_rows_f32(src.data_ptr(), n, D, ld_src, dst.data_ptr(), ld_dst, int(bool(normalize)),
+                                           _stream_ptr(src.device))
+        elif src.dtype == dst.dtype:
             if not normalize:
                 dst[:, :D].copy_(src)
                 if dst.shape[1] > D:
                     dst[:, D:].zero_()
                 return dst
-            rc = L.ccr_normalize_rows_bf16(src.data_ptr(), n, D, ld_src, dst.data_ptr(), ld_dst,
-                                           _stream_ptr(src.device))
+            fn = L.ccr_normalize_rows_f16 if f16 else L.ccr_normalize_rows_bf16
+            rc = fn(src.data_ptr(), n, D, ld_src, dst.data_ptr(), ld_dst, _stream_ptr(src.device))
         else:
             raise TypeError(f"unsupported source dtype {src.dtype}")
     _lib.check(rc)
@@ -451,8 +478,9 @@ def ingest_rows(src, dst, normalize=False):
 
 
 def score_dense(q, items, n_items=None, D=None):
-    """Dense fp32 [B, N] scores (small reranking sets / LazyScore.as_tensor)."""
+    """Dense fp32 [B, N] scores (small reranking sets / LazyScore.as_tensor); bf16 or fp16 operands."""
     _require_cuda(q, "q")
+    f16 = _operand_f16(q, items)
     B = q.shape[0]
     N = items.shape[0] if n_items is None else n_items
     D = q.shape[1] if D is None else D
@@ -462,7 +490,7 @@ def score_dense(q, items, n_items=None, D=None):
     ldq = q.stride(0) if B > 1 else max(q.stride(0), q.shape[1])
     ldi = items.stride(0) if items.shape[0] > 1 else max(items.stride(0), items.shape[1])
     with torch.cuda.device(q.device):
-        rc = _lib.lib().ccr_score_dense_f32(q.data_ptr(), B, ldq, items.data_ptr(), N, ldi, D, out.data_ptr(), N,
-                                            _stream_ptr(q.device))
+        fn = _lib.lib().ccr_score_dense_f16 if f16 else _lib.lib().ccr_score_dense_f32
+        rc = fn(q.data_ptr(), B, ldq, items.data_ptr(), N, ldi, D, out.data_ptr(), N, _stream_ptr(q.device))
     _lib.check(rc)
     return out

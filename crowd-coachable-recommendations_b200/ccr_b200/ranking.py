@@ -9,6 +9,8 @@ straight into a device-resident bf16 table and one fused kernel does score + mas
 Deliberate deviations (documented in DESIGN.md): scores come from bf16-rounded embeddings with
 fp32 accumulation (the reference's GPU path under autocast is fp16-in/fp16-out,
 scripts/al_0_rank.py:125); exact ties are ordered by corpus position (reference: unspecified).
+``table_dtype=torch.float16`` rounds the embeddings to fp16 instead, the reference's own operand
+format, so the ranking matches its autocast run up to accumulation order; the scores stay fp32.
 """
 from __future__ import annotations
 
@@ -20,7 +22,7 @@ import numpy as np
 import torch
 
 from . import engine
-from .table import EmbeddingTable
+from .table import EmbeddingTable, check_table_dtype
 
 RANKING_TOPN = 1001  # scripts/ms_marco_eval.py:230
 BLOCK_VALUE = -1e6   # scripts/ms_marco_eval.py:227
@@ -55,8 +57,9 @@ def generate_embeddings(data_indices, data_dic, embedding_func, batch_size, embe
 
 
 def generate_embeddings_device(data_indices, data_dic, embedding_func, batch_size, normalize=False,
-                               device="cuda", id_offset=0, name=None):
-    """Encoder batches -> device bf16 table without the host round trip (SURVEY.md §8f-1)."""
+                               device="cuda", id_offset=0, name=None, dtype=torch.bfloat16):
+    """Encoder batches -> device bf16 (or ``dtype``) table without the host round trip (SURVEY.md §8f-1)."""
+    check_table_dtype(dtype)
     table = None
     with torch.no_grad():
         for step in range(math.ceil(len(data_indices) / batch_size)):
@@ -64,10 +67,10 @@ def generate_embeddings_device(data_indices, data_dic, embedding_func, batch_siz
             emb = torch.as_tensor(embedding_func([data_dic[i] for i in idx]))
             if table is None:
                 table = EmbeddingTable(len(data_indices), emb.shape[1], device=device, normalize=normalize,
-                                       id_offset=id_offset)
+                                       id_offset=id_offset, dtype=dtype)
             table.append(emb)
     if table is None:
-        table = EmbeddingTable(0, 768, device=device, normalize=normalize, id_offset=id_offset)
+        table = EmbeddingTable(0, 768, device=device, normalize=normalize, id_offset=id_offset, dtype=dtype)
     if name is not None:
         table.save(name)
     return table
@@ -151,12 +154,18 @@ def ranking_tensors(query_table, passage_table, k, mask=None, algo=0):
     return scores, order
 
 
-def ranking(corpus, queries, embedding_func, batch_size, block_dict=None, device="cuda", algo=0):
+def ranking(corpus, queries, embedding_func, batch_size, block_dict=None, device="cuda", algo=0,
+            table_dtype=torch.bfloat16):
+    """``table_dtype``: element type of the device tables, bf16 (default) or fp16 (the reference's
+    autocast operand format); scores are fp32 either way."""
+    check_table_dtype(table_dtype)
     sim = os.environ["CCREC_SIM_TYPE"]  # KeyError when unset, like ms_marco_eval.py:212
     normalize = sim == "cos"
     queries_ids, corpus_ids = list(queries.keys()), list(corpus.keys())
-    q_table = generate_embeddings_device(queries_ids, queries, embedding_func, batch_size, normalize, device)
-    p_table = generate_embeddings_device(corpus_ids, corpus, embedding_func, batch_size, normalize, device)
+    q_table = generate_embeddings_device(queries_ids, queries, embedding_func, batch_size, normalize, device,
+                                         dtype=table_dtype)
+    p_table = generate_embeddings_device(corpus_ids, corpus, embedding_func, batch_size, normalize, device,
+                                         dtype=table_dtype)
     if len(queries_ids) == 0:
         return {}
     mask = None
@@ -201,15 +210,16 @@ def mrr_at_k(order, corpus_ids, queries_ids, qrels, k_values=(1, 5, 10, 100), de
 
 
 def ranking_sharded(corpus, queries, embedding_func, batch_size, block_dict=None, group=None, device=None,
-                    index_cls=None):
+                    index_cls=None, table_dtype=torch.bfloat16):
     """``ranking`` with the passage table row-sharded over the ranks of a torch.distributed group
     (one process per GPU): every rank encodes the queries and ONLY its own contiguous slice of the
     corpus (``shard_bounds``) straight into its device shard -- the encoder pass, which dominates the
     reference's wall clock, is split G ways and no rank ever holds the whole table -- then the
     fused local top-k, one all-gather and the G-way merge produce the global result.  Every rank
-    returns the same ``{qid: {pid: score}}`` as the single-table call."""
+    returns the same ``{qid: {pid: score}}`` as the single-table call (``table_dtype`` as in ``ranking``)."""
     from .dist import ShardedIndex
 
+    check_table_dtype(table_dtype)
     sim = os.environ["CCREC_SIM_TYPE"]  # KeyError when unset, like ms_marco_eval.py:212
     normalize = sim == "cos"
     queries_ids, corpus_ids = list(queries.keys()), list(corpus.keys())
@@ -219,7 +229,7 @@ def ranking_sharded(corpus, queries, embedding_func, batch_size, block_dict=None
         q_emb = torch.cat([torch.as_tensor(embedding_func([queries[i] for i in queries_ids[s:s + batch_size]]))
                            for s in range(0, len(queries_ids), batch_size)])
         index = (index_cls or ShardedIndex)(len(corpus_ids), q_emb.shape[1], normalize=normalize, device=device,
-                                            group=group)
+                                            group=group, dtype=table_dtype)
         for s in range(index.lo, index.hi, batch_size):
             e = min(index.hi, s + batch_size)
             index.add_local(torch.as_tensor(embedding_func([corpus[i] for i in corpus_ids[s:e]])))

@@ -1,4 +1,4 @@
-"""Embedding-table residency layer: a device-resident bf16 [N, ld] item/passage table.
+"""Embedding-table residency layer: a device-resident bf16 (or, opt-in, fp16) [N, ld] item/passage table.
 
 Replaces the reference's pageable host fp32 table (scripts/ms_marco_eval.py:123-152
 ``generate_embeddings`` -> ``.to("cpu")`` -> ``vstack``; src/ccrec/models/bbpr.py:466-483
@@ -16,11 +16,28 @@ def _round_up(x, m):
     return (x + m - 1) // m * m
 
 
+TABLE_DTYPES = (torch.bfloat16, torch.float16)
+_DTYPE_NAMES = {torch.bfloat16: "bfloat16", torch.float16: "float16"}
+
+
+def check_table_dtype(dtype):
+    """The element type of a device table: bf16 (default) or fp16; anything else is a ValueError."""
+    if dtype not in TABLE_DTYPES:
+        raise ValueError(f"table dtype must be torch.bfloat16 or torch.float16, not {dtype}")
+    return dtype
+
+
 class EmbeddingTable:
     """Row-major bf16 table on one GPU.  ``id_offset`` is the global id of local row 0
-    (row-sharded tables: scripts-level corpus position = id_offset + local row)."""
+    (row-sharded tables: scripts-level corpus position = id_offset + local row).
 
-    def __init__(self, capacity, dim=768, device="cuda", normalize=False, id_offset=0):
+    ``dtype=torch.float16`` stores IEEE fp16 instead: the operand format of the reference's autocast GPU
+    matmul (scripts/al_0_rank.py:125), 11 significant bits instead of 8, same 2 bytes per element and
+    the same kernels (fp32 accumulation, fp32 scores).  fp16 overflows above 65504: an append or a
+    query batch with a value that rounds to inf is refused with ValueError."""
+
+    def __init__(self, capacity, dim=768, device="cuda", normalize=False, id_offset=0, dtype=torch.bfloat16):
+        self.dtype = check_table_dtype(dtype)
         self.dim = int(dim)
         self.ld = _round_up(self.dim, 8)
         self.device = torch.device(device)
@@ -28,7 +45,7 @@ class EmbeddingTable:
             raise RuntimeError("EmbeddingTable lives on a CUDA device (ccr_b200 has no CPU path)")
         self.normalize = bool(normalize)
         self.id_offset = int(id_offset)
-        self.data = torch.empty((int(capacity), self.ld), dtype=torch.bfloat16, device=self.device)
+        self.data = torch.empty((int(capacity), self.ld), dtype=self.dtype, device=self.device)
         self.n = 0
 
     def __len__(self):
@@ -50,39 +67,48 @@ class EmbeddingTable:
         if emb.shape[1] != self.dim:
             raise ValueError(f"embedding dim {emb.shape[1]} != table dim {self.dim}")
         if self.n + m > self.data.shape[0]:
-            grown = torch.empty((max(self.n + m, 2 * self.data.shape[0]), self.ld), dtype=torch.bfloat16,
+            grown = torch.empty((max(self.n + m, 2 * self.data.shape[0]), self.ld), dtype=self.dtype,
                                 device=self.device)
             grown[: self.n].copy_(self.data[: self.n])
             self.data = grown
-        if emb.dtype not in (torch.float32, torch.bfloat16):
-            emb = emb.float()
-        emb = emb.to(self.device, non_blocking=True)
-        if emb.stride(1) != 1:
-            emb = emb.contiguous()
-        engine.ingest_rows(emb, self.data[self.n : self.n + m], normalize=self.normalize)
+        self._ingest(emb, self.data[self.n : self.n + m])
         self.n += m
         return self
 
+    def _ingest(self, src, dst):
+        """Rows of any float dtype -> ``dst`` under the table's dtype and similarity convention.  fp32 and
+        table-dtype sources go to the kernels as they are; everything else is widened to fp32 first."""
+        if src.dtype not in (torch.float32, self.dtype):
+            src = src.float()
+        src = src.to(self.device, non_blocking=True)
+        if src.stride(1) != 1:
+            src = src.contiguous()
+        if self.dtype == torch.bfloat16 or src.dtype != torch.float32:
+            return engine.ingest_rows(src, dst, normalize=self.normalize)
+        # fp32 -> fp16 may overflow: count the values that round to inf (one device -> host read)
+        overflow = torch.zeros(1, dtype=torch.int32, device=self.device)
+        engine.ingest_rows(src, dst, normalize=self.normalize, overflow=overflow)
+        bad = int(overflow.item())
+        if bad:
+            raise ValueError(f"{bad} value(s) overflow fp16 (|x| >= 65520 after normalisation, or not finite); "
+                             "nothing was added")
+        return dst
+
     @classmethod
-    def from_tensor(cls, emb, device="cuda", normalize=False, id_offset=0, chunk=1 << 18):
+    def from_tensor(cls, emb, device="cuda", normalize=False, id_offset=0, chunk=1 << 18, dtype=torch.bfloat16):
         emb = torch.as_tensor(emb)
-        t = cls(emb.shape[0], emb.shape[1], device=device, normalize=normalize, id_offset=id_offset)
+        t = cls(emb.shape[0], emb.shape[1], device=device, normalize=normalize, id_offset=id_offset, dtype=dtype)
         for s in range(0, emb.shape[0], chunk):
             t.append(emb[s : s + chunk])
         return t
 
     def encode_queries(self, q):
-        """Query/user embeddings -> bf16 [B, ld] under the table's similarity convention."""
+        """Query/user embeddings -> [B, ld] of the table's dtype under its similarity convention."""
         q = torch.as_tensor(q)
         if q.dim() == 1:
             q = q.unsqueeze(0)
-        if q.dtype not in (torch.float32, torch.bfloat16):
-            q = q.float()
-        q = q.to(self.device, non_blocking=True)
-        if q.stride(1) != 1:
-            q = q.contiguous()
-        out = torch.empty((q.shape[0], self.ld), dtype=torch.bfloat16, device=self.device)
-        return engine.ingest_rows(q, out, normalize=self.normalize)
+        out = torch.empty((q.shape[0], self.ld), dtype=self.dtype, device=self.device)
+        return self._ingest(q, out)
 
     def search(self, queries, k, mask=None, algo=0, allow_short=False, want_f64=False, encoded=False,
                want_keys=False):
@@ -99,13 +125,14 @@ class EmbeddingTable:
     # ---- persistence: the `name=` analogue of generate_embeddings (ms_marco_eval.py:150-151) ----
     def save(self, path):
         torch.save({"rows": self.rows.cpu(), "dim": self.dim, "normalize": self.normalize,
-                    "id_offset": self.id_offset}, path)
+                    "id_offset": self.id_offset, "dtype": _DTYPE_NAMES[self.dtype]}, path)
 
     @classmethod
     def load(cls, path, device="cuda"):
         blob = torch.load(path)
+        dtype = getattr(torch, blob.get("dtype", "bfloat16"))  # files written before fp16 tables: bf16
         t = cls(blob["rows"].shape[0], blob["dim"], device=device, normalize=blob["normalize"],
-                id_offset=blob["id_offset"])
+                id_offset=blob["id_offset"], dtype=dtype)
         t.data[: blob["rows"].shape[0]].copy_(blob["rows"])
         t.n = blob["rows"].shape[0]
         return t

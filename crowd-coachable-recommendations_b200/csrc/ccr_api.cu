@@ -346,6 +346,7 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   SelectParams sp = {};
   sp.q = (const __nv_bfloat16*)q; sp.ldq = ldq; sp.B = (int)B; sp.q_rows = (int)B;
   sp.items = (const __nv_bfloat16*)items; sp.ldi = ldi; sp.n_items = n_items; sp.D = D;
+  sp.f16 = (flags & CCR_FLAG_F16) ? 1 : 0;
   sp.k = k; sp.k_keep = pl.k_keep; sp.C = pl.C; sp.S = pl.S; sp.n_q_tiles = pl.n_q_tiles; sp.two_cta = pl.two_cta;
   sp.mask_indptr = has_mask ? (const long long*)mask_indptr : nullptr;
   sp.mask_cols = (has_mask && !pl.include_mask) ? mask_cols : nullptr;
@@ -383,7 +384,7 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   if (pl.algo == CCR_ALGO_TCGEN05 && B < kQTile && n_items > 0) {
     // short batch: stage the queries in a [128, D] block so that no TMA box of the query operand is
     // out of bounds (measurably faster than hardware zero-fill of 120+ rows); only the padding rows
-    // are zeroed
+    // are zeroed.  A plain copy of 2-byte elements: the same for fp16, whose +0 has bf16's bits
     __nv_bfloat16* qp = (__nv_bfloat16*)(ws + pl.off_qpad);
     e = cudaMemsetAsync(qp + (size_t)B * D, 0, (size_t)(kQTile - B) * D * sizeof(__nv_bfloat16), st);
     if (e == cudaSuccess)
@@ -407,6 +408,7 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
     OverrideParams op = {};
     // sp.q may be the padded staging block of a short batch: use ITS pitch (sp.ldq), not the caller's
     op.q = sp.q; op.ldq = sp.ldq; op.B = (int)B; op.items = sp.items; op.ldi = ldi; op.n_items = n_items; op.D = D;
+    op.f16 = sp.f16;
     op.mask_indptr = sp.mask_indptr; op.mask_cols = mask_cols; op.mask_vals = mask_vals; op.nnz = nnz;
     op.mode = mask_mode; op.ovr_hi = (u64*)(ws + pl.off_ovr_hi); op.ovr_lo = (u32*)(ws + pl.off_ovr_lo);
     lr = launch_overrides(op, st);
@@ -480,6 +482,17 @@ int ccr_ingest_rows_f32(const float* src, int64_t n, int D, int64_t ld_src, void
   return CCR_OK;
 }
 
+int ccr_ingest_rows_f32_f16(const float* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
+                            int normalize, int32_t* overflow_count, void* stream) {
+  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad ingest shape");
+  if (n == 0) return CCR_OK;
+  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
+  int lr = launch_ingest_f32_f16(src, n, D, ld_src, (__half*)dst, ld_dst, normalize, (int*)overflow_count,
+                                 (cudaStream_t)stream);
+  if (lr) return fail(CCR_ECUDA, "ingest kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+  return CCR_OK;
+}
+
 int ccr_normalize_rows_bf16(const void* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
                             void* stream) {
   if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad normalize shape");
@@ -491,8 +504,21 @@ int ccr_normalize_rows_bf16(const void* src, int64_t n, int D, int64_t ld_src, v
   return CCR_OK;
 }
 
-int ccr_score_dense_f32(const void* q, int64_t B, int64_t ldq, const void* items, int64_t n_items,
-                        int64_t ldi, int D, float* out, int64_t ld_out, void* stream) {
+int ccr_normalize_rows_f16(const void* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
+                           void* stream) {
+  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad normalize shape");
+  if (n == 0) return CCR_OK;
+  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
+  int lr = launch_normalize_f16((const __half*)src, n, D, ld_src, (__half*)dst, ld_dst, (cudaStream_t)stream);
+  if (lr) return fail(CCR_ECUDA, "normalize kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+  return CCR_OK;
+}
+
+}  // extern "C"
+
+// ccr_score_dense_f32 / ccr_score_dense_f16: f16 selects the operand format
+static int score_dense(const void* q, int64_t B, int64_t ldq, const void* items, int64_t n_items, int64_t ldi, int D,
+                       float* out, int64_t ld_out, int f16, void* stream) {
   if (B < 0 || n_items < 0 || D <= 0 || D % 8 || ldq < D || ldi < D || ldq % 8 || ldi % 8 || ld_out < n_items)
     return fail(CCR_EINVAL, "bad dense shape");
   if (B == 0 || n_items == 0) return CCR_OK;
@@ -503,7 +529,7 @@ int ccr_score_dense_f32(const void* q, int64_t B, int64_t ldq, const void* items
     // large tiles: the TMA + tcgen05 pipeline of the fused kernel with a store epilogue
     SelectParams sp = {};
     sp.q = (const __nv_bfloat16*)q; sp.ldq = ldq; sp.B = (int)B; sp.q_rows = (int)B;
-    sp.items = (const __nv_bfloat16*)items; sp.ldi = ldi; sp.n_items = n_items; sp.D = D;
+    sp.items = (const __nv_bfloat16*)items; sp.ldi = ldi; sp.n_items = n_items; sp.D = D; sp.f16 = f16;
     sp.k = 1; sp.k_keep = 1; sp.C = 0;
     sp.n_q_tiles = (int)((B + kQTile - 1) / kQTile);
     sp.S = splits_tc(sp.n_q_tiles, (n_items + kITile - 1) / kITile, device_sm_count());
@@ -514,10 +540,24 @@ int ccr_score_dense_f32(const void* q, int64_t B, int64_t ldq, const void* items
     if (lr) return fail(CCR_ECUDA, "dense tile launch failed (%d)", lr);
     return CCR_OK;
   }
-  int lr = launch_dense_f32((const __nv_bfloat16*)q, B, ldq, (const __nv_bfloat16*)items, n_items, ldi, D, out,
-                            ld_out, (cudaStream_t)stream);
+  int lr = f16 ? launch_dense_f32_f16((const __half*)q, B, ldq, (const __half*)items, n_items, ldi, D, out, ld_out,
+                                      (cudaStream_t)stream)
+               : launch_dense_f32((const __nv_bfloat16*)q, B, ldq, (const __nv_bfloat16*)items, n_items, ldi, D, out,
+                                  ld_out, (cudaStream_t)stream);
   if (lr) return fail(CCR_ECUDA, "dense kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   return CCR_OK;
+}
+
+extern "C" {
+
+int ccr_score_dense_f32(const void* q, int64_t B, int64_t ldq, const void* items, int64_t n_items,
+                        int64_t ldi, int D, float* out, int64_t ld_out, void* stream) {
+  return score_dense(q, B, ldq, items, n_items, ldi, D, out, ld_out, 0, stream);
+}
+
+int ccr_score_dense_f16(const void* q, int64_t B, int64_t ldq, const void* items, int64_t n_items,
+                        int64_t ldi, int D, float* out, int64_t ld_out, void* stream) {
+  return score_dense(q, B, ldq, items, n_items, ldi, D, out, ld_out, 1, stream);
 }
 
 size_t ccr_argsort_workspace_bytes(int64_t n_elements) {

@@ -2,6 +2,7 @@
 // in-place compaction) on candidate buffers, small PTX wrappers.
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -336,6 +337,24 @@ __device__ __forceinline__ uint4 ldg_nc_v4(const void* p) {
 }
 __device__ __forceinline__ float bf16_lo(u32 w) { return __uint_as_float(w << 16); }
 __device__ __forceinline__ float bf16_hi(u32 w) { return __uint_as_float(w & 0xffff0000u); }
+__device__ __forceinline__ float f16_lo(u32 w) { return __half2float(__ushort_as_half((unsigned short)(w & 0xffffu))); }
+__device__ __forceinline__ float f16_hi(u32 w) { return __half2float(__ushort_as_half((unsigned short)(w >> 16))); }
+
+// Stored table / query element (2 bytes): bf16 (default) or IEEE binary16 (CCR_FLAG_F16).  lo / hi
+// widen the low / high element of a packed pair exactly; from_float rounds to nearest even.
+template <typename T> struct Elem;
+template <> struct Elem<__nv_bfloat16> {
+  static __device__ __forceinline__ float lo(u32 w) { return bf16_lo(w); }
+  static __device__ __forceinline__ float hi(u32 w) { return bf16_hi(w); }
+  static __device__ __forceinline__ float to_float(__nv_bfloat16 v) { return __bfloat162float(v); }
+  static __device__ __forceinline__ __nv_bfloat16 from_float(float v) { return __float2bfloat16_rn(v); }
+};
+template <> struct Elem<__half> {
+  static __device__ __forceinline__ float lo(u32 w) { return f16_lo(w); }
+  static __device__ __forceinline__ float hi(u32 w) { return f16_hi(w); }
+  static __device__ __forceinline__ float to_float(__half v) { return __half2float(v); }
+  static __device__ __forceinline__ __half from_float(float v) { return __float2half_rn(v); }
+};
 
 // error slots written by device-side watchdogs (workspace tail)
 struct DeviceStatus {

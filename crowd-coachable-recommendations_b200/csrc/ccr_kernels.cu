@@ -18,9 +18,12 @@ namespace ccr {
 // appended to the row's candidate buffer.  A row whose buffer is nearly full is pruned to
 // its exact top-k by one warp (radix select in place), raising the row's threshold.
 // =======================================================================================
+template <typename T>
 __global__ void __launch_bounds__(256, 2) select_simt_kernel(SelectParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int D = p.D;
+  const T* __restrict__ pq = reinterpret_cast<const T*>(p.q);
+  const T* __restrict__ pitems = reinterpret_cast<const T*>(p.items);
   float* qs = reinterpret_cast<float*>(smem_raw);  // [8][D]
   __shared__ int s_cnt[kSimtRows];
   __shared__ float s_tau_f[kSimtRows];
@@ -39,7 +42,7 @@ __global__ void __launch_bounds__(256, 2) select_simt_kernel(SelectParams p) {
     int row = row0 + r;
     int c = d >> 3, h = (d >> 2) & 1, e = d & 3;
     qs[((r * 2 + h) * chunks + c) * 4 + e] =
-        (row < p.B) ? __bfloat162float(p.q[(long long)row * p.ldq + d]) : 0.f;
+        (row < p.B) ? Elem<T>::to_float(pq[(long long)row * p.ldq + d]) : 0.f;
   }
   if (tid < kSimtRows) {
     s_cnt[tid] = 0;
@@ -70,7 +73,7 @@ __global__ void __launch_bounds__(256, 2) select_simt_kernel(SelectParams p) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         long long it = it0 + j;
-        if (it < i1) w[j] = ldg_nc_v4(p.items + it * p.ldi + c * 8);
+        if (it < i1) w[j] = ldg_nc_v4(pitems + it * p.ldi + c * 8);
         else w[j] = make_uint4(0, 0, 0, 0);
       }
 #pragma unroll
@@ -80,14 +83,14 @@ __global__ void __launch_bounds__(256, 2) select_simt_kernel(SelectParams p) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           float a = acc[j * 8 + r];
-          a = fmaf(bf16_lo(w[j].x), qa.x, a);
-          a = fmaf(bf16_hi(w[j].x), qa.y, a);
-          a = fmaf(bf16_lo(w[j].y), qa.z, a);
-          a = fmaf(bf16_hi(w[j].y), qa.w, a);
-          a = fmaf(bf16_lo(w[j].z), qb.x, a);
-          a = fmaf(bf16_hi(w[j].z), qb.y, a);
-          a = fmaf(bf16_lo(w[j].w), qb.z, a);
-          a = fmaf(bf16_hi(w[j].w), qb.w, a);
+          a = fmaf(Elem<T>::lo(w[j].x), qa.x, a);
+          a = fmaf(Elem<T>::hi(w[j].x), qa.y, a);
+          a = fmaf(Elem<T>::lo(w[j].y), qa.z, a);
+          a = fmaf(Elem<T>::hi(w[j].y), qa.w, a);
+          a = fmaf(Elem<T>::lo(w[j].z), qb.x, a);
+          a = fmaf(Elem<T>::hi(w[j].z), qb.y, a);
+          a = fmaf(Elem<T>::lo(w[j].w), qb.z, a);
+          a = fmaf(Elem<T>::hi(w[j].w), qb.w, a);
           acc[j * 8 + r] = a;
         }
       }
@@ -135,19 +138,25 @@ __global__ void __launch_bounds__(256, 2) select_simt_kernel(SelectParams p) {
   if (tid < kSimtRows) p.counts[(long long)(row0 + tid) * p.S + split] = s_cnt[tid];
 }
 
-int launch_select_simt(const SelectParams& p, cudaStream_t st) {
+template <typename T>
+static int launch_select_simt_t(const SelectParams& p, cudaStream_t st) {
   size_t smem = (size_t)kSimtRows * p.D * sizeof(float);
-  cudaError_t e = cudaFuncSetAttribute(select_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  cudaError_t e = cudaFuncSetAttribute(select_simt_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)smem);
   if (e != cudaSuccess) return (int)e;
   dim3 grid(p.S, p.n_q_tiles);
-  select_simt_kernel<<<grid, 256, smem, st>>>(p);
+  select_simt_kernel<T><<<grid, 256, smem, st>>>(p);
   return (int)cudaGetLastError();
+}
+
+int launch_select_simt(const SelectParams& p, cudaStream_t st) {
+  return p.f16 ? launch_select_simt_t<__half>(p, st) : launch_select_simt_t<__nv_bfloat16>(p, st);
 }
 
 // =======================================================================================
 // Mask overrides: one warp per CSR entry.  value = set ? v : double(q.item) + v.
 // =======================================================================================
+template <typename T>
 __global__ void __launch_bounds__(256) override_kernel(OverrideParams p) {
   const int lane = threadIdx.x & 31;
   const long long e = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
@@ -174,10 +183,10 @@ __global__ void __launch_bounds__(256) override_kernel(OverrideParams p) {
     for (int c = lane; c < (p.D >> 3); c += 32) {
       uint4 a = *reinterpret_cast<const uint4*>(qr + c * 8);
       uint4 b = ldg_nc_v4(ir + c * 8);
-      acc = fmaf(bf16_lo(a.x), bf16_lo(b.x), acc); acc = fmaf(bf16_hi(a.x), bf16_hi(b.x), acc);
-      acc = fmaf(bf16_lo(a.y), bf16_lo(b.y), acc); acc = fmaf(bf16_hi(a.y), bf16_hi(b.y), acc);
-      acc = fmaf(bf16_lo(a.z), bf16_lo(b.z), acc); acc = fmaf(bf16_hi(a.z), bf16_hi(b.z), acc);
-      acc = fmaf(bf16_lo(a.w), bf16_lo(b.w), acc); acc = fmaf(bf16_hi(a.w), bf16_hi(b.w), acc);
+      acc = fmaf(Elem<T>::lo(a.x), Elem<T>::lo(b.x), acc); acc = fmaf(Elem<T>::hi(a.x), Elem<T>::hi(b.x), acc);
+      acc = fmaf(Elem<T>::lo(a.y), Elem<T>::lo(b.y), acc); acc = fmaf(Elem<T>::hi(a.y), Elem<T>::hi(b.y), acc);
+      acc = fmaf(Elem<T>::lo(a.z), Elem<T>::lo(b.z), acc); acc = fmaf(Elem<T>::hi(a.z), Elem<T>::hi(b.z), acc);
+      acc = fmaf(Elem<T>::lo(a.w), Elem<T>::lo(b.w), acc); acc = fmaf(Elem<T>::hi(a.w), Elem<T>::hi(b.w), acc);
     }
 #pragma unroll
     for (int off = 16; off; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
@@ -193,7 +202,8 @@ __global__ void __launch_bounds__(256) override_kernel(OverrideParams p) {
 int launch_overrides(const OverrideParams& p, cudaStream_t st) {
   if (p.nnz <= 0) return 0;
   long long blocks = (p.nnz + 7) / 8;
-  override_kernel<<<(unsigned)blocks, 256, 0, st>>>(p);
+  if (p.f16) override_kernel<__half><<<(unsigned)blocks, 256, 0, st>>>(p);
+  else override_kernel<__nv_bfloat16><<<(unsigned)blocks, 256, 0, st>>>(p);
   return (int)cudaGetLastError();
 }
 
@@ -711,12 +721,15 @@ int launch_mask_shard(const long long* indptr, const int* cols, const double* va
 }
 
 // =======================================================================================
-// Table ingest / normalisation: one warp per row.
+// Table ingest / normalisation: one warp per row.  DstT = __nv_bfloat16 or __half (round to nearest
+// even; fp16 keeps subnormals).  overflow (fp16 tables, may be null): += number of stored values that
+// are not finite -- |x| >= 65520 after normalisation rounds to inf, and non-finite inputs stay so;
+// one atomic per warp that saw any.
 // =======================================================================================
-template <typename SrcT>
+template <typename SrcT, typename DstT>
 __global__ void __launch_bounds__(256) ingest_kernel(const SrcT* __restrict__ src, long long n, int D,
-                                                     long long ld_src, __nv_bfloat16* __restrict__ dst,
-                                                     long long ld_dst, int normalize) {
+                                                     long long ld_src, DstT* __restrict__ dst,
+                                                     long long ld_dst, int normalize, int* __restrict__ overflow) {
   const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= n) return;
@@ -729,47 +742,71 @@ __global__ void __launch_bounds__(256) ingest_kernel(const SrcT* __restrict__ sr
     for (int off = 16; off; off >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, off);
     scale = fmaxf(sqrtf(ss), 1e-12f);  // F.normalize: x / max(||x||, eps) -- a true division, like torch
   }
-  __nv_bfloat16* o = dst + row * ld_dst;
+  DstT* o = dst + row * ld_dst;
+  int bad = 0;
   for (int d = lane; d < ld_dst; d += 32) {
     float v = d < D ? (normalize ? (float)s[d] / scale : (float)s[d]) : 0.f;
-    o[d] = __float2bfloat16_rn(v);
+    const DstT r = Elem<DstT>::from_float(v);
+    if (overflow) bad += isfinite(Elem<DstT>::to_float(r)) ? 0 : 1;
+    o[d] = r;
+  }
+  if (overflow) {
+#pragma unroll
+    for (int off = 16; off; off >>= 1) bad += __shfl_xor_sync(0xffffffffu, bad, off);
+    if (lane == 0 && bad) atomicAdd(overflow, bad);
   }
 }
 
 int launch_ingest_f32(const float* src, long long n, int D, long long ld_src, __nv_bfloat16* dst,
                       long long ld_dst, int normalize, cudaStream_t st) {
   if (n == 0) return 0;
-  ingest_kernel<float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, normalize);
+  ingest_kernel<float, __nv_bfloat16><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst,
+                                                                              normalize, nullptr);
   return (int)cudaGetLastError();
 }
 int launch_normalize_bf16(const __nv_bfloat16* src, long long n, int D, long long ld_src,
                           __nv_bfloat16* dst, long long ld_dst, cudaStream_t st) {
   if (n == 0) return 0;
-  ingest_kernel<__nv_bfloat16><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, 1);
+  ingest_kernel<__nv_bfloat16, __nv_bfloat16><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst,
+                                                                                      ld_dst, 1, nullptr);
+  return (int)cudaGetLastError();
+}
+int launch_ingest_f32_f16(const float* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
+                          int normalize, int* overflow_count, cudaStream_t st) {
+  if (n == 0) return 0;
+  ingest_kernel<float, __half><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, normalize,
+                                                                       overflow_count);
+  return (int)cudaGetLastError();
+}
+int launch_normalize_f16(const __half* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
+                         cudaStream_t st) {
+  if (n == 0) return 0;
+  ingest_kernel<__half, __half><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, 1, nullptr);
   return (int)cudaGetLastError();
 }
 
 // =======================================================================================
 // Dense fp32 score tile (not a hot path): one warp per (row, item).
 // =======================================================================================
-__global__ void __launch_bounds__(256) dense_kernel(const __nv_bfloat16* __restrict__ q, long long B,
-                                                    long long ldq, const __nv_bfloat16* __restrict__ items,
+template <typename T>
+__global__ void __launch_bounds__(256) dense_kernel(const T* __restrict__ q, long long B,
+                                                    long long ldq, const T* __restrict__ items,
                                                     long long n, long long ldi, int D,
                                                     float* __restrict__ out, long long ld_out) {
   const int lane = threadIdx.x & 31;
   const long long item = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   const long long row = blockIdx.y;
   if (item >= n) return;
-  const __nv_bfloat16* qr = q + row * ldq;
-  const __nv_bfloat16* ir = items + item * ldi;
+  const T* qr = q + row * ldq;
+  const T* ir = items + item * ldi;
   float acc = 0.f;
   for (int c = lane; c < (D >> 3); c += 32) {
     uint4 a = *reinterpret_cast<const uint4*>(qr + c * 8);
     uint4 b = *reinterpret_cast<const uint4*>(ir + c * 8);
-    acc = fmaf(bf16_lo(a.x), bf16_lo(b.x), acc); acc = fmaf(bf16_hi(a.x), bf16_hi(b.x), acc);
-    acc = fmaf(bf16_lo(a.y), bf16_lo(b.y), acc); acc = fmaf(bf16_hi(a.y), bf16_hi(b.y), acc);
-    acc = fmaf(bf16_lo(a.z), bf16_lo(b.z), acc); acc = fmaf(bf16_hi(a.z), bf16_hi(b.z), acc);
-    acc = fmaf(bf16_lo(a.w), bf16_lo(b.w), acc); acc = fmaf(bf16_hi(a.w), bf16_hi(b.w), acc);
+    acc = fmaf(Elem<T>::lo(a.x), Elem<T>::lo(b.x), acc); acc = fmaf(Elem<T>::hi(a.x), Elem<T>::hi(b.x), acc);
+    acc = fmaf(Elem<T>::lo(a.y), Elem<T>::lo(b.y), acc); acc = fmaf(Elem<T>::hi(a.y), Elem<T>::hi(b.y), acc);
+    acc = fmaf(Elem<T>::lo(a.z), Elem<T>::lo(b.z), acc); acc = fmaf(Elem<T>::hi(a.z), Elem<T>::hi(b.z), acc);
+    acc = fmaf(Elem<T>::lo(a.w), Elem<T>::lo(b.w), acc); acc = fmaf(Elem<T>::hi(a.w), Elem<T>::hi(b.w), acc);
   }
 #pragma unroll
   for (int off = 16; off; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
@@ -780,7 +817,14 @@ int launch_dense_f32(const __nv_bfloat16* q, long long B, long long ldq, const _
                      long long n, long long ldi, int D, float* out, long long ld_out, cudaStream_t st) {
   if (B == 0 || n == 0) return 0;
   dim3 grid((unsigned)((n + 7) / 8), (unsigned)B);
-  dense_kernel<<<grid, 256, 0, st>>>(q, B, ldq, items, n, ldi, D, out, ld_out);
+  dense_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(q, B, ldq, items, n, ldi, D, out, ld_out);
+  return (int)cudaGetLastError();
+}
+int launch_dense_f32_f16(const __half* q, long long B, long long ldq, const __half* items, long long n, long long ldi,
+                         int D, float* out, long long ld_out, cudaStream_t st) {
+  if (B == 0 || n == 0) return 0;
+  dim3 grid((unsigned)((n + 7) / 8), (unsigned)B);
+  dense_kernel<__half><<<grid, 256, 0, st>>>(q, B, ldq, items, n, ldi, D, out, ld_out);
   return (int)cudaGetLastError();
 }
 

@@ -8,14 +8,16 @@ namespace ccr {
 // buffer of `C` 64-bit keys in the workspace:  cand[(row * S + split) * C + i],
 // counts[row * S + split].  rows are padded to a multiple of the row-tile of the kernel.
 struct SelectParams {
-  const __nv_bfloat16* q;
+  const __nv_bfloat16* q;      // 2-byte elements: bf16, or IEEE binary16 when f16 is set
   long long ldq;
   int B;
   int q_rows;     // rows the query tensor map may address (>= B; > B when the caller padded q)
-  const __nv_bfloat16* items;
+  const __nv_bfloat16* items;  // same element type as q
   long long ldi;
   long long n_items;
   int D;
+  int f16;        // 1: q and items hold fp16 (CCR_FLAG_F16); the tensor-core kernel clears the bf16
+                  // format bits of its instruction descriptor, the SIMT kernel is instantiated for __half
   int k;
   int k_keep;     // upper bound of the candidates one row must keep (k + mask_max_row_nnz in include
                   // mode, else k): the candidate buffers are sized for it, so per-row counts derived from
@@ -94,6 +96,7 @@ struct OverrideParams {
   long long ldi;
   long long n_items;
   int D;
+  int f16;  // q / items hold fp16 instead of bf16
   const long long* mask_indptr;
   const int* mask_cols;
   const double* mask_vals;
@@ -124,6 +127,13 @@ int launch_normalize_bf16(const __nv_bfloat16* src, long long n, int D, long lon
                           __nv_bfloat16* dst, long long ld_dst, cudaStream_t st);
 int launch_dense_f32(const __nv_bfloat16* q, long long B, long long ldq, const __nv_bfloat16* items,
                      long long n, long long ldi, int D, float* out, long long ld_out, cudaStream_t st);
+// fp16 twins; overflow_count (device int32, may be null) += outputs that are not finite
+int launch_ingest_f32_f16(const float* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
+                          int normalize, int* overflow_count, cudaStream_t st);
+int launch_normalize_f16(const __half* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
+                         cudaStream_t st);
+int launch_dense_f32_f16(const __half* q, long long B, long long ldq, const __half* items, long long n, long long ldi,
+                         int D, float* out, long long ld_out, cudaStream_t st);
 
 // whole-matrix argsort and MRR first-hit scan (ccr_sort.cu)
 size_t argsort_workspace_bytes(long long n);

@@ -4,8 +4,9 @@
 //
 // * operands staged by TMA (cp.async.bulk.tensor.2d, 128-byte swizzle) into a 4-stage
 //   shared-memory ring of (16 KB Q block + 32 KB item block), K advanced 64 elements a stage;
-// * one elected thread issues tcgen05.mma.cta_group::1.kind::f16 (bf16 x bf16 -> fp32,
-//   M=128, N=256, K=16) into one of two 256-column TMEM accumulators;
+// * one elected thread issues tcgen05.mma.cta_group::1.kind::f16 (bf16 x bf16 -> fp32, or f16 x f16
+//   -> fp32 for fp16 tables: an instruction-descriptor field set at run time; M=128, N=256, K=16)
+//   into one of two 256-column TMEM accumulators;
 // * four epilogue warps read the other accumulator with tcgen05.ld (thread == query row),
 //   compare against the row's running threshold and append survivors to the row's candidate
 //   buffer; a nearly full buffer is pruned in place to its exact top-k (warp radix select),
@@ -183,10 +184,11 @@ __device__ __forceinline__ u64 make_sw128_desc(u32 saddr) {
   d |= (u64)2 << 61;
   return d;
 }
-// instruction descriptor, kind::f16: c_format f32 (bit 4), a/b format bf16 (bits 7, 10),
+// instruction descriptor, kind::f16: c_format f32 (bit 4), a/b format bf16 (bits 7, 10; both 0 = f16),
 // both K-major (bits 15,16 = 0), N>>3 at [17,23), M>>4 at [24,29)
 template <int kCta> struct TcIdesc {
   static constexpr u32 value = (1u << 4) | (1u << 7) | (1u << 10) | ((u32)(kITile >> 3) << 17) | ((u32)((kQTile * kCta) >> 4) << 24);
+  static constexpr u32 kAbBf16 = (1u << 7) | (1u << 10);
 };
 
 // ---------------------------------------------------------------------------------------
@@ -591,6 +593,7 @@ select_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     if (lane == 0 && crank == 0) {
       int stage = 0; u32 phase = 0;
       int acc = 0; u32 acc_phase = 0;
+      const u32 idesc = p.f16 ? (TcIdesc<kCta>::value & ~TcIdesc<kCta>::kAbBf16) : TcIdesc<kCta>::value;
       for (int unit = cid; unit < n_units; unit += n_cl) {
         const int u = unit / p.n_q_tiles;
         const long long t0 = (long long)u * tiles_total / p.S, t1 = (long long)(u + 1) * tiles_total / p.S;
@@ -608,9 +611,9 @@ select_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             for (int kk = 0; kk < kKBlock / 16; ++kk) {
               // +32 bytes (16 bf16) along K inside the 128-byte swizzle row: +2 in 16-byte units
               if (kCta == 2)
-                tc_mma_bf16_2cta(d_tmem, adesc + (u64)(kk * 2), bdesc + (u64)(kk * 2), TcIdesc<2>::value, (kb | kk) ? 1u : 0u);
+                tc_mma_bf16_2cta(d_tmem, adesc + (u64)(kk * 2), bdesc + (u64)(kk * 2), idesc, (kb | kk) ? 1u : 0u);
               else
-                tc_mma_bf16(d_tmem, adesc + (u64)(kk * 2), bdesc + (u64)(kk * 2), TcIdesc<1>::value, (kb | kk) ? 1u : 0u);
+                tc_mma_bf16(d_tmem, adesc + (u64)(kk * 2), bdesc + (u64)(kk * 2), idesc, (kb | kk) ? 1u : 0u);
             }
             // frees the smem slot (in both CTAs of a pair) once these MMAs retire
             if (kCta == 2) tc_commit_2cta(&sh->empty[stage]); else tc_commit(&sh->empty[stage]);
@@ -908,15 +911,17 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// 2-D bf16 row-major [rows, D] with row pitch ld elements; box = 64 x box_rows, 128B swizzle
-static int make_tmap(CUtensorMap* m, const void* base, long long rows, int D, long long ld, int box_rows) {
+// 2-D row-major [rows, D] of 2-byte elements (BFLOAT16 or FLOAT16) with row pitch ld elements;
+// box = 64 x box_rows, 128B swizzle
+static int make_tmap(CUtensorMap* m, CUtensorMapDataType dtype, const void* base, long long rows, int D, long long ld,
+                     int box_rows) {
   EncodeTiledFn fn = get_encode_fn();
   if (!fn) return -1;
   cuuint64_t dims[2] = {(cuuint64_t)D, (cuuint64_t)rows};
   cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
   cuuint32_t box[2] = {(cuuint32_t)kKBlock, (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+  CUresult r = fn(m, dtype, 2, const_cast<void*>(base), dims, strides, box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? 0 : -(int)r - 1000;
@@ -958,9 +963,10 @@ static int launch_variant(const CUtensorMap& tq, const CUtensorMap& ti, const Se
 // p.n_q_tiles counts 128-row tiles for one-CTA units and 256-row tiles when p.two_cta is set
 int launch_select_tc(const SelectParams& p, cudaStream_t st, int num_sms) {
   CUtensorMap tq, ti;
-  int r = make_tmap(&tq, p.q, p.q_rows > p.B ? p.q_rows : p.B, p.D, p.ldq, kQTile);
+  const CUtensorMapDataType dt = p.f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  int r = make_tmap(&tq, dt, p.q, p.q_rows > p.B ? p.q_rows : p.B, p.D, p.ldq, kQTile);
   if (r) return r;
-  r = make_tmap(&ti, p.items, p.n_items, p.D, p.ldi, p.two_cta ? kITile / 2 : kITile);
+  r = make_tmap(&ti, dt, p.items, p.n_items, p.D, p.ldi, p.two_cta ? kITile / 2 : kITile);
   if (r) return r;
   if (p.dense_out) return p.store_max8 ? launch_variant<3, 1>(tq, ti, p, st, num_sms) : launch_variant<2, 1>(tq, ti, p, st, num_sms);
   if (p.two_cta) return p.mask_cols ? launch_variant<1, 2>(tq, ti, p, st, num_sms) : launch_variant<0, 2>(tq, ti, p, st, num_sms);

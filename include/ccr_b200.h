@@ -66,6 +66,13 @@ extern "C" {
                                        needs id_offset + n_items <= 2^32 and no CCR_MASK_ADD (float64
                                        priors do not fit a float32 key)                           */
 
+#define CCR_FLAG_F16 0x40 /* q and items hold IEEE binary16 (fp16) instead of bf16.  Numerics: fp16 in,
+                             fp32 accumulate, fp32 out -- the operand format of the reference's
+                             autocast GPU matmul (scripts/al_0_rank.py:125), 11 significant bits
+                             instead of bf16's 8.  Same 2 bytes per element: the launch plan and
+                             the workspace size do not depend on it (ccr_plan_info /
+                             ccr_score_topk_workspace_bytes accept it and return the same values) */
+
 #define CCR_MAX_K 2048
 
 int ccr_abi_version(void);
@@ -81,9 +88,10 @@ const char* ccr_last_error_string(void);
  *   src/rime_lite/util/__init__.py:135-141 (as_tensor of MatMul+prior, topk(k).indices)
  *   src/ccrec/models/bbpr.py:528-545  (BertBPR.transform tile loop)
  *
- *   q        [B, ldq]  bf16 row-major queries / user embeddings (ldq >= D, ldq % 8 == 0)
+ *   q        [B, ldq]  bf16 row-major queries / user embeddings (ldq >= D, ldq % 8 == 0); fp16 with
+ *            CCR_FLAG_F16
  *   items    [n_items, ldi] bf16 row-major item / passage table shard (ldi >= D, ldi % 8 == 0,
- *            base 16-byte aligned)
+ *            base 16-byte aligned); fp16 with CCR_FLAG_F16 (both operands in the same format)
  *   D        embedding dim (768 in the reference: ms_marco_eval.py:190), D % 8 == 0, D <= 4096
  *   k        1 .. CCR_MAX_K
  *   mask_*   CSR over the LOCAL item columns of this shard: indptr[B+1] (int64), cols sorted
@@ -162,12 +170,30 @@ int ccr_normalize_rows_bf16(const void* src, int64_t n, int D, int64_t ld_src,
                             void* dst, int64_t ld_dst, void* stream);
 
 /*
+ * fp16 tables (CCR_FLAG_F16): fp32 rows -> IEEE binary16 rows, optionally L2-normalised first (in
+ * fp32, as ccr_ingest_rows_f32).  Rounds to nearest even and keeps subnormals, bit for bit what
+ * torch's .to(torch.float16) gives.  Columns D..ld_dst-1 of dst are zeroed.  overflow_count (a DEVICE
+ * int32, may be NULL): the number of stored values that are not finite (|x| >= 65520 after
+ * normalisation, or a non-finite input) is ADDED to it, so the caller can refuse such a batch.
+ */
+int ccr_ingest_rows_f32_f16(const float* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
+                            int normalize, int32_t* overflow_count, void* stream);
+
+/* Same for rows that are already fp16 (normalisation computed in fp32). */
+int ccr_normalize_rows_f16(const void* src, int64_t n, int D, int64_t ld_src,
+                           void* dst, int64_t ld_dst, void* stream);
+
+/*
  * Dense score tile  out[B, n] = Q . items^T  (fp32) for callers that really want the matrix
  * (LazyScore.as_tensor / _argsort on reranking sets: score_array.py:291-293).  Tiles of at least
  * 2^20 scores run on the TMA + tcgen05 pipeline of the fused kernel with a store epilogue, smaller
  * ones on a CUDA-core kernel.
  */
 int ccr_score_dense_f32(const void* q, int64_t B, int64_t ldq, const void* items, int64_t n_items,
+                        int64_t ldi, int D, float* out, int64_t ld_out, void* stream);
+
+/* The same with fp16 operands (fp16 in, fp32 accumulate, fp32 out); same two paths. */
+int ccr_score_dense_f16(const void* q, int64_t B, int64_t ldq, const void* items, int64_t n_items,
                         int64_t ldi, int D, float* out, int64_t ld_out, void* stream);
 
 /*
