@@ -1,5 +1,6 @@
-// Shared device helpers: sortable keys, warp-cooperative exact selection (radix select +
-// in-place compaction) on candidate buffers, small PTX wrappers.
+// Shared device helpers: sortable keys; the 256-bin histogram select steps every top-k path
+// uses; warp-cooperative selection on candidate buffers (exact radix select, in-place
+// compaction, approximate histogram prune); small PTX wrappers.
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -109,6 +110,70 @@ struct SharedKeys {
 };
 
 // ---------------------------------------------------------------------------------------
+// 256-bin histogram select, shared by every prune, seed and finalize step.  Lane L owns bins
+// [8L, 8L+8), so higher lanes hold higher bins.  warp_hist_scan loads the lane's bins into c
+// and returns the count in the bins of the lanes above it; warp_hist_locate then finds the bin
+// where the count from the top reaches `need` (1-based).  All 32 lanes call both.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ u32 warp_hist_scan(u32 hist_s, u32 (&c)[8]) {
+  const int lane = threadIdx.x & 31;
+  u32 lane_sum = 0;
+#pragma unroll
+  for (int t = 0; t < 8; ++t) { c[t] = sm_ld32(hist_s + (u32)(lane * 8 + t) * 4u); lane_sum += c[t]; }
+  u32 incl = lane_sum;  // keys in bins owned by lanes >= lane
+#pragma unroll
+  for (int off = 1; off < 32; off <<= 1) {
+    const u32 t = __shfl_down_sync(0xffffffffu, incl, off);
+    if (lane + off < 32) incl += t;
+  }
+  return incl - lane_sum;
+}
+
+struct HistBin {
+  u32 bin;    // the bin where the count from the top reaches `need`
+  u32 above;  // keys in the bins above it
+  u32 count;  // keys in it
+};
+
+// Every lane gets the same answer.  When need exceeds the total, no lane owns it and the result
+// is lane 31's {0, 0, 0}.
+__device__ __forceinline__ HistBin warp_hist_locate(const u32 (&c)[8], u32 above, u32 need) {
+  const int lane = threadIdx.x & 31;
+  u32 lane_sum = 0;
+#pragma unroll
+  for (int t = 0; t < 8; ++t) lane_sum += c[t];
+  const bool mine = above < need && need <= above + lane_sum;
+  HistBin r = {0u, 0u, 0u};
+  u32 run = above;
+  bool done = !mine;
+#pragma unroll
+  for (int t = 7; t >= 0; --t) {
+    const u32 prev = run;
+    run += c[t];
+    if (!done && run >= need) { r.bin = lane * 8 + t; r.above = prev; r.count = c[t]; done = true; }
+  }
+  const int src = __ffs(__ballot_sync(0xffffffffu, mine)) - 1;
+  r.bin = __shfl_sync(0xffffffffu, r.bin, src);
+  r.above = __shfl_sync(0xffffffffu, r.above, src);
+  r.count = __shfl_sync(0xffffffffu, r.count, src);
+  return r;
+}
+
+// m-th largest (1-based, repeats counted) of the nonzero values the 32 lanes hold; 0 when fewer
+// than m are nonzero.  Lanes without a value pass 0.
+__device__ __forceinline__ u32 warp_mth_largest(u32 v, int m) {
+  int gt = 0, ge = 0;
+#pragma unroll 4
+  for (int i = 0; i < 32; ++i) {
+    const u32 o = __shfl_sync(0xffffffffu, v, i);
+    gt += (o > v);
+    ge += (o >= v);
+  }
+  const unsigned who = __ballot_sync(0xffffffffu, v != 0u && gt < m && m <= ge);
+  return who ? __shfl_sync(0xffffffffu, v, __ffs(who) - 1) : 0u;
+}
+
+// ---------------------------------------------------------------------------------------
 // Warp-cooperative exact selection on n unique 64-bit keys.  Returns the `kth` largest key
 // (1-based).  hist_s: shared address of 256 x u32 private to the warp.  MSB-first 8-bit radix
 // select with early exit once the target bin holds one key.  All 32 lanes call it with
@@ -128,40 +193,14 @@ __device__ __forceinline__ u64 warp_select_kth(Keys keys, int n, int kth, u32 hi
       if ((key & pmask) == prefix) sm_red_inc(hist_s + ((u32)(key >> shift) & 255u) * 4u);
     }
     __syncwarp();
-    // lane L owns digits [8L, 8L+8); higher lanes = higher digits
     u32 c[8];
-    u32 lane_sum = 0;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) { c[j] = sm_ld32(hist_s + (u32)(lane * 8 + j) * 4u); lane_sum += c[j]; }
-    u32 incl = lane_sum;  // sum over lanes >= lane
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-      u32 t = __shfl_down_sync(0xffffffffu, incl, off);
-      if (lane + off < 32) incl += t;
-    }
-    u32 above = incl - lane_sum;
-    bool mine = (above < (u32)need) && ((u32)need <= incl);
-    u32 d = 0, newneed = 0, binc = 0;
-    if (mine) {
-      u32 run = above;
-#pragma unroll
-      for (int j = 7; j >= 0; --j) {
-        if (binc == 0) {
-          if (run + c[j] >= (u32)need) { d = lane * 8 + j; newneed = need - run; binc = c[j]; }
-          else run += c[j];
-        }
-      }
-    }
-    unsigned who = __ballot_sync(0xffffffffu, mine);
-    int src = __ffs(who) - 1;  // exactly one lane when kth <= n
-    d = __shfl_sync(0xffffffffu, d, src);
-    newneed = __shfl_sync(0xffffffffu, newneed, src);
-    binc = __shfl_sync(0xffffffffu, binc, src);
-    prefix |= (u64)d << shift;
+    const u32 above = warp_hist_scan(hist_s, c);
+    const HistBin b = warp_hist_locate(c, above, (u32)need);  // kth <= n: found
+    prefix |= (u64)b.bin << shift;
     pmask |= 0xFFull << shift;
-    need = (int)newneed;
+    need -= (int)b.above;
     __syncwarp();
-    if (binc == 1 && shift > 0) {
+    if (b.count == 1 && shift > 0) {
       // unique key with this prefix: find it
       u64 found = 0;
       for (int i = lane; i < n; i += 32) {
@@ -218,21 +257,24 @@ __device__ __forceinline__ u64 warp_prune(u64* buf, int n, int k, u32 hist_s, u3
 }
 
 // ---------------------------------------------------------------------------------------
-// One-pass approximate prune (the common case).  Keys are staged in shared memory, bucketed by
-// the 8 score bits just below the bits all n keys share, and everything at or above the bucket
-// where the running count from the top reaches k is kept: between k and k + (that bucket's
-// population - 1) survivors, which is all a *threshold* needs (any value with >= k candidates at
-// or above it is a valid lower bound of the k-th best).  The same histogram gives, for free, a
-// value with >= j candidates at or above it (the stream's contribution to the shared row bound).
+// Approximate histogram prune (the common case).  Keys are bucketed by the 8 score bits just
+// below the bits all n keys share, and everything at or above the bucket where the running count
+// from the top reaches k is kept: between k and k + (that bucket's population - 1) survivors,
+// which is all a *threshold* needs (any value with >= k candidates at or above it is a valid lower
+// bound of the k-th best).  The same histogram gives, for free, a value with >= j candidates at or
+// above it (the stream's contribution to the shared row bound).
+// kLevels = 2 refines once: when the boundary bucket is too crowded to keep whole, that bucket
+// alone is split into 256 finer ones by one more pass (BM25 scores of a young stream span many
+// binades, so its boundary bucket often is).
 // Returns false (nothing modified) when the keys do not spread over buckets (ties) or the
-// boundary bucket is too crowded; the caller then falls back to the exact radix select.
+// boundary bucket is still too crowded; the caller then falls back to the exact radix select.
 //   out_pivot_ord : ord32 score threshold; survivors are exactly the keys with ord >= it
 //   out_kept      : survivors, compacted to buf[0, kept)
 //   out_j_ord     : ord32 value with at least j keys >= it
-// ---------------------------------------------------------------------------------------
 // kStaged: keys are first copied to shared memory (stage_s) and the later passes read them there;
 // otherwise (buffers larger than the staging area) every pass streams the keys from global memory.
-template <bool kStaged>
+// ---------------------------------------------------------------------------------------
+template <bool kStaged, int kLevels>
 __device__ __forceinline__ bool warp_prune_hist(u64* buf, int n, int k, int j, int max_keep, u32 hist_s,
                                                 u32 stage_s, u32* out_pivot_ord, int* out_kept, u32* out_j_ord) {
   const int lane = threadIdx.x & 31;
@@ -254,63 +296,43 @@ __device__ __forceinline__ bool warp_prune_hist(u64* buf, int n, int k, int j, i
   const u32 d = mx ^ mn;
   if (d == 0u) return false;
   const int hb = 31 - __clz(d);
-  const int shift = hb > 7 ? hb - 7 : 0;
-  const u32 base = mn >> shift;  // digit = (ord >> shift) - base  in [0, 255]
+  int shift = hb > 7 ? hb - 7 : 0;
+  u32 edge = (mn >> shift) << shift;  // ord of bucket 0's lower edge; bucket = (ord - edge) >> shift in [0, 255]
+  u32 width = 0u;                     // level 1: ord span of the crowded bucket it splits
+  u32 need = (u32)k, kept_above = 0u;  // still to find inside the current range / keys kept above it
+  u32 pivot_ord = 0u, j_ord = 0u;
 #pragma unroll
-  for (int t = 0; t < 8; ++t) sm_st32(hist_s + (u32)(lane * 8 + t) * 4u, 0u);
-  __syncwarp();
-  for (int i = lane; i < n; i += 32) {
-    const u32 o = kStaged ? (u32)(sm_ld64(stage_s + (u32)i * 8u) >> 32) : (u32)(buf[i] >> 32);
-    sm_red_inc(hist_s + ((o >> shift) - base) * 4u);
-  }
-  __syncwarp();
-  u32 c[8], lane_sum = 0;
+  for (int level = 0; level < kLevels; ++level) {
 #pragma unroll
-  for (int t = 0; t < 8; ++t) { c[t] = sm_ld32(hist_s + (u32)(lane * 8 + t) * 4u); lane_sum += c[t]; }
-  u32 incl = lane_sum;  // keys in bins owned by lanes >= lane
-#pragma unroll
-  for (int off = 1; off < 32; off <<= 1) {
-    const u32 t = __shfl_down_sync(0xffffffffu, incl, off);
-    if (lane + off < 32) incl += t;
-  }
-  const u32 above = incl - lane_sum;
-  // bin where the count from the top reaches `need`, and that cumulative count
-  u32 bin_k = 0, cum_k = 0, bin_j = 0;
-  {
-    u32 run = above;
-    bool done_k = !((above < (u32)k) && ((u32)k <= incl)), done_j = !((above < (u32)j) && ((u32)j <= incl));
-#pragma unroll
-    for (int t = 7; t >= 0; --t) {
-      run += c[t];
-      if (!done_k && run >= (u32)k) { bin_k = lane * 8 + t; cum_k = run; done_k = true; }
-      if (!done_j && run >= (u32)j) { bin_j = lane * 8 + t; done_j = true; }
+    for (int t = 0; t < 8; ++t) sm_st32(hist_s + (u32)(lane * 8 + t) * 4u, 0u);
+    __syncwarp();
+    for (int i = lane; i < n; i += 32) {
+      const u32 o = kStaged ? (u32)(sm_ld64(stage_s + (u32)i * 8u) >> 32) : (u32)(buf[i] >> 32);
+      if (level == 0 || o - edge < width) sm_red_inc(hist_s + ((o - edge) >> shift) * 4u);  // unsigned: o < edge fails too
     }
+    __syncwarp();
+    u32 c[8];
+    const u32 above = warp_hist_scan(hist_s, c);
+    const HistBin bk = warp_hist_locate(c, above, need);
+    if (level == 0) j_ord = edge + (warp_hist_locate(c, above, (u32)j).bin << shift);  // level 0 sees every key
+    pivot_ord = edge + (bk.bin << shift);
+    if ((int)(kept_above + bk.above + bk.count) <= max_keep) break;  // keep the boundary bucket whole
+    if (level == kLevels - 1 || shift == 0) return false;
+    // split the boundary bucket: the keys above it are kept anyway
+    kept_above += bk.above;
+    need -= bk.above;
+    edge = pivot_ord;
+    width = 1u << shift;
+    shift = shift > 8 ? shift - 8 : 0;
+    __syncwarp();
   }
-  const unsigned who_k = __ballot_sync(0xffffffffu, (above < (u32)k) && ((u32)k <= incl));
-  const unsigned who_j = __ballot_sync(0xffffffffu, (above < (u32)j) && ((u32)j <= incl));
-  const int src_k = __ffs(who_k) - 1, src_j = __ffs(who_j) - 1;
-  bin_k = __shfl_sync(0xffffffffu, bin_k, src_k);
-  cum_k = __shfl_sync(0xffffffffu, cum_k, src_k);
-  bin_j = __shfl_sync(0xffffffffu, bin_j, src_j);
-  if ((int)cum_k > max_keep) return false;
-  u32 pivot_ord = (base + bin_k) << shift;
   if (pivot_ord < 0x00800000u) pivot_ord = 0x00800000u;  // never below ord32(-FLT_MAX): stays a finite float
-  // stable compaction to buf[0, kept); in place it only ever writes at or below the index it read
-  int wbase = 0;
-  for (int i0 = 0; i0 < n; i0 += 32) {
-    const int i = i0 + lane;
-    const u64 key = (i < n) ? (kStaged ? sm_ld64(stage_s + (u32)i * 8u) : buf[i]) : 0ull;
-    const bool keep = (i < n) && ((u32)(key >> 32) >= pivot_ord);
-    const unsigned m = __ballot_sync(0xffffffffu, keep);
-    __syncwarp();
-    if (keep) buf[wbase + __popc(m & ((1u << lane) - 1u))] = key;
-    wbase += __popc(m);
-    __syncwarp();
-  }
-  *out_pivot_ord = pivot_ord;
-  *out_kept = wbase;
-  u32 j_ord = (base + bin_j) << shift;
   if (j_ord < 0x00800000u) j_ord = 0x00800000u;
+  // (u32)(key >> 32) >= pivot_ord  <=>  key >= (u64)pivot_ord << 32
+  const u64 pivot = (u64)pivot_ord << 32;
+  *out_kept = kStaged ? warp_compact_ge(SharedKeys{stage_s}, GlobalKeys{buf}, n, pivot)
+                      : warp_compact_ge(GlobalKeys{buf}, GlobalKeys{buf}, n, pivot);
+  *out_pivot_ord = pivot_ord;
   *out_j_ord = j_ord;
   return true;
 }

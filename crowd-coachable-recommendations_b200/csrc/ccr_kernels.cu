@@ -361,27 +361,10 @@ __global__ void __launch_bounds__(kFinMaxThreads) finalize_kernel(FinalizeParams
       });
       __syncthreads();
       if (warp == 0) {
-        u32 c[8], lane_sum = 0;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) { c[j] = hist[lane * 8 + j]; lane_sum += c[j]; }
-        u32 incl = lane_sum;
-#pragma unroll
-        for (int off = 1; off < 32; off <<= 1) {
-          u32 t = __shfl_down_sync(0xffffffffu, incl, off);
-          if (lane + off < 32) incl += t;
-        }
-        u32 above = incl - lane_sum;
-        if (above < (u32)need && (u32)need <= incl) {
-          u32 run = above;
-          bool done = false;
-#pragma unroll
-          for (int j = 7; j >= 0; --j) {
-            if (!done) {
-              if (run + c[j] >= (u32)need) { s_d = lane * 8 + j; s_need = need - run; s_binc = c[j]; done = true; }
-              else run += c[j];
-            }
-          }
-        }
+        u32 c[8];
+        const u32 above = warp_hist_scan(smem_addr(hist), c);
+        const HistBin b = warp_hist_locate(c, above, (u32)need);  // need <= entries with the prefix: found
+        if (lane == 0) { s_d = b.bin; s_need = need - b.above; s_binc = b.count; }
       }
       __syncthreads();
       const u32 d = s_d;
@@ -1049,110 +1032,6 @@ int launch_bm25_topk(const long long* post_indptr, const int* post_docs, const d
 // still applied in q_terms order and a doc has at most one posting per term, so every float64 sum is
 // bit-identical to the block-wide kernel's and to the reference's.
 // =======================================================================================
-// One- or two-level histogram prune of a stream's candidate buffer (keys in global memory; all 32 lanes
-// call it with identical arguments).  Level 1 = warp_prune_hist's scheme: 256 buckets over the 8 score bits
-// below the bits all keys share.  BM25 scores of a young stream span many binades, so the bucket that holds
-// the k-th best is often too crowded to keep whole; instead of giving up (exact radix select: 4-6 more
-// passes over the keys) that bucket alone is split into 256 finer ones by one more pass.
-//   out_pivot_ord : survivors are exactly the keys with ord32(score) >= it (>= k of them, <= max_keep)
-//   out_j_ord     : ord32 value with at least j keys at or above it
-static __device__ __noinline__ bool bm25_prune_hist(u64* buf, int n, int k, int j, int max_keep, u32 hist_s,
-                                                    u32* out_pivot_ord, int* out_kept, u32* out_j_ord) {
-  const int lane = threadIdx.x & 31;
-  __syncwarp();
-  u32 mx = 0u, mn = 0xFFFFFFFFu;
-  for (int i = lane; i < n; i += 32) {
-    const u32 o = (u32)(buf[i] >> 32);
-    mx = o > mx ? o : mx;
-    mn = o < mn ? o : mn;
-  }
-#pragma unroll
-  for (int off = 16; off; off >>= 1) {
-    const u32 a = __shfl_xor_sync(0xffffffffu, mx, off), b = __shfl_xor_sync(0xffffffffu, mn, off);
-    mx = a > mx ? a : mx;
-    mn = b < mn ? b : mn;
-  }
-  const u32 d = mx ^ mn;
-  if (d == 0u) return false;
-  const int hb = 31 - __clz(d);
-  int shift = hb > 7 ? hb - 7 : 0;
-  u32 edge = (mn >> shift) << shift;   // ord of bucket 0's lower edge; bucket = (ord - edge) >> shift in [0, 255]
-  u32 width = 0xFFFFFFFFu;             // ord span the current histogram covers (level 1: the crowded bucket)
-  int need = k, above = 0;             // still to find inside the current bucket range / keys above it
-  u32 pivot_ord = 0u, j_ord = 0u;
-  bool have_j = false;
-  for (int level = 0; level < 2; ++level) {
-#pragma unroll
-    for (int t = 0; t < 8; ++t) sm_st32(hist_s + (u32)(lane * 8 + t) * 4u, 0u);
-    __syncwarp();
-    for (int i = lane; i < n; i += 32) {
-      const u32 o = (u32)(buf[i] >> 32);
-      if (o >= edge && o - edge < width) sm_red_inc(hist_s + ((o - edge) >> shift) * 4u);   // level 1: the crowded bucket only
-    }
-    __syncwarp();
-    u32 c[8], lane_sum = 0;
-#pragma unroll
-    for (int t = 0; t < 8; ++t) { c[t] = sm_ld32(hist_s + (u32)(lane * 8 + t) * 4u); lane_sum += c[t]; }
-    u32 incl = lane_sum;  // keys in bins owned by lanes >= lane
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-      const u32 t = __shfl_down_sync(0xffffffffu, incl, off);
-      if (lane + off < 32) incl += t;
-    }
-    const u32 hi = incl - lane_sum;   // keys in bins above this lane's
-    u32 bin_k = 0, cum_k = 0, cnt_k = 0, bin_j = 0;
-    {
-      u32 run = hi;
-      bool done_k = !((hi < (u32)need) && ((u32)need <= incl)), done_j = have_j || !((hi < (u32)j) && ((u32)j <= incl));
-#pragma unroll
-      for (int t = 7; t >= 0; --t) {
-        run += c[t];
-        if (!done_k && run >= (u32)need) { bin_k = lane * 8 + t; cum_k = run; cnt_k = c[t]; done_k = true; }
-        if (!done_j && run >= (u32)j) { bin_j = lane * 8 + t; done_j = true; }
-      }
-    }
-    const unsigned who_k = __ballot_sync(0xffffffffu, (hi < (u32)need) && ((u32)need <= incl));
-    const int src_k = __ffs(who_k) - 1;
-    bin_k = __shfl_sync(0xffffffffu, bin_k, src_k);
-    cum_k = __shfl_sync(0xffffffffu, cum_k, src_k);
-    cnt_k = __shfl_sync(0xffffffffu, cnt_k, src_k);
-    if (!have_j) {   // level 0 sees every key: its histogram also yields the j-th best bucket
-      const unsigned who_j = __ballot_sync(0xffffffffu, (hi < (u32)j) && ((u32)j <= incl));
-      bin_j = __shfl_sync(0xffffffffu, bin_j, __ffs(who_j) - 1);
-      j_ord = edge + (bin_j << shift);
-      have_j = true;
-    }
-    __syncwarp();
-    pivot_ord = edge + (bin_k << shift);
-    if (above + (int)cum_k <= max_keep) { above += (int)cum_k; break; }   // keep the boundary bucket whole
-    if (level == 1 || shift == 0) return false;                          // still too crowded (ties): exact select
-    // split the boundary bucket: the keys above it are kept anyway
-    above += (int)(cum_k - cnt_k);
-    need -= (int)(cum_k - cnt_k);
-    edge = pivot_ord;
-    width = 1u << shift;
-    shift = shift > 8 ? shift - 8 : 0;
-  }
-  if (pivot_ord < 0x00800000u) pivot_ord = 0x00800000u;  // never below ord32(-FLT_MAX): stays a finite float
-  if (j_ord < 0x00800000u) j_ord = 0x00800000u;
-  // stable compaction to buf[0, kept); in place it only ever writes at or below the index it read
-  int wbase = 0;
-  for (int i0 = 0; i0 < n; i0 += 32) {
-    const int i = i0 + lane;
-    const u64 key = (i < n) ? buf[i] : 0ull;
-    const bool keep = (i < n) && ((u32)(key >> 32) >= pivot_ord);
-    const unsigned m = __ballot_sync(0xffffffffu, keep);
-    __syncwarp();
-    if (keep) buf[wbase + __popc(m & ((1u << lane) - 1u))] = key;
-    wbase += __popc(m);
-    __syncwarp();
-  }
-  *out_pivot_ord = pivot_ord;
-  *out_kept = wbase;
-  *out_j_ord = j_ord;
-  return true;
-}
-
 __global__ void __launch_bounds__(kBmwWarps * 32, kBmwBlocksPerSm) bm25_topk_warp_kernel(
     const long long* __restrict__ post_indptr, const int* __restrict__ post_docs, const double* __restrict__ post_val,
     const int* __restrict__ head_slot, const double* __restrict__ head_rows, long long ld_head,
@@ -1318,13 +1197,13 @@ __global__ void __launch_bounds__(kBmwWarps * 32, kBmwBlocksPerSm) bm25_topk_war
       }
       __syncwarp();
       if (cnt > C - kBmwMini) {  // C >= 2k + kBmwMini: room for the next mini-chunk after a prune
-        // one histogram pass over the keys (keeps everything at or above the bucket where the count from
-        // the top reaches k: a score threshold with >= k docs at or above it); tie-heavy or crowded
-        // buffers fall back to the exact radix select
+        // one histogram pass over the keys, and a second one over a crowded boundary bucket (keeps everything
+        // at or above the bucket where the count from the top reaches k: a score threshold with >= k docs at
+        // or above it); tie-heavy or still crowded buffers fall back to the exact radix select
         u32 pivot_ord = 0u, j_ord = 0u;
         int kept = 0;
-        if (bm25_prune_hist(buf, cnt, k, (k + kBmwSketchM - 1) / kBmwSketchM, (k + C - kBmwMini) / 2,
-                            smem_addr(s_hist[warp]), &pivot_ord, &kept, &j_ord)) {
+        if (warp_prune_hist<false, 2>(buf, cnt, k, (k + kBmwSketchM - 1) / kBmwSketchM, (k + C - kBmwMini) / 2,
+                                      smem_addr(s_hist[warp]), 0u, &pivot_ord, &kept, &j_ord)) {
           cnt = kept;
           tau_key = 0ull;
           tau_f = unord32(pivot_ord);
@@ -1334,18 +1213,8 @@ __global__ void __launch_bounds__(kBmwWarps * 32, kBmwBlocksPerSm) bm25_topk_war
           __syncwarp();
           u32 v = 0u;
           if (lane < kBmwWarps) asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(v) : "r"(smem_addr(&s_jth[lane])) : "memory");
-          int gt = 0, ge = 0;
-#pragma unroll
-          for (int i = 0; i < kBmwWarps; ++i) {
-            const u32 o = __shfl_sync(0xffffffffu, v, i);
-            gt += (o > v);
-            ge += (o >= v);
-          }
-          const unsigned who = __ballot_sync(0xffffffffu, lane < kBmwWarps && v != 0u && gt < kBmwSketchM && kBmwSketchM <= ge);
-          if (who) {
-            const u32 bound = __shfl_sync(0xffffffffu, v, __ffs(who) - 1);
-            if (lane == 0) atomicMax(&s_tau_blk, bound);
-          }
+          const u32 bound = warp_mth_largest(v, kBmwSketchM);
+          if (bound != 0u && lane == 0) atomicMax(&s_tau_blk, bound);
         } else {
           const u64 pivot = warp_prune(buf, cnt, k, smem_addr(s_hist[warp]), 0u);
           cnt = k;
@@ -1377,16 +1246,9 @@ __global__ void __launch_bounds__(kBmwWarps * 32, kBmwBlocksPerSm) bm25_topk_war
     __syncthreads();   // (every stream is past its last in-loop use of s_jth)
     if (lane == 0) s_jth[warp] = jv;
     __syncthreads();
-    if (threadIdx.x == 0) {
-      u32 v[kBmwWarps];
-#pragma unroll
-      for (int i = 0; i < kBmwWarps; ++i) v[i] = s_jth[i];
-#pragma unroll
-      for (int a = 0; a < kBmwSketchM; ++a)      // partial selection sort: v[0..M) = the M largest, descending
-#pragma unroll
-        for (int b = a + 1; b < kBmwWarps; ++b)
-          if (v[b] > v[a]) { const u32 t = v[a]; v[a] = v[b]; v[b] = t; }
-      if (v[kBmwSketchM - 1] != 0u) atomicMax(row_tau + row, v[kBmwSketchM - 1]);
+    if (warp == 0) {
+      const u32 bound = warp_mth_largest(lane < kBmwWarps ? s_jth[lane] : 0u, kBmwSketchM);
+      if (bound != 0u && lane == 0) atomicMax(row_tau + row, bound);
     }
   }
 }
@@ -1519,8 +1381,8 @@ __global__ void __launch_bounds__(kDenseThreads) select_dense_kernel(const float
         u32 pivot_ord = 0u, j_ord = 0u;
         int kept = 0;
         const int n_now = s_cnt;
-        if (warp_prune_hist<false>(buf, n_now, k_row, k_row, (k_row + C - kDenseSlack) / 2, smem_addr(s_hist), 0u,
-                                   &pivot_ord, &kept, &j_ord)) {
+        if (warp_prune_hist<false, 1>(buf, n_now, k_row, k_row, (k_row + C - kDenseSlack) / 2, smem_addr(s_hist), 0u,
+                                      &pivot_ord, &kept, &j_ord)) {
           if (tid == 0) { s_cnt = kept; s_tau_key = 0ull; s_tau_f = unord32(pivot_ord); }
         } else {
           const u64 pivot = warp_prune(buf, n_now, k_row, smem_addr(s_hist), 0u);

@@ -326,15 +326,7 @@ static __device__ __noinline__ u32 sketch_bound(const u32* gq, int S_row, int m,
   if (S_row <= 32) {
     u32 v = 0u;
     if (lane < S_row) v = (lane == own_stream) ? own_val : __ldcg(gq + lane);
-    int gt = 0, ge = 0;
-#pragma unroll 4
-    for (int i = 0; i < 32; ++i) {
-      const u32 o = __shfl_sync(0xffffffffu, v, i);
-      gt += (o > v);
-      ge += (o >= v);
-    }
-    const unsigned who = __ballot_sync(0xffffffffu, gt < m && m <= ge);
-    return who ? __shfl_sync(0xffffffffu, v, __ffs(who) - 1) : 0u;
+    return warp_mth_largest(v, m);
   }
   const int ns = S_row < kStageKeys ? S_row : kStageKeys;
   for (int i = lane; i < ns; i += 32) {
@@ -369,8 +361,8 @@ static __device__ __noinline__ u64 prune_stream(u64* b, int n, int k, int C, int
   u32 j_ord = 0u, pivot_ord = 0u;
   // fast path: one histogram pass; leaves between k and (k + C-128)/2 survivors
   const bool fast =
-      staged ? warp_prune_hist<true>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord)
-             : warp_prune_hist<false>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord);
+      staged ? warp_prune_hist<true, 1>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord)
+             : warp_prune_hist<false, 1>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord);
   if (fast) {
     new_tau = unord32(pivot_ord);  // ">=": every key at or above the pivot bucket was kept
   } else {
@@ -843,27 +835,10 @@ __global__ void __launch_bounds__(256) seed_tau_kernel(const float* __restrict__
     }
     __syncthreads();
     if (tid < 32) {
-      u32 c[8], lane_sum = 0;
-#pragma unroll
-      for (int t = 0; t < 8; ++t) { c[t] = hist[lane * 8 + t]; lane_sum += c[t]; }
-      u32 incl = lane_sum;
-#pragma unroll
-      for (int off = 1; off < 32; off <<= 1) {
-        const u32 t = __shfl_down_sync(0xffffffffu, incl, off);
-        if (lane + off < 32) incl += t;
-      }
-      const u32 above = incl - lane_sum;
-      if (above < (u32)need && (u32)need <= incl) {
-        u32 run = above;
-        bool done = false;
-#pragma unroll
-        for (int t = 7; t >= 0; --t) {
-          if (!done) {
-            if (run + c[t] >= (u32)need) { s_d = lane * 8 + t; s_need = need - run; done = true; }
-            else run += c[t];
-          }
-        }
-      }
+      u32 c[8];
+      const u32 above = warp_hist_scan(smem_addr(hist), c);
+      const HistBin b = warp_hist_locate(c, above, (u32)need);  // kth <= m: found
+      if (lane == 0) { s_d = b.bin; s_need = need - b.above; }
     }
     __syncthreads();
     prefix |= s_d << shift;
