@@ -256,6 +256,16 @@ __device__ __forceinline__ u64 warp_prune(u64* buf, int n, int k, u32 hist_s, u3
   return pivot;
 }
 
+// The outcome of one prune step (warp_prune_stream below): a later candidate (s, id) of the
+// stream passes when s >= tau_f and make_key(s, id) > tau_key.
+struct PruneResult {
+  int kept;      // keys left in buf[0, kept)
+  float tau_f;
+  u64 tau_key;
+  u32 j_ord;     // histogram path: ord32 score with >= j kept keys at or above it
+  bool hist;     // the histogram path ran
+};
+
 // ---------------------------------------------------------------------------------------
 // Approximate histogram prune (the common case).  Keys are bucketed by the 8 score bits just
 // below the bits all n keys share, and everything at or above the bucket where the running count
@@ -268,15 +278,14 @@ __device__ __forceinline__ u64 warp_prune(u64* buf, int n, int k, u32 hist_s, u3
 // binades, so its boundary bucket often is).
 // Returns false (nothing modified) when the keys do not spread over buckets (ties) or the
 // boundary bucket is still too crowded; the caller then falls back to the exact radix select.
-//   out_pivot_ord : ord32 score threshold; survivors are exactly the keys with ord >= it
-//   out_kept      : survivors, compacted to buf[0, kept)
-//   out_j_ord     : ord32 value with at least j keys >= it
+// Otherwise the survivors, exactly the keys with ord32 score >= pivot_ord, are compacted to
+// buf[0, r.kept), and r.tau_f = unord32(pivot_ord).
 // kStaged: keys are first copied to shared memory (stage_s) and the later passes read them there;
 // otherwise (buffers larger than the staging area) every pass streams the keys from global memory.
 // ---------------------------------------------------------------------------------------
 template <bool kStaged, int kLevels>
 __device__ __forceinline__ bool warp_prune_hist(u64* buf, int n, int k, int j, int max_keep, u32 hist_s,
-                                                u32 stage_s, u32* out_pivot_ord, int* out_kept, u32* out_j_ord) {
+                                                u32 stage_s, PruneResult& r) {
   const int lane = threadIdx.x & 31;
   __syncwarp();
   u32 mx = 0u, mn = 0xFFFFFFFFu;
@@ -330,23 +339,61 @@ __device__ __forceinline__ bool warp_prune_hist(u64* buf, int n, int k, int j, i
   if (j_ord < 0x00800000u) j_ord = 0x00800000u;
   // (u32)(key >> 32) >= pivot_ord  <=>  key >= (u64)pivot_ord << 32
   const u64 pivot = (u64)pivot_ord << 32;
-  *out_kept = kStaged ? warp_compact_ge(SharedKeys{stage_s}, GlobalKeys{buf}, n, pivot)
-                      : warp_compact_ge(GlobalKeys{buf}, GlobalKeys{buf}, n, pivot);
-  *out_pivot_ord = pivot_ord;
-  *out_j_ord = j_ord;
+  const int kept = kStaged ? warp_compact_ge(SharedKeys{stage_s}, GlobalKeys{buf}, n, pivot)
+                           : warp_compact_ge(GlobalKeys{buf}, GlobalKeys{buf}, n, pivot);
+  r = {kept, unord32(pivot_ord), 0ull, j_ord, true};
   return true;
 }
 
-// Append one candidate (noinline: keeps the unrolled per-column hit tests small).
-static __device__ __noinline__ int cand_insert(float s, u32 col, int cnt, u64 tau_key, u64* buf,
-                                        const int* mask_cols, long long mbeg, long long mend) {
-  const u64 key = make_key(s, col);
-  if (key > tau_key && !(mask_cols && mask_contains(mask_cols, mbeg, mend, (int)col))) {
-    buf[cnt] = key;
-    return cnt + 1;
+// ---------------------------------------------------------------------------------------
+// One prune step of a streaming top-k: shrink a candidate buffer and raise the bound later
+// candidates of the stream must pass (PruneResult).  Both forms keep every key that can still
+// rank in the top k:
+//   exact path (warp_prune): buf keeps the k largest keys and the k-th, `pivot`, becomes a *strict*
+//     key bound: tau_f = key_score(pivot), tau_key = pivot.  Keys are unique, so a new key ranks
+//     in the top k only if it is larger than the pivot -- including a score tied with the pivot's
+//     whose id is lower.  A stream that visits ids in ascending order can drop the key compare: a
+//     later id never beats a tied pivot, so s >= next_up(key_score(pivot)) is the same bound.
+//   histogram path (warp_prune_hist): buf keeps every key whose score is >= unord32(pivot_ord),
+//     at least k of them, so tau_f = unord32(pivot_ord) and tau_key = 0.  A score equal to that
+//     edge may tie a kept key and still rank, so it passes (>=) and no key compare applies.
+// kLevels = 0: exact path only.  Otherwise the histogram prune is tried first with that refinement
+// depth; ties or a boundary bucket too crowded for max_keep fall back to the exact path.  j and
+// max_keep are read by the histogram path only.  All 32 lanes call it with identical arguments.
+// ---------------------------------------------------------------------------------------
+template <bool kStaged, int kLevels>
+__device__ __forceinline__ PruneResult warp_prune_stream(u64* buf, int n, int k, int j, int max_keep, u32 hist_s,
+                                                         u32 stage_s) {
+  PruneResult r;
+  if constexpr (kLevels > 0) {
+    if (warp_prune_hist<kStaged, kLevels>(buf, n, k, j, max_keep, hist_s, stage_s, r)) return r;
   }
-  return cnt;
+  const u64 pivot = warp_prune(buf, n, k, hist_s, kStaged ? stage_s : 0u);
+  return {k, key_score(pivot), pivot, 0u, false};
 }
+
+// The state of one candidate stream that every thread of a block appends to, in shared memory.
+// One thread calls init; one warp prunes with warp_prune_stream and hands the result to apply.
+struct BlockStream {
+  int cnt;        // keys in the stream's buffer
+  float tau_f;    // the PruneResult bound: -inf before the first prune
+  u64 tau_key;
+  u32 hist[256];  // the pruning warp's histogram
+
+  __device__ __forceinline__ void init() { cnt = 0; tau_f = -INFINITY; tau_key = 0ull; }
+  // Append (s, id) when it passes the bound (tf, tk): the record's own, or a copy of it read
+  // before a block vote.
+  __device__ __forceinline__ void append(u64* buf, float s, u32 id, float tf, u64 tk) {
+    if (s >= tf) {
+      const u64 key = make_key(s, id);
+      if (key > tk) buf[atomicAdd(&cnt, 1)] = key;
+    }
+  }
+  // lane 0 of the pruning warp publishes the new count and bound
+  __device__ __forceinline__ void apply(const PruneResult& r) {
+    if ((threadIdx.x & 31) == 0) { cnt = r.kept; tau_f = r.tau_f; tau_key = r.tau_key; }
+  }
+};
 
 // ---------------------------------------------------------------------------------------
 // misc

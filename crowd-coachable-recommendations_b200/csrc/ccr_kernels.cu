@@ -25,6 +25,8 @@ __global__ void __launch_bounds__(256, 2) select_simt_kernel(SelectParams p) {
   const T* __restrict__ pq = reinterpret_cast<const T*>(p.q);
   const T* __restrict__ pitems = reinterpret_cast<const T*>(p.items);
   float* qs = reinterpret_cast<float*>(smem_raw);  // [8][D]
+  // one stream per row, kept as separate arrays rather than BlockStream records: with the records
+  // ptxas holds a row address across the dot-product loop (127 instead of 122 registers)
   __shared__ int s_cnt[kSimtRows];
   __shared__ float s_tau_f[kSimtRows];
   __shared__ u64 s_tau_key[kSimtRows];
@@ -123,11 +125,11 @@ __global__ void __launch_bounds__(256, 2) select_simt_kernel(SelectParams p) {
         int n = s_cnt[warp];
         if (n > p.C - kSimtChunk) {
           u64* b = p.cand + ((long long)(row0 + warp) * p.S + split) * p.C;
-          u64 pivot = warp_prune(b, n, p.k, smem_addr(s_hist[warp]), 0u);
+          const PruneResult r = warp_prune_stream<false, 0>(b, n, p.k, 0, 0, smem_addr(s_hist[warp]), 0u);
           if (lane == 0) {
-            s_cnt[warp] = p.k;
-            s_tau_key[warp] = pivot;
-            s_tau_f[warp] = key_score(pivot);
+            s_cnt[warp] = r.kept;
+            s_tau_key[warp] = r.tau_key;
+            s_tau_f[warp] = r.tau_f;
           }
         }
       }
@@ -854,7 +856,6 @@ int launch_bm25_impacts(const long long* post_indptr, const int* post_docs, cons
 }
 
 constexpr int kBmUnroll = 4;      // postings per thread and iteration (memory-level parallelism)
-constexpr int kBmScan = kBmSlack;  // accumulators ranked between two prune checks
 
 // dynamic shared memory: double acc[kBmChunk]; long long cur[kBmMaxTerms], pend[kBmMaxTerms]; int nxt[kBmMaxTerms]
 constexpr size_t kBmSmem = (size_t)kBmChunk * 8 + (size_t)kBmMaxTerms * (8 + 8 + 4);
@@ -873,10 +874,7 @@ __global__ void __launch_bounds__(kBmThreads) bm25_topk_kernel(const long long* 
   long long* cur = reinterpret_cast<long long*>(acc + kBmChunk);
   long long* pend = cur + kBmMaxTerms;
   int* nxt = reinterpret_cast<int*>(pend + kBmMaxTerms);
-  __shared__ int s_cnt;
-  __shared__ float s_tau_f;
-  __shared__ u64 s_tau_key;
-  __shared__ u32 s_hist[256];
+  __shared__ BlockStream s_st;
 
   const int tid = threadIdx.x, split = blockIdx.x;
   const long long row = blockIdx.y;
@@ -905,7 +903,7 @@ __global__ void __launch_bounds__(kBmThreads) bm25_topk_kernel(const long long* 
     pend[t] = end;
     nxt[t] = lo < end ? post_docs[lo] : 0x7fffffff;
   }
-  if (tid == 0) { s_cnt = 0; s_tau_f = -INFINITY; s_tau_key = 0ull; }
+  if (tid == 0) s_st.init();
   __syncthreads();
 
   for (long long c0 = d0; c0 < d1; c0 += kBmChunk) {
@@ -982,31 +980,22 @@ __global__ void __launch_bounds__(kBmThreads) bm25_topk_kernel(const long long* 
       double* o = dense_out + row * ld_out + c0;
       for (int j = tid; j < len; j += kBmThreads) o[j] = acc[j];
     } else {
-      for (int base = 0; base < len; base += kBmScan) {
+      for (int base = 0; base < len; base += kBmSlack) {
 #pragma unroll
-        for (int u = 0; u < kBmScan / kBmThreads; ++u) {
+        for (int u = 0; u < kBmSlack / kBmThreads; ++u) {
           const int j = base + u * kBmThreads + tid;
-          if (j < len) {
-            const float sc = (float)acc[j];
-            if (sc >= s_tau_f) {
-              const u64 key = make_key(sc, (u32)(c0 + j));
-              if (key > s_tau_key) buf[atomicAdd(&s_cnt, 1)] = key;
-            }
-          }
+          if (j < len) s_st.append(buf, (float)acc[j], (u32)(c0 + j), s_st.tau_f, s_st.tau_key);
         }
         __syncthreads();
-        if (s_cnt > C - kBmScan) {  // uniform: read after the barrier
-          if (tid < 32) {
-            const u64 pivot = warp_prune(buf, s_cnt, k, smem_addr(s_hist), 0u);
-            if (tid == 0) { s_cnt = k; s_tau_key = pivot; s_tau_f = key_score(pivot); }
-          }
+        if (s_st.cnt > C - kBmSlack) {  // uniform: read after the barrier
+          if (tid < 32) s_st.apply(warp_prune_stream<false, 0>(buf, s_st.cnt, k, 0, 0, smem_addr(s_st.hist), 0u));
         }
         __syncthreads();
       }
     }
     __syncthreads();
   }
-  if (counts && tid == 0) counts[(long long)row * S + split] = s_cnt;
+  if (counts && tid == 0) counts[(long long)row * S + split] = s_st.cnt;
 }
 
 int launch_bm25_topk(const long long* post_indptr, const int* post_docs, const double* post_val,
@@ -1197,29 +1186,20 @@ __global__ void __launch_bounds__(kBmwWarps * 32, kBmwBlocksPerSm) bm25_topk_war
       }
       __syncwarp();
       if (cnt > C - kBmwMini) {  // C >= 2k + kBmwMini: room for the next mini-chunk after a prune
-        // one histogram pass over the keys, and a second one over a crowded boundary bucket (keeps everything
-        // at or above the bucket where the count from the top reaches k: a score threshold with >= k docs at
-        // or above it); tie-heavy or still crowded buffers fall back to the exact radix select
-        u32 pivot_ord = 0u, j_ord = 0u;
-        int kept = 0;
-        if (warp_prune_hist<false, 2>(buf, cnt, k, (k + kBmwSketchM - 1) / kBmwSketchM, (k + C - kBmwMini) / 2,
-                                      smem_addr(s_hist[warp]), 0u, &pivot_ord, &kept, &j_ord)) {
-          cnt = kept;
-          tau_key = 0ull;
-          tau_f = unord32(pivot_ord);
+        // one histogram pass over the keys, and a second one over a crowded boundary bucket; tie-heavy or
+        // still crowded buffers fall back to the exact radix select
+        const PruneResult r = warp_prune_stream<false, 2>(buf, cnt, k, (k + kBmwSketchM - 1) / kBmwSketchM,
+                                                          (k + C - kBmwMini) / 2, smem_addr(s_hist[warp]), 0u);
+        cnt = r.kept; tau_f = r.tau_f; tau_key = r.tau_key;
+        if (r.hist) {
           // sketch bound: this stream has >= ceil(k/M) docs at or above j_ord; the M-th largest of the block's
           // published values therefore has >= k docs of the query at or above it
-          if (lane == 0) atomicMax(&s_jth[warp], j_ord);
+          if (lane == 0) atomicMax(&s_jth[warp], r.j_ord);
           __syncwarp();
           u32 v = 0u;
           if (lane < kBmwWarps) asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(v) : "r"(smem_addr(&s_jth[lane])) : "memory");
           const u32 bound = warp_mth_largest(v, kBmwSketchM);
           if (bound != 0u && lane == 0) atomicMax(&s_tau_blk, bound);
-        } else {
-          const u64 pivot = warp_prune(buf, cnt, k, smem_addr(s_hist[warp]), 0u);
-          cnt = k;
-          tau_key = pivot;
-          tau_f = key_score(pivot);
         }
         pruned = true;
         if (lane == 0) atomicMax(&s_tau_blk, ord32(tau_f));
@@ -1321,10 +1301,7 @@ __global__ void __launch_bounds__(kDenseThreads) select_dense_kernel(const float
                                                                      long long N, int k, int k_keep,
                                                                      const long long* __restrict__ mask_indptr, int C,
                                                                      int S, u64* cand, int* counts) {
-  __shared__ int s_cnt;
-  __shared__ float s_tau_f;
-  __shared__ u64 s_tau_key;
-  __shared__ u32 s_hist[256];
+  __shared__ BlockStream s_st;
   const int tid = threadIdx.x, split = blockIdx.x;
   const long long row = blockIdx.y;
   // buffers are sized for k_keep = k + mask_max_row_nnz: never trust the CSR beyond that
@@ -1337,7 +1314,7 @@ __global__ void __launch_bounds__(kDenseThreads) select_dense_kernel(const float
   if (i1 > N) i1 = N;
   u64* buf = cand + ((long long)row * S + split) * C;
   const float* r = scores + row * ld;
-  if (tid == 0) { s_cnt = 0; s_tau_f = -INFINITY; s_tau_key = 0ull; }
+  if (tid == 0) s_st.init();
   __syncthreads();
   // kDenseSlack columns per iteration: 16 per thread as four 16-byte loads in flight (scalar loads at a
   // ragged end or an unaligned row), one max + ONE block vote, and only an iteration that holds a
@@ -1362,37 +1339,24 @@ __global__ void __launch_bounds__(kDenseThreads) select_dense_kernel(const float
     float mx = v[0];
 #pragma unroll
     for (int j = 1; j < kPer; ++j) mx = fmaxf(mx, v[j]);   // NaN scores never rank (torch would put them first; the reference has none)
-    const float tau_f = s_tau_f;
-    const u64 tau_key = s_tau_key;
+    const float tau_f = s_st.tau_f;
+    const u64 tau_key = s_st.tau_key;
     if (!__syncthreads_or(mx >= tau_f)) continue;
 #pragma unroll
     for (int j = 0; j < kPer; ++j) {
-      if (v[j] >= tau_f) {
-        const long long i = base + ((j >> 2) * kDenseThreads + tid) * 4 + (j & 3);
-        const u64 key = make_key(v[j], (u32)i);
-        if (key > tau_key) buf[atomicAdd(&s_cnt, 1)] = key;
-      }
+      const long long i = base + ((j >> 2) * kDenseThreads + tid) * 4 + (j & 3);
+      s_st.append(buf, v[j], (u32)i, tau_f, tau_key);
     }
     __syncthreads();
-    if (s_cnt > C - kDenseSlack) {  // uniform: read after the barrier; C >= 2 * k_row + slack
-      if (tid < 32) {
-        // one histogram pass first (a score threshold with >= k_row candidates at or above it is all the
-        // stream needs); the exact radix select only for tie-heavy or crowded buffers
-        u32 pivot_ord = 0u, j_ord = 0u;
-        int kept = 0;
-        const int n_now = s_cnt;
-        if (warp_prune_hist<false, 1>(buf, n_now, k_row, k_row, (k_row + C - kDenseSlack) / 2, smem_addr(s_hist), 0u,
-                                      &pivot_ord, &kept, &j_ord)) {
-          if (tid == 0) { s_cnt = kept; s_tau_key = 0ull; s_tau_f = unord32(pivot_ord); }
-        } else {
-          const u64 pivot = warp_prune(buf, n_now, k_row, smem_addr(s_hist), 0u);
-          if (tid == 0) { s_cnt = k_row; s_tau_key = pivot; s_tau_f = key_score(pivot); }
-        }
-      }
+    if (s_st.cnt > C - kDenseSlack) {  // uniform: read after the barrier; C >= 2 * k_row + slack
+      // one histogram pass first; the exact radix select only for tie-heavy or crowded buffers
+      if (tid < 32)
+        s_st.apply(warp_prune_stream<false, 1>(buf, s_st.cnt, k_row, k_row, (k_row + C - kDenseSlack) / 2,
+                                               smem_addr(s_st.hist), 0u));
     }
     __syncthreads();
   }
-  if (tid == 0) counts[(long long)row * S + split] = s_cnt;
+  if (tid == 0) counts[(long long)row * S + split] = s_st.cnt;
 }
 
 __global__ void __launch_bounds__(256) override_dense_kernel(const float* __restrict__ scores, long long ld, int B,

@@ -154,14 +154,9 @@ int launch_override_dense(const float* scores, long long ld, int B, long long N,
 // BM25 (ccr_kernels.cu)
 // block shape, measured at the NQ shape (profiles/r01_bm25_bench.json): 4096 docs x 256 threads x 5 blocks
 // per SM 45.3 ms per 3,452 queries; 8192 x 512 x 2: 56.7 ms; 4096 x 512 x 2: 70.9; 8192 x 256 x 3: 65.7
-#ifndef CCR_BM_CHUNK
-#define CCR_BM_CHUNK 4096
-#define CCR_BM_THREADS 256
-#define CCR_BM_BLOCKS_PER_SM 5
-#endif
-constexpr int kBmChunk = CCR_BM_CHUNK;     // docs per shared-memory accumulator pass (8 bytes each)
-constexpr int kBmThreads = CCR_BM_THREADS;
-constexpr int kBmBlocksPerSm = CCR_BM_BLOCKS_PER_SM;
+constexpr int kBmChunk = 4096;     // docs per shared-memory accumulator pass (8 bytes each)
+constexpr int kBmThreads = 256;
+constexpr int kBmBlocksPerSm = 5;
 constexpr int kBmMaxTerms = 512;   // distinct vocabulary terms per query
 constexpr int kBmSlack = 1024;     // accumulators ranked between two prune checks
 // warp-private variant: 8 independent warps per block, 512-doc mini-chunks, <= 32 distinct query terms
@@ -170,11 +165,8 @@ constexpr int kBmwMini = 512;
 constexpr int kBmwMaxTerms = 32;   // one lane per term
 constexpr int kBmwSketchM = 5;       // query bound = the 5th largest of the streams' ceil(k/5)-th best scores (7, 8: same speed)
 constexpr int kBmwDepth = 4;         // batches of 32 postings in flight per warp on a dense term
-#ifndef CCR_BMW_BLOCKS_PER_SM
-#define CCR_BMW_BLOCKS_PER_SM 4
-#endif
-constexpr int kBmwBlocksPerSm = CCR_BMW_BLOCKS_PER_SM;   // 42.5 KB of static shared memory per block; 64 registers per
-                                                         // thread (5 blocks = 48 registers spill: 46.7 vs 39.1 ms, r02_bm25.md)
+constexpr int kBmwBlocksPerSm = 4;   // 42.5 KB of static shared memory per block; 64 registers per
+                                     // thread (5 blocks = 48 registers spill: 46.7 vs 39.1 ms, r02_bm25.md)
 int launch_bm25_topk_warp(const long long* post_indptr, const int* post_docs, const double* post_val,
                           const int* head_slot, const double* head_rows, long long ld_head,
                           const long long* q_indptr, const int* q_terms, long long Bq, long long N, int k, int C, int S,

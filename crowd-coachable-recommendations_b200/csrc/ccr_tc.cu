@@ -337,18 +337,6 @@ static __device__ __noinline__ u32 sketch_bound(const u32* gq, int S_row, int m,
   return (u32)(warp_select_kth(SharedKeys{stage_s}, ns, m, hist_s) >> 32);
 }
 
-static __device__ __noinline__ u64 exact_prune(u64* b, int n, int k, int j, bool staged, u32 hist_s, u32 stage_s,
-                                               u32* j_ord) {
-  const u64 pivot = warp_prune(b, n, k, hist_s, staged ? stage_s : 0u);
-  if (j > 0) {
-    u64 kj;
-    if (staged) kj = warp_select_kth(SharedKeys{stage_s}, n, j, hist_s);
-    else kj = warp_select_kth(GlobalKeys{b}, k, j, hist_s);
-    *j_ord = (u32)(kj >> 32);
-  }
-  return pivot;
-}
-
 // Prune one stream's buffer (all 32 lanes cooperate), publish its share_j-th best, refresh the
 // row's shared bound.  Returns (kept << 32) | float bits of the stream's new threshold.
 static __device__ __noinline__ u64 prune_stream(u64* b, int n, int k, int C, int row_s, int stream_s, ShareArgs sh,
@@ -356,19 +344,17 @@ static __device__ __noinline__ u64 prune_stream(u64* b, int n, int k, int C, int
   const int lane = threadIdx.x & 31;
   const bool staged = C <= kStageKeys;
   const int jj = sh.share_j > 0 ? sh.share_j : k;
-  float new_tau;
-  int kept = k;
-  u32 j_ord = 0u, pivot_ord = 0u;
-  // fast path: one histogram pass; leaves between k and (k + C-128)/2 survivors
-  const bool fast =
-      staged ? warp_prune_hist<true, 1>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord)
-             : warp_prune_hist<false, 1>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s, &pivot_ord, &kept, &j_ord);
-  if (fast) {
-    new_tau = unord32(pivot_ord);  // ">=": every key at or above the pivot bucket was kept
-  } else {
-    const u64 pivot = exact_prune(b, n, k, sh.share_j, staged, hist_s, stage_s, &j_ord);
-    new_tau = next_up(key_score(pivot));
-    kept = k;
+  // histogram path: leaves between k and (k + C-128)/2 survivors
+  const PruneResult r =
+      staged ? warp_prune_stream<true, 1>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s)
+             : warp_prune_stream<false, 1>(b, n, k, jj, (k + C - 128) / 2, hist_s, stage_s);
+  // the stream visits item ids in ascending order: the exact pivot's key bound is a float bound
+  float new_tau = r.hist ? r.tau_f : next_up(r.tau_f);
+  u32 j_ord = r.j_ord;
+  if (!r.hist && sh.share_j > 0) {  // the staging area still holds all n keys; buf holds the top k
+    const u64 kj = staged ? warp_select_kth(SharedKeys{stage_s}, n, sh.share_j, hist_s)
+                          : warp_select_kth(GlobalKeys{b}, k, sh.share_j, hist_s);
+    j_ord = (u32)(kj >> 32);
   }
   if (sh.share_j > 0) {
     u32* gq = sh.g_q + (long long)row_s * sh.S_row;
@@ -379,7 +365,7 @@ static __device__ __noinline__ u64 prune_stream(u64* b, int n, int k, int C, int
       if (bound > ord32(new_tau)) new_tau = unord32(bound);
     }
   }
-  return ((u64)(u32)kept << 32) | (u64)__float_as_uint(new_tau);
+  return ((u64)(u32)r.kept << 32) | (u64)__float_as_uint(new_tau);
 }
 
 // Prune every stream of this warp whose buffer could overflow during the next half tile.  Runs
