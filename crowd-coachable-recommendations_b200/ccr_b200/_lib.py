@@ -51,6 +51,14 @@ EXPORTS = [
     "ccr_bm25_topk_workspace_bytes",
     "ccr_bm25_topk",
     "ccr_bm25_scores_f64",
+    "ccr_exact_k_candidates",
+    "ccr_exact_error_bound",
+    "ccr_score_topk_exact_workspace_bytes",
+    "ccr_score_topk_exact",
+    "ccr_ingest_rows_f32_f32",
+    "ccr_rerank_exact_workspace_bytes",
+    "ccr_rerank_exact",
+    "ccr_threshold_compact",
 ]
 
 _lib = None
@@ -136,6 +144,24 @@ def lib():
     L.ccr_bm25_head_row_pitch.argtypes = [i64]
     L.ccr_bm25_build_head_rows.restype = i32
     L.ccr_bm25_build_head_rows.argtypes = [vp, vp, vp, vp, i32, i64, i64, vp, vp, vp]
+    L.ccr_exact_k_candidates.restype = i32
+    L.ccr_exact_k_candidates.argtypes = [i64, i64, i32, i32, i32]
+    L.ccr_exact_error_bound.restype = f64
+    L.ccr_exact_error_bound.argtypes = [f64, f64, i32, i32]
+    L.ccr_score_topk_exact_workspace_bytes.restype = sz
+    L.ccr_score_topk_exact_workspace_bytes.argtypes = [i64, i64, i32, i32, i64, i64, i32]
+    L.ccr_score_topk_exact.restype = i32
+    L.ccr_score_topk_exact.argtypes = [vp, vp, i64, i64, vp, vp, i64, i64, i32, i32, vp, vp, vp, vp, i64, i64, i32,
+                                       i64, vp, vp, vp, vp, vp, vp, vp, sz, i32, vp]
+    L.ccr_ingest_rows_f32_f32.restype = i32
+    L.ccr_ingest_rows_f32_f32.argtypes = [vp, i64, i32, i64, vp, i64, i32, vp, vp]
+    L.ccr_rerank_exact_workspace_bytes.restype = sz
+    L.ccr_rerank_exact_workspace_bytes.argtypes = [i64, i64, i64]
+    L.ccr_rerank_exact.restype = i32
+    L.ccr_rerank_exact.argtypes = [vp, i64, i64, vp, i64, i64, i32, i32, vp, vp, i64, vp, vp, vp, i64, i32, i64,
+                                   vp, vp, vp, vp, sz, i32, vp]
+    L.ccr_threshold_compact.restype = i32
+    L.ccr_threshold_compact.argtypes = [vp, i64, i64, i64, vp, vp, vp, vp]
     if L.ccr_abi_version() != ABI_VERSION:
         raise RuntimeError("libccr_b200 ABI version mismatch")
     _lib = L
@@ -157,6 +183,14 @@ def plan_info(B, n_items, D, k, flags=0, mask_nnz=0, mask_max_row_nnz=-1):
     check(lib().ccr_plan_info(B, n_items, D, k, mask_nnz, mask_max_row_nnz, flags, arr))
     return {"n_q_tiles": arr[0], "n_splits": arr[1], "cand_capacity": arr[2], "algo": arr[3], "two_cta": arr[4],
             "seed_items": arr[5], "n_kernel_launches": arr[6], "lead_tiles": arr[7]}
+
+
+def exact_k_candidates(B, n_items, D, k, flags=0):
+    """k': candidates per row the scan stage of an exact search returns (the plan's rule, no GPU needed)."""
+    kc = lib().ccr_exact_k_candidates(B, n_items, D, k, flags)
+    if kc < 0:
+        check(kc)
+    return kc
 
 
 def reload_env():

@@ -238,7 +238,7 @@ def generate_train_data(qids, qrels, ranking_profile, ranking_profile_2, corpus_
 
 def rank_step(corpus, queries, qrels, embedding_func, results_dir, step, ranking_profile_bm25, qids_split,
               n_repeats=3, repeat_seed=42, number_of_qid_split_batch=None, block_dict=None, landing_image=None,
-              batch_size=512, device="cuda", table_dtype=torch.bfloat16):
+              batch_size=512, device="cuda", table_dtype=torch.bfloat16, exact=False):
     """al_0_rank.py:107-218 as a function: reuse or compute ``data_iteration_{step}/ranking_profile.pt``
     (the dense retrieval runs through ccr_b200.ranking on the device, on tables of ``table_dtype``:
     bf16 by default, fp16 to rank on the reference's own autocast operand format), report MRR, write
@@ -253,7 +253,7 @@ def rank_step(corpus, queries, qrels, embedding_func, results_dir, step, ranking
         ranking_profile = torch.load(profile_path)
     else:
         ranking_profile = ranking(corpus, queries, embedding_func, batch_size, block_dict, device=device,
-                                  table_dtype=table_dtype)
+                                  table_dtype=table_dtype, exact=exact)
         # the reference's file format is the plain dict (loadable with torch.load's weights-only default)
         torch.save(ranking_profile.to_dict() if hasattr(ranking_profile, "to_dict") else ranking_profile, profile_path)
     mrr = mrr_from_profile(qrels, ranking_profile, [1, 5, 10, 100])

@@ -24,8 +24,12 @@ def shard_bounds(n_items, world_size, rank):
 class ShardedIndex:
     """Each rank holds rows [lo, hi) of the global table in an EmbeddingTable with id_offset=lo."""
 
-    def __init__(self, n_items, dim=768, normalize=False, device=None, group=None, dtype=torch.bfloat16):
+    def __init__(self, n_items, dim=768, normalize=False, device=None, group=None, dtype=torch.bfloat16,
+                 exact=False):
         self.dtype = check_table_dtype(dtype)  # element type of the local table (bf16 or fp16)
+        # exact: local exact top-k (DESIGN.md section 6b), then the (float64, int64) pair exchange; an item's
+        # exact value does not depend on the shard that holds it, so the merge equals one exact table
+        self.exact = bool(exact)
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -36,7 +40,7 @@ class ShardedIndex:
 
     def _make_table(self, capacity, dim, normalize):
         return EmbeddingTable(capacity, dim, device=self.device, normalize=normalize, id_offset=self.lo,
-                              dtype=self.dtype)
+                              dtype=self.dtype, exact=self.exact)
 
     # ---- the device steps; CPU gloo tests replace them to exercise the plumbing ----
     def _local_topk(self, q_encoded, k, mask):
@@ -81,7 +85,8 @@ class ShardedIndex:
         the CSR already lives there (no host pass, no upload), else from the host arrays."""
         if mask is None:
             return None
-        if getattr(mask, "indptr", None) is not None and mask.indptr.is_cuda:
+        if getattr(mask, "indptr", None) is not None and mask.indptr.is_cuda and not (self.exact and mask.host is not None):
+            # (an exact search's fallback selects mask rows on the host, so it keeps the host copy)
             return mask.column_shard_device(self.lo, self.hi)
         return mask.column_shard(self.lo, self.hi)
 
@@ -95,7 +100,8 @@ class ShardedIndex:
         a, b = min(B, self.rank * per), min(B, (self.rank + 1) * per)
         part = self._encode(queries[a:b]) if b > a else None
         ld = part.shape[1] if part is not None else self._encode(queries[:1]).shape[1]
-        mine = torch.zeros((per, ld), dtype=self.dtype if part is None else part.dtype,
+        enc_dtype = torch.float32 if self.exact else self.dtype  # exact tables encode queries as fp32 rows
+        mine = torch.zeros((per, ld), dtype=enc_dtype if part is None else part.dtype,
                            device=self.device if part is None else part.device)
         if part is not None:
             mine[: b - a].copy_(part)
@@ -112,7 +118,7 @@ class ShardedIndex:
         """One all-gather of packed 8-byte (float32 score, uint32 id) keys is exact when the order is
         decided in float32: no mask, or SET values that are float32 numbers; ADD priors (float64
         sums) take the (float64, int64) pair exchange."""
-        return self.n_items <= (1 << 32) and (mask is None or mask.f32_exact)
+        return not self.exact and self.n_items <= (1 << 32) and (mask is None or mask.f32_exact)
 
     def search(self, queries, k, mask: engine.SparseMask | None = None, want_f64=False):
         """queries replicated on every rank; mask is the GLOBAL CSR (sharded here by column range).

@@ -191,6 +191,17 @@ class SparseMask:
         a, b = ip[start], ip[stop]
         return SparseMask(ip[start : stop + 1] - a, c[a:b], v[a:b], self.n_cols, self.mode, self.device)
 
+    def take_rows(self, rows):
+        """The CSR of the given rows (host int array), in that order."""
+        if self.host is None:
+            raise NotImplementedError("take_rows needs the host copy of the CSR")
+        ip, c, v = self.host
+        rows = np.asarray(rows, dtype=np.int64)
+        lengths = ip[rows + 1] - ip[rows]
+        new_ip = np.concatenate([[0], np.cumsum(lengths)]).astype(np.int64)
+        src = np.repeat(ip[rows] - new_ip[:-1], lengths) + np.arange(new_ip[-1], dtype=np.int64)
+        return SparseMask(new_ip, c[src], v[src], self.n_cols, self.mode, self.device)
+
     def column_shard_device(self, lo, hi):
         """column_shard on the device (C ABI: ccr_mask_column_shard): no host pass, no upload.  The
         shard's entry count stays on the device; nnz / max_row_nnz of the result are upper bounds."""
@@ -494,3 +505,143 @@ def score_dense(q, items, n_items=None, D=None):
         rc = fn(q.data_ptr(), B, ldq, items.data_ptr(), N, ldi, D, out.data_ptr(), N, _stream_ptr(q.device))
     _lib.check(rc)
     return out
+
+
+# ---- exact fp32 ranking (DESIGN.md section 6b) ----
+
+def exact_error_bound(q_norm, v_max, D, f16):
+    """Python mirror of ``exact_error_bound`` (csrc/ccr_common.cuh, exported as ccr_exact_error_bound): a
+    bound of |scan score - exact value| for a query of norm ``q_norm`` against a table whose largest fp32
+    row norm is ``v_max``.  Works elementwise on numpy arrays."""
+    u = 2.0 ** -11 if f16 else 2.0 ** -8
+    eta = 2.0 ** -25 if f16 else 2.0 ** -134
+    d = float(D)
+    qv = np.asarray(q_norm, dtype=np.float64) * v_max
+    under = (1.0 + u) * eta * np.sqrt(d) * (np.asarray(q_norm, dtype=np.float64) + v_max) + d * eta * eta
+    a = (1.0 + u) * (1.0 + u) * qv + under
+    e = (2.0 * u + u * u) * qv + under + d * 2.0 ** -22 * a + d * 2.0 ** -149 + (2.0 ** -24 + d * 2.0 ** -53) * qv
+    return e * (1.0 + 2.0 ** -20)
+
+
+# scan-score rows of the fallback are computed in blocks of at most this many bytes: every block streams the
+# whole scan table once, so larger blocks mean fewer passes (4 GB: ~120 rows per pass at 8.84 M items)
+EXACT_FALLBACK_BLOCK_BYTES = 4 << 30
+
+
+def ingest_rows_f32(src, dst, normalize=False, v_max=None):
+    """fp32 rows -> fp32 rows of an exact table (optional fp32 L2 normalisation, zeroed padding columns);
+    ``v_max`` (device float64 [1], optional) is raised to the largest stored row norm (rounded up)."""
+    _require_cuda(src, "src")
+    _require_cuda(dst, "dst")
+    if src.dtype != torch.float32 or dst.dtype != torch.float32 or src.stride(1) != 1 or dst.stride(1) != 1:
+        raise ValueError("src and dst must be float32 with a contiguous last dimension")
+    n, D = src.shape
+    if dst.shape[0] != n or dst.shape[1] < D or (n > 1 and dst.stride(0) != dst.shape[1]):
+        raise ValueError("dst must be dense rows [n, >= D]")
+    if v_max is not None and (v_max.dtype != torch.float64 or not v_max.is_cuda):
+        raise ValueError("v_max must be a device float64 tensor")
+    ld_src = src.stride(0) if n > 1 else max(src.stride(0), D)
+    ld_dst = dst.stride(0) if n > 1 else max(dst.stride(0), dst.shape[1])
+    with torch.cuda.device(src.device):
+        rc = _lib.lib().ccr_ingest_rows_f32_f32(src.data_ptr(), n, D, ld_src, dst.data_ptr(), ld_dst,
+                                                int(bool(normalize)), v_max.data_ptr() if v_max is not None else None,
+                                                _stream_ptr(src.device))
+    _lib.check(rc)
+    return dst
+
+
+def _rows_pitch(t):
+    return t.stride(0) if t.shape[0] > 1 else max(t.stride(0), t.shape[1])
+
+
+def score_topk_exact(q, q_scan, items, items_scan, k, v_max, mask: SparseMask | None = None, id_offset=0,
+                     algo=_lib.ALGO_AUTO, allow_short=False, n_items=None, D=None):
+    """Exact fp32 top-k (C ABI: ccr_score_topk_exact, then the fallback for uncertified rows).
+
+    q [B, ld] / items [N, ld] fp32 rows, q_scan / items_scan their bf16 or fp16 rounding (same pitch),
+    v_max the device float64 [1] largest fp32 row norm of items.  Returns (scores float32, ids int64,
+    values float64, number of rows that went through the fallback)."""
+    for t, name in ((q, "q"), (items, "items"), (q_scan, "q_scan"), (items_scan, "items_scan")):
+        _require_cuda(t, name)
+    f16 = _operand_f16(q_scan, items_scan)
+    if q.dtype != torch.float32 or items.dtype != torch.float32:
+        raise TypeError("q and items must be the float32 rows of an exact table")
+    if q.stride() != q_scan.stride() or items.stride() != items_scan.stride():
+        raise ValueError("the fp32 rows and their scan copies must share one row pitch")
+    dev = q.device
+    B = q.shape[0]
+    N = items.shape[0] if n_items is None else int(n_items)
+    D = q.shape[1] if D is None else int(D)
+    k = int(k)
+    ldq, ldi = _rows_pitch(q), _rows_pitch(items)
+    flags = int(algo) | (_lib.FLAG_ALLOW_SHORT if allow_short else 0) | (_lib.FLAG_F16 if f16 else 0)
+    if mask is not None and (mask.n_rows != B or mask.n_cols != N):
+        raise ValueError(f"mask shape ({mask.n_rows}, {mask.n_cols}) does not match ({B}, {N})")
+    nnz = mask.nnz if mask is not None else 0
+    hmax = mask.max_row_nnz if mask is not None else -1
+    out_s = torch.empty((B, k), dtype=torch.float32, device=dev)
+    out_i = torch.empty((B, k), dtype=torch.int64, device=dev)
+    out_d = torch.empty((B, k), dtype=torch.float64, device=dev)
+    uncert = torch.empty(B, dtype=torch.int32, device=dev)
+    tau = torch.empty(B, dtype=torch.float64, device=dev)
+    count = torch.zeros(1, dtype=torch.int32, device=dev)
+    L = _lib.lib()
+    _status()
+    mp = (lambda t: t.data_ptr() if mask is not None and nnz else None)
+    with torch.cuda.device(dev):
+        need = L.ccr_score_topk_exact_workspace_bytes(B, N, D, k, nnz, hmax, flags)
+        ws = workspace.get(dev, max(need, 256))
+        rc = L.ccr_score_topk_exact(
+            q.data_ptr(), q_scan.data_ptr(), B, ldq, items.data_ptr() if N else None,
+            items_scan.data_ptr() if N else None, N, ldi, D, k, v_max.data_ptr(),
+            mp(mask.indptr) if mask is not None else None, mp(mask.cols) if mask is not None else None,
+            mp(mask.vals) if mask is not None else None, nnz, hmax, mask.mode if mask is not None else MASK_NONE,
+            int(id_offset), out_s.data_ptr(), out_d.data_ptr(), out_i.data_ptr(), uncert.data_ptr(), tau.data_ptr(),
+            count.data_ptr(), ws.data_ptr(), ws.numel(), flags, _stream_ptr(dev))
+    _lib.check(rc)
+    n_fallback = int(count.item()) if B else 0
+    if n_fallback:
+        rows = torch.nonzero(uncert, as_tuple=True)[0]
+        block = max(1, min(65535, EXACT_FALLBACK_BLOCK_BYTES // (4 * max(N, 1))))
+        for r0 in range(0, rows.numel(), block):
+            r = rows[r0 : r0 + block]
+            s_r, i_r, d_r = _exact_fallback_rows(q[r], q_scan[r], items, items_scan, k, tau[r], mask, r, id_offset,
+                                                 allow_short, N, D)
+            out_s[r], out_i[r], out_d[r] = s_r, i_r, d_r
+    return out_s, out_i, out_d, n_fallback
+
+
+def _exact_fallback_rows(q, q_scan, items, items_scan, k, tau, mask, rows, id_offset, allow_short, N, D):
+    """The complete path of uncertified rows: dense scan scores, the columns at or above each row's tau,
+    exact re-rank of those and the row's mask entries."""
+    dev = q.device
+    R = q.shape[0]
+    L = _lib.lib()
+    scores = score_dense(q_scan, items_scan, n_items=N, D=D)
+    indptr = torch.empty(R + 1, dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(L.ccr_threshold_compact(scores.data_ptr(), R, N, N, tau.data_ptr(), indptr.data_ptr(), None,
+                                           _stream_ptr(dev)))
+        total = int(indptr[-1].item())
+        ids = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
+        _lib.check(L.ccr_threshold_compact(scores.data_ptr(), R, N, N, tau.data_ptr(), indptr.data_ptr(),
+                                           ids.data_ptr(), _stream_ptr(dev)))
+    del scores
+    sub = mask.take_rows(rows.cpu().numpy()) if mask is not None else None
+    nnz = sub.nnz if sub is not None else 0
+    out_s = torch.empty((R, k), dtype=torch.float32, device=dev)
+    out_i = torch.empty((R, k), dtype=torch.int64, device=dev)
+    out_d = torch.empty((R, k), dtype=torch.float64, device=dev)
+    mp = (lambda t: t.data_ptr() if sub is not None and nnz else None)
+    with torch.cuda.device(dev):
+        need = L.ccr_rerank_exact_workspace_bytes(R, total, nnz)
+        ws = workspace.get(dev, max(need, 256))
+        rc = L.ccr_rerank_exact(
+            q.data_ptr(), R, _rows_pitch(q), items.data_ptr() if N else None, N, _rows_pitch(items), D, k,
+            indptr.data_ptr(), ids.data_ptr(), total, mp(sub.indptr) if sub is not None else None,
+            mp(sub.cols) if sub is not None else None, mp(sub.vals) if sub is not None else None, nnz,
+            sub.mode if sub is not None else MASK_NONE, int(id_offset), out_s.data_ptr(), out_d.data_ptr(),
+            out_i.data_ptr(), ws.data_ptr(), ws.numel(), _lib.FLAG_ALLOW_SHORT if allow_short else 0,
+            _stream_ptr(dev))
+    _lib.check(rc)
+    return out_s, out_i, out_d

@@ -43,9 +43,9 @@ def evaluate_assigned(target_csr, assigned_csr, score_mat=None, axis=None, min_t
     return out
 
 
-def evaluate_item_rec(target_csr, score_mat, topk, device="cpu", **kw):
+def evaluate_item_rec(target_csr, score_mat, topk, device="cpu", exact=False, **kw):
     S = score_mat if isinstance(score_mat, LazyScoreBase) else auto_cast_lazy_score(score_mat)
-    res = topk_lazy(S, topk, want_scores=True)
+    res = topk_lazy(S, topk, want_scores=True, exact=exact)
     if res is None:
         _assign_topk(S, topk)  # raises the descriptive NotImplementedError
     ids, vals = res

@@ -57,8 +57,9 @@ def generate_embeddings(data_indices, data_dic, embedding_func, batch_size, embe
 
 
 def generate_embeddings_device(data_indices, data_dic, embedding_func, batch_size, normalize=False,
-                               device="cuda", id_offset=0, name=None, dtype=torch.bfloat16):
-    """Encoder batches -> device bf16 (or ``dtype``) table without the host round trip (SURVEY.md §8f-1)."""
+                               device="cuda", id_offset=0, name=None, dtype=torch.bfloat16, exact=False):
+    """Encoder batches -> device bf16 (or ``dtype``) table without the host round trip (SURVEY.md §8f-1);
+    ``exact``: the table also keeps the fp32 rows and searches rank exactly (DESIGN.md section 6b)."""
     check_table_dtype(dtype)
     table = None
     with torch.no_grad():
@@ -67,10 +68,11 @@ def generate_embeddings_device(data_indices, data_dic, embedding_func, batch_siz
             emb = torch.as_tensor(embedding_func([data_dic[i] for i in idx]))
             if table is None:
                 table = EmbeddingTable(len(data_indices), emb.shape[1], device=device, normalize=normalize,
-                                       id_offset=id_offset, dtype=dtype)
+                                       id_offset=id_offset, dtype=dtype, exact=exact)
             table.append(emb)
     if table is None:
-        table = EmbeddingTable(0, 768, device=device, normalize=normalize, id_offset=id_offset, dtype=dtype)
+        table = EmbeddingTable(0, 768, device=device, normalize=normalize, id_offset=id_offset, dtype=dtype,
+                               exact=exact)
     if name is not None:
         table.save(name)
     return table
@@ -148,24 +150,26 @@ def ranking_tensors(query_table, passage_table, k, mask=None, algo=0):
     for s in range(0, Q, QUERY_CHUNK):
         e = min(Q, s + QUERY_CHUNK)
         m = mask.rows(s, e) if mask is not None else None
-        sc, ids = passage_table.search(query_table.data[s:e], k, mask=m, algo=algo, encoded=True)
+        q = query_table.data32 if query_table.exact else query_table.data
+        sc, ids = passage_table.search(q[s:e], k, mask=m, algo=algo, encoded=True)
         scores[s:e] = sc.cpu().numpy()
         order[s:e] = ids.cpu().numpy()
     return scores, order
 
 
 def ranking(corpus, queries, embedding_func, batch_size, block_dict=None, device="cuda", algo=0,
-            table_dtype=torch.bfloat16):
+            table_dtype=torch.bfloat16, exact=False):
     """``table_dtype``: element type of the device tables, bf16 (default) or fp16 (the reference's
-    autocast operand format); scores are fp32 either way."""
+    autocast operand format); scores are fp32 either way.  ``exact``: rank by the exact fp32 scores of the
+    reference's CPU path (DESIGN.md section 6b); ``table_dtype`` is then the format of the scan copy."""
     check_table_dtype(table_dtype)
     sim = os.environ["CCREC_SIM_TYPE"]  # KeyError when unset, like ms_marco_eval.py:212
     normalize = sim == "cos"
     queries_ids, corpus_ids = list(queries.keys()), list(corpus.keys())
     q_table = generate_embeddings_device(queries_ids, queries, embedding_func, batch_size, normalize, device,
-                                         dtype=table_dtype)
+                                         dtype=table_dtype, exact=exact)
     p_table = generate_embeddings_device(corpus_ids, corpus, embedding_func, batch_size, normalize, device,
-                                         dtype=table_dtype)
+                                         dtype=table_dtype, exact=exact)
     if len(queries_ids) == 0:
         return {}
     mask = None
@@ -210,13 +214,14 @@ def mrr_at_k(order, corpus_ids, queries_ids, qrels, k_values=(1, 5, 10, 100), de
 
 
 def ranking_sharded(corpus, queries, embedding_func, batch_size, block_dict=None, group=None, device=None,
-                    index_cls=None, table_dtype=torch.bfloat16):
+                    index_cls=None, table_dtype=torch.bfloat16, exact=False):
     """``ranking`` with the passage table row-sharded over the ranks of a torch.distributed group
     (one process per GPU): every rank encodes the queries and ONLY its own contiguous slice of the
     corpus (``shard_bounds``) straight into its device shard -- the encoder pass, which dominates the
     reference's wall clock, is split G ways and no rank ever holds the whole table -- then the
     fused local top-k, one all-gather and the G-way merge produce the global result.  Every rank
-    returns the same ``{qid: {pid: score}}`` as the single-table call (``table_dtype`` as in ``ranking``)."""
+    returns the same ``{qid: {pid: score}}`` as the single-table call (``table_dtype`` and ``exact`` as in
+    ``ranking``)."""
     from .dist import ShardedIndex
 
     check_table_dtype(table_dtype)
@@ -229,7 +234,7 @@ def ranking_sharded(corpus, queries, embedding_func, batch_size, block_dict=None
         q_emb = torch.cat([torch.as_tensor(embedding_func([queries[i] for i in queries_ids[s:s + batch_size]]))
                            for s in range(0, len(queries_ids), batch_size)])
         index = (index_cls or ShardedIndex)(len(corpus_ids), q_emb.shape[1], normalize=normalize, device=device,
-                                            group=group, dtype=table_dtype)
+                                            group=group, dtype=table_dtype, exact=exact)
         for s in range(index.lo, index.hi, batch_size):
             e = min(index.hi, s + batch_size)
             index.add_local(torch.as_tensor(embedding_func([corpus[i] for i in corpus_ids[s:e]])))

@@ -24,14 +24,26 @@ from .table import EmbeddingTable
 ROW_CHUNK = 8192
 
 
-def _device_table_for(right):
+def _device_table_for(right, exact=False):
     """bf16 device table for the right factor ([D, N] LazyDenseMatrix), cached on the leaf so the
-    row-batch slices of one expression (which share ``right``) upload it once."""
-    t = getattr(right, "_ccr_table", None)
+    row-batch slices of one expression (which share ``right``) upload it once.  ``exact``: an exact
+    table (fp32 rows + scan copy, DESIGN.md section 6b), cached apart from the bf16 one.  Its scan copy is
+    fp16, which needs far fewer candidates than bf16 for the same certified share, unless the factor
+    holds values that fp16 cannot represent; the ranking is exact either way."""
+    attr = "_ccr_table_exact" if exact else "_ccr_table"
+    t = getattr(right, attr, None)
     if t is None:
-        t = EmbeddingTable.from_tensor(torch.as_tensor(np.ascontiguousarray(right.c.T)))
-        right._ccr_table = t
+        rows = torch.as_tensor(np.ascontiguousarray(right.c.T))
+        if exact:
+            big = rows.numel() and not bool(torch.isfinite(rows).all() and rows.abs().max() < EXACT_F16_LIMIT)
+            t = EmbeddingTable.from_tensor(rows, dtype=torch.bfloat16 if big else torch.float16, exact=True)
+        else:
+            t = EmbeddingTable.from_tensor(rows)
+        setattr(right, attr, t)
     return t
+
+
+EXACT_F16_LIMIT = 32768.0  # factor values at or above this take a bf16 scan copy (fp16 overflows at 65520)
 
 
 DENSE_CHUNK_ELEMS = 1 << 27  # dense score elements ranked per device pass (1 GB of float64)
@@ -83,9 +95,11 @@ def _topk_materialised(plan, k, want_scores):
     return (ids, vals) if want_scores else ids
 
 
-def topk_lazy(S, k, want_scores=False, algo=0):
+def topk_lazy(S, k, want_scores=False, algo=0, exact=False):
     """(ids [B,k] int64 numpy[, scores64 [B,k]]) for a fused-plan expression (factor pair: the
-    fused kernel) or a materialised dense matrix (+ priors); None if S is neither."""
+    fused kernel) or a materialised dense matrix (+ priors); None if S is neither.  ``exact``: a factor
+    pair is ranked by its exact fp32 scores (DESIGN.md section 6b); a materialised matrix is already
+    ranked exactly by its given values, so there it changes nothing."""
     plan = fused_plan(S)
     if plan is None:
         dplan = dense_plan(S)
@@ -93,7 +107,7 @@ def topk_lazy(S, k, want_scores=False, algo=0):
     B, N = plan.shape
     if k > N:
         raise RuntimeError("selected index k out of range")
-    table = _device_table_for(plan.right)
+    table = _device_table_for(plan.right, exact=exact)
     U = torch.as_tensor(np.ascontiguousarray(plan.left.c))
     ids = np.empty((B, k), dtype=np.int64)
     vals = np.empty((B, k), dtype=np.float64) if want_scores else None
@@ -110,11 +124,12 @@ def topk_lazy(S, k, want_scores=False, algo=0):
     return (ids, vals) if want_scores else ids
 
 
-def _assign_topk(S, k, tie_breaker=1e-10, device="cpu", batch_size=None):
-    """Return a sparse matrix where each row contains k non-zero values (see module docstring)."""
+def _assign_topk(S, k, tie_breaker=1e-10, device="cpu", batch_size=None, exact=False):
+    """Return a sparse matrix where each row contains k non-zero values (see module docstring);
+    ``exact`` ranks a factor pair by its exact fp32 scores (``topk_lazy``)."""
     if not isinstance(S, LazyScoreBase):
         S = auto_cast_lazy_score(S)
-    indices = topk_lazy(S, k)
+    indices = topk_lazy(S, k, exact=exact)
     if indices is None:
         raise NotImplementedError(
             f"_assign_topk: expression {S!r} is outside the accelerated score-and-rank path "

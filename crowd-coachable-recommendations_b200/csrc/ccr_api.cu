@@ -20,7 +20,7 @@ static thread_local cudaEvent_t g_prof_start = nullptr, g_prof_stop = nullptr;  
 // test that changes it inside a live process calls ccr_debug_reload_env().  None is needed in production.
 namespace {
 struct Knobs {
-  int two_cta = -1, lead = 0, no_hist = 0, bm25_blockwide = 0;
+  int two_cta = -1, lead = 0, no_hist = 0, bm25_blockwide = 0, exact_fallback = 0;
 };
 Knobs g_knobs;
 std::once_flag g_knobs_once;
@@ -32,6 +32,7 @@ void load_knobs() {
   k.lead = env_int("CCR_LEAD", 0);
   k.no_hist = getenv("CCR_NO_HIST") != nullptr;
   k.bm25_blockwide = getenv("CCR_BM25_BLOCKWIDE") != nullptr;
+  k.exact_fallback = env_int("CCR_EXACT_FALLBACK", 0) != 0;
   g_knobs = k;
 }
 const Knobs& knobs() {
@@ -83,6 +84,7 @@ struct Plan {
   int lead_tiles;        // throttle: max lead (item tiles) of a producer over its slowest peer
   int lead_every;        // throttle: progress is published / checked every lead_every tiles (power of two)
   int throttle_poller;   // throttle: 1 a dedicated warp watches the peers, 0 the producer polls inline
+  int k_cand;            // exact ranking: candidates the scan stage returns per row (k' >= k, <= n_items)
   size_t off_seed;
   size_t off_progress;
   size_t off_qpad;       // zero-padded copy of a short query batch (B < 128): every TMA box in bounds
@@ -117,6 +119,17 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
   const int sms = device_sm_count();
   const Knobs& kn = knobs();
   pl->algo = algo;
+  {
+    // Exact ranking (DESIGN.md section 6b): a row is certified when its k-th exact value beats the scan
+    // score of the k'-th candidate by the error bound E of the scan format.  E is ~8x smaller for fp16
+    // (u = 2^-11) than for bf16 (2^-8), so fp16 needs far fewer extra candidates for the same share of
+    // certified rows.  See DESIGN.md section 6b for the measured shares behind the two rules.
+    long long kc = (flags & CCR_FLAG_F16) ? k + k / 4 + 32 : 3LL * k + 32;
+    if (kc > CCR_MAX_K) kc = CCR_MAX_K;
+    if (kc < k) kc = k;
+    if (kc > n_items) kc = n_items;
+    pl->k_cand = (int)kc;
+  }
   pl->include_mask = (algo == CCR_ALGO_TCGEN05 && nnz > 0 && h_max >= 0 && h_max <= 256 && k + h_max <= CCR_MAX_K) ? 1 : 0;
   pl->k_keep = pl->include_mask ? (int)(k + h_max) : k;
   if (algo == CCR_ALGO_TCGEN05) {
@@ -821,6 +834,203 @@ int ccr_bm25_scores_f64(const int64_t* post_indptr, const int32_t* post_docs, co
                                    ccr_bm25_head_row_pitch(n_docs), (const long long*)q_indptr, q_terms,
                                    Bq, n_docs, 1, pl.C, pl.S, nullptr, nullptr, scores, ld, (cudaStream_t)stream);
   if (lr) return fail(CCR_ECUDA, "bm25 scores launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+  return CCR_OK;
+}
+
+}  // extern "C"
+
+// ---- exact fp32 ranking (DESIGN.md section 6b) ----
+namespace {
+struct ExactLayout { size_t off_scores, off_ids, off_neg, off_ent_ip, off_hi, off_lo, total; };
+
+// entry records after `off`: B + 1 row offsets, then 12 bytes per entry
+void entry_layout(size_t off, long long B, long long n_entries, ExactLayout* L) {
+  L->off_ent_ip = off; off = align_up(off + (size_t)(B + 1) * sizeof(long long), 256);
+  L->off_hi = off;     off = align_up(off + (size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u64), 256);
+  L->off_lo = off;     off = align_up(off + (size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u32), 256);
+  L->total = off;
+}
+
+// stage-1 workspace, its [B, k'] outputs, the -inf values of its SET mask, the entry records
+void exact_layout(const Plan& pl1, long long B, int kc, long long nnz, ExactLayout* L) {
+  size_t off = align_up(pl1.total, 256);
+  L->off_scores = off; off = align_up(off + (size_t)B * kc * sizeof(float), 256);
+  L->off_ids = off;    off = align_up(off + (size_t)B * kc * sizeof(long long), 256);
+  L->off_neg = off;    off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(double), 256);
+  entry_layout(off, B, B * (long long)kc + (nnz > 0 ? nnz : 0), L);
+}
+
+int check_exact_rows(const void* q, int64_t ldq, const void* items, int64_t ldi, int D) {
+  if (ldq < D || ldi < D || ldq % 8 || ldi % 8) return fail(CCR_EINVAL, "ldq/ldi must be >= D and multiples of 8");
+  if (((uintptr_t)q & 15) || ((uintptr_t)items & 15)) return fail(CCR_EINVAL, "q/items must be 16-byte aligned");
+  return CCR_OK;
+}
+
+// entry records of (candidates U mask entries) -> exact values -> finalize_kernel with no stream candidates
+int rerank(const float* q, long long B, long long ldq, const float* items, long long n_items, long long ldi, int D,
+           int k, const long long* cand_indptr, const long long* cand_ids, long long cand_stride, long long cand_nnz,
+           const long long* mask_indptr, const int* mask_cols, const double* mask_vals, long long nnz, int mode,
+           long long id_offset, float* out_scores, double* out_scores64, long long* out_ids, unsigned char* ws,
+           const ExactLayout& L, cudaStream_t st) {
+  ExactParams ep = {};
+  ep.q = q; ep.ldq = ldq; ep.B = (int)B; ep.items = items; ep.ldi = ldi; ep.n_items = n_items; ep.D = D;
+  ep.cand_indptr = cand_indptr; ep.cand_ids = cand_ids; ep.cand_stride = cand_stride;
+  ep.mask_indptr = nnz > 0 ? mask_indptr : nullptr; ep.mask_cols = mask_cols; ep.mask_vals = mask_vals; ep.mode = mode;
+  ep.ent_indptr = (const long long*)(ws + L.off_ent_ip); ep.max_entries = cand_nnz + (nnz > 0 ? nnz : 0);
+  ep.ent_hi = (u64*)(ws + L.off_hi); ep.ent_lo = (u32*)(ws + L.off_lo);
+  int lr = launch_exact_entries(ep, st);
+  if (lr) return fail(CCR_ECUDA, "exact value kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+  FinalizeParams fp = {};
+  fp.B = (int)B; fp.k = k; fp.C = 0; fp.S = 0; fp.cand = nullptr; fp.counts = nullptr; fp.g_tau = nullptr;
+  fp.drop_cols = nullptr; fp.mask_indptr = ep.ent_indptr; fp.ovr_hi = ep.ent_hi; fp.ovr_lo = ep.ent_lo;
+  fp.id_offset = id_offset; fp.out_scores = out_scores; fp.out_scores64 = out_scores64; fp.out_keys = nullptr;
+  fp.out_ids = out_ids;
+  lr = launch_finalize(fp, st);
+  if (lr) return fail(CCR_ECUDA, "finalize launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+  return CCR_OK;
+}
+
+int check_exact_mask(int mask_mode, const int64_t* mask_indptr, const int32_t* mask_cols, const double* mask_vals,
+                     int64_t mask_nnz, bool* has_mask) {
+  if (mask_mode != CCR_MASK_NONE && mask_mode != CCR_MASK_SET && mask_mode != CCR_MASK_ADD)
+    return fail(CCR_EINVAL, "bad mask_mode %d", mask_mode);
+  *has_mask = mask_mode != CCR_MASK_NONE && mask_indptr != nullptr && mask_nnz > 0;
+  if (*has_mask && (!mask_cols || !mask_vals)) return fail(CCR_EINVAL, "mask_cols / mask_vals null");
+  if (mask_nnz < 0) return fail(CCR_EINVAL, "mask_nnz = %lld", (long long)mask_nnz);
+  return CCR_OK;
+}
+}  // namespace
+
+extern "C" {
+
+double ccr_exact_error_bound(double q_norm, double max_row_norm, int D, int flags) {
+  return exact_error_bound(q_norm, max_row_norm, D, (flags & CCR_FLAG_F16) ? 1 : 0);
+}
+
+int ccr_exact_k_candidates(int64_t B, int64_t n_items, int D, int k, int flags) {
+  int rc = check_shape(B, n_items, D, k, flags | CCR_FLAG_ALLOW_SHORT);
+  if (rc) return rc;
+  Plan pl;
+  make_plan(B, n_items, D, k, 0, -1, flags, &pl);
+  return pl.k_cand;
+}
+
+int ccr_ingest_rows_f32_f32(const float* src, int64_t n, int D, int64_t ld_src, float* dst, int64_t ld_dst,
+                            int normalize, double* max_row_norm, void* stream) {
+  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad ingest shape");
+  if (n == 0) return CCR_OK;
+  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
+  cudaStream_t st = (cudaStream_t)stream;
+  int lr = launch_ingest_f32_f32(src, n, D, ld_src, dst, ld_dst, normalize, st);
+  if (!lr && max_row_norm) lr = launch_row_norm_max(dst, n, D, ld_dst, max_row_norm, st);
+  if (lr) return fail(CCR_ECUDA, "ingest kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+  return CCR_OK;
+}
+
+size_t ccr_score_topk_exact_workspace_bytes(int64_t B, int64_t n_items, int D, int k, int64_t mask_nnz,
+                                            int64_t mask_max_row_nnz, int flags) {
+  if (check_shape(B, n_items, D, k, flags | CCR_FLAG_ALLOW_SHORT) != CCR_OK || mask_nnz < 0) return 0;
+  Plan pl0, pl1;
+  make_plan(B, n_items, D, k, 0, -1, flags, &pl0);
+  pl1.total = 0;
+  if (pl0.k_cand > 0) make_plan(B, n_items, D, pl0.k_cand, mask_nnz, mask_nnz > 0 ? mask_max_row_nnz : -1, flags, &pl1);
+  ExactLayout L;
+  exact_layout(pl1, B, pl0.k_cand, mask_nnz, &L);
+  return L.total;
+}
+
+int ccr_score_topk_exact(const float* q, const void* q_scan, int64_t B, int64_t ldq, const float* items,
+                         const void* items_scan, int64_t n_items, int64_t ldi, int D, int k,
+                         const double* max_row_norm, const int64_t* mask_indptr, const int32_t* mask_cols,
+                         const double* mask_vals, int64_t mask_nnz, int64_t mask_max_row_nnz, int mask_mode,
+                         int64_t id_offset, float* out_scores, double* out_scores64, int64_t* out_ids,
+                         int32_t* out_uncertified, double* out_tau, int32_t* uncertified_count, void* workspace,
+                         size_t workspace_bytes, int flags, void* stream) {
+  int rc = check_shape(B, n_items, D, k, flags);
+  if (rc) return rc;
+  if (flags & CCR_FLAG_PACKED_KEYS) return fail(CCR_EINVAL, "exact ranking returns float64 values, not packed keys");
+  if (B == 0) return CCR_OK;
+  if (!q || !q_scan || !out_ids || !out_scores64 || !out_uncertified || !out_tau || !uncertified_count || !max_row_norm)
+    return fail(CCR_EINVAL, "null q / q_scan / out_ids / out_scores64 / certificate outputs / max_row_norm");
+  if (n_items > 0 && (!items || !items_scan)) return fail(CCR_EINVAL, "null items");
+  if ((rc = check_exact_rows(q, ldq, items, ldi, D)) || (rc = check_exact_rows(q_scan, ldq, items_scan, ldi, D))) return rc;
+  bool has_mask;
+  if ((rc = check_exact_mask(mask_mode, mask_indptr, mask_cols, mask_vals, mask_nnz, &has_mask))) return rc;
+  const long long nnz = has_mask ? mask_nnz : 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  Plan pl0, pl1;
+  make_plan(B, n_items, D, k, 0, -1, flags, &pl0);
+  const int kc = pl0.k_cand;
+  pl1.total = 0;
+  if (kc > 0) make_plan(B, n_items, D, kc, nnz, nnz > 0 ? mask_max_row_nnz : -1, flags, &pl1);
+  ExactLayout L;
+  exact_layout(pl1, B, kc, nnz, &L);
+  if (!workspace || workspace_bytes < L.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, L.total);
+  unsigned char* ws = (unsigned char*)workspace;
+  float* s1_scores = (float*)(ws + L.off_scores);
+  long long* s1_ids = (long long*)(ws + L.off_ids);
+  if (kc > 0) {
+    // stage 1: the unchanged scan on the scan copies, every mask entry ranked last (SET -inf) so that none
+    // takes a candidate slot; the re-rank below gives each its true value
+    double* neg = (double*)(ws + L.off_neg);
+    int lr = launch_fill_f64(neg, nnz, -INFINITY, st);
+    if (lr) return fail(CCR_ECUDA, "fill launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+    rc = ccr_score_topk_bf16(q_scan, B, ldq, items_scan, n_items, ldi, D, kc, has_mask ? mask_indptr : nullptr,
+                             has_mask ? mask_cols : nullptr, has_mask ? neg : nullptr, nnz,
+                             nnz > 0 ? mask_max_row_nnz : -1, has_mask ? CCR_MASK_SET : CCR_MASK_NONE, 0, s1_scores,
+                             nullptr, (int64_t*)s1_ids, ws, pl1.total, flags & (CCR_ALGO_MASK | CCR_FLAG_F16), stream);
+    if (rc) return rc;
+  }
+  rc = rerank(q, B, ldq, items, n_items, ldi, D, k, nullptr, s1_ids, kc, B * (long long)kc,
+              (const long long*)mask_indptr, mask_cols, mask_vals, nnz, mask_mode, id_offset, out_scores, out_scores64,
+              (long long*)out_ids, ws, L, st);
+  if (rc) return rc;
+  int lr = launch_exact_certify(q, ldq, (int)B, D, (flags & CCR_FLAG_F16) ? 1 : 0, max_row_norm, k, kc, n_items,
+                                s1_scores, s1_ids, has_mask ? (const long long*)mask_indptr : nullptr, mask_cols,
+                                out_scores64, knobs().exact_fallback, out_uncertified, out_tau, uncertified_count, st);
+  if (lr) return fail(CCR_ECUDA, "certify kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+  return CCR_OK;
+}
+
+size_t ccr_rerank_exact_workspace_bytes(int64_t B, int64_t cand_nnz, int64_t mask_nnz) {
+  if (B < 0 || cand_nnz < 0 || mask_nnz < 0) return 0;
+  ExactLayout L;
+  entry_layout(0, B, cand_nnz + mask_nnz, &L);
+  return L.total;
+}
+
+int ccr_rerank_exact(const float* q, int64_t B, int64_t ldq, const float* items, int64_t n_items, int64_t ldi, int D,
+                     int k, const int64_t* cand_indptr, const int64_t* cand_ids, int64_t cand_nnz,
+                     const int64_t* mask_indptr, const int32_t* mask_cols, const double* mask_vals, int64_t mask_nnz,
+                     int mask_mode, int64_t id_offset, float* out_scores, double* out_scores64, int64_t* out_ids,
+                     void* workspace, size_t workspace_bytes, int flags, void* stream) {
+  int rc = check_shape(B, n_items, D, k, flags);
+  if (rc) return rc;
+  if (B > 0x7fffffff) return fail(CCR_EUNSUPPORTED, "B=%lld", (long long)B);
+  if (B == 0) return CCR_OK;
+  if (!q || !out_ids || !cand_indptr || (cand_nnz > 0 && !cand_ids)) return fail(CCR_EINVAL, "null q / out_ids / candidates");
+  if (cand_nnz < 0) return fail(CCR_EINVAL, "cand_nnz = %lld", (long long)cand_nnz);
+  if (n_items > 0 && !items) return fail(CCR_EINVAL, "null items");
+  if ((rc = check_exact_rows(q, ldq, items, ldi, D))) return rc;
+  bool has_mask;
+  if ((rc = check_exact_mask(mask_mode, mask_indptr, mask_cols, mask_vals, mask_nnz, &has_mask))) return rc;
+  const long long nnz = has_mask ? mask_nnz : 0;
+  ExactLayout L;
+  entry_layout(0, B, cand_nnz + nnz, &L);
+  if (!workspace || workspace_bytes < L.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, L.total);
+  return rerank(q, B, ldq, items, n_items, ldi, D, k, (const long long*)cand_indptr, (const long long*)cand_ids, 0,
+                cand_nnz, (const long long*)mask_indptr, mask_cols, mask_vals, nnz, mask_mode, id_offset, out_scores,
+                out_scores64, (long long*)out_ids, (unsigned char*)workspace, L, (cudaStream_t)stream);
+}
+
+int ccr_threshold_compact(const float* scores, int64_t R, int64_t N, int64_t ld, const double* tau,
+                          int64_t* out_indptr, int64_t* out_ids, void* stream) {
+  if (R < 0 || N < 0 || ld < N) return fail(CCR_EINVAL, "bad compaction shape");
+  if (R == 0) return CCR_OK;
+  if (!tau || !out_indptr || (N > 0 && !scores)) return fail(CCR_EINVAL, "null pointer");
+  int lr = launch_threshold_compact(scores, R, N, ld, tau, (long long*)out_indptr, (long long*)out_ids,
+                                    (cudaStream_t)stream);
+  if (lr) return fail(CCR_ECUDA, "compaction launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   return CCR_OK;
 }
 

@@ -424,6 +424,35 @@ template <> struct Elem<__half> {
   static __device__ __forceinline__ float to_float(__half v) { return __half2float(v); }
   static __device__ __forceinline__ __half from_float(float v) { return __float2half_rn(v); }
 };
+// fp32 rows of an exact table (ingest only)
+template <> struct Elem<float> {
+  static __device__ __forceinline__ float to_float(float v) { return v; }
+  static __device__ __forceinline__ float from_float(float v) { return v; }
+};
+
+// Exact ranking (DESIGN.md section 6b): a bound E on |s^ - s| for one query row, where s^ is the fp32
+// score any scan kernel computes from the scan-format copies (bf16, or fp16 when f16) of the fp32 rows q
+// and v, and s = fp32(sum q_i v_i summed in float64) is the exact value.  q_norm = ||q||_2, v_max = the
+// largest ||v||_2 of the table (both of the fp32 rows, rounded up).  Terms, with u the unit roundoff of
+// the scan format and eta its largest absolute rounding error below the normal range (gradual underflow):
+//   operand rounding        (2u + u^2) ||q|| V + (1 + u) eta sqrt(D) (||q|| + V) + D eta^2
+//   fp32 accumulation       D 2^-22 A, A >= sum |q^_i v^_i|: ASSUMED for the tensor cores (undocumented;
+//                           4x the round-to-nearest bound D 2^-24 of the CUDA-core kernels)
+//   fp32 underflow          D 2^-149 (bf16 products and partial sums below fp32's normal range)
+//   rounding of s itself    (2^-24 + D 2^-53) ||q|| V
+// times (1 + 2^-20) for the round-to-nearest arithmetic of this function.  The one implementation: the
+// certify kernel calls it, ccr_exact_error_bound exports it, ccr_b200.engine.exact_error_bound mirrors
+// it for the tests.
+__host__ __device__ inline double exact_error_bound(double q_norm, double v_max, int D, int f16) {
+  const double u = f16 ? 0x1p-11 : 0x1p-8;
+  const double eta = f16 ? 0x1p-25 : 0x1p-134;
+  const double d = (double)D;
+  const double qv = q_norm * v_max;
+  const double under = (1.0 + u) * eta * sqrt(d) * (q_norm + v_max) + d * eta * eta;
+  const double a = (1.0 + u) * (1.0 + u) * qv + under;
+  const double e = (2.0 * u + u * u) * qv + under + d * 0x1p-22 * a + d * 0x1p-149 + (0x1p-24 + d * 0x1p-53) * qv;
+  return e * (1.0 + 0x1p-20);
+}
 
 // error slots written by device-side watchdogs (workspace tail)
 struct DeviceStatus {

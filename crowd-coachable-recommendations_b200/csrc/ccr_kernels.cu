@@ -763,6 +763,13 @@ int launch_ingest_f32_f16(const float* src, long long n, int D, long long ld_src
                                                                        overflow_count);
   return (int)cudaGetLastError();
 }
+int launch_ingest_f32_f32(const float* src, long long n, int D, long long ld_src, float* dst, long long ld_dst,
+                          int normalize, cudaStream_t st) {
+  if (n == 0) return 0;
+  ingest_kernel<float, float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, normalize,
+                                                                      nullptr);
+  return (int)cudaGetLastError();
+}
 int launch_normalize_f16(const __half* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
                          cudaStream_t st) {
   if (n == 0) return 0;

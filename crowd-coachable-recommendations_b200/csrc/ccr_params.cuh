@@ -135,6 +135,43 @@ int launch_normalize_f16(const __half* src, long long n, int D, long long ld_src
 int launch_dense_f32_f16(const __half* q, long long B, long long ldq, const __half* items, long long n, long long ldi,
                          int D, float* out, long long ld_out, cudaStream_t st);
 
+// exact tables: fp32 rows (ingest_kernel<float, float>, ccr_kernels.cu) and the exact ranking stages (ccr_exact.cu)
+int launch_ingest_f32_f32(const float* src, long long n, int D, long long ld_src, float* dst, long long ld_dst,
+                          int normalize, cudaStream_t st);
+struct ExactParams {
+  const float* q;        // fp32 query rows [B, ldq]
+  long long ldq;
+  int B;
+  const float* items;    // fp32 table rows [n_items, ldi]
+  long long ldi;
+  long long n_items;
+  int D;
+  // candidates of row r: cand_ids[c(r) .. c(r+1)), c(r) = cand_indptr[r], or r * cand_stride when
+  // cand_indptr is null (the dense [B, k'] ids of the scan stage); ids < 0 or inside the row's mask are
+  // skipped (the mask entry carries the value)
+  const long long* cand_indptr;
+  const long long* cand_ids;
+  long long cand_stride;
+  const long long* mask_indptr;  // null: no mask
+  const int* mask_cols;
+  const double* mask_vals;
+  int mode;
+  const long long* ent_indptr;   // [B+1]: c(r) + m(r), the entry CSR finalize reads as its override CSR
+  long long max_entries;         // upper bound of ent_indptr[B]
+  u64* ent_hi;                   // finalize's 96-bit records: ord64(value) (0 = skipped), ~id
+  u32* ent_lo;
+};
+int launch_exact_entries(const ExactParams& p, cudaStream_t st);
+int launch_row_norm_max(const float* rows, long long n, int D, long long ld, double* v_max, cudaStream_t st);
+int launch_fill_f64(double* dst, long long n, double v, cudaStream_t st);
+// per row: certified (0) or not (1), tau = RD(L_k - E); uncertified rows are added to *count
+int launch_exact_certify(const float* q, long long ldq, int B, int D, int f16, const double* v_max, int k, int k_cand,
+                         long long n_items, const float* s1_scores, const long long* s1_ids, const long long* mask_indptr,
+                         const int* mask_cols, const double* out_scores64, int force_fallback, int* uncert,
+                         double* tau, int* count, cudaStream_t st);
+int launch_threshold_compact(const float* scores, long long R, long long N, long long ld, const double* tau,
+                             long long* indptr, long long* ids, cudaStream_t st);
+
 // whole-matrix argsort and MRR first-hit scan (ccr_sort.cu)
 size_t argsort_workspace_bytes(long long n);
 int launch_argsort(const float* scores, long long B, long long N, long long ld, const long long* indptr, const int* cols,

@@ -293,6 +293,70 @@ int ccr_bm25_scores_f64(const int64_t* post_indptr, const int32_t* post_docs, co
                         const int32_t* q_terms, int64_t max_query_terms, int64_t Bq,
                         int64_t n_docs, double* scores, int64_t ld, void* stream);
 
+/*
+ * Exact fp32 ranking (DESIGN.md section 6b).  An exact table keeps its fp32 rows (ccr_ingest_rows_f32_f32)
+ * and a scan copy: the bf16 / fp16 rounding of those stored rows (ccr_ingest_rows_f32 /
+ * ccr_ingest_rows_f32_f16 with normalize = 0); queries likewise.  A row is ranked by the exact value of
+ * each item:
+ *   unmasked item      fp32(sum q_i * v_i), the fp32 rows multiplied and summed in float64 in an order that
+ *                      depends on D only (products of two fp32 values are exact in float64, so this is
+ *                      the correctly rounded fp32 score but for rare double roundings)
+ *   CCR_MASK_SET entry the mask value
+ *   CCR_MASK_ADD entry double(score) + value (the reference's float64 promotion)
+ * descending, ties -> lowest id.  The value depends on (query row, item row) only: not on the launch plan,
+ * the test levers, the path an item took or the table's sharding.
+ *
+ * ccr_score_topk_exact: the unchanged scan (ccr_score_topk_bf16 with these flags' algo / CCR_FLAG_F16 on
+ * q_scan / items_scan, masked items ranked last) returns k' = ccr_exact_k_candidates(...) candidates per
+ * row; they and the row's mask entries are re-scored exactly from q / items and the best k written out.
+ * The row is CERTIFIED when the scan returned every unmasked item, or when its k-th exact value L_k
+ * exceeds RU(t + E) strictly (t: scan score of the k'-th candidate, an upper bound of every item left
+ * out; E = ccr_exact_error_bound(||q||, max_row_norm, D, flags), a bound of |scan score - exact value|).
+ * Otherwise out_uncertified[row] = 1, out_tau[row] = RD(L_k - E) and *uncertified_count (device int32,
+ * ADDED to) counts it: every item whose exact value reaches L_k has a scan score >= out_tau[row], so
+ * re-ranking (ccr_rerank_exact) the columns that ccr_threshold_compact keeps from the row's dense scan
+ * scores (ccr_score_dense_f32 / _f16) gives the exact result.  out_scores64 is required.
+ *   q, items          fp32 rows; q_scan, items_scan their scan copies, same pitches ldq / ldi (>= D,
+ *                     multiples of 8, 16-byte aligned bases)
+ *   max_row_norm      device double: the largest ||v||_2 of the table's fp32 rows (rounded up),
+ *                     maintained by ccr_ingest_rows_f32_f32
+ *   other arguments   as ccr_score_topk_bf16 (no CCR_FLAG_PACKED_KEYS)
+ * The test lever CCR_EXACT_FALLBACK=1 marks every row uncertified.
+ */
+int ccr_exact_k_candidates(int64_t B, int64_t n_items, int D, int k, int flags);
+double ccr_exact_error_bound(double q_norm, double max_row_norm, int D, int flags);
+size_t ccr_score_topk_exact_workspace_bytes(int64_t B, int64_t n_items, int D, int k, int64_t mask_nnz,
+                                            int64_t mask_max_row_nnz, int flags);
+int ccr_score_topk_exact(const float* q, const void* q_scan, int64_t B, int64_t ldq, const float* items,
+                         const void* items_scan, int64_t n_items, int64_t ldi, int D, int k,
+                         const double* max_row_norm, const int64_t* mask_indptr, const int32_t* mask_cols,
+                         const double* mask_vals, int64_t mask_nnz, int64_t mask_max_row_nnz, int mask_mode,
+                         int64_t id_offset, float* out_scores, double* out_scores64, int64_t* out_ids,
+                         int32_t* out_uncertified, double* out_tau, int32_t* uncertified_count, void* workspace,
+                         size_t workspace_bytes, int flags, void* stream);
+
+/* fp32 rows -> fp32 table rows of an exact table, optionally L2-normalised (as ccr_ingest_rows_f32);
+ * columns D..ld_dst-1 zeroed.  max_row_norm (device double, may be NULL) = max(itself, RU(||row||_2)) over
+ * the stored rows. */
+int ccr_ingest_rows_f32_f32(const float* src, int64_t n, int D, int64_t ld_src, float* dst, int64_t ld_dst,
+                            int normalize, double* max_row_norm, void* stream);
+
+/* Exact top-k of given candidates: row r ranks cand_ids[cand_indptr[r] .. cand_indptr[r+1]) (int64 local
+ * ids; duplicates, ids outside [0, n_items) and ids inside the row's mask are ignored) together with every
+ * mask entry of the row, by the exact values defined above.  cand_nnz >= cand_indptr[B]. */
+size_t ccr_rerank_exact_workspace_bytes(int64_t B, int64_t cand_nnz, int64_t mask_nnz);
+int ccr_rerank_exact(const float* q, int64_t B, int64_t ldq, const float* items, int64_t n_items, int64_t ldi, int D,
+                     int k, const int64_t* cand_indptr, const int64_t* cand_ids, int64_t cand_nnz,
+                     const int64_t* mask_indptr, const int32_t* mask_cols, const double* mask_vals, int64_t mask_nnz,
+                     int mask_mode, int64_t id_offset, float* out_scores, double* out_scores64, int64_t* out_ids,
+                     void* workspace, size_t workspace_bytes, int flags, void* stream);
+
+/* Columns of a dense fp32 score block scores [R, ld] with double(score) >= tau[r] (device float64 [R]), as a
+ * CSR.  First call with out_ids = NULL: out_indptr [R+1] receives the row offsets.  Second call with the
+ * same out_indptr and out_ids [out_indptr[R]]: the column ids, in no particular order within a row. */
+int ccr_threshold_compact(const float* scores, int64_t R, int64_t N, int64_t ld, const double* tau,
+                          int64_t* out_indptr, int64_t* out_ids, void* stream);
+
 /* Which kernel ccr_score_topk_bf16 picks under CCR_ALGO_AUTO: CCR_ALGO_SIMT or CCR_ALGO_TCGEN05. */
 int ccr_choose_algo(int64_t B, int64_t n_items, int D, int k);
 
