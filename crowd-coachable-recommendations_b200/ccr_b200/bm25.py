@@ -212,8 +212,7 @@ class BM25(object):
                 res_s = out_s[s:e] if whole else torch.empty((n_q, k), dtype=torch.float32, device=dev)
                 res_i = out_i[s:e] if whole else torch.empty((n_q, k), dtype=torch.int64, device=dev)
                 with torch.cuda.device(dev):
-                    need = L.ccr_bm25_topk_workspace_bytes(n_q, N, k)
-                    ws = workspace.get(dev, max(need, 256))
+                    ws = workspace.get(dev, L.ccr_bm25_topk_workspace_bytes(n_q, N, k))
                     rc = L.ccr_bm25_topk(self._indptr.data_ptr(), self._docs.data_ptr(), self._val.data_ptr(),
                                          *self._head_ptrs(), d_indptr.data_ptr(), d_terms.data_ptr(),
                                          int(lengths[rows].max()), n_q, N, k,

@@ -4,6 +4,8 @@ PyTorch is used for device memory, streams and (in dist.py) torch.distributed on
 """
 from __future__ import annotations
 
+from collections import namedtuple
+
 import numpy as np
 import torch
 
@@ -29,13 +31,16 @@ class _Workspace:
         self._buf = {}
 
     def get(self, device, nbytes):
+        # never smaller than 256 bytes: a size query that rejected its arguments returns 0, and the call
+        # itself, given a valid buffer, then reports why
+        nbytes = max(int(nbytes), 256)
         index = device.index if device.index is not None else torch.cuda.current_device()
         key = (device.type, index, torch.cuda.current_stream(device).cuda_stream)
         b = self._buf.get(key)
         if b is None or b.numel() < nbytes:
             b = None
             self._buf[key] = None
-            b = torch.empty(int(nbytes) + 256, dtype=torch.uint8, device=device)
+            b = torch.empty(nbytes + 256, dtype=torch.uint8, device=device)
             # the old block may still be in use by work queued on this stream; the caching allocator
             # only recycles it for the same stream, i.e. after that work
             self._buf[key] = b
@@ -228,6 +233,28 @@ class SparseMask:
         return SparseMask(new_ip, c[keep] - lo, v[keep], hi - lo, self.mode, self.device)
 
 
+_MaskABI = namedtuple("_MaskABI", "indptr cols vals nnz h_max mode")
+_NO_MASK = _MaskABI(None, None, None, 0, -1, MASK_NONE)
+
+
+def _mask_abi(mask, B, N):
+    """The C ABI arguments of ``mask`` for B rows and N columns: raw pointers, nnz, max row nnz and mode, or
+    None when there is no mask to apply (None, MASK_NONE or no entries): the rule the C ABI applies, so every
+    wrapper passes the same arguments for the same mask."""
+    if mask is None:
+        return None
+    if mask.n_rows != B or mask.n_cols != N:
+        raise ValueError(f"mask shape ({mask.n_rows}, {mask.n_cols}) does not match ({B}, {N})")
+    if mask.mode == MASK_NONE or mask.nnz <= 0:
+        return None
+    return _MaskABI(mask.indptr.data_ptr(), mask.cols.data_ptr(), mask.vals.data_ptr(), mask.nnz, mask.max_row_nnz,
+                    mask.mode)
+
+
+def _rows_pitch(t):
+    return t.stride(0) if t.shape[0] > 1 else max(t.stride(0), t.shape[1])
+
+
 def _operand_f16(q, items):
     """True for two fp16 operands, False for two bf16 ones; anything else is a TypeError."""
     if q.dtype == items.dtype == torch.float16:
@@ -259,8 +286,7 @@ def score_topk(q, items, k, mask: SparseMask | None = None, id_offset=0, algo=_l
     B = q.shape[0]
     N = items.shape[0] if n_items is None else int(n_items)
     D = q.shape[1] if D is None else int(D)
-    ldq = q.stride(0) if B > 1 else max(q.stride(0), q.shape[1])
-    ldi = items.stride(0) if items.shape[0] > 1 else max(items.stride(0), items.shape[1])
+    ldq, ldi = _rows_pitch(q), _rows_pitch(items)
     k = int(k)
     flags = int(algo) | (_lib.FLAG_ALLOW_SHORT if allow_short else 0) | (_lib.FLAG_F16 if f16 else 0)
     if want_keys:
@@ -268,12 +294,7 @@ def score_topk(q, items, k, mask: SparseMask | None = None, id_offset=0, algo=_l
             raise ValueError("want_keys and want_f64 are exclusive (one 8-byte slot per entry)")
         flags |= _lib.FLAG_PACKED_KEYS
     L = _lib.lib()
-    if mask is not None:
-        if mask.n_rows != B:
-            raise ValueError(f"mask has {mask.n_rows} rows, queries {B}")
-        if mask.n_cols != N:
-            raise ValueError(f"mask has {mask.n_cols} columns, table shard {N}")
-    nnz = mask.nnz if mask is not None else 0
+    m = _mask_abi(mask, B, N) or _NO_MASK
     out_s = torch.empty((B, k), dtype=torch.float32, device=dev)
     out_i = torch.empty((B, k), dtype=torch.int64, device=dev)
     out_d = torch.empty((B, k), dtype=torch.float64, device=dev) if want_f64 else None
@@ -281,18 +302,10 @@ def score_topk(q, items, k, mask: SparseMask | None = None, id_offset=0, algo=_l
         out_d = torch.empty((B, k), dtype=torch.int64, device=dev)
     _status()
     with torch.cuda.device(dev):
-        hmax = mask.max_row_nnz if mask is not None else -1
-        need = L.ccr_score_topk_workspace_bytes(B, N, D, k, nnz, hmax, flags)
-        if need == 0 and B > 0:
-            # invalid shape: let the real call produce the error message
-            need = 256
-        ws = workspace.get(dev, need)
+        ws = workspace.get(dev, L.ccr_score_topk_workspace_bytes(B, N, D, k, m.nnz, m.h_max, flags))
         rc = L.ccr_score_topk_bf16(
             q.data_ptr(), B, ldq, items.data_ptr() if N > 0 else None, N, ldi, D, k,
-            mask.indptr.data_ptr() if mask is not None else None,
-            mask.cols.data_ptr() if mask is not None and nnz else (mask.indptr.data_ptr() if mask is not None else None),
-            mask.vals.data_ptr() if mask is not None and nnz else (mask.indptr.data_ptr() if mask is not None else None),
-            nnz, hmax, mask.mode if mask is not None else MASK_NONE, int(id_offset),
+            m.indptr, m.cols, m.vals, m.nnz, m.h_max, m.mode, int(id_offset),
             out_s.data_ptr(), out_d.data_ptr() if out_d is not None else None, out_i.data_ptr(),
             ws.data_ptr(), ws.numel(), flags, _stream_ptr(dev))
     _lib.check(rc)
@@ -363,22 +376,15 @@ def topk_dense(scores, k, mask: SparseMask | None = None):
     B, N = scores.shape
     k = int(k)
     dev = scores.device
-    ld = scores.stride(0) if B > 1 else max(scores.stride(0), N)
-    if mask is not None and (mask.n_rows != B or mask.n_cols != N):
-        raise ValueError("mask shape does not match the score matrix")
-    nnz = mask.nnz if mask is not None else 0
-    hmax = mask.max_row_nnz if mask is not None else 0
+    m = _mask_abi(mask, B, N) or _NO_MASK
     out_s = torch.empty((B, k), dtype=torch.float32, device=dev)
     out_d = torch.empty((B, k), dtype=torch.float64, device=dev)
     out_i = torch.empty((B, k), dtype=torch.int64, device=dev)
     L = _lib.lib()
     with torch.cuda.device(dev):
-        need = L.ccr_topk_dense_workspace_bytes(B, N, k, nnz, hmax)
-        ws = workspace.get(dev, max(need, 256))
+        ws = workspace.get(dev, L.ccr_topk_dense_workspace_bytes(B, N, k, m.nnz, m.h_max))
         rc = L.ccr_topk_dense_f32(
-            scores.data_ptr(), B, N, ld, k,
-            mask.indptr.data_ptr() if nnz else None, mask.cols.data_ptr() if nnz else None,
-            mask.vals.data_ptr() if nnz else None, nnz, hmax, mask.mode if nnz else MASK_NONE,
+            scores.data_ptr(), B, N, _rows_pitch(scores), k, m.indptr, m.cols, m.vals, m.nnz, m.h_max, m.mode,
             out_s.data_ptr(), out_d.data_ptr(), out_i.data_ptr(), ws.data_ptr(), ws.numel(), _stream_ptr(dev))
     _lib.check(rc)
     return out_s, out_i, out_d
@@ -394,10 +400,7 @@ def argsort_scores(scores, mask: SparseMask | None = None):
     B, N = scores.shape
     dev = scores.device
     n = B * N
-    ld = scores.stride(0) if B > 1 else max(scores.stride(0), N)
-    if mask is not None and (mask.n_rows != B or mask.n_cols != N):
-        raise ValueError("mask shape does not match the score matrix")
-    nnz = mask.nnz if mask is not None else 0
+    m = _mask_abi(mask, B, N) or _NO_MASK
     rows = torch.empty(n, dtype=torch.int64, device=dev)
     cols = torch.empty(n, dtype=torch.int64, device=dev)
     L = _lib.lib()
@@ -405,11 +408,10 @@ def argsort_scores(scores, mask: SparseMask | None = None):
         need = L.ccr_argsort_workspace_bytes(n)
         if need == 0 and n > 0:
             raise ValueError("argsort: more than 2^31 matrix elements")
-        ws = workspace.get(dev, max(need, 256))
-        rc = L.ccr_argsort_scores_f32(scores.data_ptr(), B, N, ld,
-                                      mask.indptr.data_ptr() if nnz else None, mask.cols.data_ptr() if nnz else None,
-                                      mask.vals.data_ptr() if nnz else None, nnz, mask.mode if nnz else MASK_NONE,
-                                      rows.data_ptr(), cols.data_ptr(), ws.data_ptr(), ws.numel(), _stream_ptr(dev))
+        ws = workspace.get(dev, need)
+        rc = L.ccr_argsort_scores_f32(scores.data_ptr(), B, N, _rows_pitch(scores), m.indptr, m.cols, m.vals, m.nnz,
+                                      m.mode, rows.data_ptr(), cols.data_ptr(), ws.data_ptr(), ws.numel(),
+                                      _stream_ptr(dev))
     _lib.check(rc)
     return rows, cols
 
@@ -461,8 +463,7 @@ def ingest_rows(src, dst, normalize=False, overflow=None):
         raise TypeError("fp16 rows do not go into a bf16 table: pass them as float32")
     if overflow is not None and (not f16 or overflow.dtype != torch.int32 or not overflow.is_cuda):
         raise ValueError("overflow must be a device int32 tensor, for fp16 destinations only")
-    ld_src = src.stride(0) if n > 1 else max(src.stride(0), D)
-    ld_dst = dst.stride(0) if n > 1 else max(dst.stride(0), dst.shape[1])
+    ld_src, ld_dst = _rows_pitch(src), _rows_pitch(dst)
     L = _lib.lib()
     with torch.cuda.device(src.device):
         if src.dtype == torch.float32:
@@ -498,11 +499,10 @@ def score_dense(q, items, n_items=None, D=None):
     out = torch.empty((B, N), dtype=torch.float32, device=q.device)
     if B == 0 or N == 0:
         return out
-    ldq = q.stride(0) if B > 1 else max(q.stride(0), q.shape[1])
-    ldi = items.stride(0) if items.shape[0] > 1 else max(items.stride(0), items.shape[1])
     with torch.cuda.device(q.device):
         fn = _lib.lib().ccr_score_dense_f16 if f16 else _lib.lib().ccr_score_dense_f32
-        rc = fn(q.data_ptr(), B, ldq, items.data_ptr(), N, ldi, D, out.data_ptr(), N, _stream_ptr(q.device))
+        rc = fn(q.data_ptr(), B, _rows_pitch(q), items.data_ptr(), N, _rows_pitch(items), D, out.data_ptr(), N,
+                _stream_ptr(q.device))
     _lib.check(rc)
     return out
 
@@ -540,18 +540,13 @@ def ingest_rows_f32(src, dst, normalize=False, v_max=None):
         raise ValueError("dst must be dense rows [n, >= D]")
     if v_max is not None and (v_max.dtype != torch.float64 or not v_max.is_cuda):
         raise ValueError("v_max must be a device float64 tensor")
-    ld_src = src.stride(0) if n > 1 else max(src.stride(0), D)
-    ld_dst = dst.stride(0) if n > 1 else max(dst.stride(0), dst.shape[1])
     with torch.cuda.device(src.device):
-        rc = _lib.lib().ccr_ingest_rows_f32_f32(src.data_ptr(), n, D, ld_src, dst.data_ptr(), ld_dst,
-                                                int(bool(normalize)), v_max.data_ptr() if v_max is not None else None,
+        rc = _lib.lib().ccr_ingest_rows_f32_f32(src.data_ptr(), n, D, _rows_pitch(src), dst.data_ptr(),
+                                                _rows_pitch(dst), int(bool(normalize)),
+                                                v_max.data_ptr() if v_max is not None else None,
                                                 _stream_ptr(src.device))
     _lib.check(rc)
     return dst
-
-
-def _rows_pitch(t):
-    return t.stride(0) if t.shape[0] > 1 else max(t.stride(0), t.shape[1])
 
 
 def score_topk_exact(q, q_scan, items, items_scan, k, v_max, mask: SparseMask | None = None, id_offset=0,
@@ -575,10 +570,7 @@ def score_topk_exact(q, q_scan, items, items_scan, k, v_max, mask: SparseMask | 
     k = int(k)
     ldq, ldi = _rows_pitch(q), _rows_pitch(items)
     flags = int(algo) | (_lib.FLAG_ALLOW_SHORT if allow_short else 0) | (_lib.FLAG_F16 if f16 else 0)
-    if mask is not None and (mask.n_rows != B or mask.n_cols != N):
-        raise ValueError(f"mask shape ({mask.n_rows}, {mask.n_cols}) does not match ({B}, {N})")
-    nnz = mask.nnz if mask is not None else 0
-    hmax = mask.max_row_nnz if mask is not None else -1
+    m = _mask_abi(mask, B, N) or _NO_MASK
     out_s = torch.empty((B, k), dtype=torch.float32, device=dev)
     out_i = torch.empty((B, k), dtype=torch.int64, device=dev)
     out_d = torch.empty((B, k), dtype=torch.float64, device=dev)
@@ -587,17 +579,14 @@ def score_topk_exact(q, q_scan, items, items_scan, k, v_max, mask: SparseMask | 
     count = torch.zeros(1, dtype=torch.int32, device=dev)
     L = _lib.lib()
     _status()
-    mp = (lambda t: t.data_ptr() if mask is not None and nnz else None)
     with torch.cuda.device(dev):
-        need = L.ccr_score_topk_exact_workspace_bytes(B, N, D, k, nnz, hmax, flags)
-        ws = workspace.get(dev, max(need, 256))
+        ws = workspace.get(dev, L.ccr_score_topk_exact_workspace_bytes(B, N, D, k, m.nnz, m.h_max, flags))
         rc = L.ccr_score_topk_exact(
             q.data_ptr(), q_scan.data_ptr(), B, ldq, items.data_ptr() if N else None,
             items_scan.data_ptr() if N else None, N, ldi, D, k, v_max.data_ptr(),
-            mp(mask.indptr) if mask is not None else None, mp(mask.cols) if mask is not None else None,
-            mp(mask.vals) if mask is not None else None, nnz, hmax, mask.mode if mask is not None else MASK_NONE,
-            int(id_offset), out_s.data_ptr(), out_d.data_ptr(), out_i.data_ptr(), uncert.data_ptr(), tau.data_ptr(),
-            count.data_ptr(), ws.data_ptr(), ws.numel(), flags, _stream_ptr(dev))
+            m.indptr, m.cols, m.vals, m.nnz, m.h_max, m.mode, int(id_offset), out_s.data_ptr(), out_d.data_ptr(),
+            out_i.data_ptr(), uncert.data_ptr(), tau.data_ptr(), count.data_ptr(), ws.data_ptr(), ws.numel(), flags,
+            _stream_ptr(dev))
     _lib.check(rc)
     n_fallback = int(count.item()) if B else 0
     if n_fallback:
@@ -627,21 +616,16 @@ def _exact_fallback_rows(q, q_scan, items, items_scan, k, tau, mask, rows, id_of
         _lib.check(L.ccr_threshold_compact(scores.data_ptr(), R, N, N, tau.data_ptr(), indptr.data_ptr(),
                                            ids.data_ptr(), _stream_ptr(dev)))
     del scores
-    sub = mask.take_rows(rows.cpu().numpy()) if mask is not None else None
-    nnz = sub.nnz if sub is not None else 0
+    m = _mask_abi(mask.take_rows(rows.cpu().numpy()) if mask is not None else None, R, N) or _NO_MASK
     out_s = torch.empty((R, k), dtype=torch.float32, device=dev)
     out_i = torch.empty((R, k), dtype=torch.int64, device=dev)
     out_d = torch.empty((R, k), dtype=torch.float64, device=dev)
-    mp = (lambda t: t.data_ptr() if sub is not None and nnz else None)
     with torch.cuda.device(dev):
-        need = L.ccr_rerank_exact_workspace_bytes(R, total, nnz)
-        ws = workspace.get(dev, max(need, 256))
+        ws = workspace.get(dev, L.ccr_rerank_exact_workspace_bytes(R, total, m.nnz))
         rc = L.ccr_rerank_exact(
             q.data_ptr(), R, _rows_pitch(q), items.data_ptr() if N else None, N, _rows_pitch(items), D, k,
-            indptr.data_ptr(), ids.data_ptr(), total, mp(sub.indptr) if sub is not None else None,
-            mp(sub.cols) if sub is not None else None, mp(sub.vals) if sub is not None else None, nnz,
-            sub.mode if sub is not None else MASK_NONE, int(id_offset), out_s.data_ptr(), out_d.data_ptr(),
-            out_i.data_ptr(), ws.data_ptr(), ws.numel(), _lib.FLAG_ALLOW_SHORT if allow_short else 0,
-            _stream_ptr(dev))
+            indptr.data_ptr(), ids.data_ptr(), total, m.indptr, m.cols, m.vals, m.nnz, m.mode, int(id_offset),
+            out_s.data_ptr(), out_d.data_ptr(), out_i.data_ptr(), ws.data_ptr(), ws.numel(),
+            _lib.FLAG_ALLOW_SHORT if allow_short else 0, _stream_ptr(dev))
     _lib.check(rc)
     return out_s, out_i, out_d

@@ -266,6 +266,25 @@ int check_shape(long long B, long long n_items, int D, int k, int flags) {
     return fail(CCR_EINVAL, "unknown algo flag %d", algo);
   return CCR_OK;
 }
+
+// h_max of a plan: the largest number of mask entries in one row (or a bound), < 0 when unknown or no mask
+long long mask_h_max(long long nnz, long long max_row_nnz) { return nnz > 0 ? max_row_nnz : -1; }
+
+// The mask CSR of an entry point.  A mask is present exactly when mode != CCR_MASK_NONE, indptr is set and
+// nnz > 0; otherwise every field is the empty mask (null pointers, nnz 0, h_max -1, CCR_MASK_NONE).
+struct MaskArgs { const long long* indptr; const int* cols; const double* vals; long long nnz, h_max; int mode; };
+
+int parse_mask(const int64_t* indptr, const int32_t* cols, const double* vals, int64_t nnz, int64_t max_row_nnz,
+               int mode, MaskArgs* m) {
+  *m = {nullptr, nullptr, nullptr, 0, -1, CCR_MASK_NONE};
+  if (mode != CCR_MASK_NONE && mode != CCR_MASK_SET && mode != CCR_MASK_ADD)
+    return fail(CCR_EINVAL, "bad mask_mode %d", mode);
+  if (mode != CCR_MASK_NONE && nnz < 0) return fail(CCR_EINVAL, "mask_nnz = %lld", (long long)nnz);
+  if (mode == CCR_MASK_NONE || !indptr || nnz == 0) return CCR_OK;
+  if (!cols || !vals) return fail(CCR_EINVAL, "mask_cols / mask_vals null");
+  *m = {(const long long*)indptr, cols, vals, nnz, mask_h_max(nnz, max_row_nnz), mode};
+  return CCR_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -295,7 +314,7 @@ size_t ccr_score_topk_workspace_bytes(int64_t B, int64_t n_items, int D, int k, 
                                       int64_t mask_max_row_nnz, int flags) {
   if (check_shape(B, n_items, D, k, flags | CCR_FLAG_ALLOW_SHORT) != CCR_OK) return 0;
   Plan pl;
-  make_plan(B, n_items, D, k, mask_nnz, mask_nnz > 0 ? mask_max_row_nnz : -1, flags, &pl);
+  make_plan(B, n_items, D, k, mask_nnz, mask_h_max(mask_nnz, mask_max_row_nnz), flags, &pl);
   return pl.total;
 }
 
@@ -305,7 +324,7 @@ int ccr_plan_info(int64_t B, int64_t n_items, int D, int k, int64_t mask_nnz, in
   if (rc) return rc;
   if (!info8) return fail(CCR_EINVAL, "info8 is null");
   Plan pl;
-  make_plan(B, n_items, D, k, mask_nnz, mask_nnz > 0 ? mask_max_row_nnz : -1, flags, &pl);
+  make_plan(B, n_items, D, k, mask_nnz, mask_h_max(mask_nnz, mask_max_row_nnz), flags, &pl);
   info8[0] = pl.n_q_tiles;
   info8[1] = pl.S;
   info8[2] = pl.C;
@@ -332,20 +351,16 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   if (n_items > 0 && !items) return fail(CCR_EINVAL, "null items");
   if (ldq < D || ldi < D || ldq % 8 || ldi % 8) return fail(CCR_EINVAL, "ldq/ldi must be >= D and multiples of 8");
   if (((uintptr_t)q & 15) || ((uintptr_t)items & 15)) return fail(CCR_EINVAL, "q/items must be 16-byte aligned");
-  if (mask_mode != CCR_MASK_NONE && mask_mode != CCR_MASK_SET && mask_mode != CCR_MASK_ADD)
-    return fail(CCR_EINVAL, "bad mask_mode %d", mask_mode);
-  const bool has_mask = mask_mode != CCR_MASK_NONE && mask_indptr != nullptr;
-  if (has_mask && (!mask_cols || !mask_vals)) return fail(CCR_EINVAL, "mask_cols / mask_vals null");
+  MaskArgs m;
+  if ((rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, mask_max_row_nnz, mask_mode, &m))) return rc;
   if (flags & CCR_FLAG_PACKED_KEYS) {
-    if (mask_mode == CCR_MASK_ADD) return fail(CCR_EINVAL, "CCR_FLAG_PACKED_KEYS: float64 priors do not fit a float32 key");
+    if (m.mode == CCR_MASK_ADD) return fail(CCR_EINVAL, "CCR_FLAG_PACKED_KEYS: float64 priors do not fit a float32 key");
     if (id_offset < 0 || id_offset + n_items > (1LL << 32)) return fail(CCR_EUNSUPPORTED, "CCR_FLAG_PACKED_KEYS: global ids must be < 2^32");
   }
   cudaStream_t st = (cudaStream_t)stream;
 
-  const long long nnz = has_mask ? mask_nnz : 0;
-  if (nnz < 0) return fail(CCR_EINVAL, "mask_nnz = %lld", nnz);
   Plan pl;
-  make_plan(B, n_items, D, k, nnz, nnz > 0 ? mask_max_row_nnz : -1, flags, &pl);
+  make_plan(B, n_items, D, k, m.nnz, m.h_max, flags, &pl);
   if (!workspace || workspace_bytes < pl.total)
     return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, pl.total);
   unsigned char* ws = (unsigned char*)workspace;
@@ -361,8 +376,8 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   sp.items = (const __nv_bfloat16*)items; sp.ldi = ldi; sp.n_items = n_items; sp.D = D;
   sp.f16 = (flags & CCR_FLAG_F16) ? 1 : 0;
   sp.k = k; sp.k_keep = pl.k_keep; sp.C = pl.C; sp.S = pl.S; sp.n_q_tiles = pl.n_q_tiles; sp.two_cta = pl.two_cta;
-  sp.mask_indptr = has_mask ? (const long long*)mask_indptr : nullptr;
-  sp.mask_cols = (has_mask && !pl.include_mask) ? mask_cols : nullptr;
+  sp.mask_indptr = m.indptr;
+  sp.mask_cols = pl.include_mask ? nullptr : m.cols;
   sp.cand = (u64*)(ws + pl.off_cand);
   sp.counts = (int*)(ws + pl.off_counts);
   sp.status = status;
@@ -389,8 +404,8 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
     int lr0 = launch_select_tc(ss, st, device_sm_count());
     if (lr0) return fail(CCR_ECUDA, "seed GEMM launch failed (%d)", lr0);
     // per row: the (k + h)-th largest of the seed_m / 8 group maxima
-    lr0 = launch_seed_tau(ss.dense_out, pl.seed_ld, (int)pl.seed_ld, (int)B, k, has_mask ? (const long long*)mask_indptr : nullptr,
-                          sp.g_tau, pl.use_hist ? (uint2*)(ws + pl.off_hpar) : nullptr, st);
+    lr0 = launch_seed_tau(ss.dense_out, pl.seed_ld, (int)pl.seed_ld, (int)B, k, m.indptr, sp.g_tau,
+                          pl.use_hist ? (uint2*)(ws + pl.off_hpar) : nullptr, st);
     if (lr0) return fail(CCR_ECUDA, "seed select launch failed: %s", cudaGetErrorString((cudaError_t)lr0));
   }
 
@@ -417,13 +432,13 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   }
   if (lr) return fail(CCR_ECUDA, "select kernel launch failed (%d: %s)", lr, lr > 0 ? cudaGetErrorString((cudaError_t)lr) : "tensor map");
 
-  if (has_mask && nnz > 0) {
+  if (m.nnz > 0) {
     OverrideParams op = {};
     // sp.q may be the padded staging block of a short batch: use ITS pitch (sp.ldq), not the caller's
     op.q = sp.q; op.ldq = sp.ldq; op.B = (int)B; op.items = sp.items; op.ldi = ldi; op.n_items = n_items; op.D = D;
     op.f16 = sp.f16;
-    op.mask_indptr = sp.mask_indptr; op.mask_cols = mask_cols; op.mask_vals = mask_vals; op.nnz = nnz;
-    op.mode = mask_mode; op.ovr_hi = (u64*)(ws + pl.off_ovr_hi); op.ovr_lo = (u32*)(ws + pl.off_ovr_lo);
+    op.mask_indptr = m.indptr; op.mask_cols = m.cols; op.mask_vals = m.vals; op.nnz = m.nnz;
+    op.mode = m.mode; op.ovr_hi = (u64*)(ws + pl.off_ovr_hi); op.ovr_lo = (u32*)(ws + pl.off_ovr_lo);
     lr = launch_overrides(op, st);
     if (lr) return fail(CCR_ECUDA, "override kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   }
@@ -431,8 +446,8 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   FinalizeParams fp = {};
   fp.B = (int)B; fp.k = k; fp.C = pl.C; fp.S = pl.S * pl.halves; fp.cand = sp.cand; fp.counts = sp.counts;
   fp.g_tau = sp.g_tau;
-  fp.drop_cols = (has_mask && nnz > 0 && pl.include_mask) ? mask_cols : nullptr;
-  fp.mask_indptr = (has_mask && nnz > 0) ? sp.mask_indptr : nullptr;
+  fp.drop_cols = pl.include_mask ? m.cols : nullptr;
+  fp.mask_indptr = m.indptr;
   fp.ovr_hi = (u64*)(ws + pl.off_ovr_hi); fp.ovr_lo = (u32*)(ws + pl.off_ovr_lo);
   fp.id_offset = id_offset; fp.out_scores = out_scores; fp.out_scores64 = out_scores64;
   fp.out_keys = nullptr;
@@ -583,17 +598,14 @@ int ccr_argsort_scores_f32(const float* scores, int64_t B, int64_t n_cols, int64
                            int64_t* out_rows, int64_t* out_cols, void* workspace, size_t workspace_bytes, void* stream) {
   if (B < 0 || n_cols < 0 || ld < n_cols) return fail(CCR_EINVAL, "bad argsort shape");
   if (B * n_cols > (1LL << 31)) return fail(CCR_EUNSUPPORTED, "argsort: more than 2^31 matrix elements");
-  if (mask_mode != CCR_MASK_NONE && mask_mode != CCR_MASK_SET && mask_mode != CCR_MASK_ADD)
-    return fail(CCR_EINVAL, "bad mask_mode %d", mask_mode);
+  MaskArgs m;
+  if (int rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, -1, mask_mode, &m)) return rc;
   if (B * n_cols == 0) return CCR_OK;
   if (!scores || !out_rows || !out_cols) return fail(CCR_EINVAL, "null pointer");
-  const bool has_mask = mask_mode != CCR_MASK_NONE && mask_indptr != nullptr && mask_nnz > 0;
-  if (has_mask && (!mask_cols || !mask_vals)) return fail(CCR_EINVAL, "mask_cols / mask_vals null");
   const size_t need = argsort_workspace_bytes(B * n_cols);
   if (!workspace || workspace_bytes < need) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, need);
-  int lr = launch_argsort(scores, B, n_cols, ld, has_mask ? (const long long*)mask_indptr : nullptr, mask_cols, mask_vals,
-                          has_mask ? mask_nnz : 0, mask_mode, (long long*)out_rows, (long long*)out_cols, workspace,
-                          (cudaStream_t)stream);
+  int lr = launch_argsort(scores, B, n_cols, ld, m.indptr, m.cols, m.vals, m.nnz, m.mode, (long long*)out_rows,
+                          (long long*)out_cols, workspace, (cudaStream_t)stream);
   if (lr) return fail(CCR_ECUDA, "argsort launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   return CCR_OK;
 }
@@ -646,34 +658,30 @@ int ccr_topk_dense_f32(const float* scores, int64_t B, int64_t n_cols, int64_t l
   if (k < 1 || k > CCR_MAX_K) return fail(CCR_EUNSUPPORTED, "k=%d outside [1,%d]", k, CCR_MAX_K);
   if (k > n_cols) return fail(CCR_EK_RANGE, "selected index k out of range (k=%d > n=%lld)", k, (long long)n_cols);
   if (n_cols > (1LL << 31) - 512) return fail(CCR_EUNSUPPORTED, "n_cols must be < 2^31");
-  if (mask_mode != CCR_MASK_NONE && mask_mode != CCR_MASK_SET && mask_mode != CCR_MASK_ADD)
-    return fail(CCR_EINVAL, "bad mask_mode %d", mask_mode);
+  MaskArgs m;
+  if (int rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, mask_max_row_nnz, mask_mode, &m)) return rc;
   if (B == 0) return CCR_OK;
   if (!scores || !out_ids) return fail(CCR_EINVAL, "null pointer");
-  const bool has_mask = mask_mode != CCR_MASK_NONE && mask_indptr != nullptr && mask_nnz > 0;
-  if (has_mask && (!mask_cols || !mask_vals)) return fail(CCR_EINVAL, "mask_cols / mask_vals null");
-  const long long nnz = has_mask ? mask_nnz : 0;
-  const long long h = has_mask ? mask_max_row_nnz : 0;
+  const long long h = m.indptr ? m.h_max : 0;  // masked columns are dropped at the end: k + h candidates per row
   if (h < 0 || k + h > CCR_MAX_K)
     return fail(CCR_EUNSUPPORTED, "dense top-k: k + max row nnz = %lld outside [1,%d]", (long long)(k + h), CCR_MAX_K);
   DensePlanC pl;
-  dense_plan(B, n_cols, (int)(k + h), nnz, &pl);
+  dense_plan(B, n_cols, (int)(k + h), m.nnz, &pl);
   if (!workspace || workspace_bytes < pl.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, pl.total);
   unsigned char* ws = (unsigned char*)workspace;
   cudaStream_t st = (cudaStream_t)stream;
-  const long long* indptr = has_mask ? (const long long*)mask_indptr : nullptr;
-  int lr = launch_select_dense(scores, ld, B, n_cols, k, (int)(k + h), indptr, pl.C, pl.S, (u64*)ws, (int*)(ws + pl.off_counts), st);
+  int lr = launch_select_dense(scores, ld, B, n_cols, k, (int)(k + h), m.indptr, pl.C, pl.S, (u64*)ws, (int*)(ws + pl.off_counts), st);
   if (lr) return fail(CCR_ECUDA, "dense select launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  if (has_mask) {
-    lr = launch_override_dense(scores, ld, (int)B, n_cols, indptr, mask_cols, mask_vals, nnz, mask_mode,
+  if (m.indptr) {
+    lr = launch_override_dense(scores, ld, (int)B, n_cols, m.indptr, m.cols, m.vals, m.nnz, m.mode,
                                (u64*)(ws + pl.off_ovr_hi), (u32*)(ws + pl.off_ovr_lo), st);
     if (lr) return fail(CCR_ECUDA, "dense override launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   }
   FinalizeParams fp = {};
   fp.B = (int)B; fp.k = k; fp.C = pl.C; fp.S = pl.S; fp.cand = (u64*)ws; fp.counts = (int*)(ws + pl.off_counts);
   fp.g_tau = nullptr;
-  fp.drop_cols = has_mask ? mask_cols : nullptr;
-  fp.mask_indptr = indptr;
+  fp.drop_cols = m.cols;
+  fp.mask_indptr = m.indptr;
   fp.ovr_hi = (u64*)(ws + pl.off_ovr_hi); fp.ovr_lo = (u32*)(ws + pl.off_ovr_lo);
   fp.id_offset = 0; fp.out_keys = nullptr; fp.out_scores = out_scores; fp.out_scores64 = out_scores64; fp.out_ids = (long long*)out_ids;
   lr = launch_finalize(fp, st);
@@ -869,14 +877,13 @@ int check_exact_rows(const void* q, int64_t ldq, const void* items, int64_t ldi,
 // entry records of (candidates U mask entries) -> exact values -> finalize_kernel with no stream candidates
 int rerank(const float* q, long long B, long long ldq, const float* items, long long n_items, long long ldi, int D,
            int k, const long long* cand_indptr, const long long* cand_ids, long long cand_stride, long long cand_nnz,
-           const long long* mask_indptr, const int* mask_cols, const double* mask_vals, long long nnz, int mode,
-           long long id_offset, float* out_scores, double* out_scores64, long long* out_ids, unsigned char* ws,
-           const ExactLayout& L, cudaStream_t st) {
+           const MaskArgs& m, long long id_offset, float* out_scores, double* out_scores64, long long* out_ids,
+           unsigned char* ws, const ExactLayout& L, cudaStream_t st) {
   ExactParams ep = {};
   ep.q = q; ep.ldq = ldq; ep.B = (int)B; ep.items = items; ep.ldi = ldi; ep.n_items = n_items; ep.D = D;
   ep.cand_indptr = cand_indptr; ep.cand_ids = cand_ids; ep.cand_stride = cand_stride;
-  ep.mask_indptr = nnz > 0 ? mask_indptr : nullptr; ep.mask_cols = mask_cols; ep.mask_vals = mask_vals; ep.mode = mode;
-  ep.ent_indptr = (const long long*)(ws + L.off_ent_ip); ep.max_entries = cand_nnz + (nnz > 0 ? nnz : 0);
+  ep.mask_indptr = m.indptr; ep.mask_cols = m.cols; ep.mask_vals = m.vals; ep.mode = m.mode;
+  ep.ent_indptr = (const long long*)(ws + L.off_ent_ip); ep.max_entries = cand_nnz + m.nnz;
   ep.ent_hi = (u64*)(ws + L.off_hi); ep.ent_lo = (u32*)(ws + L.off_lo);
   int lr = launch_exact_entries(ep, st);
   if (lr) return fail(CCR_ECUDA, "exact value kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
@@ -887,16 +894,6 @@ int rerank(const float* q, long long B, long long ldq, const float* items, long 
   fp.out_ids = out_ids;
   lr = launch_finalize(fp, st);
   if (lr) return fail(CCR_ECUDA, "finalize launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
-}
-
-int check_exact_mask(int mask_mode, const int64_t* mask_indptr, const int32_t* mask_cols, const double* mask_vals,
-                     int64_t mask_nnz, bool* has_mask) {
-  if (mask_mode != CCR_MASK_NONE && mask_mode != CCR_MASK_SET && mask_mode != CCR_MASK_ADD)
-    return fail(CCR_EINVAL, "bad mask_mode %d", mask_mode);
-  *has_mask = mask_mode != CCR_MASK_NONE && mask_indptr != nullptr && mask_nnz > 0;
-  if (*has_mask && (!mask_cols || !mask_vals)) return fail(CCR_EINVAL, "mask_cols / mask_vals null");
-  if (mask_nnz < 0) return fail(CCR_EINVAL, "mask_nnz = %lld", (long long)mask_nnz);
   return CCR_OK;
 }
 }  // namespace
@@ -933,7 +930,8 @@ size_t ccr_score_topk_exact_workspace_bytes(int64_t B, int64_t n_items, int D, i
   Plan pl0, pl1;
   make_plan(B, n_items, D, k, 0, -1, flags, &pl0);
   pl1.total = 0;
-  if (pl0.k_cand > 0) make_plan(B, n_items, D, pl0.k_cand, mask_nnz, mask_nnz > 0 ? mask_max_row_nnz : -1, flags, &pl1);
+  if (pl0.k_cand > 0)
+    make_plan(B, n_items, D, pl0.k_cand, mask_nnz, mask_h_max(mask_nnz, mask_max_row_nnz), flags, &pl1);
   ExactLayout L;
   exact_layout(pl1, B, pl0.k_cand, mask_nnz, &L);
   return L.total;
@@ -954,17 +952,16 @@ int ccr_score_topk_exact(const float* q, const void* q_scan, int64_t B, int64_t 
     return fail(CCR_EINVAL, "null q / q_scan / out_ids / out_scores64 / certificate outputs / max_row_norm");
   if (n_items > 0 && (!items || !items_scan)) return fail(CCR_EINVAL, "null items");
   if ((rc = check_exact_rows(q, ldq, items, ldi, D)) || (rc = check_exact_rows(q_scan, ldq, items_scan, ldi, D))) return rc;
-  bool has_mask;
-  if ((rc = check_exact_mask(mask_mode, mask_indptr, mask_cols, mask_vals, mask_nnz, &has_mask))) return rc;
-  const long long nnz = has_mask ? mask_nnz : 0;
+  MaskArgs m;
+  if ((rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, mask_max_row_nnz, mask_mode, &m))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Plan pl0, pl1;
   make_plan(B, n_items, D, k, 0, -1, flags, &pl0);
   const int kc = pl0.k_cand;
   pl1.total = 0;
-  if (kc > 0) make_plan(B, n_items, D, kc, nnz, nnz > 0 ? mask_max_row_nnz : -1, flags, &pl1);
+  if (kc > 0) make_plan(B, n_items, D, kc, m.nnz, m.h_max, flags, &pl1);
   ExactLayout L;
-  exact_layout(pl1, B, kc, nnz, &L);
+  exact_layout(pl1, B, kc, m.nnz, &L);
   if (!workspace || workspace_bytes < L.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, L.total);
   unsigned char* ws = (unsigned char*)workspace;
   float* s1_scores = (float*)(ws + L.off_scores);
@@ -973,21 +970,19 @@ int ccr_score_topk_exact(const float* q, const void* q_scan, int64_t B, int64_t 
     // stage 1: the unchanged scan on the scan copies, every mask entry ranked last (SET -inf) so that none
     // takes a candidate slot; the re-rank below gives each its true value
     double* neg = (double*)(ws + L.off_neg);
-    int lr = launch_fill_f64(neg, nnz, -INFINITY, st);
+    int lr = launch_fill_f64(neg, m.nnz, -INFINITY, st);
     if (lr) return fail(CCR_ECUDA, "fill launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-    rc = ccr_score_topk_bf16(q_scan, B, ldq, items_scan, n_items, ldi, D, kc, has_mask ? mask_indptr : nullptr,
-                             has_mask ? mask_cols : nullptr, has_mask ? neg : nullptr, nnz,
-                             nnz > 0 ? mask_max_row_nnz : -1, has_mask ? CCR_MASK_SET : CCR_MASK_NONE, 0, s1_scores,
-                             nullptr, (int64_t*)s1_ids, ws, pl1.total, flags & (CCR_ALGO_MASK | CCR_FLAG_F16), stream);
+    rc = ccr_score_topk_bf16(q_scan, B, ldq, items_scan, n_items, ldi, D, kc, (const int64_t*)m.indptr, m.cols, neg,
+                             m.nnz, m.h_max, CCR_MASK_SET, 0, s1_scores, nullptr, (int64_t*)s1_ids, ws, pl1.total,
+                             flags & (CCR_ALGO_MASK | CCR_FLAG_F16), stream);
     if (rc) return rc;
   }
-  rc = rerank(q, B, ldq, items, n_items, ldi, D, k, nullptr, s1_ids, kc, B * (long long)kc,
-              (const long long*)mask_indptr, mask_cols, mask_vals, nnz, mask_mode, id_offset, out_scores, out_scores64,
-              (long long*)out_ids, ws, L, st);
+  rc = rerank(q, B, ldq, items, n_items, ldi, D, k, nullptr, s1_ids, kc, B * (long long)kc, m, id_offset, out_scores,
+              out_scores64, (long long*)out_ids, ws, L, st);
   if (rc) return rc;
   int lr = launch_exact_certify(q, ldq, (int)B, D, (flags & CCR_FLAG_F16) ? 1 : 0, max_row_norm, k, kc, n_items,
-                                s1_scores, s1_ids, has_mask ? (const long long*)mask_indptr : nullptr, mask_cols,
-                                out_scores64, knobs().exact_fallback, out_uncertified, out_tau, uncertified_count, st);
+                                s1_scores, s1_ids, m.indptr, m.cols, out_scores64, knobs().exact_fallback,
+                                out_uncertified, out_tau, uncertified_count, st);
   if (lr) return fail(CCR_ECUDA, "certify kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   return CCR_OK;
 }
@@ -1012,15 +1007,14 @@ int ccr_rerank_exact(const float* q, int64_t B, int64_t ldq, const float* items,
   if (cand_nnz < 0) return fail(CCR_EINVAL, "cand_nnz = %lld", (long long)cand_nnz);
   if (n_items > 0 && !items) return fail(CCR_EINVAL, "null items");
   if ((rc = check_exact_rows(q, ldq, items, ldi, D))) return rc;
-  bool has_mask;
-  if ((rc = check_exact_mask(mask_mode, mask_indptr, mask_cols, mask_vals, mask_nnz, &has_mask))) return rc;
-  const long long nnz = has_mask ? mask_nnz : 0;
+  MaskArgs m;
+  if ((rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, -1, mask_mode, &m))) return rc;
   ExactLayout L;
-  entry_layout(0, B, cand_nnz + nnz, &L);
+  entry_layout(0, B, cand_nnz + m.nnz, &L);
   if (!workspace || workspace_bytes < L.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, L.total);
   return rerank(q, B, ldq, items, n_items, ldi, D, k, (const long long*)cand_indptr, (const long long*)cand_ids, 0,
-                cand_nnz, (const long long*)mask_indptr, mask_cols, mask_vals, nnz, mask_mode, id_offset, out_scores,
-                out_scores64, (long long*)out_ids, (unsigned char*)workspace, L, (cudaStream_t)stream);
+                cand_nnz, m, id_offset, out_scores, out_scores64, (long long*)out_ids, (unsigned char*)workspace, L,
+                (cudaStream_t)stream);
 }
 
 int ccr_threshold_compact(const float* scores, int64_t R, int64_t N, int64_t ld, const double* tau,

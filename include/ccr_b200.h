@@ -101,7 +101,10 @@ const char* ccr_last_error_string(void);
  *            true count from indptr, the bound sizes the workspace);
  *            mask_max_row_nnz = largest number of entries in one row, or an upper bound (lets the kernel stream masked
  *            items through and drop them at the end instead of testing every candidate; pass -1 if
- *            unknown); all NULL / 0 when mask_mode == CCR_MASK_NONE
+ *            unknown).  The mask applies exactly when mask_mode != CCR_MASK_NONE, mask_indptr != NULL
+ *            and mask_nnz > 0 (the same rule for every entry point that takes a mask); otherwise it
+ *            is ignored, and with mask_nnz == 0 mask_cols and mask_vals may be NULL.  mask_nnz < 0
+ *            with a mode set is CCR_EINVAL
  *   id_offset added to local item ids on output (row-sharded tables)
  *   out_scores   [B, k] float32, descending           (may be NULL)
  *   out_scores64 [B, k] float64 exact value the order was decided on (may be NULL)
