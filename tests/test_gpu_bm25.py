@@ -14,6 +14,7 @@ import torch
 
 import cases
 from oracle import ccr_oracle as O
+from select_oracle import lever  # noqa: F401  (fixture)
 
 pytestmark = pytest.mark.gpu
 
@@ -74,17 +75,11 @@ def _synthetic(seed, n, q, vocab, doc_len):
 
 
 @pytest.fixture(params=["auto", "blockwide"])
-def bm25_kernel(request):
+def bm25_kernel(request, lever):
     """auto: queries of <= 32 distinct terms take the warp-private kernel, longer ones the block-wide
     kernel (the batches below hold both kinds); blockwide: everything on the block-wide kernel."""
-    from ccr_b200 import _lib
-
-    if request.param == "blockwide":
-        os.environ["CCR_BM25_BLOCKWIDE"] = "1"
-        _lib.reload_env()
-    yield request.param
-    os.environ.pop("CCR_BM25_BLOCKWIDE", None)
-    _lib.reload_env()
+    lever(CCR_BM25_BLOCKWIDE="1" if request.param == "blockwide" else None)
+    return request.param
 
 
 @pytest.mark.parametrize("n,q,k", [(40000, 40, 1001), (150000, 300, 100), (9000, 700, 10)])

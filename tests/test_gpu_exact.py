@@ -8,6 +8,7 @@ import torch
 
 import cases
 from oracle import ccr_oracle as O
+from select_oracle import lever, levers  # noqa: F401  (fixture)
 from test_gpu_parity import CASES, _mask  # the parity shapes
 
 pytestmark = pytest.mark.gpu
@@ -21,19 +22,6 @@ def ccr():
 
     assert torch.cuda.is_available()
     return ccr_b200
-
-
-@pytest.fixture
-def lever(monkeypatch):
-    from ccr_b200 import _lib
-
-    def setenv(name, value):
-        monkeypatch.setenv(name, value)
-        _lib.reload_env()
-
-    yield setenv
-    monkeypatch.undo()
-    _lib.reload_env()
 
 
 def _rows32(table, q32):
@@ -114,7 +102,7 @@ def test_exact_matches_float64_oracle(ccr, scan, algo, B, N, D, k, mode, sim, le
     check_exact(table, q32, k, mask, s, i, d)
     print(f"{scan} algo={algo} B={B} N={N} k={k}: {n_fb} fallback rows")
     # forced fallback: every row through the dense scan + compaction + re-rank, bit-identical
-    lever("CCR_EXACT_FALLBACK", "1")
+    lever(CCR_EXACT_FALLBACK="1")
     s2, i2, d2, n_fb2 = table._search_exact(q32, k, mask=mask, algo=algo, want_f64=True, encoded=True)
     assert n_fb2 == B
     assert torch.equal(i, i2) and torch.equal(d, d2) and torch.equal(s, s2)
@@ -398,19 +386,9 @@ def test_exact_bench_workload_fp16(ccr, lever):
     del s64, s32, val
     for name, value in (("CCR_2CTA", "0"), ("CCR_2CTA", "1"), ("CCR_LEAD", "4"), ("CCR_NO_HIST", "1"),
                         ("CCR_EXACT_FALLBACK", "1")):
-        lever(name, value)
-        s2, i2, d2, _ = table._search_exact(q32, k, mask=mask, want_f64=True, encoded=True)
+        with levers(**{name: value}):
+            s2, i2, d2, _ = table._search_exact(q32, k, mask=mask, want_f64=True, encoded=True)
         assert torch.equal(i, i2) and torch.equal(d, d2) and torch.equal(s, s2), (name, value)
-        os_env_pop(name)
-
-
-def os_env_pop(name):
-    import os
-
-    from ccr_b200 import _lib
-
-    os.environ.pop(name, None)
-    _lib.reload_env()
 
 
 @pytest.mark.parametrize("world", [2, 4, 8])

@@ -11,7 +11,9 @@ import torch
 
 import cases
 import f16_ref
+import select_oracle as SO
 from oracle import ccr_oracle as O
+from select_oracle import lever, levers  # noqa: F401  (fixture)
 from test_gpu_parity import CASES, SEEDED_CASES, _mask  # the same shapes as the bf16 parity tests
 
 pytestmark = pytest.mark.gpu
@@ -29,24 +31,6 @@ def ccr():
     return ccr_b200
 
 
-@pytest.fixture
-def knobs(monkeypatch):
-    """Set CCR_* test levers for one test and make the library re-read them (before and after)."""
-    from ccr_b200 import _lib
-
-    def setenv(**kv):
-        for key, v in kv.items():
-            if v is None:
-                monkeypatch.delenv(key, raising=False)
-            else:
-                monkeypatch.setenv(key, v)
-        _lib.reload_env()
-
-    yield setenv
-    monkeypatch.undo()
-    _lib.reload_env()
-
-
 @pytest.mark.parametrize("algo", [1, 2])
 @pytest.mark.parametrize("B,N,D,k,mode,sim", CASES)
 def test_f16_score_topk_matches_oracle(ccr, algo, B, N, D, k, mode, sim):
@@ -57,18 +41,21 @@ def test_f16_score_topk_matches_oracle(ccr, algo, B, N, D, k, mode, sim):
     table = ccr.EmbeddingTable.from_tensor(torch.as_tensor(P), device=dev, normalize=(sim == "cos"), dtype=F16)
     assert table.dtype == F16 and table.data.dtype == F16
     mask = _mask(rs, B, N, mode, dev, ccr) if mode != O.MASK_NONE else None
-    s, i, d = table.search(torch.as_tensor(Q), k, mask=mask, algo=algo, want_f64=True)
+    q = table.encode_queries(torch.as_tensor(Q))
+    s, i, d = table.search(q, k, mask=mask, algo=algo, want_f64=True, encoded=True)
     torch.cuda.synchronize()
     full = f16_ref.full_scores_ref_f16(Q, P, mask=mask.host if mask else None, mode=mode, sim=sim).numpy()
     live = np.abs(f16_ref.full_scores_ref_f16(Q, P, sim=sim).numpy()).max()
     errs = O.check_topk(d.cpu().numpy(), i.cpu().numpy(), full_scores=full, rtol=RTOL, atol=RTOL * float(live))
     assert not errs, errs[:5]
     np.testing.assert_allclose(s.cpu().numpy(), d.cpu().numpy().astype(np.float32), rtol=1e-6)
+    errs = SO.check_kernel(algo, s, i, d, q, table.data, table.ld, k, mask, n_items=N)
+    assert not errs, errs
 
 
 @pytest.mark.parametrize("B,N,D,k,mode,sim,two", SEEDED_CASES)
-def test_f16_seeded_pair_throttle_paths_match_oracle(ccr, B, N, D, k, mode, sim, two, knobs):
-    knobs(CCR_2CTA=two, CCR_NO_HIST=None)
+def test_f16_seeded_pair_throttle_paths_match_oracle(ccr, B, N, D, k, mode, sim, two, lever):
+    lever(CCR_2CTA=two, CCR_NO_HIST=None)
     dev = torch.device("cuda:0")
     rs = np.random.RandomState(B + k)
     P = cases.embeddings(B * 7 + k, N, D, clustered=(sim == "cos"))
@@ -76,7 +63,8 @@ def test_f16_seeded_pair_throttle_paths_match_oracle(ccr, B, N, D, k, mode, sim,
     P[rs.randint(0, N, size=2000)] = P[rs.randint(0, N, size=2000)]  # some exact ties
     table = ccr.EmbeddingTable.from_tensor(torch.as_tensor(P), device=dev, normalize=(sim == "cos"), dtype=F16)
     mask = _mask(rs, B, N, mode, dev, ccr) if mode != O.MASK_NONE else None
-    s, i, d = table.search(torch.as_tensor(Q), k, mask=mask, algo=2, want_f64=True)
+    q = table.encode_queries(torch.as_tensor(Q))
+    s, i, d = table.search(q, k, mask=mask, algo=2, want_f64=True, encoded=True)
     torch.cuda.synchronize()
     rs_, ri_ = f16_ref.score_topk_ref_f16(Q, P, k, mask=mask.host if mask else None, mode=mode, sim=sim)
     plain = np.abs(rs_.numpy())
@@ -84,10 +72,12 @@ def test_f16_seeded_pair_throttle_paths_match_oracle(ccr, B, N, D, k, mode, sim,
     errs = O.check_topk(d.cpu().numpy(), i.cpu().numpy(), ref_scores=rs_.numpy(), ref_ids=ri_.numpy(), rtol=RTOL,
                         atol=RTOL * live)
     assert not errs, errs[:3]
+    errs = SO.check_kernel(2, s, i, d, q, table.data, table.ld, k, mask, n_items=N)
+    assert not errs, errs
     # histogram sharing changes scheduling only
-    knobs(CCR_NO_HIST="1")
-    s0, i0, d0 = table.search(torch.as_tensor(Q), k, mask=mask, algo=2, want_f64=True)
-    assert torch.equal(i, i0) and torch.equal(d, d0)
+    lever(CCR_NO_HIST="1")
+    s0, i0, d0 = table.search(q, k, mask=mask, algo=2, want_f64=True, encoded=True)
+    assert torch.equal(i, i0) and torch.equal(d.view(torch.int64), d0.view(torch.int64))
 
 
 def test_f16_bench_workload_every_row(ccr):
@@ -125,15 +115,9 @@ def test_f16_bench_workload_every_row(ccr):
     rows_of = np.repeat(np.arange(B), np.diff(indptr))
     assert not (i.cpu().numpy()[rows_of] == cols[:, None].astype(np.int64)).any()  # no blocked id
     for env in ({"CCR_LEAD": "4"}, {"CCR_2CTA": "0"}, {"CCR_NO_HIST": "1"}):
-        os.environ.update(env)
-        _lib.reload_env()
-        try:
+        with levers(**env):
             s2, i2, d2 = ccr.score_topk(q, table.data, k, mask=mask, n_items=N, D=table.ld, want_f64=True)
-            assert torch.equal(i, i2) and torch.equal(d, d2), env
-        finally:
-            for key in env:
-                del os.environ[key]
-            _lib.reload_env()
+        assert torch.equal(i, i2) and torch.equal(d, d2), env
     del table
     torch.cuda.empty_cache()
 

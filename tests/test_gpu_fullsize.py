@@ -22,6 +22,7 @@ import torch
 
 import cases
 from oracle import ccr_oracle as O
+from select_oracle import levers
 
 pytestmark = pytest.mark.gpu
 
@@ -98,15 +99,9 @@ def test_bench_workload_every_row_vs_fp32_oracle(ccr, bench, big):
     assert not hit
     # the throttle lead, the single-CTA variant and histogram sharing change scheduling only: same bits
     for env in ({"CCR_LEAD": "4"}, {"CCR_2CTA": "0"}, {"CCR_NO_HIST": "1"}):
-        os.environ.update(env)
-        _lib.reload_env()
-        try:
+        with levers(**env):
             s2, i2, d2 = ccr.score_topk(q, big.data, k, mask=mask, n_items=N_MARCO, D=big.ld, want_f64=True)
-            assert torch.equal(i, i2) and torch.equal(d, d2), env
-        finally:
-            for key in env:
-                del os.environ[key]
-            _lib.reload_env()
+        assert torch.equal(i, i2) and torch.equal(d, d2), env
 
 
 def test_nq_shape_k1001_vs_fp32_oracle(ccr, bench, big):

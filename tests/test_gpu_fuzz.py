@@ -1,23 +1,28 @@
 """Randomised small-shape parity sweep through the C ABI against the CPU oracle: tile-boundary
 batch / corpus sizes, odd dims, k up to N, light and heavy masks (include and exclude modes),
-SET and ADD (positive priors), dot and cos, both kernels, 1-CTA and 2-CTA tensor-core variants."""
+SET and ADD (positive priors), dot and cos, bf16 and fp16 tables, both kernels, 1-CTA and 2-CTA tensor-core
+variants; besides the tolerance rule, every case is checked bit-exactly (tensor-core kernel) or against the fp32
+summation bound (CUDA-core kernel) by select_oracle."""
 import numpy as np
 import pytest
 import torch
 
 import cases
+import f16_ref
+import select_oracle as SO
 from oracle import ccr_oracle as O
+from select_oracle import lever  # noqa: F401  (fixture)
 
 pytestmark = pytest.mark.gpu
 
 
-def _one_case(ccr, rs, B, N, D, k, mode, heavy, sim, algo):
+def _one_case(ccr, rs, B, N, D, k, mode, heavy, sim, algo, dtype):
     dev = torch.device("cuda:0")
     P = cases.embeddings(int(rs.randint(1 << 30)), N, D, clustered=(sim == "cos"))
     Q = cases.embeddings(int(rs.randint(1 << 30)), B, D, clustered=(sim == "cos"))
     if rs.rand() < 0.3:  # exact ties: duplicate some items
         P[rs.randint(0, N, size=N // 4)] = P[rs.randint(0, N, size=N // 4)]
-    table = ccr.EmbeddingTable.from_tensor(torch.as_tensor(P), device=dev, normalize=(sim == "cos"))
+    table = ccr.EmbeddingTable.from_tensor(torch.as_tensor(P), device=dev, normalize=(sim == "cos"), dtype=dtype)
     mask = None
     if mode != O.MASK_NONE:
         hi = min(N, 600 if heavy else 40)
@@ -29,9 +34,14 @@ def _one_case(ccr, rs, B, N, D, k, mode, heavy, sim, algo):
             cols = np.concatenate([np.sort(r) for r in rows]) if B else np.zeros(0)
             vals = np.where(rs.rand(len(cols)) < 0.5, -1e10, rs.choice([1.0, 1e5], size=len(cols)))
             mask = ccr.SparseMask(indptr, cols, vals, N, ccr.MASK_ADD, dev)
-    s, i, d = table.search(torch.as_tensor(Q), k, mask=mask, algo=algo, want_f64=True)
+    q = table.encode_queries(torch.as_tensor(Q))
+    s, i, d = table.search(q, k, mask=mask, algo=algo, want_f64=True, encoded=True)
     torch.cuda.synchronize()
-    full = O.full_scores_ref(Q, P, mask=mask.host if mask else None, mode=mode, sim=sim).numpy()
+    errs = SO.check_kernel(algo, s, i, d, q, table.data, table.ld, k, mask, n_items=N)
+    if errs:
+        return errs
+    ref = f16_ref.full_scores_ref_f16 if dtype == torch.float16 else O.full_scores_ref
+    full = ref(Q, P, mask=mask.host if mask else None, mode=mode, sim=sim).numpy()
     # cos: the fp32 norm is summed in a different order than torch's, so a normalised element can land
     # on the other side of a bf16 rounding boundary (1 bf16 ulp of one factor) -> absolute slack on the
     # unit-scale cos scores; dot: the bf16 inputs are bit-identical, only fp32 summation order differs
@@ -41,7 +51,7 @@ def _one_case(ccr, rs, B, N, D, k, mode, heavy, sim, algo):
 
 
 @pytest.mark.parametrize("seed", range(6))
-def test_fuzz_against_oracle(seed, monkeypatch):
+def test_fuzz_against_oracle(seed, lever):
     import ccr_b200 as ccr
 
     rs = np.random.RandomState(1000 + seed)
@@ -56,6 +66,8 @@ def test_fuzz_against_oracle(seed, monkeypatch):
         sim = "cos" if rs.rand() < 0.25 else "dot"
         algo = int(rs.choice([1, 2, 2]))
         two = str(int(rs.rand() < 0.5))
-        monkeypatch.setenv("CCR_2CTA", two)
-        errs = _one_case(ccr, rs, B, N, D, k, mode, heavy, sim, algo)
-        assert not errs, (dict(B=B, N=N, D=D, k=k, mode=mode, heavy=heavy, sim=sim, algo=algo, two_cta=two), errs[:3])
+        dtype = torch.float16 if rs.rand() < 0.5 else torch.bfloat16
+        lever(CCR_2CTA=two)
+        errs = _one_case(ccr, rs, B, N, D, k, mode, heavy, sim, algo, dtype)
+        assert not errs, (dict(B=B, N=N, D=D, k=k, mode=mode, heavy=heavy, sim=sim, algo=algo, two_cta=two,
+                               dtype=dtype), errs[:3])

@@ -7,6 +7,8 @@ import numpy as np
 import pytest
 import torch
 
+from select_oracle import lever  # noqa: F401  (fixture)
+
 pytestmark = pytest.mark.gpu
 
 B, N, D, K = 4, 1024, 64, 8
@@ -20,19 +22,6 @@ def ccr():
 
     assert torch.cuda.is_available()
     return ccr_b200
-
-
-@pytest.fixture
-def lever(monkeypatch):
-    from ccr_b200 import _lib
-
-    def setenv(name, value):
-        monkeypatch.setenv(name, value)
-        _lib.reload_env()
-
-    yield setenv
-    monkeypatch.undo()
-    _lib.reload_env()
 
 
 @pytest.fixture(scope="module")
@@ -159,7 +148,7 @@ def test_dense_wrappers_empty_mask_equals_no_mask(ccr):
 @pytest.mark.parametrize("fallback", [False, True])
 def test_score_topk_exact_empty_mask_equals_no_mask(ccr, lever, fallback):
     if fallback:
-        lever("CCR_EXACT_FALLBACK", "1")
+        lever(CCR_EXACT_FALLBACK="1")
     rs = np.random.RandomState(13)
     P = torch.as_tensor(rs.standard_normal((3000, 128)).astype(np.float32))
     Q = torch.as_tensor(rs.standard_normal((5, 128)).astype(np.float32))

@@ -7,7 +7,9 @@ import scipy.sparse as sps
 import torch
 
 import cases
+import select_oracle as SO
 from oracle import ccr_oracle as O
+from select_oracle import lever  # noqa: F401  (fixture)
 
 pytestmark = pytest.mark.gpu
 
@@ -55,12 +57,15 @@ def test_score_topk_matches_oracle(ccr, algo, B, N, D, k, mode, sim):
     Q = cases.embeddings(N + 2, B, D, clustered=(sim == "cos"))
     table = ccr.EmbeddingTable.from_tensor(torch.as_tensor(P), device=dev, normalize=(sim == "cos"))
     mask = _mask(rs, B, N, mode, dev, ccr) if mode != O.MASK_NONE else None
-    s, i, d = table.search(torch.as_tensor(Q), k, mask=mask, algo=algo, want_f64=True)
+    q = table.encode_queries(torch.as_tensor(Q))
+    s, i, d = table.search(q, k, mask=mask, algo=algo, want_f64=True, encoded=True)
     torch.cuda.synchronize()
     full = O.full_scores_ref(Q, P, mask=mask.host if mask else None, mode=mode, sim=sim).numpy()
     errs = O.check_topk(d.cpu().numpy(), i.cpu().numpy(), full_scores=full, rtol=RTOL)
     assert not errs, errs[:5]
     np.testing.assert_allclose(s.cpu().numpy(), d.cpu().numpy().astype(np.float32), rtol=1e-6)
+    errs = SO.check_kernel(algo, s, i, d, q, table.data, table.ld, k, mask, n_items=N)
+    assert not errs, errs
 
 
 @pytest.mark.parametrize("algo", [1, 2])
@@ -310,9 +315,8 @@ SEEDED_CASES = [
 
 
 @pytest.mark.parametrize("B,N,D,k,mode,sim,two", SEEDED_CASES)
-def test_seeded_histogram_path_matches_oracle(ccr, B, N, D, k, mode, sim, two, monkeypatch):
-    if two is not None:
-        monkeypatch.setenv("CCR_2CTA", two)
+def test_seeded_histogram_path_matches_oracle(ccr, B, N, D, k, mode, sim, two, lever):
+    lever(CCR_2CTA=two, CCR_NO_HIST=None)
     dev = torch.device("cuda:0")
     rs = np.random.RandomState(B + k)
     P = cases.embeddings(B * 7 + k, N, D, clustered=(sim == "cos"))
@@ -320,16 +324,19 @@ def test_seeded_histogram_path_matches_oracle(ccr, B, N, D, k, mode, sim, two, m
     P[rs.randint(0, N, size=2000)] = P[rs.randint(0, N, size=2000)]  # some exact ties
     table = ccr.EmbeddingTable.from_tensor(torch.as_tensor(P), device=dev, normalize=(sim == "cos"))
     mask = _mask(rs, B, N, mode, dev, ccr) if mode != O.MASK_NONE else None
-    s, i, d = table.search(torch.as_tensor(Q), k, mask=mask, algo=2, want_f64=True)
+    q = table.encode_queries(torch.as_tensor(Q))
+    s, i, d = table.search(q, k, mask=mask, algo=2, want_f64=True, encoded=True)
     torch.cuda.synchronize()
     rs_, ri_ = O.score_topk_ref(Q, P, k, mask=mask.host if mask else None, mode=mode, sim=sim)
     errs = O.check_topk(d.cpu().numpy(), i.cpu().numpy(), ref_scores=rs_.numpy(), ref_ids=ri_.numpy(), rtol=RTOL,
                         atol=2e-3 if sim == "cos" else 1e-4)
     assert not errs, errs[:3]
+    errs = SO.check_kernel(2, s, i, d, q, table.data, table.ld, k, mask, n_items=N)
+    assert not errs, errs
     # and the histogram sharing must not change a single bit of the result
-    monkeypatch.setenv("CCR_NO_HIST", "1")
-    s0, i0, d0 = table.search(torch.as_tensor(Q), k, mask=mask, algo=2, want_f64=True)
-    assert torch.equal(i, i0) and torch.equal(d, d0)
+    lever(CCR_NO_HIST="1")
+    s0, i0, d0 = table.search(q, k, mask=mask, algo=2, want_f64=True, encoded=True)
+    assert torch.equal(i, i0) and torch.equal(d.view(torch.int64), d0.view(torch.int64))
 
 
 def test_seeded_path_degenerate_scores(ccr):

@@ -51,16 +51,14 @@ def test_planning_entry_points_work_without_gpu():
 def test_env_knobs_are_parsed_once_and_reloadable():
     from ccr_b200 import _lib
 
+    from select_oracle import levers
+
     base = _lib.plan_info(512, 8841823, 768, 100)
     assert base["two_cta"] == 1
-    os.environ["CCR_2CTA"] = "0"
-    try:
+    with levers(_reload=False, CCR_2CTA="0"):
         assert _lib.plan_info(512, 8841823, 768, 100)["two_cta"] == 1   # cached knobs: no effect yet
         _lib.reload_env()
         assert _lib.plan_info(512, 8841823, 768, 100)["two_cta"] == 0
-    finally:
-        del os.environ["CCR_2CTA"]
-        _lib.reload_env()
     assert _lib.plan_info(512, 8841823, 768, 100) == base
 
 
