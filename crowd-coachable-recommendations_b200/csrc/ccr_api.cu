@@ -88,7 +88,7 @@ struct Plan {
   size_t off_seed;
   size_t off_progress;
   size_t off_qpad;       // zero-padded copy of a short query batch (B < 128): every TMA box in bounds
-  size_t off_cand, off_counts, off_ovr_hi, off_ovr_lo, off_status, off_gtau, off_gq, off_hist, off_hpar, total;
+  size_t off_cand, off_counts, off_rec_hi, off_rec_lo, off_status, off_gtau, off_gq, off_hist, off_hpar, total;
 };
 
 size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -209,8 +209,8 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
   size_t off = 0;
   pl->off_cand = off;   off = align_up(off + (size_t)pl->rows_pad * pl->S * pl->halves * pl->C * sizeof(u64), 256);
   pl->off_counts = off; off = align_up(off + (size_t)pl->rows_pad * pl->S * pl->halves * sizeof(int), 256);
-  pl->off_ovr_hi = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u64), 256);
-  pl->off_ovr_lo = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u32), 256);
+  pl->off_rec_hi = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u64), 256);
+  pl->off_rec_lo = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u32), 256);
   // [off_status, off_qpad) is zeroed by ONE memset per call: status, throttle counters, sharing state
   pl->off_status = off; off = align_up(off + sizeof(DeviceStatus), 256);
   pl->off_progress = off; off = align_up(off + (size_t)pl->n_q_tiles * pl->S * sizeof(int), 256);
@@ -332,7 +332,7 @@ int ccr_plan_info(int64_t B, int64_t n_items, int D, int k, int64_t mask_nnz, in
   info8[4] = pl.two_cta;
   info8[5] = pl.seed_m;
   // kernels one ccr_score_topk_bf16 call launches: [seeding GEMM, seed select,] fused score+select,
-  // [mask overrides,] finalize  (memsets / the short-batch query copy are not kernels of this library)
+  // [mask-entry records,] finalize  (memsets / the short-batch query copy are not kernels of this library)
   info8[6] = (B > 0) ? (pl.seed_m > 0 ? 2 : 0) + (n_items > 0 ? 1 : 0) + (mask_nnz > 0 ? 1 : 0) + 1 : 0;
   info8[7] = pl.lead_tiles;
   return CCR_OK;
@@ -432,23 +432,25 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   }
   if (lr) return fail(CCR_ECUDA, "select kernel launch failed (%d: %s)", lr, lr > 0 ? cudaGetErrorString((cudaError_t)lr) : "tensor map");
 
+  // one record per mask entry: the record CSR is the mask CSR
+  u64* rec_hi = (u64*)(ws + pl.off_rec_hi);
+  u32* rec_lo = (u32*)(ws + pl.off_rec_lo);
   if (m.nnz > 0) {
-    OverrideParams op = {};
+    RecordParams rp = {};
+    rp.B = (int)B; rp.src = sp.f16 ? kRecF16Dot : kRecBf16Dot;
     // sp.q may be the padded staging block of a short batch: use ITS pitch (sp.ldq), not the caller's
-    op.q = sp.q; op.ldq = sp.ldq; op.B = (int)B; op.items = sp.items; op.ldi = ldi; op.n_items = n_items; op.D = D;
-    op.f16 = sp.f16;
-    op.mask_indptr = m.indptr; op.mask_cols = m.cols; op.mask_vals = m.vals; op.nnz = m.nnz;
-    op.mode = m.mode; op.ovr_hi = (u64*)(ws + pl.off_ovr_hi); op.ovr_lo = (u32*)(ws + pl.off_ovr_lo);
-    lr = launch_overrides(op, st);
-    if (lr) return fail(CCR_ECUDA, "override kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+    rp.q = sp.q; rp.ldq = sp.ldq; rp.items = sp.items; rp.ldi = ldi; rp.D = D; rp.n_cols = n_items;
+    rp.mask_indptr = m.indptr; rp.mask_cols = m.cols; rp.mask_vals = m.vals; rp.mode = m.mode;
+    rp.max_entries = m.nnz; rp.rec_hi = rec_hi; rp.rec_lo = rec_lo;
+    lr = launch_entry_records(rp, st);
+    if (lr) return fail(CCR_ECUDA, "mask record kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   }
 
   FinalizeParams fp = {};
   fp.B = (int)B; fp.k = k; fp.C = pl.C; fp.S = pl.S * pl.halves; fp.cand = sp.cand; fp.counts = sp.counts;
   fp.g_tau = sp.g_tau;
-  fp.drop_cols = pl.include_mask ? m.cols : nullptr;
-  fp.mask_indptr = m.indptr;
-  fp.ovr_hi = (u64*)(ws + pl.off_ovr_hi); fp.ovr_lo = (u32*)(ws + pl.off_ovr_lo);
+  fp.rec_indptr = m.indptr; fp.rec_hi = rec_hi; fp.rec_lo = rec_lo;
+  fp.drop_cols = pl.include_mask ? m.cols : nullptr;  // searched in the record CSR: the records are the mask entries
   fp.id_offset = id_offset; fp.out_scores = out_scores; fp.out_scores64 = out_scores64;
   fp.out_keys = nullptr;
   if (flags & CCR_FLAG_PACKED_KEYS) { fp.out_keys = (u64*)out_scores64; fp.out_scores64 = nullptr; }
@@ -622,7 +624,7 @@ int ccr_first_hit_rank(const int64_t* ids, int64_t B, int k, const int64_t* rel_
 }
 
 // ---- top-k of a materialised dense score matrix ----
-struct DensePlanC { int S, C; size_t off_counts, off_ovr_hi, off_ovr_lo, total; };
+struct DensePlanC { int S, C; size_t off_counts, off_rec_hi, off_rec_lo, total; };
 static void dense_plan(long long B, long long N, int k_keep, long long nnz, DensePlanC* pl) {
   const int sms = device_sm_count();
   const long long rows = B > 0 ? B : 1;
@@ -635,8 +637,8 @@ static void dense_plan(long long B, long long N, int k_keep, long long nnz, Dens
   pl->C = cand_capacity(k_keep, kDenseSlack);
   size_t off = align_up((size_t)rows * s * pl->C * sizeof(u64), 256);
   pl->off_counts = off; off = align_up(off + (size_t)rows * s * sizeof(int), 256);
-  pl->off_ovr_hi = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u64), 256);
-  pl->off_ovr_lo = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u32), 256);
+  pl->off_rec_hi = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u64), 256);
+  pl->off_rec_lo = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u32), 256);
   pl->total = off;
 }
 
@@ -672,17 +674,22 @@ int ccr_topk_dense_f32(const float* scores, int64_t B, int64_t n_cols, int64_t l
   cudaStream_t st = (cudaStream_t)stream;
   int lr = launch_select_dense(scores, ld, B, n_cols, k, (int)(k + h), m.indptr, pl.C, pl.S, (u64*)ws, (int*)(ws + pl.off_counts), st);
   if (lr) return fail(CCR_ECUDA, "dense select launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+  // one record per mask entry: the record CSR is the mask CSR
+  u64* rec_hi = (u64*)(ws + pl.off_rec_hi);
+  u32* rec_lo = (u32*)(ws + pl.off_rec_lo);
   if (m.indptr) {
-    lr = launch_override_dense(scores, ld, (int)B, n_cols, m.indptr, m.cols, m.vals, m.nnz, m.mode,
-                               (u64*)(ws + pl.off_ovr_hi), (u32*)(ws + pl.off_ovr_lo), st);
-    if (lr) return fail(CCR_ECUDA, "dense override launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+    RecordParams rp = {};
+    rp.B = (int)B; rp.src = kRecMatrix; rp.scores = scores; rp.ld = ld; rp.n_cols = n_cols;
+    rp.mask_indptr = m.indptr; rp.mask_cols = m.cols; rp.mask_vals = m.vals; rp.mode = m.mode;
+    rp.max_entries = m.nnz; rp.rec_hi = rec_hi; rp.rec_lo = rec_lo;
+    lr = launch_entry_records(rp, st);
+    if (lr) return fail(CCR_ECUDA, "dense mask record launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   }
   FinalizeParams fp = {};
   fp.B = (int)B; fp.k = k; fp.C = pl.C; fp.S = pl.S; fp.cand = (u64*)ws; fp.counts = (int*)(ws + pl.off_counts);
   fp.g_tau = nullptr;
-  fp.drop_cols = m.cols;
-  fp.mask_indptr = m.indptr;
-  fp.ovr_hi = (u64*)(ws + pl.off_ovr_hi); fp.ovr_lo = (u32*)(ws + pl.off_ovr_lo);
+  fp.rec_indptr = m.indptr; fp.rec_hi = rec_hi; fp.rec_lo = rec_lo;
+  fp.drop_cols = m.cols;  // searched in the record CSR: the records are the mask entries
   fp.id_offset = 0; fp.out_keys = nullptr; fp.out_scores = out_scores; fp.out_scores64 = out_scores64; fp.out_ids = (long long*)out_ids;
   lr = launch_finalize(fp, st);
   if (lr) return fail(CCR_ECUDA, "finalize launch failed: %s", cudaGetErrorString((cudaError_t)lr));
@@ -816,7 +823,7 @@ int ccr_bm25_topk(const int64_t* post_indptr, const int32_t* post_docs, const do
   if (lr) return fail(CCR_ECUDA, "bm25 top-k launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   FinalizeParams fp = {};
   fp.B = (int)Bq; fp.k = k; fp.C = pl.C; fp.S = pl.streams; fp.cand = cand; fp.counts = counts;
-  fp.g_tau = warp ? row_tau : nullptr; fp.drop_cols = nullptr; fp.mask_indptr = nullptr; fp.ovr_hi = nullptr; fp.ovr_lo = nullptr;
+  fp.g_tau = warp ? row_tau : nullptr; fp.rec_indptr = nullptr; fp.rec_hi = nullptr; fp.rec_lo = nullptr; fp.drop_cols = nullptr;
   fp.id_offset = 0; fp.out_keys = nullptr; fp.out_scores = out_scores; fp.out_scores64 = nullptr; fp.out_ids = (long long*)out_ids;
   lr = launch_finalize(fp, st);
   if (lr) return fail(CCR_ECUDA, "finalize launch failed: %s", cudaGetErrorString((cudaError_t)lr));
@@ -849,13 +856,13 @@ int ccr_bm25_scores_f64(const int64_t* post_indptr, const int32_t* post_docs, co
 
 // ---- exact fp32 ranking (DESIGN.md section 6b) ----
 namespace {
-struct ExactLayout { size_t off_scores, off_ids, off_neg, off_ent_ip, off_hi, off_lo, total; };
+struct ExactLayout { size_t off_scores, off_ids, off_neg, off_rec_ip, off_rec_hi, off_rec_lo, total; };
 
-// entry records after `off`: B + 1 row offsets, then 12 bytes per entry
+// entry records after `off`: the record CSR (B + 1 row offsets), then 12 bytes per entry
 void entry_layout(size_t off, long long B, long long n_entries, ExactLayout* L) {
-  L->off_ent_ip = off; off = align_up(off + (size_t)(B + 1) * sizeof(long long), 256);
-  L->off_hi = off;     off = align_up(off + (size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u64), 256);
-  L->off_lo = off;     off = align_up(off + (size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u32), 256);
+  L->off_rec_ip = off; off = align_up(off + (size_t)(B + 1) * sizeof(long long), 256);
+  L->off_rec_hi = off; off = align_up(off + (size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u64), 256);
+  L->off_rec_lo = off; off = align_up(off + (size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u32), 256);
   L->total = off;
 }
 
@@ -879,17 +886,18 @@ int rerank(const float* q, long long B, long long ldq, const float* items, long 
            int k, const long long* cand_indptr, const long long* cand_ids, long long cand_stride, long long cand_nnz,
            const MaskArgs& m, long long id_offset, float* out_scores, double* out_scores64, long long* out_ids,
            unsigned char* ws, const ExactLayout& L, cudaStream_t st) {
-  ExactParams ep = {};
-  ep.q = q; ep.ldq = ldq; ep.B = (int)B; ep.items = items; ep.ldi = ldi; ep.n_items = n_items; ep.D = D;
-  ep.cand_indptr = cand_indptr; ep.cand_ids = cand_ids; ep.cand_stride = cand_stride;
-  ep.mask_indptr = m.indptr; ep.mask_cols = m.cols; ep.mask_vals = m.vals; ep.mode = m.mode;
-  ep.ent_indptr = (const long long*)(ws + L.off_ent_ip); ep.max_entries = cand_nnz + m.nnz;
-  ep.ent_hi = (u64*)(ws + L.off_hi); ep.ent_lo = (u32*)(ws + L.off_lo);
-  int lr = launch_exact_entries(ep, st);
+  RecordParams rp = {};
+  rp.B = (int)B; rp.src = kRecExactDot; rp.q = q; rp.ldq = ldq; rp.items = items; rp.ldi = ldi; rp.D = D;
+  rp.n_cols = n_items;
+  rp.mask_indptr = m.indptr; rp.mask_cols = m.cols; rp.mask_vals = m.vals; rp.mode = m.mode;
+  rp.cand_indptr = cand_indptr; rp.cand_ids = cand_ids; rp.cand_stride = cand_stride;
+  rp.rec_indptr = (long long*)(ws + L.off_rec_ip); rp.max_entries = cand_nnz + m.nnz;
+  rp.rec_hi = (u64*)(ws + L.off_rec_hi); rp.rec_lo = (u32*)(ws + L.off_rec_lo);
+  int lr = launch_entry_records(rp, st);
   if (lr) return fail(CCR_ECUDA, "exact value kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
   FinalizeParams fp = {};
   fp.B = (int)B; fp.k = k; fp.C = 0; fp.S = 0; fp.cand = nullptr; fp.counts = nullptr; fp.g_tau = nullptr;
-  fp.drop_cols = nullptr; fp.mask_indptr = ep.ent_indptr; fp.ovr_hi = ep.ent_hi; fp.ovr_lo = ep.ent_lo;
+  fp.rec_indptr = rp.rec_indptr; fp.rec_hi = rp.rec_hi; fp.rec_lo = rp.rec_lo; fp.drop_cols = nullptr;
   fp.id_offset = id_offset; fp.out_scores = out_scores; fp.out_scores64 = out_scores64; fp.out_keys = nullptr;
   fp.out_ids = out_ids;
   lr = launch_finalize(fp, st);

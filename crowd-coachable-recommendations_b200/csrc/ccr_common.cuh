@@ -1,12 +1,12 @@
-// Shared device helpers: sortable keys; the 256-bin histogram select steps every top-k path
-// uses; warp-cooperative selection on candidate buffers (exact radix select, in-place
-// compaction, approximate histogram prune); small PTX wrappers.
+// Shared device helpers: sortable keys; mask lookup, CSR row lookup and the mask value rule; the
+// 256-bin histogram select steps every top-k path uses; warp-cooperative selection on candidate
+// buffers (exact radix select, in-place compaction, approximate histogram prune); small PTX wrappers.
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-
+#include "../../include/ccr_b200.h"
 namespace ccr {
 
 typedef unsigned long long u64;
@@ -461,5 +461,21 @@ struct DeviceStatus {
   int block;
   int extra;
 };
+
+// ---------------------------------------------------------------------------------------
+// sparse rows: CSR row lookup and the value rule of mask entries
+// ---------------------------------------------------------------------------------------
+// row of flat entry e of a CSR with n_rows rows: the largest r with indptr[r] <= e (indptr[0] <= e < indptr[n_rows])
+template <typename I>
+__device__ __forceinline__ I csr_row_of(const long long* __restrict__ indptr, I n_rows, long long e) {
+  I lo = 0, hi = n_rows;  // invariant: indptr[lo] <= e < indptr[hi]
+  while (hi - lo > 1) { const I mid = (lo + hi) >> 1; if (indptr[mid] <= e) lo = mid; else hi = mid; }
+  return lo;
+}
+
+// the value a mask entry ranks by: CCR_MASK_SET the mask value, CCR_MASK_ADD double(score) + value
+__device__ __forceinline__ double mask_value(int mode, float score, double v) {
+  return mode == CCR_MASK_SET ? v : (double)score + v;
+}
 
 }  // namespace ccr

@@ -1,92 +1,11 @@
-// Exact fp32 ranking (DESIGN.md section 6b): the stages around the unchanged scan kernels.
-//   exact_entries_kernel : exact value of every (row, candidate) and (row, mask entry) pair, written as
-//                          finalize_kernel's 96-bit records; finalize then selects and sorts them
+// Exact fp32 ranking (DESIGN.md section 6b): the stages around the unchanged scan kernels and the
+// exact re-rank (entry_records_kernel with the ExactDot source + finalize_kernel, ccr_kernels.cu).
 //   certify_kernel       : per row, does the k-th exact value beat every item the scan stage left out?
 //   compact_kernel       : columns of a dense scan-score block at or above a per-row threshold, as a CSR
 //   row_norm_max_kernel  : largest fp32 row norm of an appended batch (the V of the error bound)
 #include "ccr_params.cuh"
 
 namespace ccr {
-
-// sum of a[i] * b[i] over i < D in float64; the order depends on D only (lane-strided float4 chunks, then
-// a butterfly that leaves the same sum in every lane).  Products of two fp32 values are exact in float64.
-__device__ __forceinline__ double dot_f64(const float* __restrict__ a, const float* __restrict__ b, int D, int lane) {
-  double acc = 0.0;
-  for (int c = lane; c < (D >> 2); c += 32) {
-    const float4 x = *reinterpret_cast<const float4*>(a + c * 4);
-    const float4 y = __ldg(reinterpret_cast<const float4*>(b + c * 4));
-    acc = fma((double)x.x, (double)y.x, acc);
-    acc = fma((double)x.y, (double)y.y, acc);
-    acc = fma((double)x.z, (double)y.z, acc);
-    acc = fma((double)x.w, (double)y.w, acc);
-  }
-#pragma unroll
-  for (int off = 16; off; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-  return acc;
-}
-
-__global__ void entry_indptr_kernel(ExactParams p) {
-  const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (r > p.B) return;
-  const long long c = p.cand_indptr ? p.cand_indptr[r] : r * p.cand_stride;
-  const long long m = p.mask_indptr ? p.mask_indptr[r] : 0;
-  const_cast<long long*>(p.ent_indptr)[r] = c + m;
-}
-
-// One warp per entry.  Row r's entries: its candidates, then its mask entries.
-//   candidate (not in the mask)  fp32(q . v in float64)
-//   SET mask entry               the mask value
-//   ADD mask entry               double(fp32(q . v in float64)) + value
-__global__ void __launch_bounds__(256) exact_entries_kernel(ExactParams p) {
-  const int lane = threadIdx.x & 31;
-  const long long e = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
-  if (e >= p.max_entries || e >= p.ent_indptr[p.B]) return;
-  int lo = 0, hi = p.B;  // invariant: ent_indptr[lo] <= e < ent_indptr[hi]
-  while (hi - lo > 1) {
-    const int mid = (lo + hi) >> 1;
-    if (p.ent_indptr[mid] <= e) lo = mid; else hi = mid;
-  }
-  const int row = lo;
-  const long long c0 = p.cand_indptr ? p.cand_indptr[row] : row * p.cand_stride;
-  const long long c1 = p.cand_indptr ? p.cand_indptr[row + 1] : (row + 1) * p.cand_stride;
-  const long long m0 = p.mask_indptr ? p.mask_indptr[row] : 0;
-  const long long m1 = p.mask_indptr ? p.mask_indptr[row + 1] : 0;
-  const long long j = e - p.ent_indptr[row];
-  long long col;
-  long long me = -1;  // mask entry, or -1 for a candidate
-  if (j < c1 - c0) {
-    col = p.cand_ids[c0 + j];
-    if (col >= 0 && col < p.n_items && p.mask_indptr && mask_contains(p.mask_cols, m0, m1, (int)col)) col = -1;
-  } else {
-    me = m0 + (j - (c1 - c0));
-    col = p.mask_cols[me];
-  }
-  if (col < 0 || col >= p.n_items) {
-    if (lane == 0) { p.ent_hi[e] = 0ull; p.ent_lo[e] = 0u; }  // ignored by finalize (hi == 0)
-    return;
-  }
-  double val;
-  if (me >= 0 && p.mode == 1 /* CCR_MASK_SET */) {
-    val = p.mask_vals[me];
-  } else {
-    val = (double)(float)dot_f64(p.q + (long long)row * p.ldq, p.items + col * p.ldi, p.D, lane);
-    if (me >= 0) val += p.mask_vals[me];
-  }
-  if (lane == 0) {
-    const u64 h = ord64(val);
-    p.ent_hi[e] = h ? h : 1ull;  // 0 is reserved for "skipped"
-    p.ent_lo[e] = 0xFFFFFFFFu - (u32)col;
-  }
-}
-
-int launch_exact_entries(const ExactParams& p, cudaStream_t st) {
-  if (p.B <= 0) return 0;
-  entry_indptr_kernel<<<(unsigned)((p.B + 256) / 256), 256, 0, st>>>(p);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess || p.max_entries <= 0) return (int)e;
-  exact_entries_kernel<<<(unsigned)((p.max_entries + 7) / 8), 256, 0, st>>>(p);
-  return (int)cudaGetLastError();
-}
 
 // One warp per row.  Certified when the scan stage returned every item (k_cand == n_items), fewer than
 // k_cand unmasked items (every unmasked item), or when the k-th exact value L_k beats RU(t + E) strictly,

@@ -1,8 +1,8 @@
 // CUDA-core kernels of the score-and-rank path:
 //   select_simt_kernel  : streaming score + mask-exclusion + running top-k, B <= 8 rows per pass
 //                         (bandwidth-bound small-query-batch regime; 128-bit coalesced loads)
-//   override_kernel     : exact scores of the sparse mask entries (set / add in float64)
-//   finalize_kernel     : per row, exact top-k of (unit candidates U mask overrides), sorted
+//   entry_records_kernel: finalize's records of mask entries (and exact-path candidates), float64 values
+//   finalize_kernel     : per row, exact top-k of (unit candidates U entry records), sorted
 //   merge_topk_kernel   : G-way merge of per-shard sorted lists (multi-GPU exchange step)
 //   ingest / normalize / dense helpers
 #include "ccr_params.cuh"
@@ -156,32 +156,20 @@ int launch_select_simt(const SelectParams& p, cudaStream_t st) {
 }
 
 // =======================================================================================
-// Mask overrides: one warp per CSR entry.  value = set ? v : double(q.item) + v.
+// Entry records (RecordParams): finalize's 96-bit records of the mask entries of the fused and
+// dense paths, and of the candidates and mask entries of the exact re-rank.  The kernel owns the
+// row lookup, the skip rules, the value rule and the record format; a score source supplies only
+// the fp32 score of (row, col) and how many lanes compute it together (kLanes, 1 or 32).
 // =======================================================================================
+// 2-byte table rows, one warp per entry: lane-strided 8-element chunks, fmaf in element order, then
+// the xor butterfly (tests/select_oracle.py: override_values repeats this order bit for bit)
 template <typename T>
-__global__ void __launch_bounds__(256) override_kernel(OverrideParams p) {
-  const int lane = threadIdx.x & 31;
-  const long long e = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
-  if (e >= p.nnz || e >= p.mask_indptr[p.B]) return;  // nnz may be an upper bound of indptr[B]
-  // row of entry e: largest r with indptr[r] <= e
-  int lo = 0, hi = p.B;  // invariant: indptr[lo] <= e < indptr[hi]
-  while (hi - lo > 1) {
-    int mid = (lo + hi) >> 1;
-    if (p.mask_indptr[mid] <= e) lo = mid; else hi = mid;
-  }
-  const int row = lo;
-  const int col = p.mask_cols[e];
-  double val;
-  if (col < 0 || (long long)col >= p.n_items) {
-    if (lane == 0) { p.ovr_hi[e] = 0ull; p.ovr_lo[e] = 0u; }  // ignored by finalize (hi == 0)
-    return;
-  }
-  if (p.mode == 1) {
-    val = p.mask_vals[e];
-  } else {
+struct TableDot {
+  static constexpr int kLanes = 32;
+  static __device__ __forceinline__ float score(const RecordParams& p, int row, long long col, int lane) {
+    const T* qr = reinterpret_cast<const T*>(p.q) + (long long)row * p.ldq;
+    const T* ir = reinterpret_cast<const T*>(p.items) + col * p.ldi;
     float acc = 0.f;
-    const __nv_bfloat16* qr = p.q + (long long)row * p.ldq;
-    const __nv_bfloat16* ir = p.items + (long long)col * p.ldi;
     for (int c = lane; c < (p.D >> 3); c += 32) {
       uint4 a = *reinterpret_cast<const uint4*>(qr + c * 8);
       uint4 b = ldg_nc_v4(ir + c * 8);
@@ -192,31 +180,117 @@ __global__ void __launch_bounds__(256) override_kernel(OverrideParams p) {
     }
 #pragma unroll
     for (int off = 16; off; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-    val = (double)acc + p.mask_vals[e];
+    return acc;
   }
+};
+
+// sum of a[i] * b[i] over i < D in float64; the order depends on D only (lane-strided float4 chunks, then
+// a butterfly that leaves the same sum in every lane).  Products of two fp32 values are exact in float64.
+__device__ __forceinline__ double dot_f64(const float* __restrict__ a, const float* __restrict__ b, int D, int lane) {
+  double acc = 0.0;
+  for (int c = lane; c < (D >> 2); c += 32) {
+    const float4 x = *reinterpret_cast<const float4*>(a + c * 4);
+    const float4 y = __ldg(reinterpret_cast<const float4*>(b + c * 4));
+    acc = fma((double)x.x, (double)y.x, acc);
+    acc = fma((double)x.y, (double)y.y, acc);
+    acc = fma((double)x.z, (double)y.z, acc);
+    acc = fma((double)x.w, (double)y.w, acc);
+  }
+#pragma unroll
+  for (int off = 16; off; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+  return acc;
+}
+
+// fp32 rows of an exact table, one warp per entry: fp32(q . v summed in float64)
+struct ExactDot {
+  static constexpr int kLanes = 32;
+  static __device__ __forceinline__ float score(const RecordParams& p, int row, long long col, int lane) {
+    return (float)dot_f64(reinterpret_cast<const float*>(p.q) + (long long)row * p.ldq,
+                          reinterpret_cast<const float*>(p.items) + col * p.ldi, p.D, lane);
+  }
+};
+
+// materialised score matrix, one thread per entry
+struct ScoreMatrix {
+  static constexpr int kLanes = 1;
+  static __device__ __forceinline__ float score(const RecordParams& p, int row, long long col, int) {
+    return __ldg(p.scores + (long long)row * p.ld + col);
+  }
+};
+
+// at least 8 blocks of 256 per SM: <= 32 registers, so all 64 warps of an SM gather rows (ptxas would give
+// ExactDot 40 registers and 48 warps otherwise)
+template <class Src>
+__global__ void __launch_bounds__(256, 8) entry_records_kernel(RecordParams p) {
+  const int lane = threadIdx.x % Src::kLanes;
+  const long long e = (long long)blockIdx.x * (256 / Src::kLanes) + threadIdx.x / Src::kLanes;
+  const long long* ip = p.rec_indptr ? p.rec_indptr : p.mask_indptr;
+  if (e >= p.max_entries || e >= ip[p.B]) return;  // max_entries may be an upper bound of ip[B]
+  const int row = csr_row_of(ip, p.B, e);
+  const long long j = e - ip[row];
+  long long c0 = 0, nc = 0;  // the row's candidates: cand_ids[c0, c0 + nc)
+  if (p.rec_indptr) {
+    c0 = p.cand_indptr ? p.cand_indptr[row] : row * p.cand_stride;
+    nc = (p.cand_indptr ? p.cand_indptr[row + 1] : (row + 1) * p.cand_stride) - c0;
+  }
+  const long long m0 = p.mask_indptr ? p.mask_indptr[row] : 0;
+  const long long me = j < nc ? -1 : m0 + (j - nc);  // mask entry, or -1 for a candidate
+  const long long col = me < 0 ? p.cand_ids[c0 + j] : p.mask_cols[me];
+  bool skip = col < 0 || col >= p.n_cols;
+  if (!skip && me < 0 && p.mask_indptr) skip = mask_contains(p.mask_cols, m0, p.mask_indptr[row + 1], (int)col);
+  if (skip) {
+    if (lane == 0) { p.rec_hi[e] = 0ull; p.rec_lo[e] = 0u; }  // ignored by finalize (hi == 0)
+    return;
+  }
+  const float s = (me >= 0 && p.mode == CCR_MASK_SET) ? 0.f : Src::score(p, row, col, lane);
+  const double val = me < 0 ? (double)s : mask_value(p.mode, s, p.mask_vals[me]);
   if (lane == 0) {
-    u64 h = ord64(val);
-    p.ovr_hi[e] = h ? h : 1ull;  // 0 is reserved for "invalid"
-    p.ovr_lo[e] = 0xFFFFFFFFu - (u32)col;
+    const u64 h = ord64(val);
+    p.rec_hi[e] = h ? h : 1ull;  // 0 is reserved for "skipped"
+    p.rec_lo[e] = 0xFFFFFFFFu - (u32)col;
   }
 }
 
-int launch_overrides(const OverrideParams& p, cudaStream_t st) {
-  if (p.nnz <= 0) return 0;
-  long long blocks = (p.nnz + 7) / 8;
-  if (p.f16) override_kernel<__half><<<(unsigned)blocks, 256, 0, st>>>(p);
-  else override_kernel<__nv_bfloat16><<<(unsigned)blocks, 256, 0, st>>>(p);
+// the record CSR of rows with candidates: c(r) + m(r)
+__global__ void entry_indptr_kernel(RecordParams p) {
+  const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r > p.B) return;
+  const long long c = p.cand_indptr ? p.cand_indptr[r] : r * p.cand_stride;
+  p.rec_indptr[r] = c + (p.mask_indptr ? p.mask_indptr[r] : 0);
+}
+
+template <class Src>
+static void launch_entry_records_t(const RecordParams& p, cudaStream_t st) {
+  constexpr int kPerBlock = 256 / Src::kLanes;
+  entry_records_kernel<Src><<<(unsigned)((p.max_entries + kPerBlock - 1) / kPerBlock), 256, 0, st>>>(p);
+}
+
+int launch_entry_records(const RecordParams& p, cudaStream_t st) {
+  if (p.B <= 0) return 0;
+  if (p.rec_indptr) {
+    entry_indptr_kernel<<<(unsigned)((p.B + 256) / 256), 256, 0, st>>>(p);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return (int)e;
+  }
+  if (p.max_entries <= 0) return 0;
+  switch (p.src) {
+    case kRecBf16Dot: launch_entry_records_t<TableDot<__nv_bfloat16>>(p, st); break;
+    case kRecF16Dot: launch_entry_records_t<TableDot<__half>>(p, st); break;
+    case kRecExactDot: launch_entry_records_t<ExactDot>(p, st); break;
+    case kRecMatrix: launch_entry_records_t<ScoreMatrix>(p, st); break;
+    default: return (int)cudaErrorInvalidValue;
+  }
   return (int)cudaGetLastError();
 }
 
 // =======================================================================================
 // Finalize: one block (256 threads) per query row.
-// Entries: dense candidates of every stream (64-bit keys) and the row's mask overrides, unified
+// Entries: dense candidates of every stream (64-bit keys) and the row's entry records, unified
 // as 96-bit sort keys (hi = ord64(double value), lo = ~id).
 //   1. prefix-sum the stream counts so the candidates can be walked as one flat, fully parallel
 //      index space (one independent global load per entry instead of a serial loop over streams);
 //   2. gather into shared memory every dense candidate at or above the row's shared lower bound
-//      g_tau (the global top-k is a subset of those) plus all overrides;
+//      g_tau (the global top-k is a subset of those) plus all records;
 //   3. exact k-th largest by MSB-first radix select (<= 12 passes, early exit) in shared memory,
 //      winners compacted, bitonic sorted, written out.
 // If the gathered list does not fit (loose bound), the select runs over global memory instead.
@@ -226,7 +300,7 @@ constexpr int kFinMaxStreams = 1024;
 
 struct RowEntries {
   const u64* cand; const int* prefix; int S, C, total;
-  const u64* ovr_hi; const u32* ovr_lo; long long obeg, oend;
+  const u64* rec_hi; const u32* rec_lo; long long rbeg, rend;
   const u64* l_hi; const u32* l_lo; int l_n;  // shared-memory list (when l_n >= 0)
   const int* drop_cols;                        // include mode: skip dense candidates in the row's mask
   template <class F> __device__ __forceinline__ void for_each(F f) const {
@@ -238,12 +312,12 @@ struct RowEntries {
       int lo = 0, hi = S;  // stream u with prefix[u] <= i < prefix[u+1]
       while (hi - lo > 1) { int mid = (lo + hi) >> 1; if (prefix[mid] <= i) lo = mid; else hi = mid; }
       const u64 key = cand[(long long)lo * C + (i - prefix[lo])];
-      if (drop_cols && mask_contains(drop_cols, obeg, oend, (int)key_id(key))) continue;
+      if (drop_cols && mask_contains(drop_cols, rbeg, rend, (int)key_id(key))) continue;
       f(ord64((double)key_score(key)), (u32)key);
     }
-    for (long long e = obeg + threadIdx.x; e < oend; e += blockDim.x) {
-      u64 h = ovr_hi[e];
-      if (h) f(h, ovr_lo[e]);
+    for (long long e = rbeg + threadIdx.x; e < rend; e += blockDim.x) {
+      u64 h = rec_hi[e];
+      if (h) f(h, rec_lo[e]);
     }
   }
 };
@@ -292,9 +366,9 @@ __global__ void __launch_bounds__(kFinMaxThreads) finalize_kernel(FinalizeParams
   RowEntries E;
   E.cand = p.cand + (long long)row * S * p.C;
   E.prefix = s_prefix; E.S = S; E.C = p.C; E.total = s_prefix[S];
-  E.ovr_hi = p.ovr_hi; E.ovr_lo = p.ovr_lo;
-  E.obeg = p.mask_indptr ? p.mask_indptr[row] : 0;
-  E.oend = p.mask_indptr ? p.mask_indptr[row + 1] : 0;
+  E.rec_hi = p.rec_hi; E.rec_lo = p.rec_lo;
+  E.rbeg = p.rec_indptr ? p.rec_indptr[row] : 0;
+  E.rend = p.rec_indptr ? p.rec_indptr[row + 1] : 0;
   E.l_hi = s_hi; E.l_lo = s_lo; E.l_n = -1;
   E.drop_cols = p.drop_cols;
   const int k = p.k;
@@ -318,18 +392,18 @@ __global__ void __launch_bounds__(kFinMaxThreads) finalize_kernel(FinalizeParams
 #pragma unroll
       for (int b = 0; b < 4; ++b) {
         bool take = i0 + b * NT < E.total && (u32)(key[b] >> 32) >= tau;
-        if (take && p.drop_cols) take = !mask_contains(p.drop_cols, E.obeg, E.oend, (int)key_id(key[b]));
+        if (take && p.drop_cols) take = !mask_contains(p.drop_cols, E.rbeg, E.rend, (int)key_id(key[b]));
         if (take) {
           int pos = atomicAdd(&s_nlist, 1);
           if (pos < kFinList) { s_hi[pos] = ord64((double)key_score(key[b])); s_lo[pos] = (u32)key[b]; }
         }
       }
     }
-    for (long long e = E.obeg + tid; e < E.oend; e += NT) {  // overrides are never filtered
-      const u64 h = p.ovr_hi[e];
+    for (long long e = E.rbeg + tid; e < E.rend; e += NT) {  // records are never filtered
+      const u64 h = p.rec_hi[e];
       if (h) {
         int pos = atomicAdd(&s_nlist, 1);
-        if (pos < kFinList) { s_hi[pos] = h; s_lo[pos] = p.ovr_lo[e]; }
+        if (pos < kFinList) { s_hi[pos] = h; s_lo[pos] = p.rec_lo[e]; }
       }
     }
     __syncthreads();
@@ -847,10 +921,9 @@ __global__ void __launch_bounds__(256) bm25_impacts_kernel(const long long* __re
                                                            long long V, long long nnz, double* __restrict__ val) {
   const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= nnz) return;
-  long long lo = 0, hi = V;  // term of posting e: largest t with post_indptr[t] <= e
-  while (hi - lo > 1) { const long long mid = (lo + hi) >> 1; if (post_indptr[mid] <= e) lo = mid; else hi = mid; }
+  const long long t = csr_row_of(post_indptr, V, e);  // term of posting e
   const double tf = (double)post_tf[e];
-  val[e] = ((tf * idf[lo]) * k1p1) * (1.0 / (tf + doc_norm[post_docs[e]]));
+  val[e] = ((tf * idf[t]) * k1p1) * (1.0 / (tf + doc_norm[post_docs[e]]));
 }
 
 int launch_bm25_impacts(const long long* post_indptr, const int* post_docs, const float* post_tf, const double* idf,
@@ -1298,7 +1371,7 @@ int launch_bm25_head_rows(const long long* post_indptr, const int* post_docs, co
 //   select_dense_kernel  : block = (column split, row); streams the row, threshold filter,
 //                          candidate buffer, exact radix prune -- the protocol of the fused kernels.
 //                          Rows with priors keep k + nnz(row) candidates (include mode) ...
-//   override_dense_kernel: ... and every prior entry gets its exact float64 value
+//   entry_records_kernel : ... and every prior entry gets its exact float64 value (ScoreMatrix source)
 //                          double(score) + prior (or the prior itself in SET mode), merged and the
 //                          plain candidates of those columns dropped by finalize_kernel.
 // =======================================================================================
@@ -1366,37 +1439,11 @@ __global__ void __launch_bounds__(kDenseThreads) select_dense_kernel(const float
   if (tid == 0) counts[(long long)row * S + split] = s_st.cnt;
 }
 
-__global__ void __launch_bounds__(256) override_dense_kernel(const float* __restrict__ scores, long long ld, int B,
-                                                             long long N, const long long* __restrict__ mask_indptr,
-                                                             const int* __restrict__ mask_cols,
-                                                             const double* __restrict__ mask_vals, long long nnz,
-                                                             int mode, u64* ovr_hi, u32* ovr_lo) {
-  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= nnz) return;
-  int lo = 0, hi = B;  // row of entry e: largest r with indptr[r] <= e
-  while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (mask_indptr[mid] <= e) lo = mid; else hi = mid; }
-  const int col = mask_cols[e];
-  if (col < 0 || (long long)col >= N) { ovr_hi[e] = 0ull; ovr_lo[e] = 0u; return; }
-  const double val = mode == 1 ? mask_vals[e] : (double)scores[(long long)lo * ld + col] + mask_vals[e];
-  const u64 h = ord64(val);
-  ovr_hi[e] = h ? h : 1ull;
-  ovr_lo[e] = 0xFFFFFFFFu - (u32)col;
-}
-
 int launch_select_dense(const float* scores, long long ld, long long B, long long N, int k, int k_keep,
                         const long long* mask_indptr, int C, int S, u64* cand, int* counts, cudaStream_t st) {
   if (B <= 0) return 0;
   dim3 grid((unsigned)S, (unsigned)B);
   select_dense_kernel<<<grid, kDenseThreads, 0, st>>>(scores, ld, N, k, k_keep, mask_indptr, C, S, cand, counts);
-  return (int)cudaGetLastError();
-}
-
-int launch_override_dense(const float* scores, long long ld, int B, long long N, const long long* mask_indptr,
-                          const int* mask_cols, const double* mask_vals, long long nnz, int mode, u64* ovr_hi,
-                          u32* ovr_lo, cudaStream_t st) {
-  if (nnz <= 0) return 0;
-  override_dense_kernel<<<(unsigned)((nnz + 255) / 256), 256, 0, st>>>(scores, ld, B, N, mask_indptr, mask_cols,
-                                                                      mask_vals, nnz, mode, ovr_hi, ovr_lo);
   return (int)cudaGetLastError();
 }
 

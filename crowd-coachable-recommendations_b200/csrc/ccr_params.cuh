@@ -75,12 +75,14 @@ struct FinalizeParams {
   const u64* cand;
   const int* counts;
   const u32* g_tau;  // per-row lower bound of the k-th best dense score (ord32), or null: prefilter
-  const int* drop_cols;  // include mode: the mask's column array; dense candidates found in the row's
-                         // list are dropped here (their override record carries the final value)
-  // mask overrides (null when no mask): per mask entry e, value and ~col
-  const long long* mask_indptr;
-  const u64* ovr_hi;
-  const u32* ovr_lo;
+  // entry records (null when none), written by launch_entry_records: the record CSR and, per record,
+  // hi = ord64(value) (0 = skipped) and lo = ~col
+  const long long* rec_indptr;
+  const u64* rec_hi;
+  const u32* rec_lo;
+  const int* drop_cols;  // include mode: the mask's column array; a stream candidate is dropped when found
+                         // in its row of the RECORD CSR, which is right because there the records are the
+                         // mask entries (their record carries the final value)
   long long id_offset;
   float* out_scores;
   double* out_scores64;
@@ -88,22 +90,43 @@ struct FinalizeParams {
   long long* out_ids;
 };
 
-struct OverrideParams {
-  const __nv_bfloat16* q;
-  long long ldq;
+// Finalize's entry records (entry_records_kernel).  Row r's entries: its candidates, if any, then its mask
+// entries.  Each record ranks by
+//   candidate (not in the row's mask)  double(score)
+//   mask entry                         mask_value(mode, score, value): SET never computes the score
+// with score the fp32 score of (r, col) from `src`.  Columns outside [0, n_cols) and candidates inside the
+// row's mask get the skipped record (the mask entry carries the value).
+enum RecordSource {
+  kRecBf16Dot,   // dot of the bf16 query and table rows, summed in fp32 (the fused kernels' scan format)
+  kRecF16Dot,    // the same on fp16 rows
+  kRecExactDot,  // dot of the fp32 rows of an exact table, summed in float64, rounded to fp32
+  kRecMatrix,    // element of a materialised fp32 score matrix
+};
+struct RecordParams {
   int B;
-  const __nv_bfloat16* items;
+  int src;              // RecordSource
+  const void* q;        // *Dot: query rows [B, ldq] and table rows [n_cols, ldi] of the source's element type
+  long long ldq;
+  const void* items;
   long long ldi;
-  long long n_items;
   int D;
-  int f16;  // q / items hold fp16 instead of bf16
-  const long long* mask_indptr;
+  const float* scores;  // kRecMatrix: [B, ld]
+  long long ld;
+  long long n_cols;
+  const long long* mask_indptr;  // null: no mask
   const int* mask_cols;
   const double* mask_vals;
-  long long nnz;
   int mode;
-  u64* ovr_hi;
-  u32* ovr_lo;
+  // candidates of row r (only with rec_indptr set): cand_ids[c(r) .. c(r+1)), c(r) = cand_indptr[r], or
+  // r * cand_stride when cand_indptr is null (the dense [B, k'] ids of the exact path's scan stage)
+  const long long* cand_indptr;
+  const long long* cand_ids;
+  long long cand_stride;
+  long long* rec_indptr;  // with candidates: [B+1] for the record CSR c(r) + m(r), written by the launcher;
+                          // null: no candidates, the record CSR is the mask CSR
+  long long max_entries;  // upper bound of the record CSR's total
+  u64* rec_hi;
+  u32* rec_lo;
 };
 
 // launchers (return cudaError_t as int)
@@ -112,7 +135,7 @@ int launch_select_tc(const SelectParams& p, cudaStream_t st, int num_sms);
 constexpr int kHistBins = 128;
 int launch_seed_tau(const float* scores, long long ld, int m, int B, int k, const long long* mask_indptr,
                     u32* g_tau, uint2* g_hpar, cudaStream_t st);
-int launch_overrides(const OverrideParams& p, cudaStream_t st);
+int launch_entry_records(const RecordParams& p, cudaStream_t st);
 int launch_finalize(const FinalizeParams& p, cudaStream_t st);
 int launch_merge_topk(const double* s, const long long* ids, int G, long long B, int k_in, int k_out,
                       float* os, double* os64, long long* oi, cudaStream_t st);
@@ -138,30 +161,6 @@ int launch_dense_f32_f16(const __half* q, long long B, long long ldq, const __ha
 // exact tables: fp32 rows (ingest_kernel<float, float>, ccr_kernels.cu) and the exact ranking stages (ccr_exact.cu)
 int launch_ingest_f32_f32(const float* src, long long n, int D, long long ld_src, float* dst, long long ld_dst,
                           int normalize, cudaStream_t st);
-struct ExactParams {
-  const float* q;        // fp32 query rows [B, ldq]
-  long long ldq;
-  int B;
-  const float* items;    // fp32 table rows [n_items, ldi]
-  long long ldi;
-  long long n_items;
-  int D;
-  // candidates of row r: cand_ids[c(r) .. c(r+1)), c(r) = cand_indptr[r], or r * cand_stride when
-  // cand_indptr is null (the dense [B, k'] ids of the scan stage); ids < 0 or inside the row's mask are
-  // skipped (the mask entry carries the value)
-  const long long* cand_indptr;
-  const long long* cand_ids;
-  long long cand_stride;
-  const long long* mask_indptr;  // null: no mask
-  const int* mask_cols;
-  const double* mask_vals;
-  int mode;
-  const long long* ent_indptr;   // [B+1]: c(r) + m(r), the entry CSR finalize reads as its override CSR
-  long long max_entries;         // upper bound of ent_indptr[B]
-  u64* ent_hi;                   // finalize's 96-bit records: ord64(value) (0 = skipped), ~id
-  u32* ent_lo;
-};
-int launch_exact_entries(const ExactParams& p, cudaStream_t st);
 int launch_row_norm_max(const float* rows, long long n, int D, long long ld, double* v_max, cudaStream_t st);
 int launch_fill_f64(double* dst, long long n, double v, cudaStream_t st);
 // per row: certified (0) or not (1), tau = RD(L_k - E); uncertified rows are added to *count
@@ -184,9 +183,6 @@ int launch_first_hit_rank(const long long* ids, long long B, int k, const long l
 constexpr int kDenseSlack = 4096;  // columns one block scans between two prune checks (16 per thread)
 int launch_select_dense(const float* scores, long long ld, long long B, long long N, int k, int k_keep,
                         const long long* mask_indptr, int C, int S, u64* cand, int* counts, cudaStream_t st);
-int launch_override_dense(const float* scores, long long ld, int B, long long N, const long long* mask_indptr,
-                          const int* mask_cols, const double* mask_vals, long long nnz, int mode, u64* ovr_hi,
-                          u32* ovr_lo, cudaStream_t st);
 
 // BM25 (ccr_kernels.cu)
 // block shape, measured at the NQ shape (profiles/r01_bm25_bench.json): 4096 docs x 256 threads x 5 blocks

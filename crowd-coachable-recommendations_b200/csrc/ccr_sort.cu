@@ -54,7 +54,7 @@ __global__ void __launch_bounds__(256) sort_build_keys_kernel(const float* __res
   if ((threadIdx.x & 31) == 0 && (need & ~(u32)state[3])) atomicOr(state + 3, (int)need);
 }
 
-// mask entries overwrite their element's key: ADD ranks double(score) + value, SET the value itself
+// mask entries overwrite their element's key with ~ord64(mask_value)
 __global__ void __launch_bounds__(256) sort_override_keys_kernel(const float* __restrict__ scores, long long B,
                                                                  long long N, long long ld,
                                                                  const long long* __restrict__ indptr,
@@ -63,13 +63,11 @@ __global__ void __launch_bounds__(256) sort_override_keys_kernel(const float* __
                                                                  u64* __restrict__ keys, int* __restrict__ state) {
   const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= indptr[B]) return;
-  long long lo = 0, hi = B;  // row of entry e: largest r with indptr[r] <= e
-  while (hi - lo > 1) { const long long mid = (lo + hi) >> 1; if (indptr[mid] <= e) lo = mid; else hi = mid; }
+  const long long row = csr_row_of(indptr, B, e);
   const int col = cols[e];
   if (col < 0 || (long long)col >= N) return;
-  const double v = mode == 1 ? vals[e] : (double)scores[lo * ld + col] + vals[e];
-  const u64 key = ~ord64(v);
-  keys[lo * N + col] = key;
+  const u64 key = ~ord64(mask_value(mode, scores[row * ld + col], vals[e]));
+  keys[row * N + col] = key;
   const u32 need = sort_needed_passes(key);
   if (need & ~(u32)state[3]) atomicOr(state + 3, (int)need);
 }
