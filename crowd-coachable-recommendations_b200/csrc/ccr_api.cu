@@ -49,6 +49,14 @@ static int fail(int code, const char* fmt, ...) {
   return code;
 }
 
+// The return code of a launcher or CUDA call: 0 is success, a cudaError_t becomes CCR_ECUDA with its text, and a
+// negative code is a tensor map that could not be encoded (launch_select_tc).
+static int cuda_rc(int rc, const char* what) {
+  if (rc == 0) return CCR_OK;
+  if (rc < 0) return fail(CCR_ECUDA, "%s failed: tensor map encode error %d", what, rc);
+  return fail(CCR_ECUDA, "%s failed: %s", what, cudaGetErrorString((cudaError_t)rc));
+}
+
 static int device_sm_count() {
   static int cached[64];
   int dev = 0;
@@ -65,7 +73,18 @@ static int device_sm_count() {
 }
 
 namespace {
+// Workspace layout: regions taken one after another, each starting at a 256-byte boundary
+struct Carve {
+  size_t off = 0;
+  size_t take(size_t bytes) {
+    const size_t at = off;
+    off = (off + bytes + 255) / 256 * 256;
+    return at;
+  }
+};
+
 struct Plan {
+  int sms;        // SMs of the device the plan is made for; every launch of the call uses the same count
   int algo;
   int n_q_tiles;  // TC: query tiles of 128; SIMT: groups of 8
   int rows_pad;
@@ -85,15 +104,16 @@ struct Plan {
   int lead_every;        // throttle: progress is published / checked every lead_every tiles (power of two)
   int throttle_poller;   // throttle: 1 a dedicated warp watches the peers, 0 the producer polls inline
   int k_cand;            // exact ranking: candidates the scan stage returns per row (k' >= k, <= n_items)
-  size_t off_seed;
-  size_t off_progress;
+  size_t off_cand, off_counts, off_rec_hi, off_rec_lo;
+  // [zero_begin, zero_end) is cleared by ONE memset per call: status, throttle counters, sharing state
+  size_t zero_begin, off_status, off_progress, off_gtau, off_gq, off_hist, off_hpar, zero_end;
   size_t off_qpad;       // zero-padded copy of a short query batch (B < 128): every TMA box in bounds
-  size_t off_cand, off_counts, off_rec_hi, off_rec_lo, off_status, off_gtau, off_gq, off_hist, off_hpar, total;
+  size_t off_seed, total;
 };
 
-size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
-int splits_tc(int nq, long long tiles, int sms) {
+// item splits of the tensor-core pipeline: nq query tiles against the item tiles of n_items rows on `sms` units
+int splits_tc(int nq, long long n_items, int sms) {
+  const long long tiles = (n_items + kITile - 1) / kITile;
   long long smax = tiles < 1 ? 1 : tiles;
   long long s0 = sms / nq;  // from the largest split count that still fits ONE wave
   if (s0 < 1) s0 = 1;
@@ -118,6 +138,7 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
   if (algo == CCR_ALGO_AUTO) algo = ccr_choose_algo(B, n_items, D, k);
   const int sms = device_sm_count();
   const Knobs& kn = knobs();
+  pl->sms = sms;
   pl->algo = algo;
   {
     // Exact ranking (DESIGN.md section 6b): a row is certified when its k-th exact value beats the scan
@@ -150,8 +171,7 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
     pl->n_q_tiles = (int)((B + unit_rows - 1) / unit_rows);
     if (pl->n_q_tiles < 1) pl->n_q_tiles = 1;
     pl->rows_pad = pl->n_q_tiles * unit_rows;
-    long long tiles = (n_items + kITile - 1) / kITile;
-    pl->S = splits_tc(pl->n_q_tiles, tiles, pl->two_cta ? sms / 2 : sms);
+    pl->S = splits_tc(pl->n_q_tiles, n_items, pl->two_cta ? sms / 2 : sms);
     pl->halves = 2;
     pl->C = cand_capacity(pl->k_keep, 128);
     {
@@ -206,20 +226,21 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
   if (kn.lead >= 1 && kn.lead <= 4096) pl->lead_tiles = kn.lead;
   pl->lead_every = 1;
   while (pl->lead_every * 2 <= pl->lead_tiles && pl->lead_every < 8) pl->lead_every *= 2;  // 16 -> 8, 8 -> 8, 4 -> 4
-  size_t off = 0;
-  pl->off_cand = off;   off = align_up(off + (size_t)pl->rows_pad * pl->S * pl->halves * pl->C * sizeof(u64), 256);
-  pl->off_counts = off; off = align_up(off + (size_t)pl->rows_pad * pl->S * pl->halves * sizeof(int), 256);
-  pl->off_rec_hi = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u64), 256);
-  pl->off_rec_lo = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u32), 256);
-  // [off_status, off_qpad) is zeroed by ONE memset per call: status, throttle counters, sharing state
-  pl->off_status = off; off = align_up(off + sizeof(DeviceStatus), 256);
-  pl->off_progress = off; off = align_up(off + (size_t)pl->n_q_tiles * pl->S * sizeof(int), 256);
-  pl->off_gtau = off;   off = align_up(off + (size_t)pl->rows_pad * sizeof(u32), 256);
-  pl->off_gq = off;     off = align_up(off + (size_t)pl->rows_pad * pl->S * pl->halves * sizeof(u32), 256);
-  pl->off_hist = off;   off = align_up(off + (size_t)pl->rows_pad * kHistBins * sizeof(u32), 256);
-  pl->off_hpar = off;   off = align_up(off + (size_t)pl->rows_pad * sizeof(uint2), 256);
-  pl->off_qpad = off;     off = align_up(off + (size_t)kQTile * 4096 * sizeof(__nv_bfloat16), 256);
-  pl->seed_m = 0; pl->seed_stride = 1; pl->seed_ld = 0; pl->off_seed = off; pl->use_hist = 0;
+  Carve c;
+  pl->off_cand = c.take((size_t)pl->rows_pad * pl->S * pl->halves * pl->C * sizeof(u64));
+  pl->off_counts = c.take((size_t)pl->rows_pad * pl->S * pl->halves * sizeof(int));
+  pl->off_rec_hi = c.take((size_t)(nnz > 0 ? nnz : 0) * sizeof(u64));
+  pl->off_rec_lo = c.take((size_t)(nnz > 0 ? nnz : 0) * sizeof(u32));
+  pl->zero_begin = c.off;
+  pl->off_status = c.take(sizeof(DeviceStatus));
+  pl->off_progress = c.take((size_t)pl->n_q_tiles * pl->S * sizeof(int));
+  pl->off_gtau = c.take((size_t)pl->rows_pad * sizeof(u32));
+  pl->off_gq = c.take((size_t)pl->rows_pad * pl->S * pl->halves * sizeof(u32));
+  pl->off_hist = c.take((size_t)pl->rows_pad * kHistBins * sizeof(u32));
+  pl->off_hpar = c.take((size_t)pl->rows_pad * sizeof(uint2));
+  pl->zero_end = c.off;
+  pl->off_qpad = c.take((size_t)kQTile * 4096 * sizeof(__nv_bfloat16));
+  pl->seed_m = 0; pl->seed_stride = 1; pl->seed_ld = 0; pl->use_hist = 0;
   if (algo == CCR_ALGO_TCGEN05 && n_items >= (1 << 18)) {
     // strided sample of max(N/256, 64k) items (4096..131072, <= N/8); the pre-pass keeps one fp32 value
     // per 8 sampled items (their best score), capped so that matrix stays <= 512 MB
@@ -246,11 +267,19 @@ bool make_plan(long long B, long long n_items, int D, int k, long long nnz, long
       // the histogram needs the seed bound as its origin and counts every streamed item, so it is
       // off in exclude-mask mode (masked items must not be counted)
       pl->use_hist = hist_ok && !kn.no_hist;
-      off = align_up(off + (size_t)pl->rows_pad * (size_t)pl->seed_ld * sizeof(float), 256);
     }
   }
-  pl->total = off;
+  // the pre-pass's score matrix (seed_ld = 0 without a pre-pass)
+  pl->off_seed = c.take((size_t)pl->rows_pad * (size_t)pl->seed_ld * sizeof(float));
+  pl->total = c.off;
   return true;
+}
+
+// k of a top-k over n columns: in [1, CCR_MAX_K] and, unless short rows are allowed, <= n (torch.topk's error)
+int check_k(int k, long long n, bool allow_short) {
+  if (k < 1 || k > CCR_MAX_K) return fail(CCR_EUNSUPPORTED, "k=%d outside [1,%d]", k, CCR_MAX_K);
+  if (k > n && !allow_short) return fail(CCR_EK_RANGE, "selected index k out of range (k=%d > n=%lld)", k, n);
+  return CCR_OK;
 }
 
 int check_shape(long long B, long long n_items, int D, int k, int flags) {
@@ -258,12 +287,17 @@ int check_shape(long long B, long long n_items, int D, int k, int flags) {
   if (B > (1LL << 24)) return fail(CCR_EUNSUPPORTED, "B=%lld > 2^24", B);
   if (n_items > (1LL << 31) - 512) return fail(CCR_EUNSUPPORTED, "n_items=%lld per shard must be < 2^31", n_items);
   if (D <= 0 || D % 8 != 0 || D > 4096) return fail(CCR_EUNSUPPORTED, "D=%d must be a multiple of 8 in [8,4096]", D);
-  if (k < 1 || k > CCR_MAX_K) return fail(CCR_EUNSUPPORTED, "k=%d outside [1,%d]", k, CCR_MAX_K);
-  if (k > n_items && !(flags & CCR_FLAG_ALLOW_SHORT))
-    return fail(CCR_EK_RANGE, "selected index k out of range (k=%d > n_items=%lld)", k, n_items);
+  if (int rc = check_k(k, n_items, flags & CCR_FLAG_ALLOW_SHORT)) return rc;
   int algo = flags & CCR_ALGO_MASK;
   if (algo != CCR_ALGO_AUTO && algo != CCR_ALGO_SIMT && algo != CCR_ALGO_TCGEN05)
     return fail(CCR_EINVAL, "unknown algo flag %d", algo);
+  return CCR_OK;
+}
+
+// q [B, ldq] and items [n, ldi] of the fused and exact entries: whole 16-byte rows, 16-byte aligned (TMA boxes)
+int check_rows(const void* q, int64_t ldq, const void* items, int64_t ldi, int D) {
+  if (ldq < D || ldi < D || ldq % 8 || ldi % 8) return fail(CCR_EINVAL, "ldq/ldi must be >= D and multiples of 8");
+  if (((uintptr_t)q & 15) || ((uintptr_t)items & 15)) return fail(CCR_EINVAL, "q/items must be 16-byte aligned");
   return CCR_OK;
 }
 
@@ -284,6 +318,64 @@ int parse_mask(const int64_t* indptr, const int32_t* cols, const double* vals, i
   if (!cols || !vals) return fail(CCR_EINVAL, "mask_cols / mask_vals null");
   *m = {(const long long*)indptr, cols, vals, nnz, mask_h_max(nnz, max_row_nnz), mode};
   return CCR_OK;
+}
+
+// The operand fields of SelectParams: queries q [B, ldq] against table rows items [n_items, ldi], D wide (fp16 when
+// f16, else bf16), in n_q_tiles query tiles and S item splits
+void set_operands(SelectParams* p, const void* q, long long ldq, long long B, const void* items, long long ldi,
+                  long long n_items, int D, int f16, int n_q_tiles, int S) {
+  p->q = (const __nv_bfloat16*)q; p->ldq = ldq; p->B = (int)B; p->q_rows = (int)B;
+  p->items = (const __nv_bfloat16*)items; p->ldi = ldi; p->n_items = n_items; p->D = D; p->f16 = f16;
+  p->n_q_tiles = n_q_tiles; p->S = S;
+}
+
+// The candidate lists of a top-k call: per row, `streams` lists of C keys (cand[(row * streams + s) * C + i]) and
+// their counts.  The exact re-rank has none (streams = 0).
+struct Cands { int C, streams; u64* cand; int* counts; };
+// finalize's entry records: the record CSR and one (hi, lo) pair per record; all null when there are none
+struct Records { const long long* indptr; u64* hi; u32* lo; };
+
+// The fields every entry-record launch shares: B rows of mask `m`, columns [0, n_cols), records written to `rec`.
+// The caller adds the fields of its score source and, for the re-rank, its candidates.
+RecordParams record_params(int B, RecordSource src, long long n_cols, const MaskArgs& m, const Records& rec) {
+  RecordParams rp = {};
+  rp.B = B; rp.src = src; rp.n_cols = n_cols;
+  rp.mask_indptr = m.indptr; rp.mask_cols = m.cols; rp.mask_vals = m.vals; rp.mode = m.mode;
+  rp.max_entries = m.nnz; rp.rec_hi = rec.hi; rp.rec_lo = rec.lo;
+  return rp;
+}
+
+// One record per mask entry: the record CSR is the mask CSR.  Nothing to launch without a mask.
+int mask_records(const RecordParams& rp, cudaStream_t st) {
+  return rp.mask_indptr ? cuda_rc(launch_entry_records(rp, st), "mask record kernel launch") : CCR_OK;
+}
+
+// The last step of every top-k entry: the best k per row of the candidate lists and the entry records.  g_tau: a
+// per-row lower bound of the k-th best for the prefilter, or null.  drop_cols (include mode: the mask's column
+// array): a stream candidate is dropped when found in its row of the RECORD CSR, which is right because there the
+// records are the mask entries (their record carries the final value).  packed_keys: out_scores64 receives
+// CCR_FLAG_PACKED_KEYS keys instead of float64 values.
+int finalize(int B, int k, const Cands& cb, const u32* g_tau, const Records& rec, const int* drop_cols,
+             long long id_offset, float* out_scores, double* out_scores64, long long* out_ids, bool packed_keys,
+             cudaStream_t st) {
+  FinalizeParams fp = {};
+  fp.B = B; fp.k = k; fp.C = cb.C; fp.S = cb.streams; fp.cand = cb.cand; fp.counts = cb.counts; fp.g_tau = g_tau;
+  fp.rec_indptr = rec.indptr; fp.rec_hi = rec.hi; fp.rec_lo = rec.lo; fp.drop_cols = drop_cols;
+  fp.id_offset = id_offset; fp.out_scores = out_scores; fp.out_ids = out_ids;
+  if (packed_keys) fp.out_keys = (u64*)out_scores64;
+  else fp.out_scores64 = out_scores64;
+  return cuda_rc(launch_finalize(fp, st), "finalize kernel launch");
+}
+
+// The ingest / normalize entries: rows src [n, ld_src] -> dst [n, ld_dst]; `job` names the entry in the shape error
+template <typename SrcT, typename DstT>
+int ingest_rows(const char* job, const void* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
+                int normalize, int* overflow, void* stream) {
+  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad %s shape", job);
+  if (n == 0) return CCR_OK;
+  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
+  return cuda_rc(launch_ingest((const SrcT*)src, n, D, ld_src, (DstT*)dst, ld_dst, normalize, overflow,
+                               (cudaStream_t)stream), "ingest kernel launch");
 }
 }  // namespace
 
@@ -349,8 +441,7 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   if (B == 0) return CCR_OK;
   if (!q || !out_ids) return fail(CCR_EINVAL, "null q / out_ids");
   if (n_items > 0 && !items) return fail(CCR_EINVAL, "null items");
-  if (ldq < D || ldi < D || ldq % 8 || ldi % 8) return fail(CCR_EINVAL, "ldq/ldi must be >= D and multiples of 8");
-  if (((uintptr_t)q & 15) || ((uintptr_t)items & 15)) return fail(CCR_EINVAL, "q/items must be 16-byte aligned");
+  if ((rc = check_rows(q, ldq, items, ldi, D))) return rc;
   MaskArgs m;
   if ((rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, mask_max_row_nnz, mask_mode, &m))) return rc;
   if (flags & CCR_FLAG_PACKED_KEYS) {
@@ -368,22 +459,19 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   DeviceStatus* status = g_status_record ? (DeviceStatus*)g_status_record : (DeviceStatus*)(ws + pl.off_status);
   // one memset for everything that must start from zero: status slot, throttle counters, thresholds,
   // published quantiles, histograms and their parameters
-  cudaError_t e = cudaMemsetAsync(ws + pl.off_status, 0, pl.off_qpad - pl.off_status, st);
-  if (e != cudaSuccess) return fail(CCR_ECUDA, "memset call state: %s", cudaGetErrorString(e));
+  if ((rc = cuda_rc(cudaMemsetAsync(ws + pl.zero_begin, 0, pl.zero_end - pl.zero_begin, st), "memset call state")))
+    return rc;
 
+  const Cands cb = {pl.C, pl.S * pl.halves, (u64*)(ws + pl.off_cand), (int*)(ws + pl.off_counts)};
   SelectParams sp = {};
-  sp.q = (const __nv_bfloat16*)q; sp.ldq = ldq; sp.B = (int)B; sp.q_rows = (int)B;
-  sp.items = (const __nv_bfloat16*)items; sp.ldi = ldi; sp.n_items = n_items; sp.D = D;
-  sp.f16 = (flags & CCR_FLAG_F16) ? 1 : 0;
-  sp.k = k; sp.k_keep = pl.k_keep; sp.C = pl.C; sp.S = pl.S; sp.n_q_tiles = pl.n_q_tiles; sp.two_cta = pl.two_cta;
+  set_operands(&sp, q, ldq, B, items, ldi, n_items, D, (flags & CCR_FLAG_F16) ? 1 : 0, pl.n_q_tiles, pl.S);
+  sp.k = k; sp.k_keep = pl.k_keep; sp.C = pl.C; sp.two_cta = pl.two_cta;
   sp.mask_indptr = m.indptr;
   sp.mask_cols = pl.include_mask ? nullptr : m.cols;
-  sp.cand = (u64*)(ws + pl.off_cand);
-  sp.counts = (int*)(ws + pl.off_counts);
+  sp.cand = cb.cand;
+  sp.counts = cb.counts;
   sp.status = status;
-  sp.g_tau = nullptr; sp.g_q = nullptr; sp.S_row = pl.S * pl.halves; sp.share_j = pl.share_j; sp.share_m = pl.share_m;
-  sp.dense_out = nullptr; sp.ld_out = 0; sp.store_max8 = 0;
-  sp.g_hist = nullptr; sp.g_hpar = nullptr;
+  sp.S_row = cb.streams; sp.share_j = pl.share_j; sp.share_m = pl.share_m;
   sp.progress = pl.throttle ? (int*)(ws + pl.off_progress) : nullptr;
   sp.lead_tiles = pl.lead_tiles; sp.lead_every = pl.lead_every; sp.throttle_poller = pl.throttle_poller;
   if (pl.share_j > 0 || pl.seed_m > 0) {
@@ -393,20 +481,18 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
   if (pl.seed_m > 0) {
     // threshold seeding pre-pass: scores of a strided item sample -> per-row lower bound in g_tau
     SelectParams ss = sp;
-    ss.n_items = pl.seed_m; ss.ldi = ldi * pl.seed_stride;
+    const int nqt = pl.rows_pad / kQTile;
+    set_operands(&ss, q, ldq, B, items, ldi * pl.seed_stride, pl.seed_m, D, sp.f16, nqt,
+                 splits_tc(nqt, pl.seed_m, pl.sms));
     ss.mask_indptr = nullptr; ss.mask_cols = nullptr;
     ss.dense_out = (float*)(ws + pl.off_seed); ss.ld_out = pl.seed_ld; ss.store_max8 = 1;
-    ss.g_tau = nullptr; ss.g_q = nullptr; ss.share_j = 0; ss.progress = nullptr;
+    ss.g_tau = nullptr; ss.g_q = nullptr; ss.share_j = 0; ss.progress = nullptr; ss.two_cta = 0;
     if (pl.use_hist) { sp.g_hist = (u32*)(ws + pl.off_hist); sp.g_hpar = (const uint2*)(ws + pl.off_hpar); }
-    ss.two_cta = 0; ss.n_q_tiles = pl.rows_pad / kQTile;
-    long long tiles = (pl.seed_m + kITile - 1) / kITile;
-    ss.S = splits_tc(ss.n_q_tiles, tiles, device_sm_count());
-    int lr0 = launch_select_tc(ss, st, device_sm_count());
-    if (lr0) return fail(CCR_ECUDA, "seed GEMM launch failed (%d)", lr0);
+    if ((rc = cuda_rc(launch_select_tc(ss, st, pl.sms), "seed GEMM launch"))) return rc;
     // per row: the (k + h)-th largest of the seed_m / 8 group maxima
-    lr0 = launch_seed_tau(ss.dense_out, pl.seed_ld, (int)pl.seed_ld, (int)B, k, m.indptr, sp.g_tau,
-                          pl.use_hist ? (uint2*)(ws + pl.off_hpar) : nullptr, st);
-    if (lr0) return fail(CCR_ECUDA, "seed select launch failed: %s", cudaGetErrorString((cudaError_t)lr0));
+    rc = cuda_rc(launch_seed_tau(ss.dense_out, pl.seed_ld, (int)pl.seed_ld, (int)B, k, m.indptr, sp.g_tau,
+                                 pl.use_hist ? (uint2*)(ws + pl.off_hpar) : nullptr, st), "seed select launch");
+    if (rc) return rc;
   }
 
   if (pl.algo == CCR_ALGO_TCGEN05 && B < kQTile && n_items > 0) {
@@ -414,50 +500,29 @@ int ccr_score_topk_bf16(const void* q, int64_t B, int64_t ldq, const void* items
     // out of bounds (measurably faster than hardware zero-fill of 120+ rows); only the padding rows
     // are zeroed.  A plain copy of 2-byte elements: the same for fp16, whose +0 has bf16's bits
     __nv_bfloat16* qp = (__nv_bfloat16*)(ws + pl.off_qpad);
-    e = cudaMemsetAsync(qp + (size_t)B * D, 0, (size_t)(kQTile - B) * D * sizeof(__nv_bfloat16), st);
+    cudaError_t e = cudaMemsetAsync(qp + (size_t)B * D, 0, (size_t)(kQTile - B) * D * sizeof(__nv_bfloat16), st);
     if (e == cudaSuccess)
       e = cudaMemcpy2DAsync(qp, (size_t)D * 2, q, (size_t)ldq * 2, (size_t)D * 2, (size_t)B, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) return fail(CCR_ECUDA, "query padding: %s", cudaGetErrorString(e));
+    if ((rc = cuda_rc(e, "query padding"))) return rc;
     sp.q = qp; sp.ldq = D; sp.q_rows = kQTile;
   }
-  int lr = 0;
   if (n_items == 0) {
-    e = cudaMemsetAsync(sp.counts, 0, (size_t)pl.rows_pad * pl.S * pl.halves * sizeof(int), st);
-    if (e != cudaSuccess) return fail(CCR_ECUDA, "memset counts: %s", cudaGetErrorString(e));
+    rc = cuda_rc(cudaMemsetAsync(cb.counts, 0, (size_t)pl.rows_pad * cb.streams * sizeof(int), st), "memset counts");
   } else {
     if (g_prof_start) cudaEventRecord(g_prof_start, st);
-    if (pl.algo == CCR_ALGO_TCGEN05) lr = launch_select_tc(sp, st, device_sm_count());
-    else lr = launch_select_simt(sp, st);
+    const int lr = pl.algo == CCR_ALGO_TCGEN05 ? launch_select_tc(sp, st, pl.sms) : launch_select_simt(sp, st);
     if (g_prof_stop) cudaEventRecord(g_prof_stop, st);
+    rc = cuda_rc(lr, "select kernel launch");
   }
-  if (lr) return fail(CCR_ECUDA, "select kernel launch failed (%d: %s)", lr, lr > 0 ? cudaGetErrorString((cudaError_t)lr) : "tensor map");
+  if (rc) return rc;
 
-  // one record per mask entry: the record CSR is the mask CSR
-  u64* rec_hi = (u64*)(ws + pl.off_rec_hi);
-  u32* rec_lo = (u32*)(ws + pl.off_rec_lo);
-  if (m.nnz > 0) {
-    RecordParams rp = {};
-    rp.B = (int)B; rp.src = sp.f16 ? kRecF16Dot : kRecBf16Dot;
-    // sp.q may be the padded staging block of a short batch: use ITS pitch (sp.ldq), not the caller's
-    rp.q = sp.q; rp.ldq = sp.ldq; rp.items = sp.items; rp.ldi = ldi; rp.D = D; rp.n_cols = n_items;
-    rp.mask_indptr = m.indptr; rp.mask_cols = m.cols; rp.mask_vals = m.vals; rp.mode = m.mode;
-    rp.max_entries = m.nnz; rp.rec_hi = rec_hi; rp.rec_lo = rec_lo;
-    lr = launch_entry_records(rp, st);
-    if (lr) return fail(CCR_ECUDA, "mask record kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  }
-
-  FinalizeParams fp = {};
-  fp.B = (int)B; fp.k = k; fp.C = pl.C; fp.S = pl.S * pl.halves; fp.cand = sp.cand; fp.counts = sp.counts;
-  fp.g_tau = sp.g_tau;
-  fp.rec_indptr = m.indptr; fp.rec_hi = rec_hi; fp.rec_lo = rec_lo;
-  fp.drop_cols = pl.include_mask ? m.cols : nullptr;  // searched in the record CSR: the records are the mask entries
-  fp.id_offset = id_offset; fp.out_scores = out_scores; fp.out_scores64 = out_scores64;
-  fp.out_keys = nullptr;
-  if (flags & CCR_FLAG_PACKED_KEYS) { fp.out_keys = (u64*)out_scores64; fp.out_scores64 = nullptr; }
-  fp.out_ids = (long long*)out_ids;
-  lr = launch_finalize(fp, st);
-  if (lr) return fail(CCR_ECUDA, "finalize kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  const Records rec = {m.indptr, (u64*)(ws + pl.off_rec_hi), (u32*)(ws + pl.off_rec_lo)};
+  RecordParams rp = record_params((int)B, sp.f16 ? kRecF16Dot : kRecBf16Dot, n_items, m, rec);
+  // sp.q may be the padded staging block of a short batch: use ITS pitch (sp.ldq), not the caller's
+  rp.q = sp.q; rp.ldq = sp.ldq; rp.items = sp.items; rp.ldi = ldi; rp.D = D;
+  if ((rc = mask_records(rp, st))) return rc;
+  return finalize((int)B, k, cb, sp.g_tau, rec, pl.include_mask ? m.cols : nullptr, id_offset, out_scores,
+                  out_scores64, (long long*)out_ids, flags & CCR_FLAG_PACKED_KEYS, st);
 }
 
 int ccr_merge_topk(const double* scores64, const int64_t* ids, int G, int64_t B, int k_in, int k_out,
@@ -465,10 +530,8 @@ int ccr_merge_topk(const double* scores64, const int64_t* ids, int G, int64_t B,
   if (G < 1 || B < 0 || k_in < 1 || k_out < 1) return fail(CCR_EINVAL, "bad merge shape G=%d B=%lld k_in=%d k_out=%d", G, (long long)B, k_in, k_out);
   if (B == 0) return CCR_OK;
   if (!scores64 || !ids || !out_ids) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_merge_topk(scores64, (const long long*)ids, G, B, k_in, k_out, out_scores, out_scores64,
-                             (long long*)out_ids, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "merge kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(launch_merge_topk(scores64, (const long long*)ids, G, B, k_in, k_out, out_scores, out_scores64,
+                                   (long long*)out_ids, (cudaStream_t)stream), "merge kernel launch");
 }
 
 int ccr_merge_topk_keys(const uint64_t* keys, int G, int64_t B, int k_in, int k_out, float* out_scores,
@@ -479,69 +542,44 @@ int ccr_merge_topk_keys(const uint64_t* keys, int G, int64_t B, int k_in, int k_
   int lr = launch_merge_keys((const u64*)keys, G, B, k_in, k_out, out_scores, (long long*)out_ids, (u64*)out_keys,
                              (cudaStream_t)stream);
   if (lr == (int)cudaErrorInvalidValue) return fail(CCR_EUNSUPPORTED, "merge: G * k_in = %lld keys do not fit shared memory", (long long)G * k_in);
-  if (lr) return fail(CCR_ECUDA, "key merge kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(lr, "key merge kernel launch");
 }
 
 int ccr_unpack_topk_keys(const uint64_t* keys, int64_t n, float* out_scores, int64_t* out_ids, void* stream) {
   if (n < 0) return fail(CCR_EINVAL, "bad key count");
   if (n == 0) return CCR_OK;
   if (!keys) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_unpack_keys((const u64*)keys, n, out_scores, (long long*)out_ids, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "key unpack kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(launch_unpack_keys((const u64*)keys, n, out_scores, (long long*)out_ids, (cudaStream_t)stream),
+                 "key unpack kernel launch");
 }
 
 int ccr_mask_column_shard(const int64_t* indptr, const int32_t* cols, const double* vals, int64_t B, int64_t col_lo,
                           int64_t col_hi, int64_t* out_indptr, int32_t* out_cols, double* out_vals, void* stream) {
   if (B < 0 || col_lo < 0 || col_hi < col_lo || col_hi > (1LL << 31) - 1) return fail(CCR_EINVAL, "bad mask shard range");
   if (!indptr || !out_indptr) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_mask_shard((const long long*)indptr, cols, vals, B, (int)col_lo, (int)col_hi, (long long*)out_indptr,
-                             out_cols, out_vals, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "mask shard kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(launch_mask_shard((const long long*)indptr, cols, vals, B, (int)col_lo, (int)col_hi,
+                                   (long long*)out_indptr, out_cols, out_vals, (cudaStream_t)stream),
+                 "mask shard kernel launch");
 }
 
 int ccr_ingest_rows_f32(const float* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
                         int normalize, void* stream) {
-  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad ingest shape");
-  if (n == 0) return CCR_OK;
-  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_ingest_f32(src, n, D, ld_src, (__nv_bfloat16*)dst, ld_dst, normalize, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "ingest kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return ingest_rows<float, __nv_bfloat16>("ingest", src, n, D, ld_src, dst, ld_dst, normalize, nullptr, stream);
 }
 
 int ccr_ingest_rows_f32_f16(const float* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
                             int normalize, int32_t* overflow_count, void* stream) {
-  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad ingest shape");
-  if (n == 0) return CCR_OK;
-  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_ingest_f32_f16(src, n, D, ld_src, (__half*)dst, ld_dst, normalize, (int*)overflow_count,
-                                 (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "ingest kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return ingest_rows<float, __half>("ingest", src, n, D, ld_src, dst, ld_dst, normalize, (int*)overflow_count, stream);
 }
 
 int ccr_normalize_rows_bf16(const void* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
                             void* stream) {
-  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad normalize shape");
-  if (n == 0) return CCR_OK;
-  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_normalize_bf16((const __nv_bfloat16*)src, n, D, ld_src, (__nv_bfloat16*)dst, ld_dst,
-                                 (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "normalize kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return ingest_rows<__nv_bfloat16, __nv_bfloat16>("normalize", src, n, D, ld_src, dst, ld_dst, 1, nullptr, stream);
 }
 
 int ccr_normalize_rows_f16(const void* src, int64_t n, int D, int64_t ld_src, void* dst, int64_t ld_dst,
                            void* stream) {
-  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad normalize shape");
-  if (n == 0) return CCR_OK;
-  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_normalize_f16((const __half*)src, n, D, ld_src, (__half*)dst, ld_dst, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "normalize kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return ingest_rows<__half, __half>("normalize", src, n, D, ld_src, dst, ld_dst, 1, nullptr, stream);
 }
 
 }  // extern "C"
@@ -557,25 +595,20 @@ static int score_dense(const void* q, int64_t B, int64_t ldq, const void* items,
   if (B * n_items >= (1LL << 20) && n_items >= kITile && n_items <= (1LL << 31) - 512 && D <= 4096 &&
       !(((uintptr_t)q | (uintptr_t)items) & 15)) {
     // large tiles: the TMA + tcgen05 pipeline of the fused kernel with a store epilogue
+    const int sms = device_sm_count(), n_q_tiles = (int)((B + kQTile - 1) / kQTile);
     SelectParams sp = {};
-    sp.q = (const __nv_bfloat16*)q; sp.ldq = ldq; sp.B = (int)B; sp.q_rows = (int)B;
-    sp.items = (const __nv_bfloat16*)items; sp.ldi = ldi; sp.n_items = n_items; sp.D = D; sp.f16 = f16;
+    set_operands(&sp, q, ldq, B, items, ldi, n_items, D, f16, n_q_tiles, splits_tc(n_q_tiles, n_items, sms));
     sp.k = 1; sp.k_keep = 1; sp.C = 0;
-    sp.n_q_tiles = (int)((B + kQTile - 1) / kQTile);
-    sp.S = splits_tc(sp.n_q_tiles, (n_items + kITile - 1) / kITile, device_sm_count());
     sp.status = (DeviceStatus*)g_status_record;
     sp.dense_out = out; sp.ld_out = ld_out; sp.store_max8 = 0;
     sp.lead_tiles = 16; sp.lead_every = 8;
-    int lr = launch_select_tc(sp, (cudaStream_t)stream, device_sm_count());
-    if (lr) return fail(CCR_ECUDA, "dense tile launch failed (%d)", lr);
-    return CCR_OK;
+    return cuda_rc(launch_select_tc(sp, (cudaStream_t)stream, sms), "dense tile launch");
   }
-  int lr = f16 ? launch_dense_f32_f16((const __half*)q, B, ldq, (const __half*)items, n_items, ldi, D, out, ld_out,
-                                      (cudaStream_t)stream)
-               : launch_dense_f32((const __nv_bfloat16*)q, B, ldq, (const __nv_bfloat16*)items, n_items, ldi, D, out,
-                                  ld_out, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "dense kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  const int lr = f16 ? launch_dense((const __half*)q, B, ldq, (const __half*)items, n_items, ldi, D, out, ld_out,
+                                    (cudaStream_t)stream)
+                     : launch_dense((const __nv_bfloat16*)q, B, ldq, (const __nv_bfloat16*)items, n_items, ldi, D,
+                                    out, ld_out, (cudaStream_t)stream);
+  return cuda_rc(lr, "dense kernel launch");
 }
 
 extern "C" {
@@ -606,10 +639,8 @@ int ccr_argsort_scores_f32(const float* scores, int64_t B, int64_t n_cols, int64
   if (!scores || !out_rows || !out_cols) return fail(CCR_EINVAL, "null pointer");
   const size_t need = argsort_workspace_bytes(B * n_cols);
   if (!workspace || workspace_bytes < need) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, need);
-  int lr = launch_argsort(scores, B, n_cols, ld, m.indptr, m.cols, m.vals, m.nnz, m.mode, (long long*)out_rows,
-                          (long long*)out_cols, workspace, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "argsort launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(launch_argsort(scores, B, n_cols, ld, m.indptr, m.cols, m.vals, m.nnz, m.mode, (long long*)out_rows,
+                                (long long*)out_cols, workspace, (cudaStream_t)stream), "argsort launch");
 }
 
 int ccr_first_hit_rank(const int64_t* ids, int64_t B, int k, const int64_t* rel_indptr, const int64_t* rel_ids,
@@ -617,14 +648,13 @@ int ccr_first_hit_rank(const int64_t* ids, int64_t B, int k, const int64_t* rel_
   if (B < 0 || k < 1) return fail(CCR_EINVAL, "bad first-hit shape");
   if (B == 0) return CCR_OK;
   if (!ids || !rel_indptr || !out_rank) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_first_hit_rank((const long long*)ids, B, k, (const long long*)rel_indptr, (const long long*)rel_ids,
-                                 out_rank, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "first-hit kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(launch_first_hit_rank((const long long*)ids, B, k, (const long long*)rel_indptr,
+                                       (const long long*)rel_ids, out_rank, (cudaStream_t)stream),
+                 "first-hit kernel launch");
 }
 
 // ---- top-k of a materialised dense score matrix ----
-struct DensePlanC { int S, C; size_t off_counts, off_rec_hi, off_rec_lo, total; };
+struct DensePlanC { int S, C; size_t off_cand, off_counts, off_rec_hi, off_rec_lo, total; };
 static void dense_plan(long long B, long long N, int k_keep, long long nnz, DensePlanC* pl) {
   const int sms = device_sm_count();
   const long long rows = B > 0 ? B : 1;
@@ -635,11 +665,12 @@ static void dense_plan(long long B, long long N, int k_keep, long long nnz, Dens
   if (s < 1) s = 1;
   pl->S = (int)s;
   pl->C = cand_capacity(k_keep, kDenseSlack);
-  size_t off = align_up((size_t)rows * s * pl->C * sizeof(u64), 256);
-  pl->off_counts = off; off = align_up(off + (size_t)rows * s * sizeof(int), 256);
-  pl->off_rec_hi = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u64), 256);
-  pl->off_rec_lo = off; off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(u32), 256);
-  pl->total = off;
+  Carve c;
+  pl->off_cand = c.take((size_t)rows * s * pl->C * sizeof(u64));
+  pl->off_counts = c.take((size_t)rows * s * sizeof(int));
+  pl->off_rec_hi = c.take((size_t)(nnz > 0 ? nnz : 0) * sizeof(u64));
+  pl->off_rec_lo = c.take((size_t)(nnz > 0 ? nnz : 0) * sizeof(u32));
+  pl->total = c.off;
 }
 
 size_t ccr_topk_dense_workspace_bytes(int64_t B, int64_t n_cols, int k, int64_t mask_nnz, int64_t mask_max_row_nnz) {
@@ -657,43 +688,34 @@ int ccr_topk_dense_f32(const float* scores, int64_t B, int64_t n_cols, int64_t l
                        size_t workspace_bytes, void* stream) {
   if (B < 0 || n_cols < 0 || ld < n_cols) return fail(CCR_EINVAL, "bad dense top-k shape");
   if (B > 65535) return fail(CCR_EUNSUPPORTED, "dense top-k: more than 65535 rows per call");
-  if (k < 1 || k > CCR_MAX_K) return fail(CCR_EUNSUPPORTED, "k=%d outside [1,%d]", k, CCR_MAX_K);
-  if (k > n_cols) return fail(CCR_EK_RANGE, "selected index k out of range (k=%d > n=%lld)", k, (long long)n_cols);
+  int rc = check_k(k, n_cols, false);
+  if (rc) return rc;
   if (n_cols > (1LL << 31) - 512) return fail(CCR_EUNSUPPORTED, "n_cols must be < 2^31");
   MaskArgs m;
-  if (int rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, mask_max_row_nnz, mask_mode, &m)) return rc;
+  if ((rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, mask_max_row_nnz, mask_mode, &m))) return rc;
   if (B == 0) return CCR_OK;
   if (!scores || !out_ids) return fail(CCR_EINVAL, "null pointer");
-  const long long h = m.indptr ? m.h_max : 0;  // masked columns are dropped at the end: k + h candidates per row
-  if (h < 0 || k + h > CCR_MAX_K)
-    return fail(CCR_EUNSUPPORTED, "dense top-k: k + max row nnz = %lld outside [1,%d]", (long long)(k + h), CCR_MAX_K);
+  // masked columns are dropped at the end: k + h candidates per row, h a bound of the mask entries in one row
+  if (m.indptr && m.h_max < 0)
+    return fail(CCR_EUNSUPPORTED, "dense top-k: a mask needs a known mask_max_row_nnz (got %lld)",
+                (long long)mask_max_row_nnz);
+  const long long h = m.indptr ? m.h_max : 0;
+  if (k + h > CCR_MAX_K)
+    return fail(CCR_EUNSUPPORTED, "dense top-k: k + max row nnz = %lld > %d", (long long)(k + h), CCR_MAX_K);
   DensePlanC pl;
   dense_plan(B, n_cols, (int)(k + h), m.nnz, &pl);
   if (!workspace || workspace_bytes < pl.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, pl.total);
   unsigned char* ws = (unsigned char*)workspace;
   cudaStream_t st = (cudaStream_t)stream;
-  int lr = launch_select_dense(scores, ld, B, n_cols, k, (int)(k + h), m.indptr, pl.C, pl.S, (u64*)ws, (int*)(ws + pl.off_counts), st);
-  if (lr) return fail(CCR_ECUDA, "dense select launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  // one record per mask entry: the record CSR is the mask CSR
-  u64* rec_hi = (u64*)(ws + pl.off_rec_hi);
-  u32* rec_lo = (u32*)(ws + pl.off_rec_lo);
-  if (m.indptr) {
-    RecordParams rp = {};
-    rp.B = (int)B; rp.src = kRecMatrix; rp.scores = scores; rp.ld = ld; rp.n_cols = n_cols;
-    rp.mask_indptr = m.indptr; rp.mask_cols = m.cols; rp.mask_vals = m.vals; rp.mode = m.mode;
-    rp.max_entries = m.nnz; rp.rec_hi = rec_hi; rp.rec_lo = rec_lo;
-    lr = launch_entry_records(rp, st);
-    if (lr) return fail(CCR_ECUDA, "dense mask record launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  }
-  FinalizeParams fp = {};
-  fp.B = (int)B; fp.k = k; fp.C = pl.C; fp.S = pl.S; fp.cand = (u64*)ws; fp.counts = (int*)(ws + pl.off_counts);
-  fp.g_tau = nullptr;
-  fp.rec_indptr = m.indptr; fp.rec_hi = rec_hi; fp.rec_lo = rec_lo;
-  fp.drop_cols = m.cols;  // searched in the record CSR: the records are the mask entries
-  fp.id_offset = 0; fp.out_keys = nullptr; fp.out_scores = out_scores; fp.out_scores64 = out_scores64; fp.out_ids = (long long*)out_ids;
-  lr = launch_finalize(fp, st);
-  if (lr) return fail(CCR_ECUDA, "finalize launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  const Cands cb = {pl.C, pl.S, (u64*)(ws + pl.off_cand), (int*)(ws + pl.off_counts)};
+  rc = cuda_rc(launch_select_dense(scores, ld, B, n_cols, k, (int)(k + h), m.indptr, pl.C, pl.S, cb.cand, cb.counts, st),
+               "dense select launch");
+  if (rc) return rc;
+  const Records rec = {m.indptr, (u64*)(ws + pl.off_rec_hi), (u32*)(ws + pl.off_rec_lo)};
+  RecordParams rp = record_params((int)B, kRecMatrix, n_cols, m, rec);
+  rp.scores = scores; rp.ld = ld;
+  if ((rc = mask_records(rp, st))) return rc;
+  return finalize((int)B, k, cb, nullptr, rec, m.cols, 0, out_scores, out_scores64, (long long*)out_ids, false, st);
 }
 
 // ---- BM25 (lexical sibling of the dense path) ----
@@ -702,7 +724,7 @@ int ccr_topk_dense_f32(const float* scores, int64_t B, int64_t n_cols, int64_t l
 // lists per query handed to finalize.
 struct Bm25Plan {
   int S, C, streams;
-  size_t off_counts, off_tau, total;
+  size_t off_cand, off_counts, off_tau, total;
 };
 
 static Bm25Plan bm25_plan(long long Bq, long long N, int k, bool warp) {
@@ -730,10 +752,12 @@ static Bm25Plan bm25_plan(long long Bq, long long N, int k, bool warp) {
   if (s < 1) s = 1;
   pl.S = (int)s;
   pl.streams = (int)(s * per_block);
-  pl.off_counts = align_up((size_t)rows * (size_t)pl.streams * pl.C * sizeof(u64), 256);
-  // counts, then one u32 per query: the best stream threshold (row-level bound for finalize's prefilter)
-  pl.off_tau = align_up(pl.off_counts + (size_t)rows * (size_t)pl.streams * sizeof(int), 256);
-  pl.total = align_up(pl.off_tau + (size_t)rows * sizeof(u32), 256);
+  Carve c;
+  pl.off_cand = c.take((size_t)rows * (size_t)pl.streams * pl.C * sizeof(u64));
+  pl.off_counts = c.take((size_t)rows * (size_t)pl.streams * sizeof(int));
+  // then one u32 per query: the best stream threshold (row-level bound for finalize's prefilter)
+  pl.off_tau = c.take((size_t)rows * sizeof(u32));
+  pl.total = c.off;
   return pl;
 }
 
@@ -743,10 +767,8 @@ int ccr_bm25_build_impacts(const int64_t* post_indptr, const int32_t* post_docs,
   if (n_terms < 0 || nnz < 0) return fail(CCR_EINVAL, "bad bm25 index shape");
   if (nnz == 0) return CCR_OK;
   if (!post_indptr || !post_docs || !post_tf || !idf || !doc_norm || !post_val) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_bm25_impacts((const long long*)post_indptr, post_docs, post_tf, idf, doc_norm, k1 + 1.0, n_terms,
-                               nnz, post_val, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "bm25 impacts launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(launch_bm25_impacts((const long long*)post_indptr, post_docs, post_tf, idf, doc_norm, k1 + 1.0,
+                                     n_terms, nnz, post_val, (cudaStream_t)stream), "bm25 impacts launch");
 }
 
 size_t ccr_bm25_topk_workspace_bytes(int64_t Bq, int64_t n_docs, int k) {
@@ -756,8 +778,12 @@ size_t ccr_bm25_topk_workspace_bytes(int64_t Bq, int64_t n_docs, int k) {
   return tw > tb ? tw : tb;
 }
 
-static int bm25_check(const int64_t* post_indptr, const int64_t* q_indptr, const int32_t* q_terms, int64_t Bq,
-                      int64_t n_docs, int64_t max_query_terms) {
+// The arguments both BM25 scoring entries share, checked and put in one parameter block.  The kernel is the
+// warp-private one unless a query has more than kBmwMaxTerms distinct terms or CCR_BM25_BLOCKWIDE is set; k, C, S
+// and the outputs are the caller's to set.
+static int bm25_args(const int64_t* post_indptr, const int32_t* post_docs, const double* post_val,
+                     const int32_t* head_slot, const double* head_rows, const int64_t* q_indptr,
+                     const int32_t* q_terms, int64_t max_query_terms, int64_t Bq, int64_t n_docs, Bm25Params* p) {
   if (Bq < 0 || n_docs < 0) return fail(CCR_EINVAL, "bad bm25 shape");
   if (Bq > 65535) return fail(CCR_EUNSUPPORTED, "bm25: more than 65535 queries per call");
   if (n_docs > (1LL << 31) - 512) return fail(CCR_EUNSUPPORTED, "n_docs must be < 2^31");
@@ -766,6 +792,12 @@ static int bm25_check(const int64_t* post_indptr, const int64_t* q_indptr, const
                 kBmMaxTerms);
   if (Bq > 0 && (!q_indptr || (max_query_terms > 0 && (!q_terms || !post_indptr))))
     return fail(CCR_EINVAL, "null pointer");
+  if ((head_slot == nullptr) != (head_rows == nullptr)) return fail(CCR_EINVAL, "head_slot and head_rows go together");
+  *p = {};
+  p->post_indptr = (const long long*)post_indptr; p->post_docs = post_docs; p->post_val = post_val;
+  p->head_slot = head_slot; p->head_rows = head_rows; p->ld_head = ccr_bm25_head_row_pitch(n_docs);
+  p->q_indptr = (const long long*)q_indptr; p->q_terms = q_terms; p->Bq = Bq; p->N = n_docs;
+  p->warp = max_query_terms <= kBmwMaxTerms && !knobs().bm25_blockwide;
   return CCR_OK;
 }
 
@@ -779,16 +811,14 @@ int ccr_bm25_build_head_rows(const int64_t* post_indptr, const int32_t* post_doc
   if (n_head < 0 || n_terms < 0 || n_docs < 0) return fail(CCR_EINVAL, "bad bm25 head-row shape");
   if (n_terms > 0 && !head_slot) return fail(CCR_EINVAL, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  if (n_terms > 0 && cudaMemsetAsync(head_slot, 0xFF, (size_t)n_terms * sizeof(int32_t), st) != cudaSuccess)  // all -1
-    return fail(CCR_ECUDA, "memset bm25 head slots");
-  if (n_head == 0) return CCR_OK;
+  int rc = n_terms > 0 ? cuda_rc(cudaMemsetAsync(head_slot, 0xFF, (size_t)n_terms * sizeof(int32_t), st),  // all -1
+                                 "memset bm25 head slots") : CCR_OK;
+  if (rc || n_head == 0) return rc;
   if (!post_indptr || !post_docs || !post_val || !head_terms || !head_rows) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_bm25_head_slots(head_terms, n_head, n_terms, head_slot, st);
-  if (lr) return fail(CCR_ECUDA, "bm25 head slots launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  lr = launch_bm25_head_rows((const long long*)post_indptr, post_docs, post_val, head_terms, n_head, n_terms,
-                             ccr_bm25_head_row_pitch(n_docs), head_rows, st);
-  if (lr) return fail(CCR_ECUDA, "bm25 head rows launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  if ((rc = cuda_rc(launch_bm25_head_slots(head_terms, n_head, n_terms, head_slot, st), "bm25 head slots launch")))
+    return rc;
+  return cuda_rc(launch_bm25_head_rows((const long long*)post_indptr, post_docs, post_val, head_terms, n_head, n_terms,
+                                       ccr_bm25_head_row_pitch(n_docs), head_rows, st), "bm25 head rows launch");
 }
 
 int ccr_bm25_topk(const int64_t* post_indptr, const int32_t* post_docs, const double* post_val,
@@ -796,89 +826,79 @@ int ccr_bm25_topk(const int64_t* post_indptr, const int32_t* post_docs, const do
                   const int64_t* q_indptr, const int32_t* q_terms, int64_t max_query_terms, int64_t Bq,
                   int64_t n_docs, int k, float* out_scores, int64_t* out_ids, void* workspace,
                   size_t workspace_bytes, void* stream) {
-  int rc = bm25_check(post_indptr, q_indptr, q_terms, Bq, n_docs, max_query_terms);
-  if (rc) return rc;
-  if ((head_slot == nullptr) != (head_rows == nullptr)) return fail(CCR_EINVAL, "head_slot and head_rows go together");
-  if (k < 1 || k > CCR_MAX_K) return fail(CCR_EUNSUPPORTED, "k=%d outside [1,%d]", k, CCR_MAX_K);
-  if (k > n_docs) return fail(CCR_EK_RANGE, "selected index k out of range (k=%d > n=%lld)", k, (long long)n_docs);
+  Bm25Params p;
+  int rc = bm25_args(post_indptr, post_docs, post_val, head_slot, head_rows, q_indptr, q_terms, max_query_terms, Bq,
+                     n_docs, &p);
+  if (rc || (rc = check_k(k, n_docs, false))) return rc;
   if (Bq == 0) return CCR_OK;
   if (!out_scores || !out_ids) return fail(CCR_EINVAL, "null pointer");
-  const bool warp = max_query_terms <= kBmwMaxTerms && !knobs().bm25_blockwide;
-  const Bm25Plan pl = bm25_plan(Bq, n_docs, k, warp);
+  const Bm25Plan pl = bm25_plan(Bq, n_docs, k, p.warp);
   if (!workspace || workspace_bytes < pl.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, pl.total);
   unsigned char* ws = (unsigned char*)workspace;
   cudaStream_t st = (cudaStream_t)stream;
-  const long long* pi = (const long long*)post_indptr;
-  const long long* qi = (const long long*)q_indptr;
-  u64* cand = (u64*)ws;
-  int* counts = (int*)(ws + pl.off_counts);
+  const Cands cb = {pl.C, pl.streams, (u64*)(ws + pl.off_cand), (int*)(ws + pl.off_counts)};
+  p.k = k; p.C = pl.C; p.S = pl.S; p.cand = cb.cand; p.counts = cb.counts;
   // per query: max over its streams of the stream's k-th best score (every stream that pruned holds >= k
   // docs at or above its threshold, so the row's k-th best is at least the largest of them)
-  u32* row_tau = (u32*)(ws + pl.off_tau);
-  if (cudaMemsetAsync(row_tau, 0, (size_t)Bq * sizeof(u32), st) != cudaSuccess) return fail(CCR_ECUDA, "memset bm25 bounds");
-  int lr = warp ? launch_bm25_topk_warp(pi, post_docs, post_val, head_slot, head_rows, ccr_bm25_head_row_pitch(n_docs), qi,
-                                        q_terms, Bq, n_docs, k, pl.C, pl.S, cand, counts, row_tau, nullptr, 0, st)
-                : launch_bm25_topk(pi, post_docs, post_val, head_slot, head_rows, ccr_bm25_head_row_pitch(n_docs), qi, q_terms,
-                                   Bq, n_docs, k, pl.C, pl.S, cand, counts, nullptr, 0, st);
-  if (lr) return fail(CCR_ECUDA, "bm25 top-k launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  FinalizeParams fp = {};
-  fp.B = (int)Bq; fp.k = k; fp.C = pl.C; fp.S = pl.streams; fp.cand = cand; fp.counts = counts;
-  fp.g_tau = warp ? row_tau : nullptr; fp.rec_indptr = nullptr; fp.rec_hi = nullptr; fp.rec_lo = nullptr; fp.drop_cols = nullptr;
-  fp.id_offset = 0; fp.out_keys = nullptr; fp.out_scores = out_scores; fp.out_scores64 = nullptr; fp.out_ids = (long long*)out_ids;
-  lr = launch_finalize(fp, st);
-  if (lr) return fail(CCR_ECUDA, "finalize launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  p.row_tau = (u32*)(ws + pl.off_tau);
+  if ((rc = cuda_rc(cudaMemsetAsync(p.row_tau, 0, (size_t)Bq * sizeof(u32), st), "memset bm25 bounds"))) return rc;
+  if ((rc = cuda_rc(launch_bm25(p, st), "bm25 top-k launch"))) return rc;
+  return finalize((int)Bq, k, cb, p.warp ? p.row_tau : nullptr, {}, nullptr, 0, out_scores, nullptr,
+                  (long long*)out_ids, false, st);
 }
 
 int ccr_bm25_scores_f64(const int64_t* post_indptr, const int32_t* post_docs, const double* post_val,
                         const int32_t* head_slot, const double* head_rows,
                         const int64_t* q_indptr, const int32_t* q_terms, int64_t max_query_terms, int64_t Bq,
                         int64_t n_docs, double* scores, int64_t ld, void* stream) {
-  int rc = bm25_check(post_indptr, q_indptr, q_terms, Bq, n_docs, max_query_terms);
+  Bm25Params p;
+  int rc = bm25_args(post_indptr, post_docs, post_val, head_slot, head_rows, q_indptr, q_terms, max_query_terms, Bq,
+                     n_docs, &p);
   if (rc) return rc;
-  if ((head_slot == nullptr) != (head_rows == nullptr)) return fail(CCR_EINVAL, "head_slot and head_rows go together");
   if (ld < n_docs) return fail(CCR_EINVAL, "ld < n_docs");
   if (Bq == 0 || n_docs == 0) return CCR_OK;
   if (!scores) return fail(CCR_EINVAL, "null pointer");
-  const bool warp = max_query_terms <= kBmwMaxTerms && !knobs().bm25_blockwide;
-  const Bm25Plan pl = bm25_plan(Bq, n_docs, 1, warp);
-  int lr = warp ? launch_bm25_topk_warp((const long long*)post_indptr, post_docs, post_val, head_slot, head_rows,
-                                        ccr_bm25_head_row_pitch(n_docs), (const long long*)q_indptr,
-                                        q_terms, Bq, n_docs, 1, pl.C, pl.S, nullptr, nullptr, nullptr, scores, ld, (cudaStream_t)stream)
-                : launch_bm25_topk((const long long*)post_indptr, post_docs, post_val, head_slot, head_rows,
-                                   ccr_bm25_head_row_pitch(n_docs), (const long long*)q_indptr, q_terms,
-                                   Bq, n_docs, 1, pl.C, pl.S, nullptr, nullptr, scores, ld, (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "bm25 scores launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  const Bm25Plan pl = bm25_plan(Bq, n_docs, 1, p.warp);
+  p.k = 1; p.C = pl.C; p.S = pl.S; p.dense_out = scores; p.ld_out = ld;
+  return cuda_rc(launch_bm25(p, (cudaStream_t)stream), "bm25 scores launch");
 }
 
 }  // extern "C"
 
 // ---- exact fp32 ranking (DESIGN.md section 6b) ----
 namespace {
-struct ExactLayout { size_t off_scores, off_ids, off_neg, off_rec_ip, off_rec_hi, off_rec_lo, total; };
+// Exact ranking workspace: the scan stage's own (the fused call's for kc candidates per row), its [B, kc] outputs and
+// the -inf values of its SET mask, then the entry records: the record CSR (B + 1 row offsets) and 12 bytes per entry.
+// The re-rank alone has the records only.
+struct ExactLayout {
+  int kc;
+  size_t scan_bytes, off_scores, off_ids, off_neg, off_rec_ip, off_rec_hi, off_rec_lo, total;
+};
 
-// entry records after `off`: the record CSR (B + 1 row offsets), then 12 bytes per entry
-void entry_layout(size_t off, long long B, long long n_entries, ExactLayout* L) {
-  L->off_rec_ip = off; off = align_up(off + (size_t)(B + 1) * sizeof(long long), 256);
-  L->off_rec_hi = off; off = align_up(off + (size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u64), 256);
-  L->off_rec_lo = off; off = align_up(off + (size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u32), 256);
-  L->total = off;
+// L with the entry records of n_entries entries taken after c
+ExactLayout add_records(ExactLayout L, Carve c, long long B, long long n_entries) {
+  L.off_rec_ip = c.take((size_t)(B + 1) * sizeof(long long));
+  L.off_rec_hi = c.take((size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u64));
+  L.off_rec_lo = c.take((size_t)(n_entries > 0 ? n_entries : 0) * sizeof(u32));
+  L.total = c.off;
+  return L;
 }
 
-// stage-1 workspace, its [B, k'] outputs, the -inf values of its SET mask, the entry records
-void exact_layout(const Plan& pl1, long long B, int kc, long long nnz, ExactLayout* L) {
-  size_t off = align_up(pl1.total, 256);
-  L->off_scores = off; off = align_up(off + (size_t)B * kc * sizeof(float), 256);
-  L->off_ids = off;    off = align_up(off + (size_t)B * kc * sizeof(long long), 256);
-  L->off_neg = off;    off = align_up(off + (size_t)(nnz > 0 ? nnz : 0) * sizeof(double), 256);
-  entry_layout(off, B, B * (long long)kc + (nnz > 0 ? nnz : 0), L);
-}
-
-int check_exact_rows(const void* q, int64_t ldq, const void* items, int64_t ldi, int D) {
-  if (ldq < D || ldi < D || ldq % 8 || ldi % 8) return fail(CCR_EINVAL, "ldq/ldi must be >= D and multiples of 8");
-  if (((uintptr_t)q & 15) || ((uintptr_t)items & 15)) return fail(CCR_EINVAL, "q/items must be 16-byte aligned");
-  return CCR_OK;
+ExactLayout exact_layout(long long B, long long n_items, int D, int k, long long nnz, long long h_max, int flags) {
+  ExactLayout L = {};
+  Plan pl;
+  make_plan(B, n_items, D, k, 0, -1, flags, &pl);
+  L.kc = pl.k_cand;
+  if (L.kc > 0) {
+    make_plan(B, n_items, D, L.kc, nnz, h_max, flags, &pl);
+    L.scan_bytes = pl.total;
+  }
+  Carve c;
+  c.take(L.scan_bytes);
+  L.off_scores = c.take((size_t)B * L.kc * sizeof(float));
+  L.off_ids = c.take((size_t)B * L.kc * sizeof(long long));
+  L.off_neg = c.take((size_t)(nnz > 0 ? nnz : 0) * sizeof(double));
+  return add_records(L, c, B, B * (long long)L.kc + (nnz > 0 ? nnz : 0));
 }
 
 // entry records of (candidates U mask entries) -> exact values -> finalize_kernel with no stream candidates
@@ -886,23 +906,15 @@ int rerank(const float* q, long long B, long long ldq, const float* items, long 
            int k, const long long* cand_indptr, const long long* cand_ids, long long cand_stride, long long cand_nnz,
            const MaskArgs& m, long long id_offset, float* out_scores, double* out_scores64, long long* out_ids,
            unsigned char* ws, const ExactLayout& L, cudaStream_t st) {
-  RecordParams rp = {};
-  rp.B = (int)B; rp.src = kRecExactDot; rp.q = q; rp.ldq = ldq; rp.items = items; rp.ldi = ldi; rp.D = D;
-  rp.n_cols = n_items;
-  rp.mask_indptr = m.indptr; rp.mask_cols = m.cols; rp.mask_vals = m.vals; rp.mode = m.mode;
+  long long* rec_indptr = (long long*)(ws + L.off_rec_ip);
+  const Records rec = {rec_indptr, (u64*)(ws + L.off_rec_hi), (u32*)(ws + L.off_rec_lo)};
+  RecordParams rp = record_params((int)B, kRecExactDot, n_items, m, rec);
+  rp.q = q; rp.ldq = ldq; rp.items = items; rp.ldi = ldi; rp.D = D;
   rp.cand_indptr = cand_indptr; rp.cand_ids = cand_ids; rp.cand_stride = cand_stride;
-  rp.rec_indptr = (long long*)(ws + L.off_rec_ip); rp.max_entries = cand_nnz + m.nnz;
-  rp.rec_hi = (u64*)(ws + L.off_rec_hi); rp.rec_lo = (u32*)(ws + L.off_rec_lo);
-  int lr = launch_entry_records(rp, st);
-  if (lr) return fail(CCR_ECUDA, "exact value kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  FinalizeParams fp = {};
-  fp.B = (int)B; fp.k = k; fp.C = 0; fp.S = 0; fp.cand = nullptr; fp.counts = nullptr; fp.g_tau = nullptr;
-  fp.rec_indptr = rp.rec_indptr; fp.rec_hi = rp.rec_hi; fp.rec_lo = rp.rec_lo; fp.drop_cols = nullptr;
-  fp.id_offset = id_offset; fp.out_scores = out_scores; fp.out_scores64 = out_scores64; fp.out_keys = nullptr;
-  fp.out_ids = out_ids;
-  lr = launch_finalize(fp, st);
-  if (lr) return fail(CCR_ECUDA, "finalize launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  rp.rec_indptr = rec_indptr; rp.max_entries = cand_nnz + m.nnz;
+  int rc = cuda_rc(launch_entry_records(rp, st), "exact value kernel launch");
+  if (rc) return rc;
+  return finalize((int)B, k, {}, nullptr, rec, nullptr, id_offset, out_scores, out_scores64, out_ids, false, st);
 }
 }  // namespace
 
@@ -922,27 +934,15 @@ int ccr_exact_k_candidates(int64_t B, int64_t n_items, int D, int k, int flags) 
 
 int ccr_ingest_rows_f32_f32(const float* src, int64_t n, int D, int64_t ld_src, float* dst, int64_t ld_dst,
                             int normalize, double* max_row_norm, void* stream) {
-  if (n < 0 || D <= 0 || ld_src < D || ld_dst < D) return fail(CCR_EINVAL, "bad ingest shape");
-  if (n == 0) return CCR_OK;
-  if (!src || !dst) return fail(CCR_EINVAL, "null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  int lr = launch_ingest_f32_f32(src, n, D, ld_src, dst, ld_dst, normalize, st);
-  if (!lr && max_row_norm) lr = launch_row_norm_max(dst, n, D, ld_dst, max_row_norm, st);
-  if (lr) return fail(CCR_ECUDA, "ingest kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  int rc = ingest_rows<float, float>("ingest", src, n, D, ld_src, dst, ld_dst, normalize, nullptr, stream);
+  if (rc || !max_row_norm) return rc;
+  return cuda_rc(launch_row_norm_max(dst, n, D, ld_dst, max_row_norm, (cudaStream_t)stream), "row norm kernel launch");
 }
 
 size_t ccr_score_topk_exact_workspace_bytes(int64_t B, int64_t n_items, int D, int k, int64_t mask_nnz,
                                             int64_t mask_max_row_nnz, int flags) {
   if (check_shape(B, n_items, D, k, flags | CCR_FLAG_ALLOW_SHORT) != CCR_OK || mask_nnz < 0) return 0;
-  Plan pl0, pl1;
-  make_plan(B, n_items, D, k, 0, -1, flags, &pl0);
-  pl1.total = 0;
-  if (pl0.k_cand > 0)
-    make_plan(B, n_items, D, pl0.k_cand, mask_nnz, mask_h_max(mask_nnz, mask_max_row_nnz), flags, &pl1);
-  ExactLayout L;
-  exact_layout(pl1, B, pl0.k_cand, mask_nnz, &L);
-  return L.total;
+  return exact_layout(B, n_items, D, k, mask_nnz, mask_h_max(mask_nnz, mask_max_row_nnz), flags).total;
 }
 
 int ccr_score_topk_exact(const float* q, const void* q_scan, int64_t B, int64_t ldq, const float* items,
@@ -959,17 +959,12 @@ int ccr_score_topk_exact(const float* q, const void* q_scan, int64_t B, int64_t 
   if (!q || !q_scan || !out_ids || !out_scores64 || !out_uncertified || !out_tau || !uncertified_count || !max_row_norm)
     return fail(CCR_EINVAL, "null q / q_scan / out_ids / out_scores64 / certificate outputs / max_row_norm");
   if (n_items > 0 && (!items || !items_scan)) return fail(CCR_EINVAL, "null items");
-  if ((rc = check_exact_rows(q, ldq, items, ldi, D)) || (rc = check_exact_rows(q_scan, ldq, items_scan, ldi, D))) return rc;
+  if ((rc = check_rows(q, ldq, items, ldi, D)) || (rc = check_rows(q_scan, ldq, items_scan, ldi, D))) return rc;
   MaskArgs m;
   if ((rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, mask_max_row_nnz, mask_mode, &m))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  Plan pl0, pl1;
-  make_plan(B, n_items, D, k, 0, -1, flags, &pl0);
-  const int kc = pl0.k_cand;
-  pl1.total = 0;
-  if (kc > 0) make_plan(B, n_items, D, kc, m.nnz, m.h_max, flags, &pl1);
-  ExactLayout L;
-  exact_layout(pl1, B, kc, m.nnz, &L);
+  const ExactLayout L = exact_layout(B, n_items, D, k, m.nnz, m.h_max, flags);
+  const int kc = L.kc;
   if (!workspace || workspace_bytes < L.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, L.total);
   unsigned char* ws = (unsigned char*)workspace;
   float* s1_scores = (float*)(ws + L.off_scores);
@@ -978,28 +973,23 @@ int ccr_score_topk_exact(const float* q, const void* q_scan, int64_t B, int64_t 
     // stage 1: the unchanged scan on the scan copies, every mask entry ranked last (SET -inf) so that none
     // takes a candidate slot; the re-rank below gives each its true value
     double* neg = (double*)(ws + L.off_neg);
-    int lr = launch_fill_f64(neg, m.nnz, -INFINITY, st);
-    if (lr) return fail(CCR_ECUDA, "fill launch failed: %s", cudaGetErrorString((cudaError_t)lr));
+    if ((rc = cuda_rc(launch_fill_f64(neg, m.nnz, -INFINITY, st), "fill launch"))) return rc;
     rc = ccr_score_topk_bf16(q_scan, B, ldq, items_scan, n_items, ldi, D, kc, (const int64_t*)m.indptr, m.cols, neg,
-                             m.nnz, m.h_max, CCR_MASK_SET, 0, s1_scores, nullptr, (int64_t*)s1_ids, ws, pl1.total,
+                             m.nnz, m.h_max, CCR_MASK_SET, 0, s1_scores, nullptr, (int64_t*)s1_ids, ws, L.scan_bytes,
                              flags & (CCR_ALGO_MASK | CCR_FLAG_F16), stream);
     if (rc) return rc;
   }
   rc = rerank(q, B, ldq, items, n_items, ldi, D, k, nullptr, s1_ids, kc, B * (long long)kc, m, id_offset, out_scores,
               out_scores64, (long long*)out_ids, ws, L, st);
   if (rc) return rc;
-  int lr = launch_exact_certify(q, ldq, (int)B, D, (flags & CCR_FLAG_F16) ? 1 : 0, max_row_norm, k, kc, n_items,
-                                s1_scores, s1_ids, m.indptr, m.cols, out_scores64, knobs().exact_fallback,
-                                out_uncertified, out_tau, uncertified_count, st);
-  if (lr) return fail(CCR_ECUDA, "certify kernel launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(launch_exact_certify(q, ldq, (int)B, D, (flags & CCR_FLAG_F16) ? 1 : 0, max_row_norm, k, kc, n_items,
+                                      s1_scores, s1_ids, m.indptr, m.cols, out_scores64, knobs().exact_fallback,
+                                      out_uncertified, out_tau, uncertified_count, st), "certify kernel launch");
 }
 
 size_t ccr_rerank_exact_workspace_bytes(int64_t B, int64_t cand_nnz, int64_t mask_nnz) {
   if (B < 0 || cand_nnz < 0 || mask_nnz < 0) return 0;
-  ExactLayout L;
-  entry_layout(0, B, cand_nnz + mask_nnz, &L);
-  return L.total;
+  return add_records({}, {}, B, cand_nnz + mask_nnz).total;
 }
 
 int ccr_rerank_exact(const float* q, int64_t B, int64_t ldq, const float* items, int64_t n_items, int64_t ldi, int D,
@@ -1009,16 +999,14 @@ int ccr_rerank_exact(const float* q, int64_t B, int64_t ldq, const float* items,
                      void* workspace, size_t workspace_bytes, int flags, void* stream) {
   int rc = check_shape(B, n_items, D, k, flags);
   if (rc) return rc;
-  if (B > 0x7fffffff) return fail(CCR_EUNSUPPORTED, "B=%lld", (long long)B);
   if (B == 0) return CCR_OK;
   if (!q || !out_ids || !cand_indptr || (cand_nnz > 0 && !cand_ids)) return fail(CCR_EINVAL, "null q / out_ids / candidates");
   if (cand_nnz < 0) return fail(CCR_EINVAL, "cand_nnz = %lld", (long long)cand_nnz);
   if (n_items > 0 && !items) return fail(CCR_EINVAL, "null items");
-  if ((rc = check_exact_rows(q, ldq, items, ldi, D))) return rc;
+  if ((rc = check_rows(q, ldq, items, ldi, D))) return rc;
   MaskArgs m;
   if ((rc = parse_mask(mask_indptr, mask_cols, mask_vals, mask_nnz, -1, mask_mode, &m))) return rc;
-  ExactLayout L;
-  entry_layout(0, B, cand_nnz + m.nnz, &L);
+  const ExactLayout L = add_records({}, {}, B, cand_nnz + m.nnz);
   if (!workspace || workspace_bytes < L.total) return fail(CCR_EWORKSPACE, "workspace %zu < %zu", workspace_bytes, L.total);
   return rerank(q, B, ldq, items, n_items, ldi, D, k, (const long long*)cand_indptr, (const long long*)cand_ids, 0,
                 cand_nnz, m, id_offset, out_scores, out_scores64, (long long*)out_ids, (unsigned char*)workspace, L,
@@ -1030,10 +1018,8 @@ int ccr_threshold_compact(const float* scores, int64_t R, int64_t N, int64_t ld,
   if (R < 0 || N < 0 || ld < N) return fail(CCR_EINVAL, "bad compaction shape");
   if (R == 0) return CCR_OK;
   if (!tau || !out_indptr || (N > 0 && !scores)) return fail(CCR_EINVAL, "null pointer");
-  int lr = launch_threshold_compact(scores, R, N, ld, tau, (long long*)out_indptr, (long long*)out_ids,
-                                    (cudaStream_t)stream);
-  if (lr) return fail(CCR_ECUDA, "compaction launch failed: %s", cudaGetErrorString((cudaError_t)lr));
-  return CCR_OK;
+  return cuda_rc(launch_threshold_compact(scores, R, N, ld, tau, (long long*)out_indptr, (long long*)out_ids,
+                                          (cudaStream_t)stream), "compaction launch");
 }
 
 }  // extern "C"

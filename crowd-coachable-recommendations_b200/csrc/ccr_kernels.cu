@@ -816,40 +816,20 @@ __global__ void __launch_bounds__(256) ingest_kernel(const SrcT* __restrict__ sr
   }
 }
 
-int launch_ingest_f32(const float* src, long long n, int D, long long ld_src, __nv_bfloat16* dst,
-                      long long ld_dst, int normalize, cudaStream_t st) {
+template <typename SrcT, typename DstT>
+int launch_ingest(const SrcT* src, long long n, int D, long long ld_src, DstT* dst, long long ld_dst, int normalize,
+                  int* overflow, cudaStream_t st) {
   if (n == 0) return 0;
-  ingest_kernel<float, __nv_bfloat16><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst,
-                                                                              normalize, nullptr);
+  ingest_kernel<SrcT, DstT><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, normalize,
+                                                                     overflow);
   return (int)cudaGetLastError();
 }
-int launch_normalize_bf16(const __nv_bfloat16* src, long long n, int D, long long ld_src,
-                          __nv_bfloat16* dst, long long ld_dst, cudaStream_t st) {
-  if (n == 0) return 0;
-  ingest_kernel<__nv_bfloat16, __nv_bfloat16><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst,
-                                                                                      ld_dst, 1, nullptr);
-  return (int)cudaGetLastError();
-}
-int launch_ingest_f32_f16(const float* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
-                          int normalize, int* overflow_count, cudaStream_t st) {
-  if (n == 0) return 0;
-  ingest_kernel<float, __half><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, normalize,
-                                                                       overflow_count);
-  return (int)cudaGetLastError();
-}
-int launch_ingest_f32_f32(const float* src, long long n, int D, long long ld_src, float* dst, long long ld_dst,
-                          int normalize, cudaStream_t st) {
-  if (n == 0) return 0;
-  ingest_kernel<float, float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, normalize,
-                                                                      nullptr);
-  return (int)cudaGetLastError();
-}
-int launch_normalize_f16(const __half* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
-                         cudaStream_t st) {
-  if (n == 0) return 0;
-  ingest_kernel<__half, __half><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(src, n, D, ld_src, dst, ld_dst, 1, nullptr);
-  return (int)cudaGetLastError();
-}
+template int launch_ingest(const float*, long long, int, long long, __nv_bfloat16*, long long, int, int*, cudaStream_t);
+template int launch_ingest(const float*, long long, int, long long, __half*, long long, int, int*, cudaStream_t);
+template int launch_ingest(const float*, long long, int, long long, float*, long long, int, int*, cudaStream_t);
+template int launch_ingest(const __nv_bfloat16*, long long, int, long long, __nv_bfloat16*, long long, int, int*,
+                           cudaStream_t);
+template int launch_ingest(const __half*, long long, int, long long, __half*, long long, int, int*, cudaStream_t);
 
 // =======================================================================================
 // Dense fp32 score tile (not a hot path): one warp per (row, item).
@@ -879,20 +859,18 @@ __global__ void __launch_bounds__(256) dense_kernel(const T* __restrict__ q, lon
   if (lane == 0) out[row * ld_out + item] = acc;
 }
 
-int launch_dense_f32(const __nv_bfloat16* q, long long B, long long ldq, const __nv_bfloat16* items,
-                     long long n, long long ldi, int D, float* out, long long ld_out, cudaStream_t st) {
+template <typename T>
+int launch_dense(const T* q, long long B, long long ldq, const T* items, long long n, long long ldi, int D, float* out,
+                 long long ld_out, cudaStream_t st) {
   if (B == 0 || n == 0) return 0;
   dim3 grid((unsigned)((n + 7) / 8), (unsigned)B);
-  dense_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(q, B, ldq, items, n, ldi, D, out, ld_out);
+  dense_kernel<T><<<grid, 256, 0, st>>>(q, B, ldq, items, n, ldi, D, out, ld_out);
   return (int)cudaGetLastError();
 }
-int launch_dense_f32_f16(const __half* q, long long B, long long ldq, const __half* items, long long n, long long ldi,
-                         int D, float* out, long long ld_out, cudaStream_t st) {
-  if (B == 0 || n == 0) return 0;
-  dim3 grid((unsigned)((n + 7) / 8), (unsigned)B);
-  dense_kernel<__half><<<grid, 256, 0, st>>>(q, B, ldq, items, n, ldi, D, out, ld_out);
-  return (int)cudaGetLastError();
-}
+template int launch_dense(const __nv_bfloat16*, long long, long long, const __nv_bfloat16*, long long, long long, int,
+                          float*, long long, cudaStream_t);
+template int launch_dense(const __half*, long long, long long, const __half*, long long, long long, int, float*,
+                          long long, cudaStream_t);
 
 // =======================================================================================
 // BM25 (lexical sibling of the dense path; reference: scripts/bm_25.py:27-45 scored per query by
@@ -1076,19 +1054,6 @@ __global__ void __launch_bounds__(kBmThreads) bm25_topk_kernel(const long long* 
     __syncthreads();
   }
   if (counts && tid == 0) counts[(long long)row * S + split] = s_st.cnt;
-}
-
-int launch_bm25_topk(const long long* post_indptr, const int* post_docs, const double* post_val,
-                     const int* head_slot, const double* head_rows, long long ld_head,
-                     const long long* q_indptr, const int* q_terms, long long Bq, long long N, int k, int C, int S,
-                     u64* cand, int* counts, double* dense_out, long long ld_out, cudaStream_t st) {
-  if (Bq <= 0 || N <= 0) return 0;
-  cudaError_t e = cudaFuncSetAttribute(bm25_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBmSmem);
-  if (e != cudaSuccess) return (int)e;
-  dim3 grid((unsigned)S, (unsigned)Bq);
-  bm25_topk_kernel<<<grid, kBmThreads, kBmSmem, st>>>(post_indptr, post_docs, post_val, head_slot, head_rows, ld_head,
-                                                     q_indptr, q_terms, N, k, C, S, cand, counts, dense_out, ld_out);
-  return (int)cudaGetLastError();
 }
 
 // =======================================================================================
@@ -1313,15 +1278,20 @@ __global__ void __launch_bounds__(kBmwWarps * 32, kBmwBlocksPerSm) bm25_topk_war
   }
 }
 
-int launch_bm25_topk_warp(const long long* post_indptr, const int* post_docs, const double* post_val,
-                          const int* head_slot, const double* head_rows, long long ld_head,
-                          const long long* q_indptr, const int* q_terms, long long Bq, long long N, int k, int C, int S,
-                          u64* cand, int* counts, u32* row_tau, double* dense_out, long long ld_out, cudaStream_t st) {
-  if (Bq <= 0 || N <= 0) return 0;
-  dim3 grid((unsigned)S, (unsigned)Bq);
-  bm25_topk_warp_kernel<<<grid, kBmwWarps * 32, 0, st>>>(post_indptr, post_docs, post_val, head_slot, head_rows, ld_head,
-                                                        q_indptr, q_terms, N, k, C, S, cand, counts, row_tau, dense_out,
-                                                        ld_out);
+int launch_bm25(const Bm25Params& p, cudaStream_t st) {
+  if (p.Bq <= 0 || p.N <= 0) return 0;
+  dim3 grid((unsigned)p.S, (unsigned)p.Bq);
+  if (p.warp) {
+    bm25_topk_warp_kernel<<<grid, kBmwWarps * 32, 0, st>>>(p.post_indptr, p.post_docs, p.post_val, p.head_slot,
+                                                          p.head_rows, p.ld_head, p.q_indptr, p.q_terms, p.N, p.k, p.C,
+                                                          p.S, p.cand, p.counts, p.row_tau, p.dense_out, p.ld_out);
+  } else {
+    cudaError_t e = cudaFuncSetAttribute(bm25_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBmSmem);
+    if (e != cudaSuccess) return (int)e;
+    bm25_topk_kernel<<<grid, kBmThreads, kBmSmem, st>>>(p.post_indptr, p.post_docs, p.post_val, p.head_slot,
+                                                       p.head_rows, p.ld_head, p.q_indptr, p.q_terms, p.N, p.k, p.C,
+                                                       p.S, p.cand, p.counts, p.dense_out, p.ld_out);
+  }
   return (int)cudaGetLastError();
 }
 

@@ -144,23 +144,17 @@ int launch_merge_keys(const u64* keys, int G, long long B, int k_in, int k_out, 
 int launch_unpack_keys(const u64* keys, long long n, float* os, long long* oi, cudaStream_t st);
 int launch_mask_shard(const long long* indptr, const int* cols, const double* vals, long long B, int lo, int hi,
                       long long* out_indptr, int* out_cols, double* out_vals, cudaStream_t st);
-int launch_ingest_f32(const float* src, long long n, int D, long long ld_src, __nv_bfloat16* dst,
-                      long long ld_dst, int normalize, cudaStream_t st);
-int launch_normalize_bf16(const __nv_bfloat16* src, long long n, int D, long long ld_src,
-                          __nv_bfloat16* dst, long long ld_dst, cudaStream_t st);
-int launch_dense_f32(const __nv_bfloat16* q, long long B, long long ldq, const __nv_bfloat16* items,
-                     long long n, long long ldi, int D, float* out, long long ld_out, cudaStream_t st);
-// fp16 twins; overflow_count (device int32, may be null) += outputs that are not finite
-int launch_ingest_f32_f16(const float* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
-                          int normalize, int* overflow_count, cudaStream_t st);
-int launch_normalize_f16(const __half* src, long long n, int D, long long ld_src, __half* dst, long long ld_dst,
-                         cudaStream_t st);
-int launch_dense_f32_f16(const __half* q, long long B, long long ldq, const __half* items, long long n, long long ldi,
-                         int D, float* out, long long ld_out, cudaStream_t st);
+// table rows SrcT -> DstT (float -> bf16 / fp16 / float, bf16 -> bf16, fp16 -> fp16); overflow (device int32, may
+// be null) += outputs that are not finite
+template <typename SrcT, typename DstT>
+int launch_ingest(const SrcT* src, long long n, int D, long long ld_src, DstT* dst, long long ld_dst, int normalize,
+                  int* overflow, cudaStream_t st);
+// fp32 score tile of bf16 or fp16 rows
+template <typename T>
+int launch_dense(const T* q, long long B, long long ldq, const T* items, long long n, long long ldi, int D, float* out,
+                 long long ld_out, cudaStream_t st);
 
-// exact tables: fp32 rows (ingest_kernel<float, float>, ccr_kernels.cu) and the exact ranking stages (ccr_exact.cu)
-int launch_ingest_f32_f32(const float* src, long long n, int D, long long ld_src, float* dst, long long ld_dst,
-                          int normalize, cudaStream_t st);
+// the exact ranking stages (ccr_exact.cu)
 int launch_row_norm_max(const float* rows, long long n, int D, long long ld, double* v_max, cudaStream_t st);
 int launch_fill_f64(double* dst, long long n, double v, cudaStream_t st);
 // per row: certified (0) or not (1), tau = RD(L_k - E); uncertified rows are added to *count
@@ -200,10 +194,19 @@ constexpr int kBmwSketchM = 5;       // query bound = the 5th largest of the str
 constexpr int kBmwDepth = 4;         // batches of 32 postings in flight per warp on a dense term
 constexpr int kBmwBlocksPerSm = 4;   // 42.5 KB of static shared memory per block; 64 registers per
                                      // thread (5 blocks = 48 registers spill: 46.7 vs 39.1 ms, r02_bm25.md)
-int launch_bm25_topk_warp(const long long* post_indptr, const int* post_docs, const double* post_val,
-                          const int* head_slot, const double* head_rows, long long ld_head,
-                          const long long* q_indptr, const int* q_terms, long long Bq, long long N, int k, int C, int S,
-                          u64* cand, int* counts, u32* row_tau, double* dense_out, long long ld_out, cudaStream_t st);
+// One BM25 scoring call: Bq queries over N docs, S doc splits per query.  Top-k mode fills cand / counts (C keys
+// per stream) and, warp-private kernel only, row_tau; score mode (dense_out set) writes every score instead.
+struct Bm25Params {
+  const long long* post_indptr; const int* post_docs; const double* post_val;  // postings and their impacts
+  const int* head_slot; const double* head_rows; long long ld_head;            // dense head-term rows, or null
+  const long long* q_indptr; const int* q_terms;                               // the queries' distinct terms
+  long long Bq, N;
+  int k, C, S;
+  int warp;  // 1: the warp-private kernel (queries of <= kBmwMaxTerms distinct terms), 0: the block-wide kernel
+  u64* cand; int* counts; u32* row_tau;
+  double* dense_out; long long ld_out;
+};
+int launch_bm25(const Bm25Params& p, cudaStream_t st);
 int launch_bm25_head_slots(const int* head_terms, int n_head, long long n_terms, int* head_slot, cudaStream_t st);
 int launch_bm25_head_rows(const long long* post_indptr, const int* post_docs, const double* post_val,
                           const int* head_terms, int n_head, long long n_terms, long long ld_head, double* rows,
@@ -211,8 +214,5 @@ int launch_bm25_head_rows(const long long* post_indptr, const int* post_docs, co
 int launch_bm25_impacts(const long long* post_indptr, const int* post_docs, const float* post_tf, const double* idf,
                         const double* doc_norm, double k1p1, long long V, long long nnz, double* val,
                         cudaStream_t st);
-int launch_bm25_topk(const long long* post_indptr, const int* post_docs, const double* post_val,
-                     const int* head_slot, const double* head_rows, long long ld_head, const long long* q_indptr, const int* q_terms, long long Bq, long long N, int k, int C, int S,
-                     u64* cand, int* counts, double* dense_out, long long ld_out, cudaStream_t st);
 
 }  // namespace ccr
