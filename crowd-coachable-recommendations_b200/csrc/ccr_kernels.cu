@@ -245,8 +245,10 @@ __global__ void __launch_bounds__(256, 8) entry_records_kernel(RecordParams p) {
   const float s = (me >= 0 && p.mode == CCR_MASK_SET) ? 0.f : Src::score(p, row, col, lane);
   const double val = me < 0 ? (double)s : mask_value(p.mode, s, p.mask_vals[me]);
   if (lane == 0) {
+    // a NaN value never ranks, like a NaN score in the streams (its ord64 would rank it above +inf): the
+    // skipped record, and a masked column's stream candidate is dropped by finalize, so the column is not returned
     const u64 h = ord64(val);
-    p.rec_hi[e] = h ? h : 1ull;  // 0 is reserved for "skipped"
+    p.rec_hi[e] = isnan(val) ? 0ull : h ? h : 1ull;  // 0 is reserved for "skipped"
     p.rec_lo[e] = 0xFFFFFFFFu - (u32)col;
   }
 }

@@ -172,13 +172,22 @@ def _mask_host(mask):
     return ip, c, v, mask.mode
 
 
-def exact_topk(values, k, id_offset=0, allow_short=False):
+def exact_topk(values, k, id_offset=0, allow_short=False, drop_nan=False):
     """Top k of ``values`` [R, N] (torch float32 or float64) under the kernels' order: value descending
     (ord64), then id ascending.  Returns (float64 values, int64 ids + id_offset) [R, k]; with
-    ``allow_short`` and k > N the rows end in (-inf, -1)."""
+    ``allow_short`` and k > N the rows end in (-inf, -1).  ``drop_nan``: NaN values never rank (the
+    streaming top-k kernels' rule); a row with fewer than k other values ends in (-inf, -1) too."""
     R, N = values.shape
     kk = min(k, N)
-    if values.dtype == torch.float32 and N < (1 << 31):
+    if drop_nan:
+        key = key64(values)
+        key[torch.isnan(values)] = torch.iinfo(torch.int64).min
+        ids = torch.sort(key, dim=1, descending=True, stable=True).indices[:, :kk]
+        vals = torch.gather(values, 1, ids).to(torch.float64)
+        nan = torch.isnan(vals)
+        vals[nan] = -np.inf
+        ids = torch.where(nan, torch.full_like(ids, -1 - id_offset), ids)
+    elif values.dtype == torch.float32 and N < (1 << 31):
         # one distinct int64 per item: [ord32(score) : ~id], exactly the kernels' 64-bit candidate key
         b = values.view(torch.int32)
         hi = torch.where(b < 0, b ^ 0x7FFFFFFF, b).to(torch.int64)
@@ -187,7 +196,8 @@ def exact_topk(values, k, id_offset=0, allow_short=False):
         ids = 0xFFFFFFFF - (top & 0xFFFFFFFF)
     else:
         ids = torch.sort(key64(values), dim=1, descending=True, stable=True).indices[:, :kk]
-    vals = torch.gather(values, 1, ids).to(torch.float64)
+    if not drop_nan:
+        vals = torch.gather(values, 1, ids).to(torch.float64)
     ids = ids + id_offset
     if kk < k:
         if not allow_short:
@@ -342,3 +352,136 @@ def check_kernel(algo, s, i, d, q, items, D, k, mask=None, id_offset=0, n_items=
         return check_bounded(s, i, d, q, items, D, k, mask, id_offset=id_offset, n_items=n_items)
     want_v, want_i = exact_reference(q, items, D, k, mask, id_offset=id_offset, n_items=n_items)
     return check_exact(s, i, d, want_v, want_i)
+
+
+# ---- plan mirrors of the dense and BM25 top-k entries (csrc/ccr_api.cu: dense_plan, bm25_plan) ----
+# Neither entry exports its plan; the size queries expose it exactly (ccr_topk_dense_workspace_bytes is the dense
+# total, ccr_bm25_topk_workspace_bytes the larger BM25 total), so a test that checks the mirror against them may
+# trust its split counts and stream ranges.  Without a device the library plans for 148 SMs.
+
+DEFAULT_SMS = 148
+DENSE_SLACK = 4096        # kDenseSlack: columns a dense block scans between two prune checks
+FIN_LIST = 4096           # kFinList: finalize's shared-memory entry list
+FIN_MAX_STREAMS = 1024    # kFinMaxStreams
+BMW_WARPS, BMW_MINI, BMW_BLOCKS_PER_SM, BMW_MAX_TERMS = 8, 512, 4, 32  # warp-private BM25 kernel
+BMW_SKETCH_M = 5          # kBmwSketchM
+BM_CHUNK, BM_SLACK, BM_BLOCKS_PER_SM = 4096, 1024, 5                   # block-wide BM25 kernel
+
+
+def cand_capacity(k, slack):
+    return (2 * k + slack + 63) // 64 * 64
+
+
+def carve(*sizes):
+    """Total bytes of workspace regions taken one after another, each starting at a 256-byte boundary."""
+    off = 0
+    for s in sizes:
+        off = (off + s + 255) // 256 * 256
+    return off
+
+
+def _ceil(a, b):
+    return -(-a // b)
+
+
+def dense_plan(B, N, k, nnz=0, h=0, sms=DEFAULT_SMS):
+    """ccr_topk_dense_f32's plan for k + h candidates per row: S column splits of ``per`` columns each (whole
+    4096-column chunks; trailing splits may be empty), C keys per split."""
+    rows = max(B, 1)
+    S = max(1, min(_ceil(8 * sms, rows), _ceil(N, DENSE_SLACK), FIN_MAX_STREAMS))
+    C = cand_capacity(k + h, DENSE_SLACK)
+    per = _ceil(_ceil(N, S), DENSE_SLACK) * DENSE_SLACK
+    total = carve(rows * S * C * 8, rows * S * 4, nnz * 8, nnz * 4)
+    return dict(S=S, C=C, per=per, total=total, k_keep=k + h)
+
+
+def dense_split_cols(plan, N):
+    """[(first column, end)] of every split of a dense plan."""
+    return [(min(s * plan["per"], N), min((s + 1) * plan["per"], N)) for s in range(plan["S"])]
+
+
+def dense_finalize_entries(plan, N, k_row, nnz_row=0):
+    """(lo, hi): bounds of the entries finalize gathers for one row with k_row = k + nnz(row) and nnz(row) mask
+    records: the splits' candidates, less those in the row's mask (dropped), plus the records.  A split keeps
+    every column until its buffer passes C - 4096 keys, then at least k_row and, after a histogram prune of its
+    only chunk, at most (k_row + C - 4096) / 2.  When no split prunes, every column is a candidate and each
+    masked one is replaced by its record: exactly N."""
+    C, lo, hi = plan["C"], 0, 0
+    fill = C - DENSE_SLACK
+    for a, b in dense_split_cols(plan, N):
+        n = b - a
+        lo += n if n <= fill else k_row
+        if n <= fill:
+            hi += n
+        elif n <= DENSE_SLACK:
+            hi += max(k_row, (k_row + fill) // 2)
+        else:
+            hi += fill
+    if lo == N:
+        return N, N
+    return lo, hi + nnz_row
+
+
+def bm25_plan(Bq, N, k, warp, sms=DEFAULT_SMS):
+    """ccr_bm25_topk's plan: S doc splits (blocks) per query, ``streams`` candidate lists of C keys per query
+    (8 warps per block for the warp-private kernel), ``per`` docs per stream (whole mini-chunks / chunks)."""
+    rows = max(Bq, 1)
+    if warp:
+        s = _ceil(BMW_BLOCKS_PER_SM * sms, rows)
+        minis = _ceil(N, BMW_MINI)
+        if s * BMW_WARPS > minis:
+            s = _ceil(minis, BMW_WARPS)
+        s = max(1, min(s, FIN_MAX_STREAMS // BMW_WARPS))
+        streams, C = s * BMW_WARPS, cand_capacity(k, BMW_MINI)
+        per = _ceil(minis, streams) * BMW_MINI
+    else:
+        s = max(1, min(_ceil(BM_BLOCKS_PER_SM * sms, rows), _ceil(N, BM_CHUNK), FIN_MAX_STREAMS))
+        streams, C = s, cand_capacity(k, BM_SLACK)
+        per = _ceil(_ceil(N, BM_CHUNK), s) * BM_CHUNK
+    total = carve(rows * streams * C * 8, rows * streams * 4, rows * 4)
+    return dict(S=s, streams=streams, C=C, per=per, total=total, warp=warp)
+
+
+def bm25_stream_docs(plan, N):
+    """[(first doc, end)] of every stream of a BM25 plan; the warp-private kernel's block b runs streams
+    8b .. 8b + 7."""
+    return [(min(s * plan["per"], N), min((s + 1) * plan["per"], N)) for s in range(plan["streams"])]
+
+
+def bm25_workspace(Bq, N, k, sms=DEFAULT_SMS):
+    """ccr_bm25_topk_workspace_bytes: room for either kernel."""
+    return max(bm25_plan(Bq, N, k, True, sms)["total"], bm25_plan(Bq, N, k, False, sms)["total"])
+
+
+# ---- BM25: the float64 accumulation the header specifies ----
+
+def bm25_post_val(tf, idf_t, doc_norm_d, k1):
+    """float64 impacts in the header's operation order: ((tf * idf) * (k1 + 1)) * (1 / (tf + doc_norm))."""
+    tf = np.asarray(tf, dtype=np.float64)
+    return ((tf * idf_t) * (k1 + 1)) * (1.0 / (tf + doc_norm_d))
+
+
+def bm25_scores(post_indptr, post_docs, post_val, q_indptr, q_terms, N, device="cpu"):
+    """float64 [Bq, N] scores: per query a +0.0 accumulator, each term's postings added in q_terms order, one
+    add per (term, doc).  Term position j of every query is one scatter: a query has one term there and a term
+    one posting per doc, so each cell gets exactly one rounded add per term, in the header's order."""
+    dev = torch.device(device)
+    ip = torch.as_tensor(np.asarray(post_indptr, dtype=np.int64), device=dev)
+    docs = torch.as_tensor(np.asarray(post_docs, dtype=np.int64), device=dev)
+    vals = torch.as_tensor(np.asarray(post_val, dtype=np.float64), device=dev)
+    q_indptr = np.asarray(q_indptr, dtype=np.int64)
+    q_terms = np.asarray(q_terms, dtype=np.int64)
+    Bq = len(q_indptr) - 1
+    acc = torch.zeros((Bq, N), dtype=torch.float64, device=dev)
+    lengths = np.diff(q_indptr)
+    for j in range(int(lengths.max()) if Bq else 0):
+        qs = np.nonzero(lengths > j)[0]
+        terms = torch.as_tensor(q_terms[q_indptr[qs] + j], device=dev)
+        lo, n = ip[terms], ip[terms + 1] - ip[terms]
+        if int(n.sum()) == 0:
+            continue
+        q_of = torch.repeat_interleave(torch.as_tensor(qs, device=dev), n)
+        first = torch.repeat_interleave(lo - (torch.cumsum(n, 0) - n), n)
+        e = first + torch.arange(int(n.sum()), device=dev)
+        acc.index_put_((q_of, docs[e]), vals[e], accumulate=True)
+    return acc

@@ -13,6 +13,8 @@ import pytest
 import torch
 
 import cases
+import select_oracle as SO
+from ccr_b200 import bm25
 from oracle import ccr_oracle as O
 from select_oracle import lever  # noqa: F401  (fixture)
 
@@ -82,12 +84,27 @@ def bm25_kernel(request, lever):
     return request.param
 
 
-@pytest.mark.parametrize("n,q,k", [(40000, 40, 1001), (150000, 300, 100), (9000, 700, 10)])
+@pytest.mark.parametrize("n,q,k", [(40000, 40, 1001), (150000, 300, 100), (9000, 700, 10), (20000, 4100, 100)])
 def test_bm25_topk_vs_oracle(n, q, k, ccr, bm25_kernel):
+    """Every row: the exact top k (float32 ranking, ties to the lowest position) of the model's own float64
+    scores; sampled rows also against the reference's arithmetic.  4,100 queries cross BM25.topk's 4096-query
+    chunks; every 97th and the second-to-last are three passages long (> 32 distinct terms), so both chunks
+    split into a warp-kernel call and a block-wide call whose rows are put back in place."""
     corpus, queries = _synthetic(41 + k, n, q, vocab=20000, doc_len=60)
+    if q > bm25.QUERY_CHUNK:
+        for b in list(range(50, q, 97)) + [q - 2]:
+            queries[b] = " ".join(corpus[b % n: b % n + 3])
     model = ccr.BM25(b=0.75, k1=1.2).fit(corpus)
     ref = O.BM25Ref(b=0.75, k1=1.2).fit(corpus)
     s, i = model.topk(queries, k)
+    if q > bm25.QUERY_CHUNK:
+        lengths = np.diff(model.encode_queries(queries)[0])
+        for c in range(0, q, bm25.QUERY_CHUNK):
+            assert lengths[c: c + bm25.QUERY_CHUNK].max() > bm25.WARP_KERNEL_MAX_TERMS
+    want_v, want_i = SO.exact_topk(model.scores(queries).float(), k)
+    errs = SO.check_exact(s.cpu().numpy(), i.cpu().numpy(), s.double().cpu().numpy(), want_v.cpu().numpy(),
+                          want_i.cpu().numpy())
+    assert not errs, errs
     s, i = s.cpu().numpy(), i.cpu().numpy()
     check = range(q) if q <= 64 else list(range(8)) + list(range(8, q, max(1, q // 24)))
     for b in check:

@@ -409,34 +409,6 @@ def test_assign_topk_on_materialised_matrix_is_bit_exact(ccr, name, golden_dir):
     np.testing.assert_array_equal(csr2.indices, idx)
 
 
-@pytest.mark.parametrize("B,N,k,mode", [(7, 5000, 100, O.MASK_NONE), (300, 20000, 1001, O.MASK_ADD),
-                                        (2, 300_000, 10, O.MASK_SET), (40, 37, 37, O.MASK_ADD),
-                                        (1100, 3000, 5, O.MASK_NONE)])
-def test_topk_dense_abi_matches_float64_sort(ccr, B, N, k, mode):
-    """ccr_topk_dense_f32 (materialised score matrix + sparse prior) against the reference's
-    arithmetic: float32 scores, promoted to float64 where a prior is added / assigned, stable
-    descending order.  Heavy exact ties (scores drawn from 50 distinct values in some rows)."""
-    dev = torch.device("cuda:0")
-    rs = np.random.RandomState(B + N + k)
-    dense = rs.standard_normal((B, N)).astype(np.float32)
-    dense[::3] = rs.randint(0, 50, size=dense[::3].shape).astype(np.float32)  # tie-heavy rows
-    mask = _mask(rs, B, N, mode, dev, ccr, max_h=min(N, 30)) if mode != O.MASK_NONE else None
-    s, i, d = ccr.topk_dense(torch.as_tensor(dense).to(dev), k, mask=mask)
-    full = torch.as_tensor(dense).double()
-    if mask is not None:
-        indptr, cols, vals = mask.host
-        for r in range(B):
-            c = torch.as_tensor(cols[indptr[r]:indptr[r + 1]].astype(np.int64))
-            v = torch.as_tensor(vals[indptr[r]:indptr[r + 1]])
-            full[r, c] = v if mode == O.MASK_SET else full[r, c] + v
-    want_v, want_i = torch.sort(full, dim=1, descending=True, stable=True)
-    np.testing.assert_array_equal(i.cpu().numpy(), want_i[:, :k].numpy())
-    np.testing.assert_array_equal(d.cpu().numpy(), want_v[:, :k].numpy())
-    np.testing.assert_array_equal(s.cpu().numpy(), want_v[:, :k].float().numpy())
-    with pytest.raises(RuntimeError, match="out of range"):
-        ccr.topk_dense(torch.zeros(2, 3, device=dev), 4)
-
-
 @pytest.mark.parametrize("sim", ["dot", "cos"])
 def test_transform_scores_topk_vs_reference_matrix(ccr, sim):
     """bbpr.py:528-550 replaced by the lazy factor pair: top-k (+ prior) through the fused kernel
