@@ -59,6 +59,7 @@ EXPORTS = [
     "ccr_rerank_exact_workspace_bytes",
     "ccr_rerank_exact",
     "ccr_threshold_compact",
+    "ccr_score_dense_exact",
 ]
 
 _lib = None
@@ -162,6 +163,8 @@ def lib():
                                    vp, vp, vp, vp, sz, i32, vp]
     L.ccr_threshold_compact.restype = i32
     L.ccr_threshold_compact.argtypes = [vp, i64, i64, i64, vp, vp, vp, vp]
+    L.ccr_score_dense_exact.restype = i32
+    L.ccr_score_dense_exact.argtypes = [vp, i64, i64, vp, i64, i64, i32, vp, i64, vp]
     if L.ccr_abi_version() != ABI_VERSION:
         raise RuntimeError("libccr_b200 ABI version mismatch")
     _lib = L

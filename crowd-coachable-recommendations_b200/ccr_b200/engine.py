@@ -549,6 +549,27 @@ def ingest_rows_f32(src, dst, normalize=False, v_max=None):
     return dst
 
 
+def score_dense_exact(q32, items32, n_items=None, D=None):
+    """Exact dense fp32 [B, N] scores of fp32 rows (C ABI: ccr_score_dense_exact): every entry is the exact value
+    the exact top-k gives the pair, float64 sums in a fixed order rounded to fp32 (DESIGN.md section 6b)."""
+    _require_cuda(q32, "q32")
+    _require_cuda(items32, "items32")
+    if q32.dtype != torch.float32 or items32.dtype != torch.float32:
+        raise TypeError("q32 and items32 must be float32 rows (an exact table's data32 / encode_queries)")
+    if q32.dim() != 2 or items32.dim() != 2 or q32.stride(1) != 1 or items32.stride(1) != 1:
+        raise ValueError("q32 and items32 must be 2-d with a contiguous last dimension")
+    B = q32.shape[0]
+    N = items32.shape[0] if n_items is None else int(n_items)
+    D = q32.shape[1] if D is None else int(D)
+    out = torch.empty((B, N), dtype=torch.float32, device=q32.device)
+    with torch.cuda.device(q32.device):
+        rc = _lib.lib().ccr_score_dense_exact(q32.data_ptr() if B else None, B, _rows_pitch(q32),
+                                              items32.data_ptr() if N else None, N, _rows_pitch(items32), D,
+                                              out.data_ptr() if B and N else None, N, _stream_ptr(q32.device))
+    _lib.check(rc)
+    return out
+
+
 def score_topk_exact(q, q_scan, items, items_scan, k, v_max, mask: SparseMask | None = None, id_offset=0,
                      algo=_lib.ALGO_AUTO, allow_short=False, n_items=None, D=None):
     """Exact fp32 top-k (C ABI: ccr_score_topk_exact, then the fallback for uncertified rows).

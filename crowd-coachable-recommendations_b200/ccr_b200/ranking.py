@@ -29,16 +29,18 @@ BLOCK_VALUE = -1e6   # scripts/ms_marco_eval.py:227
 QUERY_CHUNK = 8192   # query rows per fused call (bounds workspace and the [B,k] result)
 
 
-def cos_sim(a: torch.Tensor, b: torch.Tensor):
-    """scripts/ms_marco_eval.py:155-162 on the device path: fp32 normalise -> bf16 -> dense scores."""
+def cos_sim(a: torch.Tensor, b: torch.Tensor, exact=False):
+    """scripts/ms_marco_eval.py:155-162 on the device path: fp32 normalise -> bf16 -> dense scores.
+    ``exact``: both sides normalised in fp32 into an exact table and its exact dense scores returned: the fp32
+    rounding of each float64 dot product (DESIGN.md section 6b)."""
     a = torch.as_tensor(a)
     b = torch.as_tensor(b)
     if a.dim() == 1:
         a = a.unsqueeze(0)
     if b.dim() == 1:
         b = b.unsqueeze(0)
-    t = EmbeddingTable.from_tensor(b, normalize=True)
-    return t.dense_scores(a)
+    t = EmbeddingTable.from_tensor(b, normalize=True, exact=exact)
+    return t.dense_scores(a, exact=exact)
 
 
 def generate_embeddings(data_indices, data_dic, embedding_func, batch_size, embedding_size=768, name=None):

@@ -176,10 +176,20 @@ class EmbeddingTable:
                                                 n_items=self.n, D=self.ld)
         return ((s, i, d) if want_f64 else (s, i)) + (n_fb,)
 
-    def dense_scores(self, queries, encoded=False):
+    def dense_scores(self, queries, encoded=False, exact=False):
+        """Dense fp32 [B, n] scores of queries against the resident rows.  ``exact=True`` (exact tables only):
+        every entry is the exact value ``search`` ranks the pair by (DESIGN.md section 6b), summed in float64 on
+        the FP64 units, so it costs far more than the scan-format tiles and must be asked for."""
+        if exact:
+            if not self.exact:
+                raise ValueError("exact dense scores need an exact table (EmbeddingTable(..., exact=True))")
+            q = queries if encoded else self.encode_queries(queries)
+            if q.dtype != torch.float32:
+                raise TypeError("an exact table's encoded queries are its fp32 rows (encode_queries)")
+            return engine.score_dense_exact(q, self.data32, n_items=self.n, D=self.ld)
         if self.exact:
-            raise NotImplementedError("exact tables rank exactly but have no exact dense scores; use an "
-                                      "EmbeddingTable without exact=True for dense score matrices")
+            raise NotImplementedError("an exact table computes dense scores only on request: pass exact=True "
+                                      "for the exact fp32 scores")
         q = queries if encoded else self.encode_queries(queries)
         return engine.score_dense(q, self.data, n_items=self.n, D=self.ld)
 

@@ -144,7 +144,7 @@ def _assign_topk(S, k, tie_breaker=1e-10, device="cpu", batch_size=None, exact=F
 assign_topk = _assign_topk
 
 
-def _argsort(S, tie_breaker=1e-10, device="cpu"):
+def _argsort(S, tie_breaker=1e-10, device="cpu", exact=False):
     """Drop-in for ``rime_lite.util._argsort`` (src/rime_lite/util/__init__.py:158-184): global flat
     argsort of the whole score matrix, best score first, returned as ``(row_idx, col_idx)``.
 
@@ -152,13 +152,15 @@ def _argsort(S, tie_breaker=1e-10, device="cpu"):
     with a store epilogue for tiles of >= 2^20 scores) -- or uploaded, when the expression is an already
     materialised dense matrix -- and ordered by ``ccr_argsort_scores_f32``, an LSD radix sort over
     float64-ordered keys with the sparse priors merged in float64 like the reference's promotion.
-    Ties are ordered by flat position (the reference adds unseeded jitter)."""
+    Ties are ordered by flat position (the reference adds unseeded jitter).  ``exact``: a factor pair is
+    scored by its exact fp32 scores (``ccr_score_dense_exact`` on the exact table ``_assign_topk(exact=True)``
+    uses, DESIGN.md section 6b); a materialised matrix is ordered by its given values either way."""
     if not isinstance(S, LazyScoreBase):
         S = auto_cast_lazy_score(S)
     plan = fused_plan(S)
     if plan is not None:
-        table = _device_table_for(plan.right)
-        dense = table.dense_scores(torch.as_tensor(np.ascontiguousarray(plan.left.c)))
+        table = _device_table_for(plan.right, exact=exact)
+        dense = table.dense_scores(torch.as_tensor(np.ascontiguousarray(plan.left.c)), exact=exact)
         sparse = plan.sparse
     else:
         dplan = dense_plan(S)

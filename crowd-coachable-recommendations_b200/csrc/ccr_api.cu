@@ -1013,6 +1013,19 @@ int ccr_rerank_exact(const float* q, int64_t B, int64_t ldq, const float* items,
                 (cudaStream_t)stream);
 }
 
+int ccr_score_dense_exact(const float* q, int64_t B, int64_t ldq, const float* items, int64_t n_items, int64_t ldi,
+                          int D, float* out, int64_t ld_out, void* stream) {
+  if (B < 0 || n_items < 0 || ld_out < n_items) return fail(CCR_EINVAL, "bad exact dense shape");
+  if (D <= 0 || D % 8) return fail(CCR_EINVAL, "D=%d must be a positive multiple of 8", D);
+  if (D > 4096) return fail(CCR_EUNSUPPORTED, "D=%d > 4096", D);
+  if (ldq < D || ldi < D || ldq % 8 || ldi % 8) return fail(CCR_EINVAL, "ldq/ldi must be >= D and multiples of 8");
+  if (B == 0 || n_items == 0) return CCR_OK;
+  if (!q || !items || !out) return fail(CCR_EINVAL, "null pointer");
+  if (int rc = check_rows(q, ldq, items, ldi, D)) return rc;
+  return cuda_rc(launch_dense_exact(q, B, ldq, items, n_items, ldi, D, out, ld_out, (cudaStream_t)stream),
+                 "exact dense kernel launch");
+}
+
 int ccr_threshold_compact(const float* scores, int64_t R, int64_t N, int64_t ld, const double* tau,
                           int64_t* out_indptr, int64_t* out_ids, void* stream) {
   if (R < 0 || N < 0 || ld < N) return fail(CCR_EINVAL, "bad compaction shape");

@@ -3,6 +3,7 @@
 //   certify_kernel       : per row, does the k-th exact value beat every item the scan stage left out?
 //   compact_kernel       : columns of a dense scan-score block at or above a per-row threshold, as a CSR
 //   row_norm_max_kernel  : largest fp32 row norm of an appended batch (the V of the error bound)
+//   dense_exact_kernel   : the exact value of every (query, item) pair of a [B, N] block
 #include "ccr_params.cuh"
 
 namespace ccr {
@@ -141,6 +142,112 @@ int launch_fill_f64(double* dst, long long n, double v, cudaStream_t st) {
   if (n <= 0) return 0;
   fill_f64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dst, n, v);
   return (int)cudaGetLastError();
+}
+
+// Exact dense scores.  dot_f64 (ccr_kernels.cu) fixes the value of a pair: lane l of a warp sums
+// fma(double(q_e), double(v_e), acc) over the float4 chunks c = l, l + 32, ... < D/4 (elements in order), then
+// an xor butterfly with offsets 16 .. 1.  Here one warp owns an 8 x 8 tile of pairs and lane l runs lane l's
+// chain for all 64 of them, so every sum is formed in that order by construction.  A block of 8 warps (2 x 4)
+// covers 16 queries x 32 items; per K-slice of 128 elements (one chunk per lane) its 48 rows are converted to
+// double once and staged in shared memory as [row][element of the chunk][lane], which makes every warp load
+// conflict-free.  The slice after the current one is read from global memory into registers during the FMAs.
+constexpr int kDxQ = 16, kDxI = 32, kDxRows = kDxQ + kDxI;
+constexpr int kDxSlice = 128;                                   // elements per stage: 32 chunks of 4
+constexpr int kDxLoads = kDxRows * kDxSlice / 4 / 256;          // float4 loads per thread and stage
+constexpr size_t kDxSmem = 2ull * kDxRows * kDxSlice * sizeof(double);  // two stages
+
+__global__ void __launch_bounds__(256, 1) dense_exact_kernel(const float* __restrict__ q, long long B, long long ldq,
+                                                             const float* __restrict__ items, long long N,
+                                                             long long ldi, int D, float* __restrict__ out,
+                                                             long long ld_out, long long n_qt, long long tile0) {
+  extern __shared__ double s_rows[];
+  const long long t = tile0 + blockIdx.x;  // query tiles vary fastest: the blocks in flight share item rows
+  const long long q0 = (t % n_qt) * kDxQ, i0 = (t / n_qt) * kDxI;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int n_chunks = D >> 2, n_slices = (n_chunks + 31) >> 5;
+
+  // chunks past D/4 and rows past B / N stage as zeros: fma(0, 0, acc) == acc for every acc but -0.0, and a
+  // sum that starts at +0.0 never becomes -0.0 in round-to-nearest (x + -x is +0.0), so they change no sum
+  float4 nxt[kDxLoads];
+  auto load = [&](int slice) {
+#pragma unroll
+    for (int u = 0; u < kDxLoads; ++u) {
+      const int f = threadIdx.x + 256 * u, row = f >> 5, c = (slice << 5) + (f & 31);
+      const long long r = row < kDxQ ? q0 + row : i0 + (row - kDxQ);
+      const bool ok = c < n_chunks && (row < kDxQ ? r < B : r < N);
+      const float* src = row < kDxQ ? q + r * ldq : items + r * ldi;
+      nxt[u] = ok ? __ldg(reinterpret_cast<const float4*>(src) + c) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+  };
+  auto stage = [&](int buf) {
+#pragma unroll
+    for (int u = 0; u < kDxLoads; ++u) {
+      const int f = threadIdx.x + 256 * u;
+      double* d = s_rows + ((size_t)buf * kDxRows + (f >> 5)) * kDxSlice + (f & 31);
+      d[0] = (double)nxt[u].x; d[32] = (double)nxt[u].y; d[64] = (double)nxt[u].z; d[96] = (double)nxt[u].w;
+    }
+  };
+
+  double acc[64];  // acc[a * 8 + b]: query wq * 8 + a, item wi * 8 + b of the block tile
+#pragma unroll
+  for (int o = 0; o < 64; ++o) acc[o] = 0.0;
+  const int wq = warp >> 2, wi = warp & 3;
+  load(0);
+  stage(0);
+  __syncthreads();
+  for (int sl = 0; sl < n_slices; ++sl) {
+    if (sl + 1 < n_slices) load(sl + 1);
+    const double* sq = s_rows + ((size_t)(sl & 1) * kDxRows + wq * 8) * kDxSlice + lane;
+    const double* si = s_rows + ((size_t)(sl & 1) * kDxRows + kDxQ + wi * 8) * kDxSlice + lane;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      double x[8], y[8];
+#pragma unroll
+      for (int a = 0; a < 8; ++a) x[a] = sq[a * kDxSlice + j * 32];
+#pragma unroll
+      for (int b = 0; b < 8; ++b) y[b] = si[b * kDxSlice + j * 32];
+#pragma unroll
+      for (int a = 0; a < 8; ++a)
+#pragma unroll
+        for (int b = 0; b < 8; ++b) acc[a * 8 + b] = fma(x[a], y[b], acc[a * 8 + b]);
+    }
+    if (sl + 1 < n_slices) stage((sl + 1) & 1);  // that buffer was last read before the previous barrier
+    __syncthreads();
+  }
+
+  // The butterfly as a reduce-scatter: at offset `off` each lane keeps one half of its h sums and adds the
+  // partner's value of it, the partner the other half.  Each sum is the butterfly's own a_l + a_(l^off) (the
+  // two lanes of a pair compute the same value, fp add being commutative), so after 5 steps lane l holds the
+  // butterfly result of pairs 2l and 2l + 1, with 62 shuffles instead of 320.
+#pragma unroll
+  for (int h = 32, off = 16; h >= 2; h >>= 1, off >>= 1) {
+    const bool upper = lane & off;
+#pragma unroll
+    for (int i = 0; i < h; ++i) {
+      const double send = upper ? acc[i] : acc[i + h];
+      const double mine = upper ? acc[i + h] : acc[i];
+      acc[i] = mine + __shfl_xor_sync(0xffffffffu, send, off);
+    }
+  }
+  const long long r = q0 + wq * 8 + (lane >> 2), c = i0 + wi * 8 + 2 * (lane & 3);
+  if (r < B) {
+    if (c < N) out[r * ld_out + c] = (float)acc[0];
+    if (c + 1 < N) out[r * ld_out + c + 1] = (float)acc[1];
+  }
+}
+
+int launch_dense_exact(const float* q, long long B, long long ldq, const float* items, long long n, long long ldi,
+                       int D, float* out, long long ld_out, cudaStream_t st) {
+  if (B <= 0 || n <= 0) return 0;
+  cudaError_t e = cudaFuncSetAttribute(dense_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDxSmem);
+  if (e != cudaSuccess) return (int)e;
+  const long long n_qt = (B + kDxQ - 1) / kDxQ, tiles = n_qt * ((n + kDxI - 1) / kDxI);
+  for (long long t0 = 0; t0 < tiles; t0 += 1LL << 30) {
+    const long long nb = tiles - t0 < (1LL << 30) ? tiles - t0 : (1LL << 30);
+    dense_exact_kernel<<<(unsigned)nb, 256, kDxSmem, st>>>(q, B, ldq, items, n, ldi, D, out, ld_out, n_qt, t0);
+    if ((e = cudaGetLastError()) != cudaSuccess) return (int)e;
+  }
+  return 0;
 }
 
 }  // namespace ccr

@@ -157,6 +157,9 @@ int launch_dense(const T* q, long long B, long long ldq, const T* items, long lo
 // the exact ranking stages (ccr_exact.cu)
 int launch_row_norm_max(const float* rows, long long n, int D, long long ld, double* v_max, cudaStream_t st);
 int launch_fill_f64(double* dst, long long n, double v, cudaStream_t st);
+// out[r, c] = fp32(dot_f64(q_r, items_c)) for r < B, c < n: the exact value of every pair
+int launch_dense_exact(const float* q, long long B, long long ldq, const float* items, long long n, long long ldi,
+                       int D, float* out, long long ld_out, cudaStream_t st);
 // per row: certified (0) or not (1), tau = RD(L_k - E); uncertified rows are added to *count
 int launch_exact_certify(const float* q, long long ldq, int B, int D, int f16, const double* v_max, int k, int k_cand,
                          long long n_items, const float* s1_scores, const long long* s1_ids, const long long* mask_indptr,

@@ -354,6 +354,19 @@ int ccr_rerank_exact(const float* q, int64_t B, int64_t ldq, const float* items,
                      int mask_mode, int64_t id_offset, float* out_scores, double* out_scores64, int64_t* out_ids,
                      void* workspace, size_t workspace_bytes, int flags, void* stream);
 
+/* Exact dense scores: out[r, c] = the exact value above of (query row r, item row c), unmasked, for every
+ * r < B, c < n_items -- fp32 of the float64 sum in dot_f64's order: lane l (0..31) of a warp runs
+ * acc = fma((double)q_e, (double)v_e, acc) from +0.0 over the float4 chunks l, l + 32, ... < D/4 (elements of a
+ * chunk in order), an xor butterfly with offsets 16, 8, 4, 2, 1 adds the 32 lane sums, the result is rounded
+ * to fp32.  Bit for bit (+-0.0 included) the value ccr_score_topk_exact / ccr_rerank_exact give the pair
+ * for the same D (exact tables pass their padded pitch).  fp64 FMAs on the CUDA cores, no tensor cores: the
+ * accumulation order of FP64 MMA is not documented.  q [B, ldq] / items [n_items, ldi] fp32 rows (pitches
+ * >= D, multiples of 8, 16-byte aligned bases; columns past D are not read), out [B, ld_out] fp32,
+ * ld_out >= n_items.  D % 8 != 0 -> CCR_EINVAL, D > 4096 -> CCR_EUNSUPPORTED; B == 0 or n_items == 0
+ * writes nothing. */
+int ccr_score_dense_exact(const float* q, int64_t B, int64_t ldq, const float* items, int64_t n_items, int64_t ldi,
+                          int D, float* out, int64_t ld_out, void* stream);
+
 /* Columns of a dense fp32 score block scores [R, ld] with double(score) >= tau[r] (device float64 [R]), as a
  * CSR.  First call with out_ids = NULL: out_indptr [R+1] receives the row offsets.  Second call with the
  * same out_indptr and out_ids [out_indptr[R]]: the column ids, in no particular order within a row. */
